@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s of the Skillshot hot path on B200 (driver contract).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): physics-only, 65,536 SkillshotGame envs per
 GPU, U(-1.2,1.2) float32 random actions, random starts, terminal +1/-1/0 reward,
@@ -36,6 +36,11 @@ own config (same keys, same ticks per step), and prints the same line with
 "impl": "reference"; the Python reference's figure rides along as
 cpu_baseline.python_reference (the port is ~100x faster per core than the Python
 objects and is therefore the stricter baseline for the driver's ratio).
+
+--dump-outputs DIR writes, after the timed steps, what the timed path computed in
+its last step as DIR/<name>.npy (float32 / float64; at most DUMP_STEP_BYTES of sampled
+step outputs plus the game state of every env; see dump_outputs).  The inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 
 Thread counts come from the process's CPU affinity, never from OMP_NUM_THREADS
 (torch.distributed.run exports OMP_NUM_THREADS=1).
@@ -629,6 +634,31 @@ def run_reference_arm(args):
     return 0
 
 
+DUMP_STEP_BYTES = 32 << 20     # --dump-outputs: bound on the sampled step outputs (16 B per env-tick as float32)
+
+
+def dump_outputs(path: str, envs, out: dict):
+    """--dump-outputs: what the timed path handed its caller in its last step, written as path/<name>.npy.
+    SkillshotEnvs.step reuses its output tensors from launch to launch, so once a step has returned its caller holds the
+    reward / done / winner of the step's last launch [ticks_per_launch, envs, ...]: those of every tick for as many env
+    columns as fit DUMP_STEP_BYTES, drawn with a fixed seed (their indices in env_index), as float32.  The step's earlier
+    launches are not in these buffers any more: they show only through the game state every env is left in after the
+    step (SkillshotEnvs.export_state, state_<field>), written beside them as float64."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    ticks = out["reward"].shape[0]
+    n_cols = max(1, min(envs.n_envs, DUMP_STEP_BYTES // (16 * ticks)))
+    cols = np.sort(np.random.default_rng(0).choice(envs.n_envs, n_cols, replace=False))
+    idx = torch.from_numpy(cols).to(out["reward"].device)
+    arrays = {"env_index": cols.astype(np.float64)}
+    for k in ("reward", "done", "winner"):
+        arrays[k] = out[k].index_select(1, idx).cpu().numpy().astype(np.float32)
+    for k, v in envs.export_state().items():
+        arrays["state_" + k] = np.asarray(v, dtype=np.float64)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v)
+
+
 def bind_to_gpu_numa(index: int):
     """Pin this process to the CPUs NVML reports as local to GPU `index`, BEFORE the pinned host buffers of the
     end-to-end leg are allocated (first touch then lands on the GPU's own NUMA node).  With 8 ranks streaming
@@ -684,7 +714,8 @@ def run_gpu_arm(args):
 
     def device_step():
         for c in range(launches_per_step):
-            envs.step(actions[c * KF:(c + 1) * KF], want_obs=False)
+            out = envs.step(actions[c * KF:(c + 1) * KF], want_obs=False)
+        return out
 
     # ---- device-resident throughput (value) ----
     for _ in range(max(args.warmup, 3)):
@@ -695,12 +726,14 @@ def run_gpu_arm(args):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     for _ in range(args.steps):
-        device_step()
+        out = device_step()
     ev1.record()
     barrier()
     clocks = sampler.stop()
     ms = ev0.elapsed_time(ev1)
     envs.check_status()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, envs, out)
 
     # ---- the same kernel family at one tick per launch (the literal 202 B per env-step shape), and the GPU's measured
     #      instruction-rate ceilings for the record of the bound the fused kernel is actually on ----
@@ -852,7 +885,15 @@ def main():
     ap.add_argument("--no-learner", action="store_true", help="skip the rollout / update / actor-forward legs")
     ap.add_argument("--collective", default="peer", choices=["peer", "nccl"],
                     help="gradient exchange of the update at N > 1: fused NVLink peer-memory kernels, or an NCCL all-reduce")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (rank 0's envs): per-tick reward / "
+                         "done / winner of the step's last launch for a seeded sample of envs (the step's earlier "
+                         "launches show only through the game state) and the game state of every env after the step")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm's timed path (--impl b200)")
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_gpu_arm(args)

@@ -139,6 +139,44 @@ def test_bench_report_assembles_without_a_gpu():
     assert set(cfg) == {"workload", "envs_per_gpu", "ticks_per_step", "ticks_per_launch", "l2"}
 
 
+def test_bench_dump_outputs_writes_a_seeded_float_sample(tmp_path, monkeypatch):
+    """bench.py --dump-outputs on made-up step outputs: float32 / float64 files only, the byte bound on the step outputs
+    held, the same env columns on every call, and the sampled values those of the step."""
+    import importlib.util
+    import numpy as np
+    import torch
+    spec = importlib.util.spec_from_file_location("_bench3", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    monkeypatch.setattr(bench, "DUMP_STEP_BYTES", 16 * 64 * 100)
+    n, K = 1000, 64
+    g = torch.Generator().manual_seed(0)
+    out = dict(reward=torch.randn((K, n, 2), generator=g), done=torch.randint(0, 2, (K, n), generator=g, dtype=torch.uint8),
+               winner=torch.randint(0, 3, (K, n), generator=g, dtype=torch.uint8))
+
+    class Envs:
+        n_envs = n
+
+        def export_state(self):
+            return dict(px=np.arange(2 * n, dtype=np.int64).reshape(n, 2), prot=np.full((n, 2), 0.5), ticks=np.arange(n))
+
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), Envs(), out)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == sorted(os.listdir(tmp_path / "b"))
+    step_bytes = 0
+    for f in files:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b), f
+        step_bytes += a.nbytes if f in ("reward.npy", "done.npy", "winner.npy") else 0
+    assert step_bytes <= bench.DUMP_STEP_BYTES
+    cols = np.load(tmp_path / "a" / "env_index.npy").astype(np.int64)
+    assert len(cols) == 100 and np.all(np.diff(cols) > 0)
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "reward.npy"), out["reward"].numpy()[:, cols])
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "winner.npy"), out["winner"].numpy()[:, cols])
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "state_px.npy"), Envs().export_state()["px"])
+
+
 def test_cpu_legs_ignore_omp_num_threads(monkeypatch):
     """torch.distributed.run exports OMP_NUM_THREADS=1: the CPU legs size themselves from the CPU affinity instead."""
     import importlib.util

@@ -238,16 +238,18 @@ def test_replay_ring_push_wrap_and_sample():
     assert np.array_equal(b["obs"].cpu().numpy(), mirror["obs"][idx])
 
 
-def test_reference_surface_trains_one_episode(capsys):
+def test_reference_surface_trains_one_episode(tmp_path, capsys):
     """SkillshotLearner.main-style use (SkillshotLearner.py:685-693) with a short tick limit."""
     from skillshot_learning_b200 import SkillshotLearner
     skl = SkillshotLearner(device="cuda:0", seed=2)
+    skl.save_location = str(tmp_path / "training_models")      # save_boards writes the board rasters there
     skl.model_param_game_tick_limit = 12
     skl.use_random_start = False
     before = skl.networks.actor.clone()
     prog = skl.model_train(epochs=1, save_progress=False, save_boards=True)
     assert prog["epoch_ticks"] == [12] and prog["epoch_winner"] == [0]
     assert len(prog["epoch_board_sequences"][0]) == 12 and prog["epoch_board_sequences"][0][0].shape == (250, 250)
+    assert os.path.exists(os.path.join(skl.save_location, "training_boards", "training_boards.npy"))
     assert skl.networks.step_critic == 2 and skl.networks.step_actor == 2      # 24 rows in batches of 16
     assert not torch.equal(before, skl.networks.actor)
     assert np.isfinite(skl.last_fit["critic_loss"])
