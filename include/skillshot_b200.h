@@ -549,8 +549,8 @@ int ss_ddpg_update(const ss_ddpg_update_args *args, void *stream);
 
 /* ss_ddpg_update and ss_selfplay_rollout launch their kernels as a programmatic-dependent-launch chain (each grid is placed
  * while its predecessor drains and waits, griddepcontrol.wait, before its first dependent access; csrc/ss_launch.cuh).
- * enabled = 0: ordinary launches; 1: chained; -1: back to the default (chained unless the environment says SS_UPDATE_PDL=0 /
- * SS_ROLLOUT_PDL=0).  Returns the previous setting (-1 / 0 / 1).  Results are bit-identical either way. */
+ * enabled = 0: ordinary launches; 1: chained; -1: back to the default (chained).  Returns the previous setting (-1 / 0 / 1).
+ * Results are bit-identical either way. */
 int ss_set_dependent_launch(int enabled);
 
 /* a = actor(s) -> act_out [n][2], then critic([s, a]) -> any of q_out [n] / neg_dq_da_out [n][2] / y_out [n] (the TD target

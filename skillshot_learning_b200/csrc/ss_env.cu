@@ -679,18 +679,6 @@ __global__ void apply_kernel(void *state, int64_t n, int64_t env, int player, in
     if (status && status_out) atomicOr(status_out, status);
 }
 
-// SS_STEP_PP=0 sends the physics-only fused step back to the one-thread-per-env kernel (A/B measurements only)
-inline bool getenv_pp() {
-    static int v = -1;
-    if (v < 0) { const char *e = getenv("SS_STEP_PP"); v = (e && e[0] == '0') ? 0 : 1; }
-    return v != 0;
-}
-// SS_STEP_PDL=0 launches the one-tick physics kernel without programmatic dependent launch (A/B measurements only)
-inline bool getenv_pdl() {
-    static int v = -1;
-    if (v < 0) { const char *e = getenv("SS_STEP_PDL"); v = (e && e[0] == '0') ? 0 : 1; }
-    return v != 0;
-}
 inline int check_launch() { return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA; }
 inline unsigned blocks_for(int64_t n, int block) { return (unsigned)((n + block - 1) / block); }
 // CTA size of step_pp_kernel for n_envs (see the kernel): 896 when that still makes at least ~one CTA per SM (65,536 envs
@@ -782,7 +770,7 @@ int ss_env_step_ring(void *state, int64_t n_envs, const float *actions, float *o
     }
     // (the statistics variants are separate instantiations: the bookkeeping costs the physics-only kernels a few
     //  registers and ~5 % when compiled in)
-    if (obs_out && n_ticks == 1 && !speeds && reward_mode != SS_REWARD_SIMPLE && getenv_pp()) {
+    if (obs_out && n_ticks == 1 && !speeds && reward_mode != SS_REWARD_SIMPLE) {
         // the rollout's env step: one tick with observations, one thread per player
         const dim3 grid_pp(blocks_for(2 * n_envs, kBlockPP));
         if ((A.stats ? sslaunch::launch(step_pp_obs_kernel<true>, grid_pp, dim3(kBlockPP), 0, st, A)
@@ -799,7 +787,7 @@ int ss_env_step_ring(void *state, int64_t n_envs, const float *actions, float *o
             else step_kernel<true, true, false, 8><<<grid, block, 0, st>>>(A);
         }
     } else if (n_ticks > 1 && !A.stats && !speeds && !shaped && !done_rows_out && done_out && winner_out &&
-               2 * n_envs * ((int64_t)n_ticks + 2) < (int64_t)0x7fffffff && getenv_pp()) {     // (32-bit running index)
+               2 * n_envs * ((int64_t)n_ticks + 2) < (int64_t)0x7fffffff) {     // (32-bit running index)
         // physics-only fused ticks (bench.py's timed shape): one thread per player.  (A single tick per launch stays on
         // the one-thread-per-env kernel: a launch then pays 3 sincos per lane to set up what it carries, measured 4.1 vs 3.9 us.)
         if (reward_out && reward_mode == SS_REWARD_TERMINAL) launch_step_pp<OUT_TERMINAL>(A, n_envs, st);
@@ -816,7 +804,7 @@ int ss_env_step_ring(void *state, int64_t n_envs, const float *actions, float *o
         // One physics tick per launch: a ~2 us kernel behind ~2 us of launch latency.  Launched with programmatic stream
         // serialization, the grid is scheduled while its predecessor drains and waits (griddepcontrol.wait) before its
         // first global access: back-to-back one-tick launches overlap their launch latency with the previous tick's tail.
-        if (getenv_pdl() && !A.stats && !speeds) {
+        if (!A.stats && !speeds) {
             cudaLaunchConfig_t cfg = {};
             cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = 0; cfg.stream = st;
             cudaLaunchAttribute attr[1];
@@ -845,8 +833,7 @@ int ss_env_step_ring(void *state, int64_t n_envs, const float *actions, float *o
             if (speeds) step_kernel<false, false, true, 1, true><<<grid, block, 0, st>>>(A);
             else step_kernel<false, false, false, 1, true><<<grid, block, 0, st>>>(A);
         } else {
-            if (speeds) step_kernel<false, false, true><<<grid, block, 0, st>>>(A);
-            else step_kernel<false, false, false><<<grid, block, 0, st>>>(A);
+            step_kernel<false, false, true><<<grid, block, 0, st>>>(A);
         }
     }
     return check_launch();

@@ -50,7 +50,6 @@ struct FramesArgs {
     uint8_t *h1;                 // [units][H1TILE_BYTES] scratch between the two kernels
     int64_t n, group, stride, head;
     int frames;
-    long long *trace;            // development: event timestamps of CTA 0 of the layer-1 kernel (NULL in production)
 };
 
 __host__ __device__ constexpr int frames_k1(int frames) { return (DS * frames + 2 + 15) / 16 * 16; }
@@ -177,15 +176,6 @@ __global__ void __launch_bounds__(NTH, 1) frames_l1_kernel(const FramesArgs A) {
     const uint32_t sbase = smem_u32(smem);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     auto bar = [&](int idx) -> uint32_t { return sbase + SM_BAR + (uint32_t)idx * 8; };
-    int tr_n = 0;                // development trace: role 0 = epilogue warp 0, 1 = MMA warp, 2 = copy thread
-    auto trace = [&](int role, int code) {
-        if (A.trace && blockIdx.x == 0 && lane == 0 && (warp == 0 || warp == MMA_W || warp == COPY_W) && tr_n < 256) {
-            A.trace[(role * 256 + tr_n) * 2] = clock64();
-            A.trace[(role * 256 + tr_n) * 2 + 1] = code;
-            ++tr_n;
-        }
-    };
-    trace(0, 900);
     const int k1 = frames_k1(A.frames);                     // input columns + bias pair, padded to the MMA K step
     const int nstages = (k1 + KSTAGE - 1) / KSTAGE;         // K stages in use (the last one may be partial)
     const uint32_t tile_bytes = (uint32_t)(k1 / 8) * CHUNK_A;
@@ -217,7 +207,6 @@ __global__ void __launch_bounds__(NTH, 1) frames_l1_kernel(const FramesArgs A) {
         stage_w1(A.theta + g * A.stride, A.frames, oldest, k1, smem + SM_W1);
         fence_proxy_async();
         __syncthreads();
-        trace(0, 901);
 
         if (warp < EPI_WARPS) {
             // ============ epilogue: D[slot] -> ReLU -> bf16 -> the tile's layer-2 operand image ============
@@ -227,10 +216,8 @@ __global__ void __launch_bounds__(NTH, 1) frames_l1_kernel(const FramesArgs A) {
             for (uint32_t i = 0; i < ntiles; ++i) {
                 const uint32_t tc = tcount + i, slot = tc & 1;
                 uint8_t *out = A.h1 + (u + i) * (int64_t)H1TILE_BYTES + r * 16;
-                trace(0, 100 + (int)i);
                 mbar_wait(bar(B_DFULL + slot), (tc >> 1) & 1);
                 tc_fence_after();
-                trace(0, 200 + (int)i);
                 uint32_t va[32], vb[32];
                 tmem_ld32(tl + slot * 256, va);
 #pragma unroll
@@ -243,7 +230,6 @@ __global__ void __launch_bounds__(NTH, 1) frames_l1_kernel(const FramesArgs A) {
                     else { tc_fence_before(); mbar_arrive(bar(B_DFREE + slot)); }        // D[slot] fully read
                     relu_pack_store_global(vb, out + (uint32_t)((j + 1) * 4) * CHUNK_A, keep);
                 }
-                trace(0, 300 + (int)i);
             }
         } else if (warp == MMA_W) {
             // ============ the MMA-issuing warp ============
@@ -253,7 +239,6 @@ __global__ void __launch_bounds__(NTH, 1) frames_l1_kernel(const FramesArgs A) {
             // The tensor pipe queues only a couple of MMAs, so the issuing thread cannot run ahead: whatever it waits for
             // idles the pipe unless MMAs are queued behind it.  Every wait (next stage landed, next accumulator drained) is
             // therefore placed BETWEEN the two halves of a stage's MMAs, and the commits after them.
-            trace(1, 100);
             mbar_wait(bar(B_DFREE + (tc0 & 1)), ((tc0 >> 1) & 1) ^ 1);
             mbar_wait(bar(B_XFULL + 0), tc0 & 1);
             tc_fence_after();
@@ -264,7 +249,6 @@ __global__ void __launch_bounds__(NTH, 1) frames_l1_kernel(const FramesArgs A) {
                 for (int sg = 0; sg < NSTAGE; ++sg) {             // unrolled: descriptor offsets and flags fold to constants --
                     if (sg >= nstages) break;                     // a single thread's issue loop must stay a few instructions per MMA
                     const int steps = min(KSTAGE, k1 - sg * KSTAGE) / 16;
-                    trace(1, 200 + (int)i * 4 + sg);
                     if (lane == 0) {
 #pragma unroll
                         for (int ks = 0; ks < 2; ++ks)
@@ -290,7 +274,6 @@ __global__ void __launch_bounds__(NTH, 1) frames_l1_kernel(const FramesArgs A) {
                         if (sg == nstages - 1) umma_commit(bar(B_DFULL + slot));
                     }
                     __syncwarp();
-                    trace(1, 300 + (int)i * 4 + sg);
                 }
             }
         } else if (warp == COPY_W && lane == 0) {
@@ -302,7 +285,6 @@ __global__ void __launch_bounds__(NTH, 1) frames_l1_kernel(const FramesArgs A) {
                 for (int sg = 0; sg < nstages; ++sg) {
                     const uint32_t bytes = (uint32_t)min(KSTAGE, k1 - sg * KSTAGE) / 8 * CHUNK_A;
                     mbar_wait(bar(B_XFREE + sg), (tc & 1) ^ 1);       // the previous tile's MMAs have read this stage
-                    trace(2, 100 + (int)i * 4 + sg);
                     mbar_expect_tx(bar(B_XFULL + sg), bytes);
                     bulk_load_hint(sbase + SM_X + sg * XSTAGE_BYTES, src + sg * XSTAGE_BYTES, bytes, bar(B_XFULL + sg), stream_through);
                 }
@@ -515,16 +497,16 @@ extern "C" int64_t ss_actor_frames_tc_workspace_bytes(int64_t n_rows, int64_t no
     return frame_units(n_rows, group) * (int64_t)H1TILE_BYTES;
 }
 
-static int frames_forward(const float *params, int64_t param_stride, int64_t noise_group, const void *stack_tc, int frames,
-                          int64_t head, float *act_out, int64_t n_rows, void *workspace, int64_t workspace_bytes,
-                          long long *trace, void *stream) {
+extern "C" int ss_actor_forward_frames_tc(const float *params, int64_t param_stride, int64_t noise_group, const void *stack_tc,
+                                          int frames, int64_t head, float *act_out, int64_t n_rows, void *workspace,
+                                          int64_t workspace_bytes, void *stream) {
     if (!params || !stack_tc || !act_out || !workspace || n_rows <= 0 || frames < 1 || frames > MAXF || head < 0 || param_stride < 0)
         return SS_ERR_INVALID_ARG;
     if (param_stride > 0 && (noise_group <= 0 || noise_group % TM != 0)) return SS_ERR_INVALID_ARG;
     if ((((uintptr_t)params | (uintptr_t)stack_tc | (uintptr_t)workspace) & 15) || (param_stride & 3) || ((uintptr_t)act_out & 7))
         return SS_ERR_INVALID_ARG;
     FramesArgs A{params, (const uint8_t *)stack_tc, act_out, (uint8_t *)workspace, n_rows,
-                 param_stride > 0 ? noise_group : n_rows, param_stride, head, frames, trace};
+                 param_stride > 0 ? noise_group : n_rows, param_stride, head, frames};
     if (A.group > n_rows) A.group = n_rows;
     const int64_t units = frame_units(n_rows, A.group);
     if (workspace_bytes < units * (int64_t)H1TILE_BYTES) return SS_ERR_INVALID_ARG;
@@ -540,17 +522,4 @@ static int frames_forward(const float *params, int64_t param_stride, int64_t noi
     l1::frames_l1_kernel<<<grid, l1::NTH, l1::SM_TOTAL, (cudaStream_t)stream>>>(A);
     l23::frames_l23_kernel<<<grid, l23::NTH, l23::SM_TOTAL, (cudaStream_t)stream>>>(A);
     return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA;
-}
-
-extern "C" int ss_actor_forward_frames_tc(const float *params, int64_t param_stride, int64_t noise_group, const void *stack_tc,
-                                          int frames, int64_t head, float *act_out, int64_t n_rows, void *workspace,
-                                          int64_t workspace_bytes, void *stream) {
-    return frames_forward(params, param_stride, noise_group, stack_tc, frames, head, act_out, n_rows, workspace, workspace_bytes,
-                          nullptr, stream);
-}
-
-// development: the same with an event trace of CTA 0 of the layer-1 kernel (3 roles x 256 events x {clock, code}); tools/frames_trace.py
-extern "C" int ss_debug_frames_trace(const float *params, const void *stack_tc, int frames, int64_t head, float *act_out,
-                                     int64_t n_rows, void *workspace, int64_t workspace_bytes, long long *trace, void *stream) {
-    return frames_forward(params, 0, 0, stack_tc, frames, head, act_out, n_rows, workspace, workspace_bytes, trace, stream);
 }

@@ -31,9 +31,8 @@ enum : int { kPdlOff = 0, kPdlOn = 1, kPdlEarlyWeights = 2, kPdlEarlyAfterFirst 
 
 // the launch mode of the calling host thread; set by ss_ddpg_update around each entry point it calls
 int &pdl_mode();
-// whether ss_ddpg_update / ss_selfplay_rollout chain their launches at all: ss_set_dependent_launch(), else the environment
-// (SS_UPDATE_PDL=0 / SS_ROLLOUT_PDL=0 switch the respective chain off)
-bool chain_enabled(const char *env_name);
+// whether ss_ddpg_update / ss_selfplay_rollout chain their launches at all: yes unless ss_set_dependent_launch(0)
+bool chain_enabled();
 
 struct PdlScope {                     // sets the mode for the lifetime of the object
     int saved;

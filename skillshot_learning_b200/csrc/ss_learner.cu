@@ -19,7 +19,6 @@
 // identical whatever the number of CTAs that took part).
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 
 #include "../../include/skillshot_b200.h"
 #include "ss_launch.cuh"
@@ -769,16 +768,6 @@ inline size_t smem_critic_grad(int ds) { return (size_t)(ds + H1 + DA + H2) * PI
 inline size_t smem_actor_grad(int ds) { return (size_t)(ds + H1 + H2 + DA + H1 + DA + H2 + DA) * PITCH * 4 + TB * 4; }
 
 inline int check_launch() { return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA; }
-// SS_ROLLOUT_FUSED=1 plays the rollout tick as ONE kernel (ss_actor_forward_step_tc: the env step in the forward kernel's
-// output stage).  It is correct (bit-identical, tested) and OFF by default because it is slower: 119 us per tick at 262,144
-// envs against 71 us for the two kernels -- the env tick is ~450 dependent instructions, three float64 sin / cos among them,
-// and the four output warps that would run it are one warp per scheduler: nothing hides its latency there, while the
-// stand-alone kernel runs 32 warps per SM (profiles/r2_rollout_fused_vs_two_kernels.txt).
-inline bool rollout_fused() {
-    static int v = -1;
-    if (v < 0) { const char *e = getenv("SS_ROLLOUT_FUSED"); v = (e && e[0] == '1') ? 1 : 0; }
-    return v != 0;
-}
 
 template <class K>
 int max_ctas(K kernel, size_t smem) {
@@ -1109,25 +1098,19 @@ int ss_selfplay_rollout(void *env_state, int64_t n_envs, const float *actor_para
         // The two kernels of a tick form a dependent-launch chain (ss_launch.cuh): each grid is placed while its predecessor
         // drains and holds at griddepcontrol.wait.  From the second tick on the forward kernel also stages (and perturbs) the
         // actor's parameters ahead of that wait -- its predecessor, the env step, does not write them; the first tick's
-        // forward may follow an update's Adam kernel and waits first.  SS_ROLLOUT_PDL=0 / ss_set_dependent_launch(0): ordinary launches.
-        const int kOn = (tensor_cores && sslaunch::chain_enabled("SS_ROLLOUT_PDL")) ? sslaunch::kPdlOn : sslaunch::kPdlOff;
+        // forward may follow an update's Adam kernel and waits first.  ss_set_dependent_launch(0): ordinary launches.
+        // A tick stays two kernels: the whole tick as ONE kernel (ss_actor_forward_step_tc, the env step in the forward
+        // kernel's output stage) is bit-identical and slower, 119 us per tick at 262,144 envs against 71 us -- the env tick
+        // is ~450 dependent instructions, three float64 sin / cos among them, and the four output warps that would run it
+        // are one warp per scheduler: nothing hides its latency there, while the stand-alone kernel runs 32 warps per SM
+        // (profiles/r2_rollout_fused_vs_two_kernels.txt).
+        const int kOn = (tensor_cores && sslaunch::chain_enabled()) ? sslaunch::kPdlOn : sslaunch::kPdlOff;
         sslaunch::PdlScope scope(kOn);
         for (int t = 0; t < n_ticks; ++t, seg = (seg + 1) % segs) {
             float *o = ring_obs + seg * rows * 12, *a = ring_act + seg * rows * 2;
             // the last tick's observation goes to the caller's buffer, the others to the next segment's rows
             float *o_next = (t + 1 < n_ticks) ? ring_obs + ((seg + 1) % segs) * rows * 12 : obs_a;
             sslaunch::pdl_mode() = (kOn && t > 0) ? (sslaunch::kPdlOn | sslaunch::kPdlEarlyWeights) : kOn;
-            if (tensor_cores && !speeds && reward_mode != SS_REWARD_SIMPLE && rollout_fused()) {
-                // the whole tick as ONE kernel: the forward kernel's output stage plays the env step of the rows it has
-                // just computed the actions of, and writes the transition straight into the ring (ss_mlp_tc.cu)
-                const int rc1 = ss_actor_forward_step_tc(actor_params, o, a, rows, param_noise_sd, noise_group, action_noise_sd,
-                                                         noise_seed, noise_counter + (uint64_t)t, env_state,
-                                                         ring_next_obs + seg * rows * 12, o_next, ring_reward + seg * rows, done,
-                                                         ring_done + seg * rows, winner, reward_mode, tick_limit, reset_mode,
-                                                         env_seed, env_counter + (uint64_t)t, status, step_flags, stream);
-                if (rc1 != SS_OK) return rc1;
-                continue;
-            }
             int rc = tensor_cores
                          ? ss_actor_forward_tc(actor_params, o, a, rows, param_noise_sd, noise_group, action_noise_sd, noise_seed,
                                                noise_counter + (uint64_t)t, stream)

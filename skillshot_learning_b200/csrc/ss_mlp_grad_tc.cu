@@ -33,8 +33,6 @@
 // Gradients are therefore computed from bf16 operands (products exact, fp32 accumulation):
 // relative error ~1e-3 against the float32 path of ss_learner.cu, which remains the exact one.
 // Per-CTA partial gradients go to the same workspace layout and fixed-order reduction as there.
-#include <stdlib.h>
-
 #include "ss_tc_common.cuh"
 
 namespace {
@@ -78,7 +76,6 @@ struct GradArgs {
     uint64_t seed, counter;
     int64_t n, n_global, row_offset;
     float *work;                     // [gridDim.x][params + 1]
-    long long *trace;                // development: event timestamps of CTA 0 (NULL in production)
     int early_weights;               // ss_launch.cuh: the parameters may be staged ahead of griddepcontrol.wait (set by launch_grad)
 };
 
@@ -123,16 +120,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_grad_tc_kernel(const GradArgs
     const uint32_t sbase = smem_u32(smem);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t bar_mma = sbase + SM_BAR, bar_epi = sbase + SM_BAR + 8;
-    int tr_n = 0;                    // development trace: role 0 = epilogue warp 0, role 1 = MMA warp
-    auto trace = [&](int role, int code) {
-        if (A.trace && blockIdx.x == 0 && lane == 0 && (warp == 0 || warp == MMA_WARP) && tr_n < 256) {
-            A.trace[(role * 256 + tr_n) * 2] = clock64();
-            A.trace[(role * 256 + tr_n) * 2 + 1] = code;
-            ++tr_n;
-        }
-    };
-
-    trace(0, 900);
     if (threadIdx.x == 0) {
         mbar_init(bar_mma, 32 * EPI_WARPS);
         mbar_init(bar_epi, 1);
@@ -161,7 +148,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_grad_tc_kernel(const GradArgs
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem = *reinterpret_cast<const volatile uint32_t *>(smem + SM_TMEM);
-    trace(0, 901);
 
     const int64_t tiles = (A.n + TM - 1) / TM;
     float *g = A.work + (int64_t)blockIdx.x * (PN + 1);
@@ -179,10 +165,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_grad_tc_kernel(const GradArgs
         const uint32_t thresh16 = (uint32_t)(A.rate * 65536.0f);
         uint32_t ph = 0;
         float stat = 0.f, dsum0 = 0.f, dsum1 = 0.f;      // sum of squared errors; db3 partials
-        // development trace codes: kind * 1000 + 8 * (tile of this CTA) + phase (0 L1a, 1 L1b, 2 L2, 3 G2|BXa|G3, 4 BXb, 5 G1)
-        int tl_i = 0;
-        auto to_mma = [&](int phase) { fence_proxy_async(); tc_fence_before(); mbar_arrive(bar_mma); trace(0, 1000 + tl_i * 8 + phase); };
-        auto from_mma = [&](int phase) { mbar_wait(bar_epi, ph); ph ^= 1; tc_fence_after(); trace(0, 2000 + tl_i * 8 + phase); };
+        int tl_i = 0;                                   // tiles done by this CTA
+        auto to_mma = [&]() { fence_proxy_async(); tc_fence_before(); mbar_arrive(bar_mma); };
+        auto from_mma = [&]() { mbar_wait(bar_epi, ph); ph ^= 1; tc_fence_after(); };
 
         // hidden layer 1, one 128-unit half: WORK -> ReLU (+ dropout) -> bf16 -> X2 chunks 16 * half ..
         // Inverted-dropout keep bits of this thread's row for the columns its warp handles: 2 halves x 4 steps x 16
@@ -281,16 +266,16 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_grad_tc_kernel(const GradArgs
             // every warp has arrived for the previous tile's G1 before any arrives for this tile's L1a (no wait lies between
             // the two arrivals, and a warp that arrived twice in one phase would complete it without the slowest one)
             if (tl_i > 0) asm volatile("bar.sync 1, 256;" ::: "memory");
-            to_mma(0);                                    // -> L1a
-            from_mma(0);                                  // (the commit behind L1a also retires the previous tile's G1)
+            to_mma();                                     // -> L1a
+            from_mma();                                   // (the commit behind L1a also retires the previous tile's G1)
             hidden1(0);
-            to_mma(1);                                    // -> L1b
-            from_mma(1);
+            to_mma();                                     // -> L1b
+            from_mma();
             hidden1(1);
-            to_mma(2);                                    // -> L2
+            to_mma();                                     // -> L2
             make_keep(tile + gridDim.x, 0, 0);            // in the shadow of the 17-step layer-2 chain
             make_keep(tile + gridDim.x, 0, 1);
-            from_mma(2);
+            from_mma();
             // ---- output layer, loss / upstream gradient (fp32) ----
             float z0 = 0.f, z1 = 0.f;
             sweep_work(tl + T_WORK, cs, [&](const uint32_t (&v)[16], int j) {
@@ -358,21 +343,20 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_grad_tc_kernel(const GradArgs
                         make_uint4(pack_bf16(gz[0], gz[1]), pack_bf16(gz[2], gz[3]), pack_bf16(gz[4], gz[5]), pack_bf16(gz[6], gz[7]));
                 }
             });
-            to_mma(3);                                    // -> G2 (first half), BXa | G2 (second half), G3
+            to_mma();                                     // -> G2 (first half), BXa | G2 (second half), G3
             make_keep(tile + gridDim.x, 1, 0);            // ... of G2's first half and BXa
-            from_mma(3);                                  // dx2[:, :128] is there and h1[:, :128] has been consumed
+            from_mma();                                   // dx2[:, :128] is there and h1[:, :128] has been consumed
             back1(0);                                     // (beside the rest of G2 and G3)
-            to_mma(4);                                    // -> BXb
+            to_mma();                                     // -> BXb
             make_keep(tile + gridDim.x, 1, 1);            // ... and of the rest of the weight-gradient group and BXb
-            from_mma(4);                                  // ... which also retires G2 / G3: h1[:, 128:], h2, dz2 are free
+            from_mma();                                   // ... which also retires G2 / G3: h1[:, 128:], h2, dz2 are free
             back1(1);
             store_obs_half(xin, dz2row, cs);              // X0 for G1 (the DZ2 buffer is free: BXb has retired)
-            to_mma(5);                                    // -> G1, not waited for: it retires with the next tile's L1a
+            to_mma();                                     // -> G1, not waited for: it retires with the next tile's L1a
             ++tl_i;
         }
-        from_mma(5);                                      // the last tile's G1
+        from_mma();                                       // the last tile's G1
 
-        trace(0, 902);
         // ======================= write this CTA's partial gradient =======================
         // thread r = hidden-2 unit r for dW2'^T and dW3^T, = hidden-1 unit 128 h + r for dW1'^T; columns split by slice
         {
@@ -434,7 +418,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_grad_tc_kernel(const GradArgs
                 }
             }
         }
-        trace(0, 903);
         tc_fence_before();
     } else {
         // ======================= the MMA-issuing warp =======================
@@ -445,13 +428,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_grad_tc_kernel(const GradArgs
         constexpr uint32_t kFwd = umma_idesc(TM, 128);                // K-major x K-major
         constexpr uint32_t kBx = umma_idesc(TM, 128, 0, 1);           // dz2 (K-major) x W2 image (MN-major)
         constexpr uint32_t kG128 = umma_idesc(TM, 128, 1, 1), kG16 = umma_idesc(TM, 16, 1, 1), kG32 = umma_idesc(TM, 32, 1, 1);
-        int tl_i = 0;
-        auto wait_epi = [&](int phase) { mbar_wait(bar_mma, ph); ph ^= 1; tc_fence_after(); trace(1, 3000 + tl_i * 8 + phase); };
-        auto issued = [&](int phase) { trace(1, 4000 + tl_i * 8 + phase); };
+        auto wait_epi = [&]() { mbar_wait(bar_mma, ph); ph ^= 1; tc_fence_after(); };
         uint32_t acc = 0;                                             // 0 on the CTA's first tile: accumulators start fresh
         for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x, acc = 1) {
             for (int half = 0; half < 2; ++half) {                    // L1a, L1b (X0 sits in the head of the H2 buffer)
-                wait_epi(half);
+                wait_epi();
                 if (lane == 0) {
                     const uint64_t ad = desc_kmajor(h2, CHUNK_A), bd = desc_kmajor(b1 + half * 128 * 16, CHUNK_B1);
 #pragma unroll
@@ -460,9 +441,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_grad_tc_kernel(const GradArgs
                     umma_commit(bar_epi);
                 }
                 __syncwarp();
-                issued(half);
             }
-            wait_epi(2);                                              // L2
+            wait_epi();                                               // L2
             if (lane == 0) {
                 const uint64_t ad = desc_kmajor(x2, CHUNK_A), bd = desc_kmajor(b2, CHUNK_B2);
 #pragma unroll
@@ -471,11 +451,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_grad_tc_kernel(const GradArgs
                 umma_commit(bar_epi);
             }
             __syncwarp();
-            issued(2);
             // The epilogue warps wait for nothing but dx2: what they need first goes first.  The first half of G2 consumes
             // h1[:, :128] (the chunks back1(0) overwrites with dz1), BXa delivers dx2[:, :128]; the commit behind those two
             // releases back1(0), which then runs beside the second half of G2, its bias / action columns and G3.
-            wait_epi(3);                                              // G2, BXa, G3
+            wait_epi();                                               // G2, BXa, G3
             if (lane == 0) {
                 const uint64_t h2t = desc_mnmajor(h2, CHUNK_A), dz3t = desc_mnmajor(dz3, CHUNK_A);
                 const uint64_t dz2t = desc_mnmajor(dz2, CHUNK_A), x2t = desc_mnmajor(x2, CHUNK_A);
@@ -500,8 +479,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_grad_tc_kernel(const GradArgs
                 }
             }
             __syncwarp();
-            issued(3);
-            wait_epi(4);                                              // BXb; its commit also retires the G group above
+            wait_epi();                                               // BXb; its commit also retires the G group above
             if (lane == 0) {
                 const uint64_t ad = desc_kmajor(dz2, CHUNK_A), bd = desc_mnmajor(b2 + 16 * CHUNK_B2, CHUNK_B2);
 #pragma unroll
@@ -510,8 +488,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_grad_tc_kernel(const GradArgs
                 umma_commit(bar_epi);
             }
             __syncwarp();
-            issued(4);
-            wait_epi(5);                                              // G1: no commit of its own, the next L1a's covers it
+            wait_epi();                                               // G1: no commit of its own, the next L1a's covers it
             if (lane == 0) {
                 const uint64_t x0t = desc_mnmajor(dz2, CHUNK_A);
 #pragma unroll
@@ -524,8 +501,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_grad_tc_kernel(const GradArgs
                 }
             }
             __syncwarp();
-            issued(5);
-            ++tl_i;
         }
         if (lane == 0) umma_commit(bar_epi);                          // the last tile's G1
         __syncwarp();
@@ -586,17 +561,6 @@ int launch_grad(const GradArgs &A0, float *grad_out, float *aux_out, int64_t wor
 }  // namespace
 
 extern "C" {
-
-// development: the critic gradient kernel with an event trace of CTA 0 (tools/tc_grad_trace.py)
-int ss_debug_critic_grad_trace(const float *critic_params, const float *obs, const float *act, const float *target,
-                               int64_t n, float *grad_out, void *workspace, int64_t workspace_bytes, long long *trace,
-                               void *stream) {
-    GradArgs A{};
-    A.params = critic_params; A.obs = obs; A.act = act; A.target = target; A.rate = 0.2f; A.n = n; A.n_global = n;
-    if (const char *e = getenv("SS_TRACE_RATE")) A.rate = (float)atof(e);      // 0: no dropout, the actor kernel's schedule
-    A.work = (float *)workspace; A.trace = trace;
-    return launch_grad<NET_CRITIC>(A, grad_out, nullptr, workspace_bytes, stream);
-}
 
 int ss_critic_grad_tc(const float *critic_params, const float *obs, const float *act, const float *target,
                       const uint8_t *dropout_keep, float dropout_rate, uint64_t seed, uint64_t counter,

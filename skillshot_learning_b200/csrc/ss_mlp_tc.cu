@@ -57,8 +57,6 @@ struct FwdArgs {
     const float *reward;
     const uint8_t *done;
     float gamma;
-    long long *trace;        // development: event timestamps of CTA 0 (NULL in production)
-    int dbg;                 // development ablations: 1 = output warps skip layer 3, 2 = producers skip the conversion
     // fused env step (ss_actor_forward_step_tc): rows are players in env order (row = 2 env + player); the output-warp lane
     // that has just computed a player's action plays that player's tick (ss_env_pp.cuh) and writes the transition
     void *env_state;         // packed env state of n / 2 envs
@@ -120,7 +118,7 @@ __device__ __forceinline__ void layer3(const uint32_t (&v)[32], const float4 *w3
 // epilogue 1 -> MMA2 -> epilogue 2 (tensor pipe 43-47 % busy: the chain is ~4x a tile's MMA time and there
 // is no shared memory for a third 68 KB tile); a 64-column block pipeline between the layers ran 2x SLOWER
 // (issue-bound: 25 MMAs, 10 waits, 10 commits per tile on the one issuing thread).  An event trace of this
-// version (tools/tc_trace.py) shows the MMA warp as the pacing role.
+// version (profiles/r1_actor_fwd_tc_event_trace.txt) showed the MMA warp as the pacing role.
 namespace pipe {
 
 // the "empty" word of the pair mailbox: a NaN payload no arithmetic produces (tanhf of a NaN gives the canonical 0x7fffffff)
@@ -150,17 +148,6 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
     const uint32_t sbase = smem_u32(smem);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     auto bar = [&](int idx) -> uint32_t { return sbase + SMP_BAR + (uint32_t)idx * 8; };
-    // development trace (A.trace != NULL): role 0 = producer warp 0, 1 = output warp 4, 2 = MMA warp
-    int tr_n = 0;
-    auto trace = [&](int role, int code) {
-        if (A.trace && cta == 0 && lane == 0 && (warp == 0 || warp == P_WARPS || warp == MMA_W) && tr_n < 256) {
-            A.trace[(role * 256 + tr_n) * 2] = clock64();
-            A.trace[(role * 256 + tr_n) * 2 + 1] = code;
-            ++tr_n;
-        }
-    };
-
-    trace(0, 900);
     if (threadIdx.x == 0) {
         mbar_init(bar(B_X), 128);
         mbar_init(bar(B_Z), 1);
@@ -182,7 +169,6 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem = *reinterpret_cast<const volatile uint32_t *>(smem + SMP_TMEM);
-    trace(0, 901);
 
     const bool noisy = NET == NET_ACTOR && A.param_sd > 0.f;
     const int64_t group = noisy ? A.group : A.n;
@@ -220,7 +206,6 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
         }
         fence_proxy_async();
         __syncthreads();
-        trace(0, 902);
 
         if (warp < P_WARPS) {
             // ============ producer warps: observation staging and the layer-1 epilogue ============
@@ -262,14 +247,12 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
                 } else if (NET == NET_CRITIC && row0 + i * TM + r < end) {
                     act = __ldg(reinterpret_cast<const float2 *>(A.act_in) + row0 + i * TM + r);
                 }
-                trace(0, 100 + (int)i);
                 // MMA1(tile) retired: D1 holds layer 1 and X0[tc & 1] is dead.  The tensor pipe retires one thread's MMAs
                 // in issue order and MMA2(tile - 2) was issued before MMA1(tile), so A1[tc & 1] is free as well.
                 mbar_wait(bar(B_Z), tc & 1);
                 tc_fence_after();
-                trace(0, 200 + (int)i);
                 if (NET == NET_CRITIC) *reinterpret_cast<uint4 *>(arow + (H1 / 8) * CHUNK_A) = tail_chunk_critic(act.x, act.y);
-                if (!(A.dbg & 2)) {
+                {
                     uint32_t va[32], vb[32];
                     tmem_ld32(tl, va);
 #pragma unroll
@@ -285,7 +268,6 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
                 fence_proxy_async();
                 tc_fence_before();
                 mbar_arrive(bar(B_X));                            // A1[tile] full, D1 free, X0(tile + 1) staged
-                trace(0, 500 + (int)i);
                 if (i + 2 < ntiles) stage_x0(i + 2);              // into X0[tc & 1]
                 if (NET == NET_CRITIC && A.pair_mail && i + 1 < ntiles) {
                     // the next tile's actions, if the actor role has delivered all 32 by now
@@ -302,7 +284,6 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
             for (int64_t i = 0; i < ntiles; ++i) {
                 const uint32_t tc = tcount + (uint32_t)i, slot = tc & 1;
                 const int64_t row = row0 + i * TM + r;
-                trace(1, 100 + (int)i);
                 // FUSED: this row's player.  Its state and the sin / cos of its two rotations do not depend on the action:
                 // they are fetched and evaluated here, in the time this warp would otherwise spend waiting for MMA2.
                 sspp::LaneState L;
@@ -314,8 +295,6 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
                 }
                 mbar_wait(bar(B_Y + slot), (tc >> 1) & 1);
                 tc_fence_after();
-                trace(1, 200 + (int)i);
-                if (A.dbg & 1) { tc_fence_before(); mbar_arrive(bar(B_D2E + slot)); continue; }
                 float acc[3][4] = {{b3[0], 0.f, 0.f, 0.f}, {NET == NET_ACTOR ? b3[1] : 0.f, 0.f, 0.f, 0.f}, {0.f, 0.f, 0.f, 0.f}};
                 {
                     constexpr int kW3Step = NET == NET_ACTOR ? 16 : 32;
@@ -330,7 +309,6 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
                         if (j + 2 < H2 / 32) tmem_ld32(tl + slot * 128 + (j + 2) * 32, va);
                         else { tc_fence_before(); mbar_arrive(bar(B_D2E + slot)); }     // D2[slot] fully read
                         layer3<NET>(vb, w3x + (j + 1) * kW3Step, acc);
-                        trace(1, (j == 0 ? 600 : 700) + (int)i);
                     }
                 }
                 const float out0 = (acc[0][0] + acc[0][1]) + (acc[0][2] + acc[0][3]);
@@ -382,7 +360,6 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
                         }
                     }
                 }
-                trace(1, 800 + (int)i);
             }
         } else {
             // ============ the MMA-issuing warp ============
@@ -398,11 +375,11 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
             //    producers waiting explicitly for MMA2(t-2)) -- correct, 5 % slower: the output warps' ~1.8 k cycles per
             //    tile and the producers' ~1.2 k are then the pace, not the issuing thread;
             //  * both waits first, then MMA1(t+1) and the MMA2(t) chain back to back with one fence -- no change;
-            //  * ablations (tools/tc_ablate.py, 524,288 rows): 44.5 us whole, 37.4 with the output warps' layer 3 switched
+            //  * ablations (a development build, 524,288 rows): 44.5 us whole, 37.4 with the output warps' layer 3 switched
             //    off, 40.2 with the producers' conversion off, 35.3 with both off -- the issuing loop alone (two waits,
             //    MMA1, 17 x MMA2, two commits per tile) already takes ~1.9 k cycles per tile against 1.29 k of MMA execution;
             //  * fetching the output warps' layer-3 weights eight loads ahead of their FMAs -- their pass over D2 drops
-            //    from ~1.6 k to ~1.2 k cycles per tile (trace events 600 / 700 / 800) and the KERNEL gets 6 % slower;
+            //    from ~1.6 k to ~1.2 k cycles per tile (event trace) and the KERNEL gets 6 % slower;
             //  * eight producer warps (two per tensor-memory lane quadrant) -- 12 % SLOWER;
             //  * cta_group::2 (a cluster of two CTAs, one thread issuing M = 256 pair MMAs for both, each CTA holding
             //    half of the weight images, hand-offs through the cluster address window, multicast commits) --
@@ -426,15 +403,11 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
             mma1(tc0);
             for (int64_t i = 0; i < ntiles; ++i) {
                 const uint32_t tc = __shfl_sync(0xffffffffu, tc0 + (uint32_t)i, 0), slot = tc & 1;
-                trace(2, 100 + (int)i);
                 mbar_wait_likely_done(bar(B_X), xph); xph ^= 1;   // A1[tile] full, D1 free, X0(tile + 1) staged
                 tc_fence_after();
-                trace(2, 200 + (int)i);
                 if (i + 1 < ntiles) mma1(tc + 1);
-                trace(2, 300 + (int)i);
                 mbar_wait_likely_done(bar(B_D2E + slot), ((tc >> 1) & 1) ^ 1);    // the output warps have drained D2[slot]
                 tc_fence_after();
-                trace(2, 400 + (int)i);
                 if (lane == 0) {
                     const uint64_t ad = desc_advance(a1d, slot * X2_BYTES);
 #pragma unroll
@@ -443,7 +416,6 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
                                   kI2, ks > 0);
                     umma_commit(bar(B_Y + slot));
                 }
-                trace(2, 500 + (int)i);
             }
         }
         tcount += (uint32_t)ntiles;
@@ -451,7 +423,6 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
         tc_fence_before();
         __syncthreads();                   // pipeline drained: the output warps have read the last D2
         tc_fence_after();
-        trace(0, 903);
     }
 
     if (!waited) { sslaunch::griddep_wait(); sslaunch::griddep_launch(); }      // a CTA without a tile still waits
@@ -573,14 +544,6 @@ extern "C" int ss_actor_forward_step_tc(const float *actor_params, const float *
     A.TP.seed = env_seed; A.TP.counter = env_counter; A.TP.tick_limit = tick_limit; A.TP.reward_mode = reward_mode;
     A.TP.auto_reset = 1; A.TP.reset_mode = reset_mode;
     return launch_fwd<NET_ACTOR, true>(A, stream);
-}
-
-// development: the actor forward with an event trace of CTA 0 (3 roles x 256 events x {clock, code}); tools/tc_trace.py
-extern "C" int ss_debug_actor_forward_trace(const float *actor_params, const float *obs, float *act_out, int64_t n,
-                                            long long *trace, void *stream, int dbg) {
-    FwdArgs A{};
-    A.params = actor_params; A.obs = obs; A.n = n; A.group = n; A.act_out = act_out; A.trace = trace; A.dbg = dbg;
-    return launch_fwd<NET_ACTOR>(A, stream);
 }
 
 extern "C" int ss_critic_forward_tc(const float *critic_params, const float *obs, const float *act, int64_t n,

@@ -10,7 +10,6 @@
 // arguments, from C.  Nothing here touches the device directly.
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 
 #include "../../include/skillshot_b200.h"
 #include "ss_launch.cuh"
@@ -23,14 +22,9 @@ int &sslaunch::pdl_mode() {
     return mode;
 }
 
-static std::atomic<int> g_chain_override{-1};       // -1: the environment decides
+static std::atomic<int> g_chain_override{-1};       // -1: the default (chained)
 
-bool sslaunch::chain_enabled(const char *env_name) {
-    const int o = g_chain_override.load(std::memory_order_relaxed);
-    if (o >= 0) return o != 0;
-    const char *e = getenv(env_name);
-    return !(e && e[0] == '0');
-}
+bool sslaunch::chain_enabled() { return g_chain_override.load(std::memory_order_relaxed) != 0; }
 
 extern "C" int ss_set_dependent_launch(int enabled) {
     return g_chain_override.exchange(enabled < 0 ? -1 : (enabled ? 1 : 0), std::memory_order_relaxed);
@@ -61,8 +55,8 @@ extern "C" int ss_ddpg_update(const ss_ddpg_update_args *a, void *stream) {
     //   critic(s, a) -> actor gradient -> reduce + Adam (actor, actor')
     // With the peer exchange the order is ... critic gradient -> push -> actor(s) -> peers' Adam (critic) -> critic(s, a) -> ...:
     // critic(s, a) then directly follows the kernel that writes the critic and stages behind its wait (kPdlEarlyAfterFirst).
-    // SS_UPDATE_PDL=0 or ss_set_dependent_launch(0) switches the chain off (A/B measurements, the equality test).
-    const int kOn = sslaunch::chain_enabled("SS_UPDATE_PDL") ? sslaunch::kPdlOn : sslaunch::kPdlOff;
+    // ss_set_dependent_launch(0) switches the chain off (the equality test).
+    const int kOn = sslaunch::chain_enabled() ? sslaunch::kPdlOn : sslaunch::kPdlOff;
     const int kEarly = kOn ? (sslaunch::kPdlOn | sslaunch::kPdlEarlyWeights) : sslaunch::kPdlOff;
     sslaunch::PdlScope scope(kOn);
 
@@ -98,21 +92,11 @@ extern "C" int ss_ddpg_update(const ss_ddpg_update_args *a, void *stream) {
     // the Adam kernel that waits for the peers' pushes, so that the exchange's latency (rank skew + NVLink visibility,
     // ~20 us on 8 GPUs) passes under 15 us of useful work instead of an idle spin.  (The gradient slices of the critic step
     // have been consumed by the push kernel by then; the actions land in the scratch area behind the slices.)
-    // SS_PEER_FUSED=1 (experiment, off by default) makes push, wait and Adam ONE kernel per exchange (ss_peer_reduce_adam_tf:
-    // each 64-parameter CTA goes on as soon as its own values have arrived from every rank) and runs the actor step as on a
-    // single GPU.  Bit-identical (peer_check ok) and SLOWER: 0.203 vs 0.189 ms per update on 2 GPUs
-    // (profiles/r2_peer_fused_ab_n2.txt) -- 573 CTAs each fencing and polling at system scope cost more than the kernel
-    // boundary they remove, and nothing runs under the wait any more.
-    static const bool fused_env = [] { const char *e = getenv("SS_PEER_FUSED"); return e && e[0] == '1'; }();
-    const bool fused_exchange = peers && fused_env;
-    // SS_PEER_STAGED=0 (A/B): no early actor forward; the actor step's forward pair then runs as one launch after Adam
-    static const bool staged_env = [] { const char *e = getenv("SS_PEER_STAGED"); return !(e && e[0] == '0'); }();
-    const bool early_actor_forward = peers && tc && !fused_exchange && staged_env;
-    if (fused_exchange) {
-        rc = ss_peer_reduce_adam_tf(a->workspace, rc, SS_CRITIC_PARAMS, a->stats, a->peer_bases, a->world, a->rank, a->peer_capacity,
-                                    a->epoch, a->critic, a->m_critic, a->v_critic, a->target_critic, a->grad_critic, a->step_critic,
-                                    a->lr_critic, a->beta1, a->beta2, a->eps, a->tau, 1.0f, a->status, stream);
-    } else if (peers) {
+    // Push, wait and Adam as ONE kernel per exchange (ss_peer_reduce_adam_tf) is bit-identical and was measured SLOWER:
+    // 0.203 vs 0.189 ms per update on 2 GPUs (profiles/r2_peer_fused_ab_n2.txt) -- 573 CTAs each fencing and polling at
+    // system scope cost more than the kernel boundary they remove, and nothing runs under the wait any more.
+    const bool early_actor_forward = peers && tc;
+    if (peers) {
         rc = ss_peer_reduce_push(a->workspace, rc, SS_CRITIC_PARAMS, a->stats, a->peer_bases, a->world, a->rank,
                                  a->peer_capacity, a->epoch, a->done_counter, stream);
         if (rc != SS_OK) return rc;
@@ -145,11 +129,7 @@ extern "C" int ss_ddpg_update(const ss_ddpg_update_args *a, void *stream) {
         rc = ss_actor_grad(a->actor, a->critic, a->obs, n, nullptr, a->stats + 1, a->workspace, a->workspace_bytes, stream);
     if (rc <= 0) return rc < 0 ? rc : SS_ERR_INVALID_ARG;
     sslaunch::pdl_mode() = kOn;
-    if (fused_exchange) {
-        rc = ss_peer_reduce_adam_tf(a->workspace, rc, SS_ACTOR_PARAMS, a->stats + 1, a->peer_bases, a->world, a->rank, a->peer_capacity,
-                                    a->epoch + 1, a->actor, a->m_actor, a->v_actor, a->target_actor, a->grad_actor, a->step_actor,
-                                    a->lr_actor, a->beta1, a->beta2, a->eps, a->tau, 1.0f, a->status, stream);
-    } else if (peers) {
+    if (peers) {
         rc = ss_peer_reduce_push(a->workspace, rc, SS_ACTOR_PARAMS, a->stats + 1, a->peer_bases, a->world, a->rank,
                                  a->peer_capacity, a->epoch + 1, a->done_counter, stream);
         if (rc != SS_OK) return rc;

@@ -1258,8 +1258,7 @@ class SelfPlayTrainer:
         k = self.updates & 1
         # (measured, profiles/r2_update_sample_early_ab.txt: 158.1 -> 152.1 us at 65,536 rows; at 524,288 rows the gather
         #  competes with what it runs beside, 759 -> 764 us: small minibatches only)
-        early = (self._ring_clean and self._batches[k] is not None and self.batch_size <= 131072 and
-                 os.environ.get("SS_UPDATE_SAMPLE_EARLY", "1") != "0")
+        early = self._ring_clean and self._batches[k] is not None and self.batch_size <= 131072
         self._batch = self._batches[k] = net.update_from_ring(self.replay, self.batch_size, out=self._batches[k], sample_early=early)
         self._ring_clean = True
         self.updates += 1

@@ -1,4 +1,4 @@
-"""Development: device time of one DDPG update (the bench's update leg) at a few minibatch sizes; run with SS_UPDATE_PDL=0 / 1."""
+"""Development: device time of one DDPG update (the bench's update leg) at a few minibatch sizes."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -21,6 +21,6 @@ for batch in [int(x) for x in (sys.argv[1:] or ["65536", "524288"])]:
         e1.record()
         torch.cuda.synchronize()
         best = min(best, e0.elapsed_time(e1) / 200 * 1e3)
-    print("SS_UPDATE_PDL=%s  batch %7d  update %.1f us  (sse %.6g  q %.6g)" % (os.environ.get("SS_UPDATE_PDL", "1"), batch, best,
-          float(tr.networks.stats[0]), float(tr.networks.stats[1])), flush=True)
+    print("batch %7d  update %.1f us  (sse %.6g  q %.6g)" % (batch, best, float(tr.networks.stats[0]), float(tr.networks.stats[1])),
+          flush=True)
     del tr
