@@ -427,6 +427,26 @@ int ss_critic_grad_frames(const float *critic_params, int frames, const float *o
                           void *workspace, int64_t workspace_bytes, void *stream);
 int ss_actor_grad_frames(const float *actor_params, const float *critic_params, int frames, const float *obs, int64_t n,
                          float *grad_out, float *q_sum_out, void *workspace, int64_t workspace_bytes, void *stream);
+/* The same four calls on the tensor cores (tcgen05.mma), argument for argument, with a workspace of
+ * ss_learner_frames_tc_workspace_bytes(frames, n) bytes (16-byte aligned) that holds the gradient slices and the tiles
+ * passed between the kernels of a call.  Precision: observations fp16 in the forward layer 1 and bf16 high + low halves
+ * in dW1; W1 fp16; hidden activations, dz1 / dz2 and W2 bf16; biases and the critic's action as high + low bf16 pairs;
+ * fp32 accumulation; the output layer, loss and tanh in fp32.  Results agree with the float32 path to about 2e-2 of
+ * their scale.  The gradient calls leave slices of n_params + 1 floats and return their number when grad_out is NULL,
+ * like ss_critic_grad_tc / ss_actor_grad_tc.  Dropout keep bits are those of ss_critic_grad_frames.  neg_dq_da_out
+ * [n][2] (may be NULL) receives -dQ/da. */
+int64_t ss_learner_frames_tc_workspace_bytes(int frames, int64_t n);
+int ss_critic_forward_frames_tc(const float *critic_params, int frames, const float *obs, const float *act, float *q_out,
+                                float *neg_dq_da_out, int64_t n, void *workspace, int64_t workspace_bytes, void *stream);
+int ss_ddpg_targets_frames_tc(const float *target_actor_params, const float *target_critic_params, int frames,
+                              const float *reward, const float *next_obs, const uint8_t *done, float gamma, float *y_out,
+                              int64_t n, void *workspace, int64_t workspace_bytes, void *stream);
+int ss_critic_grad_frames_tc(const float *critic_params, int frames, const float *obs, const float *act, const float *target,
+                             const uint8_t *dropout_keep, float dropout_rate, uint64_t seed, uint64_t counter,
+                             int64_t n, int64_t n_global, int64_t row_offset, float *grad_out, float *sse_out,
+                             void *workspace, int64_t workspace_bytes, void *stream);
+int ss_actor_grad_frames_tc(const float *actor_params, const float *critic_params, int frames, const float *obs, int64_t n,
+                            float *grad_out, float *q_sum_out, void *workspace, int64_t workspace_bytes, void *stream);
 int ss_replay_push_frames(float *ring_obs, float *ring_act, float *ring_reward, float *ring_next_obs, uint8_t *ring_done,
                           int64_t capacity, int64_t write_pos, int frames, const float *obs, const float *act,
                           const float *reward, const float *next_obs, const uint8_t *done, int done_div, int64_t n,

@@ -118,6 +118,12 @@ SIGNATURES = {
     "ss_ddpg_targets_frames": (_i32, [_vp, _vp, _i32, _vp, _vp, _vp, _f32, _vp, _i64, _vp]),
     "ss_critic_grad_frames": (_i32, [_vp, _i32, _vp, _vp, _vp, _vp, _f32, _u64, _u64, _i64, _i64, _i64, _vp, _vp, _vp, _i64, _vp]),
     "ss_actor_grad_frames": (_i32, [_vp, _vp, _i32, _vp, _i64, _vp, _vp, _vp, _i64, _vp]),
+    "ss_learner_frames_tc_workspace_bytes": (_i64, [_i32, _i64]),
+    "ss_critic_forward_frames_tc": (_i32, [_vp, _i32, _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp]),
+    "ss_ddpg_targets_frames_tc": (_i32, [_vp, _vp, _i32, _vp, _vp, _vp, _f32, _vp, _i64, _vp, _i64, _vp]),
+    "ss_critic_grad_frames_tc": (_i32, [_vp, _i32, _vp, _vp, _vp, _vp, _f32, _u64, _u64, _i64, _i64, _i64, _vp, _vp, _vp, _i64,
+                                         _vp]),
+    "ss_actor_grad_frames_tc": (_i32, [_vp, _vp, _i32, _vp, _i64, _vp, _vp, _vp, _i64, _vp]),
     "ss_replay_push_frames": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _i32, _i64, _vp]),
     "ss_replay_sample_frames": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _vp, _u64, _u64, _i64,
                                         _vp, _vp, _vp, _vp, _vp, _vp, _vp]),

@@ -32,6 +32,7 @@ UNITS = {
     "ss_peer.cu": [],
     "ss_update.cu": [],
     "ss_frames_tc.cu": [],
+    "ss_frames_grad_tc.cu": [],
     "ss_probe.cu": [],
 }
 

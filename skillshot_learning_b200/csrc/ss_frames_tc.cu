@@ -477,6 +477,18 @@ __global__ void obs_stack_push_tc_kernel(uint8_t *xt, int64_t n_rows, int frames
 
 }  // namespace
 
+int sstc::frames_layer1_tc(const float *params, const void *xt, int frames, int64_t n, void *h1, cudaStream_t st) {
+    FramesArgs A{params, (const uint8_t *)xt, nullptr, (uint8_t *)h1, n, n, 0, frames - 1, frames};
+    int dev = 0, sms = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) return SS_ERR_CUDA;
+    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return SS_ERR_CUDA;
+    const int64_t units = frame_units(n, n);
+    if (cudaFuncSetAttribute(l1::frames_l1_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l1::SM_TOTAL) != cudaSuccess)
+        return SS_ERR_CUDA;
+    l1::frames_l1_kernel<<<(int)(units < sms ? units : sms), l1::NTH, l1::SM_TOTAL, st>>>(A);
+    return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA;
+}
+
 extern "C" int64_t ss_obs_stack_tc_bytes(int64_t n_rows, int frames) {
     if (n_rows <= 0 || frames < 1 || frames > MAXF) return -1;
     return (n_rows + TM - 1) / TM * (int64_t)(frames_k1(frames) / 8) * CHUNK_A;

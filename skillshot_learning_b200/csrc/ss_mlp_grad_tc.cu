@@ -560,6 +560,11 @@ int launch_grad(const GradArgs &A0, float *grad_out, float *aux_out, int64_t wor
 
 }  // namespace
 
+int sstc::reduce_slices(const float *work, int parts, int n_params, float *grad, float *aux, cudaStream_t st) {
+    reduce_parts_kernel<<<(n_params + 1 + 63) / 64, dim3(64, 4), 0, st>>>(work, parts, n_params, grad, aux);
+    return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA;
+}
+
 extern "C" {
 
 int ss_critic_grad_tc(const float *critic_params, const float *obs, const float *act, const float *target,

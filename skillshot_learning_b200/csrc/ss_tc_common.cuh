@@ -369,4 +369,11 @@ __device__ __forceinline__ void stage_weights(const Stager &S) {
     }
 }
 
+// ---- launchers shared between translation units (host side) ------------------------------------
+// frames_l1_kernel (ss_frames_tc.cu) alone: H1 tiles of `params`' first layer from fp16 operand tiles whose columns are in
+// frame order (the layout ss_obs_stack_push_tc writes with ring head = frames - 1)
+int frames_layer1_tc(const float *params, const void *xt, int frames, int64_t n, void *h1, cudaStream_t st);
+// reduce_parts_kernel (ss_mlp_grad_tc.cu): grad[p] = fixed-order sum of `parts` slices of n_params + 1 floats, aux = extra slot
+int reduce_slices(const float *work, int parts, int n_params, float *grad, float *aux, cudaStream_t st);
+
 }  // namespace sstc

@@ -160,13 +160,11 @@ class ActorCritic:
             raise RuntimeError("skillshot_learning_b200 needs a CUDA device (no CPU fallback)")
         # frames > 1: the frame-stacked "planning" networks of readme.md:18-20 (no reference code): both first layers read
         # 12 * frames inputs, oldest frame first.  frames = 1 is the reference.  Their update runs on the exact float32
-        # kernels (ss_*_frames); the tensor-core gradient kernels are built for the reference's 12 inputs.
+        # kernels (ss_*_frames) or, with update_precision "bf16", on the tensor cores (ss_*_frames_tc, separate steps).
         self.frames = int(frames)
         self.a_n, self.c_n = int(lib.ss_actor_frames_params(self.frames)), int(lib.ss_critic_frames_params(self.frames))
         if self.a_n < 0 or self.c_n < 0:
             raise ValueError("frames must be 1..20")
-        if self.frames > 1 and update_precision != "f32":
-            raise ValueError("the frame-stacked networks are updated by the float32 kernels: update_precision='f32'")
         self.actor_shapes = [(12 * self.frames, 256)] + ACTOR_SHAPES[1:]
         self.critic_shapes = [(12 * self.frames, 256)] + CRITIC_SHAPES[1:]
         self.device = torch.device(device)
@@ -308,9 +306,16 @@ class ActorCritic:
         q = torch.empty(n, dtype=torch.float32, device=self.device)
         phi = self.target_critic if target else self.critic
         with torch.cuda.device(self.device):
+            if self.frames > 1 and precision == "bf16":
+                up = torch.empty((n, 2), dtype=torch.float32, device=self.device) if want_dq_da else None
+                ws = self._workspace_for(n, "bf16")
+                check(lib.ss_critic_forward_frames_tc(phi.data_ptr(), self.frames, obs.data_ptr(), act.data_ptr(), q.data_ptr(),
+                                                      _ptr(up), n, ws.data_ptr(), ws.numel(), _stream(self.device)),
+                      "ss_critic_forward_frames_tc")
+                return (q, up) if want_dq_da else q
             if self.frames > 1:
                 if precision != "f32":
-                    raise ValueError("frame-stacked networks: float32 kernels only")
+                    raise ValueError("precision must be 'f32' (exact path) or 'bf16' (tensor cores)")
                 check(lib.ss_critic_forward_frames(phi.data_ptr(), self.frames, obs.data_ptr(), act.data_ptr(), q.data_ptr(), n,
                                                    _stream(self.device)), "ss_critic_forward_frames")
                 return q
@@ -335,7 +340,12 @@ class ActorCritic:
             done = done.to(device=self.device, dtype=torch.uint8).contiguous()
         n = reward.shape[0]
         with torch.cuda.device(self.device):
-            if self.update_precision == "bf16":
+            if self.update_precision == "bf16" and self.frames > 1:
+                ws = self._workspace_for(n)
+                check(lib.ss_ddpg_targets_frames_tc(self.target_actor.data_ptr(), self.target_critic.data_ptr(), self.frames,
+                                                    reward.data_ptr(), next_obs.data_ptr(), _ptr(done), self.gamma, y.data_ptr(),
+                                                    n, ws.data_ptr(), ws.numel(), _stream(self.device)), "ss_ddpg_targets_frames_tc")
+            elif self.update_precision == "bf16":
                 ws = self._workspace_for(n)
                 check(lib.ss_ddpg_targets_tc(self.target_actor.data_ptr(), self.target_critic.data_ptr(),
                                              reward.data_ptr(), next_obs.data_ptr(), _ptr(done), self.gamma,
@@ -347,10 +357,15 @@ class ActorCritic:
                                                  _stream(self.device)), "ss_ddpg_targets")
         return y
 
-    def _workspace_for(self, n: int) -> torch.Tensor:
+    def _workspace_for(self, n: int, precision: Optional[str] = None) -> torch.Tensor:
         """Scratch for the gradient kernels: per-CTA gradient slices (+ 32 bytes per row for the
-        tensor-core entry points: actions, -dQ/da and Q of the actor step)."""
-        need = self._ws_base + (32 * n if self.update_precision == "bf16" else 0)
+        tensor-core entry points: actions, -dQ/da and Q of the actor step; frames > 1: the slices and the tiles passed
+        between the kernels of a call, ss_learner_frames_tc_workspace_bytes)."""
+        bf16 = (precision or self.update_precision) == "bf16"
+        if bf16 and self.frames > 1:
+            need = max(self._ws_base, int(lib.ss_learner_frames_tc_workspace_bytes(self.frames, n)))
+        else:
+            need = self._ws_base + (32 * n if bf16 else 0)
         if self.workspace.numel() < need:
             self.workspace = torch.empty(need, dtype=torch.uint8, device=self.device)
         return self.workspace
@@ -372,7 +387,10 @@ class ActorCritic:
         tail = (_ptr(keep), self.dropout, self.seed, self.counter, n, int(n_global), int(row_offset),
                 None if slices_only else g.data_ptr(), self.stats[0:1].data_ptr(), ws.data_ptr(), ws.numel(), _stream(self.device))
         with torch.cuda.device(self.device):
-            if self.update_precision == "bf16":
+            if self.update_precision == "bf16" and self.frames > 1:
+                rc = lib.ss_critic_grad_frames_tc(self.critic.data_ptr(), self.frames, obs.data_ptr(), act.data_ptr(), y.data_ptr(),
+                                                  *tail)
+            elif self.update_precision == "bf16":
                 rc = lib.ss_critic_grad_tc(self.critic.data_ptr(), obs.data_ptr(), act.data_ptr(), y.data_ptr(), *tail)
             else:
                 rc = lib.ss_critic_grad_frames(self.critic.data_ptr(), self.frames, obs.data_ptr(), act.data_ptr(), y.data_ptr(), *tail)
@@ -390,7 +408,9 @@ class ActorCritic:
         tail = (obs.data_ptr(), obs.shape[0], None if slices_only else g.data_ptr(), self.stats[1:2].data_ptr(), ws.data_ptr(),
                 ws.numel(), _stream(self.device))
         with torch.cuda.device(self.device):
-            if self.update_precision == "bf16":
+            if self.update_precision == "bf16" and self.frames > 1:
+                rc = lib.ss_actor_grad_frames_tc(self.actor.data_ptr(), self.critic.data_ptr(), self.frames, *tail)
+            elif self.update_precision == "bf16":
                 rc = lib.ss_actor_grad_tc(self.actor.data_ptr(), self.critic.data_ptr(), *tail)
             else:
                 rc = lib.ss_actor_grad_frames(self.actor.data_ptr(), self.critic.data_ptr(), self.frames, *tail)
@@ -1059,23 +1079,27 @@ class SelfPlayTrainer:
                  batch_size: int = 4096, gamma: float = 0.0, tau: float = 1.0, param_noise_sd: float = 0.5,
                  noise_group: int = 128, reward_mode: str = "looking", tick_limit: int = 2000,
                  random_positions: bool = True, process_group=None, precision: str = "f32", collective: str = "nccl",
-                 frames: int = 1):
+                 frames: int = 1, update_precision: Optional[str] = None):
         """frames > 1: the frame-stacked "planning" networks (readme.md:18-20, BASELINE.json configs[4]): both players act
         from their last `frames` observations (FrameStackActor; `precision` selects its float32 or tensor-core kernels),
         the replay ring stores the stacked observations, and the critic / actor update of SkillshotLearner.py:386-443 runs
-        on the 12 * frames-input networks (float32 kernels, separate steps)."""
+        on the 12 * frames-input networks in separate steps.
+        update_precision: the kernels of that update, "f32" or "bf16"; None = `precision` when frames = 1, "f32" when
+        frames > 1."""
         self.device = torch.device(device)
         self.frames = int(frames)
         self.envs = SkillshotEnvs(n_envs, device=device, random_positions=random_positions, seed=seed,
                                   reward_mode=reward_mode, tick_limit=tick_limit, auto_reset=True)
         self.envs.collect_episode_stats = True     # the reference's per-episode ticks / winner log, reduced on the device
         self.networks = ActorCritic(device=device, seed=seed if process_group is None else 0, gamma=gamma, tau=tau,
-                                    process_group=process_group, update_precision=precision if self.frames == 1 else "f32",
+                                    process_group=process_group,
+                                    update_precision=update_precision or (precision if self.frames == 1 else "f32"),
                                     collective=collective, frames=self.frames)
         self.networks.seed = seed          # exploration / dropout streams differ per rank, weights do not
         self.replay = ReplayRing(replay_capacity or 2 * n_envs * 8, device=device, seed=seed, frames=self.frames)
         self.batch_size, self.param_noise_sd, self.noise_group = int(batch_size), float(param_noise_sd), int(noise_group)
         self.precision = precision
+        self.update_precision = update_precision
         n = n_envs
         self.obs = self.envs.observe().contiguous()                       # [n,2,12] seen by the actor next
         self.prev_obs = torch.empty_like(self.obs)
@@ -1182,7 +1206,8 @@ class SelfPlayTrainer:
     def state_dict(self):
         sd = dict(envs=self.envs.state_dict(), networks=self.networks.state_dict(), replay=self.replay.state_dict(),
                   obs=self.obs.cpu(), actions=self.actions.cpu(), ticks=self.ticks, batch_size=self.batch_size,
-                  param_noise_sd=self.param_noise_sd, noise_group=self.noise_group, precision=self.precision, frames=self.frames)
+                  param_noise_sd=self.param_noise_sd, noise_group=self.noise_group, precision=self.precision, frames=self.frames,
+                  update_precision=self.update_precision)
         if self.stack is not None:      # the players' observation histories and the noise counter of the stacked actor
             st = self.stack
             sd["stack"] = dict(stack=st.stack.cpu(), stack32=None if st.stack32 is None else st.stack32.cpu(), head=st.head,
@@ -1197,6 +1222,7 @@ class SelfPlayTrainer:
         self.actions.copy_(sd["actions"].to(self.device))
         self.ticks, self.batch_size = int(sd["ticks"]), int(sd["batch_size"])
         self.param_noise_sd, self.noise_group = float(sd["param_noise_sd"]), int(sd["noise_group"])
+        self.update_precision = sd.get("update_precision")      # absent from older checkpoints: None
         if self.stack is not None:
             st, ss = self.stack, sd["stack"]
             st.stack.copy_(ss["stack"].to(self.device))
