@@ -457,6 +457,70 @@ int ss_replay_sample_frames(const float *ring_obs, const float *ring_act, const 
                             float *obs, float *act, float *reward, float *next_obs, uint8_t *done, int64_t *indices_out,
                             void *stream);
 
+/* ---- matches: two actors against each other (no reference code; the readme's "does the planning actor play better" question) ----
+ * A match is n_envs games between policy A and policy B, ONE game per env (no auto-reset: every game starts at tick 0 and
+ * is played to a hit or to tick_limit ticks, so no outcome is sampled by its length).  Seat map, split index 0 <= split <= n_envs:
+ *   env j <  split: A is player 1, B is player 2
+ *   env j >= split: B is player 1, A is player 2
+ * The seats are not symmetric -- check_collision tests player 1 first and a double hit records id 1 (SkillshotGame.py:58-94)
+ * -- so a fair match seats each policy in both.  The policies' inputs and outputs are POLICY-MAJOR, env j at row j of its half:
+ *   obs float32 [2][n_envs][12]   half 0 = A's observations, half 1 = B's
+ *   act float32 [2][n_envs][2]    the same layout for the actions
+ * so each policy's forward reads one contiguous block of rows; only the env step knows the seat map.
+ *
+ *   ss_env_step_match     one tick of every env: each env's two actions are read from `act` through the seat map, both next
+ *                         observations written to `obs_out` (policy-major).  No reward, no auto-reset; per-env speeds as for
+ *                         ss_env_step; SS_STATUS_NAN as ss_env_step raises it.  A game still live with ticks >= tick_limit
+ *                         (> 0) is NOT stepped (its observation is rewritten unchanged), so an outcome cannot change after the
+ *                         limit however many ticks are enqueued.  For up to tick_limit ticks from a fresh reset the state and
+ *                         the observations are bit-identical to ss_env_step(reward_mode NONE, auto_reset 0) under the seat
+ *                         permutation.
+ *   ss_actor_forward_groups_tc  ss_actor_forward_tc (no noise) with one parameter vector per group of rows: row i uses
+ *                         params + (i / group_rows) * param_stride (param_stride % 4 == 0; 0 = one vector for all rows).
+ *                         Each row's action is bit-identical to ss_actor_forward_tc run on its group's rows alone.
+ *   ss_match_summary      out uint64 [SS_MATCH_STATS] = [2][8] from the state (ticks, live, winner), OVERWRITTEN: block 0 = the
+ *                         envs where A is player 1 (j < split), block 1 = where A is player 2; per block
+ *                         { games, A wins (B was hit), B wins (A was hit), draws (live, ticks >= tick_limit),
+ *                           unfinished (live, ticks < tick_limit), sum of the ticks of the decided games, 0, 0 }.
+ *                         winner_id is the id of the player that was HIT (SkillshotGame.py:77).  Exact integer counts. */
+#define SS_MATCH_STATS 16
+int ss_env_step_match(void *state, int64_t n_envs, int64_t split, const float *actions, float *obs_out, int64_t tick_limit,
+                      const void *speeds, uint32_t *status, void *stream);
+int ss_actor_forward_groups_tc(const float *params, int64_t param_stride, int64_t group_rows, const float *obs, float *act_out,
+                               int64_t n, void *stream);
+int ss_match_summary(const void *state, int64_t n_envs, int64_t split, int64_t tick_limit, uint64_t *out, void *stream);
+
+/* n_ticks match ticks enqueued from one host call (as ss_selfplay_rollout does for self-play).  Per tick: the policies'
+ * forwards from `obs` (and their histories), then ss_env_step_match, then the newest observation of each frames > 1 policy
+ * pushed into its history at slot head + 1.  The forwards:
+ *   both frames 1, tensor_cores     ONE ss_actor_forward_groups_tc over 2 n_envs rows, group_rows = n_envs
+ *   a policy with frames > 1        ss_actor_forward_frames_tc (float32: ss_actor_forward_frames) on its half, param_stride 0
+ *   a frames-1 policy otherwise     ss_actor_forward_tc (float32: ss_actor_forward) on its half
+ * Histories: stack_a / stack_b (NULL for frames 1) are the layout of ss_obs_stack_push_tc (tensor_cores) or ss_obs_stack_push
+ * (float32) for n_envs rows; `head` is the slot counter of the newest frame on entry, the same for both; after the call it is
+ * head + n_ticks.  On return `obs` holds the current observations and `act` the last tick's actions.  Parameters: A's vector at
+ * `params`, B's at params + param_stride (param_stride % 4 == 0, at least the larger of the two vectors' lengths).
+ * `workspace` holds ss_match_workspace_bytes(n_envs, frames_a, frames_b, tensor_cores) bytes (16-byte aligned; NULL when 0).
+ * Every argument is checked before anything is enqueued. */
+typedef struct ss_match_args {
+    void *state;
+    int64_t n_envs, split, tick_limit;
+    const void *speeds;                        /* NULL or the per-env speeds of ss_env_step */
+    uint32_t *status;                          /* NULL or uint32[1] */
+    float *obs, *act;
+    const float *params;
+    int64_t param_stride;
+    int frames_a, frames_b;
+    void *stack_a, *stack_b;
+    int64_t head;
+    void *workspace;
+    int64_t workspace_bytes;
+    int tensor_cores;
+    int n_ticks;
+} ss_match_args;
+int64_t ss_match_workspace_bytes(int64_t n_envs, int frames_a, int frames_b, int tensor_cores);
+int ss_match_play(const ss_match_args *args, void *stream);
+
 /* ---- multi-GPU: the gradient all-reduce fused with its neighbours over NVLink peer memory ----
  * One exchange allocation per rank = flags[2][world] | inbox[2][world][capacity floats], made by
  * ss_peer_alloc and shared between the processes of one node through CUDA IPC (export on the owner,

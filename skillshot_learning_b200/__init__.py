@@ -5,6 +5,7 @@ from . import _lib  # noqa: F401  (raises ImportError when libskillshot_b200.so 
 from .game import Player, Projectile, SkillshotEnvs, SkillshotGame, render_board  # noqa: F401
 
 from .learner import ActorCritic, FrameStackActor, ReplayRing, SelfPlayTrainer, SkillshotLearner  # noqa: F401
+from .match import Match  # noqa: F401
 
 __all__ = ["SkillshotEnvs", "SkillshotGame", "Player", "Projectile", "render_board",
-           "ActorCritic", "FrameStackActor", "ReplayRing", "SelfPlayTrainer", "SkillshotLearner"]
+           "ActorCritic", "FrameStackActor", "ReplayRing", "SelfPlayTrainer", "SkillshotLearner", "Match"]

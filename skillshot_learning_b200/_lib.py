@@ -39,6 +39,8 @@ _u32 = ctypes.c_uint32
 
 
 PAIR_MAIL_EMPTY = 0x7fc0dead      # SS_PAIR_MAIL_EMPTY
+MATCH_STATS = 16                  # SS_MATCH_STATS: uint64 [2][8] of ss_match_summary
+MAX_FRAMES = 20                   # SS_MAX_FRAMES
 
 
 class DdpgUpdateArgs(ctypes.Structure):
@@ -53,6 +55,14 @@ class DdpgUpdateArgs(ctypes.Structure):
                  ("row_offset", _i64), ("workspace", _vp), ("workspace_bytes", _i64), ("tensor_cores", _i32),
                  ("world", _i32), ("rank", _i32), ("peer_bases", _vp), ("peer_capacity", _i64), ("epoch", _u32),
                  ("done_counter", _vp), ("status", _vp), ("pair_mail", _vp), ("sample_early", _i32)])
+
+
+class MatchArgs(ctypes.Structure):
+    """struct ss_match_args of include/skillshot_b200.h (same field order)."""
+    _fields_ = [("state", _vp), ("n_envs", _i64), ("split", _i64), ("tick_limit", _i64), ("speeds", _vp), ("status", _vp),
+                ("obs", _vp), ("act", _vp), ("params", _vp), ("param_stride", _i64), ("frames_a", _i32), ("frames_b", _i32),
+                ("stack_a", _vp), ("stack_b", _vp), ("head", _i64), ("workspace", _vp), ("workspace_bytes", _i64),
+                ("tensor_cores", _i32), ("n_ticks", _i32)]
 
 
 # name -> (restype, argtypes); every symbol the header declares
@@ -137,6 +147,11 @@ SIGNATURES = {
     "ss_replay_push": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _i32, _i64, _vp]),
     "ss_ddpg_update": (_i32, [ctypes.POINTER(DdpgUpdateArgs), _vp]),
     "ss_probe_rates": (_i32, [_vp, _vp, _vp]),
+    "ss_env_step_match": (_i32, [_vp, _i64, _i64, _vp, _vp, _i64, _vp, _vp, _vp]),
+    "ss_actor_forward_groups_tc": (_i32, [_vp, _i64, _i64, _vp, _vp, _i64, _vp]),
+    "ss_match_summary": (_i32, [_vp, _i64, _i64, _i64, _vp, _vp]),
+    "ss_match_workspace_bytes": (_i64, [_i64, _i32, _i32, _i32]),
+    "ss_match_play": (_i32, [ctypes.POINTER(MatchArgs), _vp]),
     "ss_replay_sample": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp, _u64, _u64, _i64,
                                  _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
 }

@@ -34,6 +34,7 @@ UNITS = {
     "ss_frames_tc.cu": [],
     "ss_frames_grad_tc.cu": [],
     "ss_probe.cu": [],
+    "ss_match.cu": [],
 }
 
 

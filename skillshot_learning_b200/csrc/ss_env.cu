@@ -679,6 +679,78 @@ __global__ void apply_kernel(void *state, int64_t n, int64_t env, int player, in
     if (status && status_out) atomicOr(status_out, status);
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Matches (ss_env_step_match, ss_match_summary): two policies, one game per env, the seat map of the header -- in env
+// i < split policy A is player 1.  Actions and observations are policy-major ([2][n] rows, env i at row i of each half).
+struct MatchStepArgs {
+    void *state;
+    int64_t n, split, tick_limit;
+    const float2 *actions;      // [2][n]
+    float4 *obs_out;            // [2][n][3]
+    const void *speeds;
+    uint32_t *status;
+};
+
+// fast_obs sink: player P's three float4 go to the row of the policy that sits in seat P
+struct SeatSink {
+    float4 *p1, *p2;
+    __device__ __forceinline__ void put(int j, float a, float b, float c, float d) {
+        (j < 3 ? p1 : p2)[j < 3 ? j : j - 3] = make_float4(a, b, c, d);
+    }
+};
+
+// One tick of one env per thread: the arithmetic of step_kernel<OBS, CARRY> with reward mode none and no auto-reset
+// (act_and_tick_carry, then fast_view / fast_obs of the post-tick state), hence the same bits.  A live game at the tick
+// limit is left as it is; its observation is written again.
+template <bool SPEEDS>
+__global__ void __launch_bounds__(kBlock, 8) match_step_kernel(const MatchStepArgs A) {
+    const int64_t i = (int64_t)blockIdx.x * kBlock + threadIdx.x;
+    if (i >= A.n) return;
+    const StatePlanes S = planes_of(A.state, A.n);
+    Env e;
+    load_env(S, i, e);
+    const Speeds k = SPEEDS ? load_speeds(A.speeds, A.n, i) : default_speeds();
+    const bool a_first = i < A.split;
+    const float2 aa = __ldg(A.actions + i), ab = __ldg(A.actions + A.n + i);
+    const float2 p1 = a_first ? aa : ab, p2 = a_first ? ab : aa;
+    Trig tr;
+    trig_of(e, tr);
+    uint32_t status = 0;
+    const bool frozen = e.live && e.ticks >= A.tick_limit;
+    if (!frozen) act_and_tick_carry(e, p1.x, p1.y, p2.x, p2.y, k, status, tr);
+    const FastView v0 = fast_view<0>(e, tr, false), v1 = fast_view<1>(e, tr, false);
+    float4 *row_a = A.obs_out + i * 3, *row_b = A.obs_out + (A.n + i) * 3;
+    SeatSink sink{a_first ? row_a : row_b, a_first ? row_b : row_a};
+    fast_obs<0>(e, v0, k, sink);
+    fast_obs<1>(e, v1, k, sink);
+    if (!frozen) store_env(S, i, e);
+    if (status && A.status) atomicOr(A.status, status);
+}
+
+// The [2][8] outcome counters of ss_match_summary: per-CTA sums in shared memory, then one atomic per counter and CTA.
+__global__ void match_summary_kernel(const void *state, int64_t n, int64_t split, int64_t tick_limit, unsigned long long *out) {
+    __shared__ unsigned long long acc[SS_MATCH_STATS];
+    if (threadIdx.x < SS_MATCH_STATS) acc[threadIdx.x] = 0;
+    __syncthreads();
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) {
+        const int4 b = planes_of((void *)state, n).ib[i];
+        const int ticks = b.z, live = (b.w >> 2) & 1, winner = (b.w >> 4) & 3;
+        const int seat = i < split ? 0 : 1;              // block 0: A is player 1
+        unsigned long long *c = acc + 8 * seat;
+        atomicAdd(c + 0, 1ull);
+        if (!live) {
+            // winner_id = the player that was hit: A was hit when it is A's seat (player 1 in block 0, player 2 in block 1)
+            atomicAdd(c + (winner == seat + 1 ? 2 : 1), 1ull);
+            atomicAdd(c + 5, (unsigned long long)ticks);
+        } else {
+            atomicAdd(c + (ticks >= tick_limit ? 3 : 4), 1ull);
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x < SS_MATCH_STATS && acc[threadIdx.x]) atomicAdd(out + threadIdx.x, acc[threadIdx.x]);
+}
+
 inline int check_launch() { return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA; }
 inline unsigned blocks_for(int64_t n, int block) { return (unsigned)((n + block - 1) / block); }
 // CTA size of step_pp_kernel for n_envs (see the kernel): 896 when that still makes at least ~one CTA per SM (65,536 envs
@@ -926,6 +998,27 @@ int ss_env_apply(void *state, int64_t n_envs, int64_t env, int player, int op, d
     if (!state || env < 0 || env >= n_envs || player < 0 || player > 1 || op < 0 || op > SS_OP_GAME_TICK)
         return SS_ERR_INVALID_ARG;
     apply_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(state, n_envs, env, player, op, value, speeds, status);
+    return check_launch();
+}
+
+int ss_env_step_match(void *state, int64_t n_envs, int64_t split, const float *actions, float *obs_out, int64_t tick_limit,
+                      const void *speeds, uint32_t *status, void *stream) {
+    if (!state || !actions || !obs_out || n_envs <= 0 || split < 0 || split > n_envs || tick_limit <= 0) return SS_ERR_INVALID_ARG;
+    if ((((uintptr_t)state | (uintptr_t)obs_out | (uintptr_t)speeds) & 15) || ((uintptr_t)actions & 7) || ((uintptr_t)status & 3))
+        return SS_ERR_INVALID_ARG;
+    MatchStepArgs A{state, n_envs, split, tick_limit, (const float2 *)actions, (float4 *)obs_out, speeds, status};
+    cudaStream_t st = (cudaStream_t)stream;
+    if (speeds) match_step_kernel<true><<<blocks_for(n_envs, kBlock), kBlock, 0, st>>>(A);
+    else match_step_kernel<false><<<blocks_for(n_envs, kBlock), kBlock, 0, st>>>(A);
+    return check_launch();
+}
+
+int ss_match_summary(const void *state, int64_t n_envs, int64_t split, int64_t tick_limit, uint64_t *out, void *stream) {
+    if (!state || !out || n_envs <= 0 || split < 0 || split > n_envs || tick_limit <= 0) return SS_ERR_INVALID_ARG;
+    if (((uintptr_t)state & 15) || ((uintptr_t)out & 7)) return SS_ERR_INVALID_ARG;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (cudaMemsetAsync(out, 0, SS_MATCH_STATS * sizeof(uint64_t), st) != cudaSuccess) return SS_ERR_CUDA;
+    match_summary_kernel<<<blocks_for(n_envs, 256), 256, 0, st>>>(state, n_envs, split, tick_limit, (unsigned long long *)out);
     return check_launch();
 }
 

@@ -75,6 +75,8 @@ struct FwdArgs {
     // the empty mark, takes them and puts the mark back.  The data is its own flag: no fence, no separate flag traffic
     // (a release store per tile cost the output warps ~700 cycles each, measured).
     int2 *pair_mail;
+    // grouped forward (ss_actor_forward_groups_tc): row i uses the parameter vector params + (i / group) * param_stride
+    int64_t param_stride;
 };
 
 // 32 accumulator columns (hidden-2 units) -> ReLU -> layer 3, four split accumulators per output.
@@ -141,8 +143,27 @@ constexpr uint32_t SMP_TMEM = SMP_BAR + B_COUNT * 8;
 constexpr uint32_t SMP_TOTAL = SMP_TMEM + 16;
 static_assert(SMP_TOTAL <= 227 * 1024, "shared memory budget");
 
+// GROUPS: this CTA's tiles [u0, u1) when the CTAs are split over the groups in proportion to the groups' tiles (the last
+// group may be shorter), every range inside one group, so that a CTA stages one parameter vector once.  With fewer CTAs
+// than groups the tiles are split evenly and a range may cross groups (the segment loop restages at each boundary).
+__device__ __forceinline__ void group_units(int64_t n, int64_t group, int64_t upg, int cta, int ncta, int64_t &u0, int64_t &u1) {
+    const int64_t G = (n + group - 1) / group;
+    const int64_t last = (n - (G - 1) * group + TM - 1) / TM;          // tiles of the last group
+    if (ncta < G) {
+        u0 = G * upg * cta / ncta; u1 = G * upg * (cta + 1) / ncta;
+        return;
+    }
+    const int64_t T = (G - 1) * upg + last;
+    // group g owns CTAs [floor(g upg ncta / T), floor((g + 1) upg ncta / T)), the last group up to ncta; each owns >= 1
+    const int64_t g = min(G - 1, ((int64_t)(cta + 1) * T - 1) / (upg * ncta));
+    const int64_t c0 = g * upg * ncta / T, c1 = g + 1 == G ? ncta : (g + 1) * upg * ncta / T;
+    const int64_t tiles = g + 1 == G ? last : upg, j = cta - c0, k = c1 - c0;
+    u0 = g * upg + tiles * j / k; u1 = g * upg + tiles * (j + 1) / k;
+}
+
 // cta / ncta: this CTA's index among the CTAs that share the work of A (the whole grid, or one role's part of a pair launch)
-template <int NET, bool FUSED>
+// GROUPS (actor only): one parameter vector per group of A.group rows instead of one perturbed vector per noise group
+template <int NET, bool FUSED, bool GROUPS = false>
 __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const int ncta) {
     extern __shared__ __align__(128) uint8_t smem[];
     const uint32_t sbase = smem_u32(smem);
@@ -170,12 +191,13 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
     tc_fence_after();
     const uint32_t tmem = *reinterpret_cast<const volatile uint32_t *>(smem + SMP_TMEM);
 
-    const bool noisy = NET == NET_ACTOR && A.param_sd > 0.f;
-    const int64_t group = noisy ? A.group : A.n;
+    const bool noisy = NET == NET_ACTOR && !GROUPS && A.param_sd > 0.f;
+    const int64_t group = (noisy || GROUPS) ? A.group : A.n;
     const int64_t upg = (group + TM - 1) / TM;
     const int64_t n_groups = (A.n + group - 1) / group;
     const int64_t units = n_groups * upg;
-    const int64_t u0 = units * cta / ncta, u1 = units * (cta + 1) / ncta;
+    int64_t u0 = units * cta / ncta, u1 = units * (cta + 1) / ncta;
+    if (GROUPS) group_units(A.n, group, upg, cta, ncta, u0, u1);
 
     uint32_t tcount = 0;                                     // tiles done by this CTA: buffers = tcount & 1, parities from tcount
     uint32_t xph = 0;                                        // MMA warp: parity of the next X hand-off
@@ -195,9 +217,9 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
         // weights are staged ahead of the wait too when the caller knows that grid does not write them
         if (!waited && !A.early_weights) { sslaunch::griddep_wait(); sslaunch::griddep_launch(); waited = true; }
         if (waited && warp < P_WARPS) load_obs(A.obs, row0 + r, end, xin);
-        stage_weights<NET, NTH, true>(Stager{A.params, smem + SMP_B1, smem + SMP_B2, reinterpret_cast<float4 *>(smem + SMP_W3),
-                                             reinterpret_cast<float *>(smem + SMP_B3), noisy, A.param_sd, A.seed, A.counter,
-                                             (uint32_t)g});
+        stage_weights<NET, NTH, true>(Stager{GROUPS ? A.params + g * A.param_stride : A.params, smem + SMP_B1, smem + SMP_B2,
+                                             reinterpret_cast<float4 *>(smem + SMP_W3), reinterpret_cast<float *>(smem + SMP_B3),
+                                             noisy, A.param_sd, A.seed, A.counter, (uint32_t)g});
         if (!waited) {
             sslaunch::griddep_wait();
             sslaunch::griddep_launch();
@@ -450,6 +472,11 @@ __global__ void __launch_bounds__(NTH, 1) mlp_fwd_pair_kernel(const FwdArgs Aa, 
     else fwd_body<NET_CRITIC, false>(Ac, (int)blockIdx.x - ga, (int)gridDim.x - ga);
 }
 
+// ss_actor_forward_groups_tc: the actor pipeline with one parameter vector per group of rows
+__global__ void __launch_bounds__(NTH, 1) mlp_fwd_groups_kernel(const FwdArgs A) {
+    fwd_body<NET_ACTOR, false, true>(A, (int)blockIdx.x, (int)gridDim.x);
+}
+
 }  // namespace pipe
 
 template <int NET, bool FUSED = false>
@@ -505,6 +532,35 @@ extern "C" int ss_actor_forward_tc_signal(const float *actor_params, const float
         if (units_out) *units_out = units;
     }
     return launch_fwd<NET_ACTOR>(A, stream);
+}
+
+// One parameter vector per group of group_rows rows.  Launch geometry: as many CTAs as launch_fwd would give the real
+// tiles, but at least one per group while the groups fit the SMs -- and the CTAs are split over the groups in proportion
+// to their tiles (group_units), not one CTA per group: a match's two groups of 131,072 rows would otherwise run on 2 SMs.
+extern "C" int ss_actor_forward_groups_tc(const float *params, int64_t param_stride, int64_t group_rows, const float *obs,
+                                          float *act_out, int64_t n, void *stream) {
+    if (!params || !obs || !act_out || n <= 0 || group_rows <= 0 || param_stride < 0) return SS_ERR_INVALID_ARG;
+    if ((param_stride & 3) || (param_stride > 0 && param_stride < SS_ACTOR_PARAMS)) return SS_ERR_INVALID_ARG;
+    if ((((uintptr_t)params | (uintptr_t)obs) & 15) || ((uintptr_t)act_out & 7)) return SS_ERR_INVALID_ARG;
+    int dev = 0, sms = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) return SS_ERR_CUDA;
+    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return SS_ERR_CUDA;
+    const int64_t group = group_rows < n ? group_rows : n;
+    const int64_t n_groups = (n + group - 1) / group;
+    const int64_t tiles = (n_groups - 1) * ((group + TM - 1) / TM) + (n - (n_groups - 1) * group + TM - 1) / TM;
+    const int64_t rounds = (tiles + sms - 1) / sms;
+    int grid = (int)((tiles + rounds - 1) / rounds);
+    if (n_groups <= sms && grid < n_groups) grid = (int)n_groups;
+    FwdArgs A{};
+    A.params = params; A.obs = obs; A.n = n; A.group = group; A.act_out = act_out; A.param_stride = param_stride;
+    if (cudaFuncSetAttribute(pipe::mlp_fwd_groups_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pipe::SMP_TOTAL) !=
+        cudaSuccess)
+        return SS_ERR_CUDA;
+    A.early_weights = sslaunch::take_early_weights();
+    if (sslaunch::launch(pipe::mlp_fwd_groups_kernel, dim3(grid), dim3(pipe::NTH), pipe::SMP_TOTAL, (cudaStream_t)stream, A) !=
+        cudaSuccess)
+        return SS_ERR_CUDA;
+    return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA;
 }
 
 extern "C" int ss_actor_forward_tc(const float *actor_params, const float *obs, float *act_out, int64_t n,

@@ -26,6 +26,7 @@ import torch
 from . import _lib
 from ._lib import check, lib
 from .game import FEATURE_KEYS, REWARD_MODES, SkillshotEnvs, SkillshotGame
+from .match import Match
 
 A_N, C_N = _lib.ACTOR_PARAMS, _lib.CRITIC_PARAMS
 ACTOR_SHAPES = [(12, 256), (256,), (256, 128), (128,), (128, 2), (2,)]       # Keras get_weights() order
@@ -1256,6 +1257,27 @@ class SelfPlayTrainer:
         """The training-progress log of the reference (per-episode ticks and winner, SkillshotLearner.py:164-180,
         365-366) for the games finished so far, reduced on the device by the step kernel (SkillshotEnvs.episode_summary)."""
         return self.envs.episode_summary(reset=reset)
+
+    def evaluate(self, opponent, n_games: int = 65536, seed: int = 0, tick_limit: Optional[int] = None) -> dict:
+        """Play the current actor (with this trainer's frames and `precision`) against `opponent` -- a flat actor vector or
+        the six get_weights() arrays, see Match -- over n_games seat-balanced games and return Match.play's result
+        (score is the current actor's).  The tick limit (default: the trainer's), start mode and per-env speeds (env j
+        takes those of the trainer's env j mod n_envs) are the trainer's.  The match has its own envs, buffers and Philox
+        stream and copies the actor: the trainer's envs, ring, networks and counters are not touched, so a run that
+        evaluates in the middle continues bit-identically."""
+        envs = self.envs
+        limit = envs.tick_limit if tick_limit is None else int(tick_limit)
+        if limit <= 0:
+            raise ValueError("a match needs a positive tick_limit (the trainer has none)")
+        speeds = None
+        if envs.speeds is not None:
+            n, buf = envs.n_envs, envs.speeds
+            idx = torch.arange(int(n_games), device=self.device) % n
+            f = buf[:16 * n].view(torch.float64).view(n, 2)
+            g = buf[16 * n:]
+            speeds = (f[idx, 0], f[idx, 1], g.view(torch.float64).view(n, 2)[idx, 0], g.view(torch.int64).view(n, 2)[idx, 1])
+        return Match(self.networks.actor, opponent, n_games, device=self.device, precision=self.precision, tick_limit=limit,
+                     random_positions=envs.random_positions, seed=seed, speeds=speeds).play()
 
     def check_exchange(self):
         """Raises if a rank's gradient failed to arrive in the fused peer exchange (the Adam kernels skip their writes from
