@@ -69,6 +69,7 @@ extern "C" {
 #define SS_STATUS_NAN 1       /* where the reference raises ValueError: int(round(nan)), Player.py:63 */
 #define SS_STATUS_PEER_TIMEOUT 2   /* ss_peer_adam_tf gave up waiting for a peer's gradient */
 #define SS_STATUS_ROLLOUT_TIMEOUT 4   /* ss_env_step_tiles gave up waiting for the actor forward kernel's actions */
+#define SS_STATUS_SEAT_RANGE 8   /* ss_env_step_seated met a seat-table row outside [0, n_rows) (that env was not stepped) */
 
 /* ops of ss_env_apply: the single-object methods of the reference */
 #define SS_OP_MOVE_DIRECTION_FLOAT 0  /* Player.move_direction_float(value), Player.py:57-68 */
@@ -520,6 +521,70 @@ typedef struct ss_match_args {
 } ss_match_args;
 int64_t ss_match_workspace_bytes(int64_t n_envs, int frames_a, int frames_b, int tensor_cores);
 int ss_match_play(const ss_match_args *args, void *stream);
+
+/* ---- leagues: up to SS_LEAGUE_MAX_POLICIES actors in one batch (a match generalised to any schedule of pairings) ----
+ * One game per env from tick 0 as in a match.  The rows of the policies' inputs and outputs are grouped in SEGMENTS, one
+ * per policy, contiguous and in order: segment s = rows [seg_start[s], seg_start[s + 1]), one row for every env in which
+ * its policy plays, and n_rows = 2 n_envs.  Which rows an env's two players read and write is device data:
+ *   seat_rows   int32 [n_envs][2]  {row of player 1, row of player 2}  (an int2 per env, 8-byte aligned)
+ *   seat_policy uint8 [n_envs][2]  {policy of player 1, policy of player 2}  (2-byte aligned; for the summary only)
+ *   obs float32 [n_rows][12], act float32 [n_rows][2]
+ *
+ *   ss_env_step_seated    ss_env_step_match with the rows taken from seat_rows instead of the split rule: no reward, no
+ *                         auto-reset, a live game with ticks >= tick_limit (> 0) is not stepped (its observation is written
+ *                         again), SS_STATUS_NAN as ss_env_step raises it.  An env with a row outside [0, n_rows) is neither
+ *                         read, stepped nor written and raises SS_STATUS_SEAT_RANGE.  n_rows < 2^31.
+ *   ss_actor_forward_segments_tc  ss_actor_forward_tc (no noise) over n_segs (1..SS_LEAGUE_MAX_POLICIES) consecutive
+ *                         segments of seg_rows_host[s] >= 1 rows each (a HOST array): segment s reads and writes the rows
+ *                         from sum_{t<s} seg_rows_host[t] on and uses the vector params + s param_stride (param_stride % 4
+ *                         == 0, 0 or >= SS_ACTOR_PARAMS).  Each row's action is bit-identical to ss_actor_forward_tc run
+ *                         on its segment alone.
+ *   ss_league_summary     out uint64 [n_policies][n_policies][8], OVERWRITTEN: cell (i, j) counts the envs with policy i in
+ *                         seat 1 and policy j in seat 2 { games, seat-1 wins (player 2 was hit), seat-2 wins, draws (live,
+ *                         ticks >= tick_limit), unfinished (live, ticks < tick_limit), sum of the ticks of the decided
+ *                         games, 0, 0 }.  winner_id is the id of the player that was HIT.  Exact integer counts; an env
+ *                         with a policy index >= n_policies is not counted.  2 <= n_policies <= SS_LEAGUE_MAX_POLICIES. */
+#define SS_LEAGUE_MAX_POLICIES 64
+int ss_env_step_seated(void *state, int64_t n_envs, const void *seat_rows, int64_t n_rows, const float *actions, float *obs_out,
+                       int64_t tick_limit, const void *speeds, uint32_t *status, void *stream);
+int ss_actor_forward_segments_tc(const float *params, int64_t param_stride, const int64_t *seg_rows_host, int n_segs,
+                                 const float *obs, float *act_out, void *stream);
+int ss_league_summary(const void *state, int64_t n_envs, const uint8_t *seat_policy, int n_policies, int64_t tick_limit,
+                      uint64_t *out, void *stream);
+
+/* n_ticks league ticks from one host call (as ss_match_play for two policies).  The arrays seg_start [n_policies + 1],
+ * frames [n_policies] and stacks [n_policies] are HOST arrays indexed by segment; segment s uses the vector
+ * params + s param_stride (param_stride % 4 == 0, at least every segment's ss_actor_frames_params).  Per tick:
+ *   tensor_cores   one ss_actor_forward_segments_tc per maximal run of consecutive frames-1 segments, and
+ *                  ss_actor_forward_frames_tc (param_stride 0) on each frames > 1 segment
+ *   float32        ss_actor_forward or ss_actor_forward_frames on each segment
+ * then ss_env_step_seated, then the newest observation of each frames > 1 segment pushed into its history stacks[s]
+ * (the layout of ss_obs_stack_push_tc / ss_obs_stack_push for that segment's rows; NULL for frames 1) at slot head + 1.
+ * `workspace` holds ss_league_workspace_bytes(args) bytes (16-byte aligned; NULL when 0; that call reads n_policies,
+ * seg_start, frames and tensor_cores and returns -1 when they are invalid).  Every argument is checked before anything is
+ * enqueued: 2 <= n_policies <= SS_LEAGUE_MAX_POLICIES, seg_start[0] == 0, every segment >= 1 row, seg_start[n_policies]
+ * == 2 n_envs. */
+typedef struct ss_league_args {
+    void *state;
+    int64_t n_envs, tick_limit;
+    const void *speeds;                        /* NULL or the per-env speeds of ss_env_step */
+    uint32_t *status;                          /* NULL or uint32[1] */
+    const void *seat_rows;                     /* int32 [n_envs][2] */
+    float *obs, *act;
+    const float *params;
+    int64_t param_stride;
+    int n_policies;
+    const int64_t *seg_start;                  /* host [n_policies + 1] */
+    const int *frames;                         /* host [n_policies] */
+    void *const *stacks;                       /* host [n_policies] */
+    int64_t head;
+    void *workspace;
+    int64_t workspace_bytes;
+    int tensor_cores;
+    int n_ticks;
+} ss_league_args;
+int64_t ss_league_workspace_bytes(const ss_league_args *args);
+int ss_league_play(const ss_league_args *args, void *stream);
 
 /* ---- multi-GPU: the gradient all-reduce fused with its neighbours over NVLink peer memory ----
  * One exchange allocation per rank = flags[2][world] | inbox[2][world][capacity floats], made by

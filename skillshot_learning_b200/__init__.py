@@ -6,6 +6,8 @@ from .game import Player, Projectile, SkillshotEnvs, SkillshotGame, render_board
 
 from .learner import ActorCritic, FrameStackActor, ReplayRing, SelfPlayTrainer, SkillshotLearner  # noqa: F401
 from .match import Match  # noqa: F401
+from .league import League, gauntlet, load_saved_actors, ratings, round_robin  # noqa: F401
 
 __all__ = ["SkillshotEnvs", "SkillshotGame", "Player", "Projectile", "render_board",
-           "ActorCritic", "FrameStackActor", "ReplayRing", "SelfPlayTrainer", "SkillshotLearner", "Match"]
+           "ActorCritic", "FrameStackActor", "ReplayRing", "SelfPlayTrainer", "SkillshotLearner", "Match",
+           "League", "round_robin", "gauntlet", "ratings", "load_saved_actors"]

@@ -41,6 +41,8 @@ _u32 = ctypes.c_uint32
 PAIR_MAIL_EMPTY = 0x7fc0dead      # SS_PAIR_MAIL_EMPTY
 MATCH_STATS = 16                  # SS_MATCH_STATS: uint64 [2][8] of ss_match_summary
 MAX_FRAMES = 20                   # SS_MAX_FRAMES
+LEAGUE_MAX_POLICIES = 64          # SS_LEAGUE_MAX_POLICIES
+STATUS_SEAT_RANGE = 8             # SS_STATUS_SEAT_RANGE
 
 
 class DdpgUpdateArgs(ctypes.Structure):
@@ -63,6 +65,14 @@ class MatchArgs(ctypes.Structure):
                 ("obs", _vp), ("act", _vp), ("params", _vp), ("param_stride", _i64), ("frames_a", _i32), ("frames_b", _i32),
                 ("stack_a", _vp), ("stack_b", _vp), ("head", _i64), ("workspace", _vp), ("workspace_bytes", _i64),
                 ("tensor_cores", _i32), ("n_ticks", _i32)]
+
+
+class LeagueArgs(ctypes.Structure):
+    """struct ss_league_args of include/skillshot_b200.h (same field order)."""
+    _fields_ = [("state", _vp), ("n_envs", _i64), ("tick_limit", _i64), ("speeds", _vp), ("status", _vp), ("seat_rows", _vp),
+                ("obs", _vp), ("act", _vp), ("params", _vp), ("param_stride", _i64), ("n_policies", _i32),
+                ("seg_start", ctypes.POINTER(_i64)), ("frames", ctypes.POINTER(_i32)), ("stacks", ctypes.POINTER(_vp)),
+                ("head", _i64), ("workspace", _vp), ("workspace_bytes", _i64), ("tensor_cores", _i32), ("n_ticks", _i32)]
 
 
 # name -> (restype, argtypes); every symbol the header declares
@@ -152,6 +162,11 @@ SIGNATURES = {
     "ss_match_summary": (_i32, [_vp, _i64, _i64, _i64, _vp, _vp]),
     "ss_match_workspace_bytes": (_i64, [_i64, _i32, _i32, _i32]),
     "ss_match_play": (_i32, [ctypes.POINTER(MatchArgs), _vp]),
+    "ss_env_step_seated": (_i32, [_vp, _i64, _vp, _i64, _vp, _vp, _i64, _vp, _vp, _vp]),
+    "ss_actor_forward_segments_tc": (_i32, [_vp, _i64, _vp, _i32, _vp, _vp, _vp]),
+    "ss_league_summary": (_i32, [_vp, _i64, _vp, _i32, _i64, _vp, _vp]),
+    "ss_league_workspace_bytes": (_i64, [ctypes.POINTER(LeagueArgs)]),
+    "ss_league_play": (_i32, [ctypes.POINTER(LeagueArgs), _vp]),
     "ss_replay_sample": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp, _u64, _u64, _i64,
                                  _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
 }

@@ -35,6 +35,7 @@ UNITS = {
     "ss_frames_grad_tc.cu": [],
     "ss_probe.cu": [],
     "ss_match.cu": [],
+    "ss_league.cu": [],
 }
 
 

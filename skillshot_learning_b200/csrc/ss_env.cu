@@ -699,19 +699,63 @@ struct SeatSink {
     }
 };
 
+// Leagues (ss_env_step_seated, ss_league_summary): any number of policies, each env's two rows given by a seat table.
+struct SeatedStepArgs {
+    void *state;
+    int64_t n, n_rows, tick_limit;
+    const int2 *seat_rows;      // [n]
+    const float2 *actions;      // [n_rows]
+    float4 *obs_out;            // [n_rows][3]
+    const void *speeds;
+    uint32_t *status;
+};
+
+// How match_step_kernel finds an env's two rows (static functions of the kernel's arguments).  ok() is false when the env
+// is not to be stepped at all; act_a / act_b and obs_a / obs_b are the two rows' actions and observations, and player 1's
+// row is the "a" row when a_first().
+// SplitSeats (ss_env_step_match): env i < split seats policy A (rows [0, n)) first, the others policy B (rows [n, 2 n)).
+struct SplitSeats {
+    using Args = MatchStepArgs;
+    __device__ __forceinline__ static bool ok(const Args &, int64_t) { return true; }
+    __device__ __forceinline__ static bool a_first(const Args &A, int64_t i) { return i < A.split; }
+    __device__ __forceinline__ static const float2 *act_a(const Args &A, int64_t i) { return A.actions + i; }
+    __device__ __forceinline__ static const float2 *act_b(const Args &A, int64_t i) { return A.actions + A.n + i; }
+    __device__ __forceinline__ static float4 *obs_a(const Args &A, int64_t i) { return A.obs_out + i * 3; }
+    __device__ __forceinline__ static float4 *obs_b(const Args &A, int64_t i) { return A.obs_out + (A.n + i) * 3; }
+};
+
+// TableSeats (ss_env_step_seated): seat_rows[i] = {row of player 1, row of player 2}.  An env with a row outside
+// [0, n_rows) is not stepped, reads and writes no row and raises SS_STATUS_SEAT_RANGE.
+struct TableSeats {
+    using Args = SeatedStepArgs;
+    __device__ __forceinline__ static bool ok(const Args &A, int64_t i) {
+        const int2 r = __ldg(A.seat_rows + i);
+        return r.x >= 0 && r.y >= 0 && r.x < A.n_rows && r.y < A.n_rows;
+    }
+    __device__ __forceinline__ static bool a_first(const Args &, int64_t) { return true; }
+    __device__ __forceinline__ static const float2 *act_a(const Args &A, int64_t i) { return A.actions + __ldg(A.seat_rows + i).x; }
+    __device__ __forceinline__ static const float2 *act_b(const Args &A, int64_t i) { return A.actions + __ldg(A.seat_rows + i).y; }
+    __device__ __forceinline__ static float4 *obs_a(const Args &A, int64_t i) { return A.obs_out + (int64_t)__ldg(A.seat_rows + i).x * 3; }
+    __device__ __forceinline__ static float4 *obs_b(const Args &A, int64_t i) { return A.obs_out + (int64_t)__ldg(A.seat_rows + i).y * 3; }
+};
+
 // One tick of one env per thread: the arithmetic of step_kernel<OBS, CARRY> with reward mode none and no auto-reset
 // (act_and_tick_carry, then fast_view / fast_obs of the post-tick state), hence the same bits.  A live game at the tick
 // limit is left as it is; its observation is written again.
-template <bool SPEEDS>
-__global__ void __launch_bounds__(kBlock, 8) match_step_kernel(const MatchStepArgs A) {
+template <bool SPEEDS, class Seats>
+__global__ void __launch_bounds__(kBlock, 8) match_step_kernel(const typename Seats::Args A) {
     const int64_t i = (int64_t)blockIdx.x * kBlock + threadIdx.x;
     if (i >= A.n) return;
+    if (!Seats::ok(A, i)) {
+        if (A.status) atomicOr(A.status, (uint32_t)SS_STATUS_SEAT_RANGE);
+        return;
+    }
     const StatePlanes S = planes_of(A.state, A.n);
     Env e;
     load_env(S, i, e);
     const Speeds k = SPEEDS ? load_speeds(A.speeds, A.n, i) : default_speeds();
-    const bool a_first = i < A.split;
-    const float2 aa = __ldg(A.actions + i), ab = __ldg(A.actions + A.n + i);
+    const bool a_first = Seats::a_first(A, i);
+    const float2 aa = __ldg(Seats::act_a(A, i)), ab = __ldg(Seats::act_b(A, i));
     const float2 p1 = a_first ? aa : ab, p2 = a_first ? ab : aa;
     Trig tr;
     trig_of(e, tr);
@@ -719,12 +763,47 @@ __global__ void __launch_bounds__(kBlock, 8) match_step_kernel(const MatchStepAr
     const bool frozen = e.live && e.ticks >= A.tick_limit;
     if (!frozen) act_and_tick_carry(e, p1.x, p1.y, p2.x, p2.y, k, status, tr);
     const FastView v0 = fast_view<0>(e, tr, false), v1 = fast_view<1>(e, tr, false);
-    float4 *row_a = A.obs_out + i * 3, *row_b = A.obs_out + (A.n + i) * 3;
+    float4 *row_a = Seats::obs_a(A, i), *row_b = Seats::obs_b(A, i);
     SeatSink sink{a_first ? row_a : row_b, a_first ? row_b : row_a};
     fast_obs<0>(e, v0, k, sink);
     fast_obs<1>(e, v1, k, sink);
     if (!frozen) store_env(S, i, e);
     if (status && A.status) atomicOr(A.status, status);
+}
+
+// The [P][P][8] counters of ss_league_summary.  The envs are pair-major, so the lanes of a warp nearly always share one
+// or two cells: the lanes of one cell (__match_any_sync) count their outcomes with ballots and sum their ticks with one
+// reduction, and the cell's lowest lane adds the totals -- one atomic per non-zero counter, cell and warp.  An env whose
+// policy index is >= P is not counted.
+__global__ void league_summary_kernel(const void *state, int64_t n, const uint8_t *seat_policy, int P, int64_t tick_limit,
+                                      unsigned long long *out) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int lane = threadIdx.x & 31;
+    int cell = -1, ticks = 0, k = -1;                 // k: the counter this env adds one to (1..4)
+    if (i < n) {
+        const uchar2 sp = __ldg(reinterpret_cast<const uchar2 *>(seat_policy) + i);
+        if (sp.x < P && sp.y < P) {
+            const int4 b = planes_of((void *)state, n).ib[i];
+            const int live = (b.w >> 2) & 1, winner = (b.w >> 4) & 3;
+            cell = sp.x * P + sp.y;
+            // winner_id = the player that was hit: seat 1 wins when player 2 was hit
+            k = !live ? (winner == 2 ? 1 : 2) : (b.z >= tick_limit ? 3 : 4);
+            ticks = live ? 0 : b.z;
+        }
+    }
+    const unsigned peers = __match_any_sync(0xffffffffu, cell);
+    const unsigned mine[5] = {peers & __ballot_sync(0xffffffffu, cell >= 0), peers & __ballot_sync(0xffffffffu, k == 1),
+                              peers & __ballot_sync(0xffffffffu, k == 2), peers & __ballot_sync(0xffffffffu, k == 3),
+                              peers & __ballot_sync(0xffffffffu, k == 4)};
+    // ticks < 2^31: the two 16-bit halves summed over at most 32 lanes cannot overflow 32 bits
+    const unsigned lo = __reduce_add_sync(peers, (unsigned)ticks & 0xffffu), hi = __reduce_add_sync(peers, (unsigned)ticks >> 16);
+    if (cell < 0 || lane != __ffs(peers) - 1) return;
+    unsigned long long *c = out + (int64_t)cell * 8;
+#pragma unroll
+    for (int j = 0; j < 5; ++j)
+        if (mine[j]) atomicAdd(c + j, (unsigned long long)__popc(mine[j]));
+    const unsigned long long t = (unsigned long long)lo + ((unsigned long long)hi << 16);
+    if (t) atomicAdd(c + 5, t);
 }
 
 // The [2][8] outcome counters of ss_match_summary: per-CTA sums in shared memory, then one atomic per counter and CTA.
@@ -1008,8 +1087,8 @@ int ss_env_step_match(void *state, int64_t n_envs, int64_t split, const float *a
         return SS_ERR_INVALID_ARG;
     MatchStepArgs A{state, n_envs, split, tick_limit, (const float2 *)actions, (float4 *)obs_out, speeds, status};
     cudaStream_t st = (cudaStream_t)stream;
-    if (speeds) match_step_kernel<true><<<blocks_for(n_envs, kBlock), kBlock, 0, st>>>(A);
-    else match_step_kernel<false><<<blocks_for(n_envs, kBlock), kBlock, 0, st>>>(A);
+    if (speeds) match_step_kernel<true, SplitSeats><<<blocks_for(n_envs, kBlock), kBlock, 0, st>>>(A);
+    else match_step_kernel<false, SplitSeats><<<blocks_for(n_envs, kBlock), kBlock, 0, st>>>(A);
     return check_launch();
 }
 
@@ -1019,6 +1098,33 @@ int ss_match_summary(const void *state, int64_t n_envs, int64_t split, int64_t t
     cudaStream_t st = (cudaStream_t)stream;
     if (cudaMemsetAsync(out, 0, SS_MATCH_STATS * sizeof(uint64_t), st) != cudaSuccess) return SS_ERR_CUDA;
     match_summary_kernel<<<blocks_for(n_envs, 256), 256, 0, st>>>(state, n_envs, split, tick_limit, (unsigned long long *)out);
+    return check_launch();
+}
+
+int ss_env_step_seated(void *state, int64_t n_envs, const void *seat_rows, int64_t n_rows, const float *actions, float *obs_out,
+                       int64_t tick_limit, const void *speeds, uint32_t *status, void *stream) {
+    if (!state || !seat_rows || !actions || !obs_out || n_envs <= 0 || n_rows <= 0 || n_rows > INT32_MAX || tick_limit <= 0)
+        return SS_ERR_INVALID_ARG;
+    if ((((uintptr_t)state | (uintptr_t)obs_out | (uintptr_t)speeds) & 15) || (((uintptr_t)actions | (uintptr_t)seat_rows) & 7) ||
+        ((uintptr_t)status & 3))
+        return SS_ERR_INVALID_ARG;
+    SeatedStepArgs A{state, n_envs, n_rows, tick_limit, (const int2 *)seat_rows, (const float2 *)actions, (float4 *)obs_out, speeds, status};
+    cudaStream_t st = (cudaStream_t)stream;
+    if (speeds) match_step_kernel<true, TableSeats><<<blocks_for(n_envs, kBlock), kBlock, 0, st>>>(A);
+    else match_step_kernel<false, TableSeats><<<blocks_for(n_envs, kBlock), kBlock, 0, st>>>(A);
+    return check_launch();
+}
+
+int ss_league_summary(const void *state, int64_t n_envs, const uint8_t *seat_policy, int n_policies, int64_t tick_limit, uint64_t *out,
+                      void *stream) {
+    if (!state || !seat_policy || !out || n_envs <= 0 || n_policies < 2 || n_policies > SS_LEAGUE_MAX_POLICIES || tick_limit <= 0)
+        return SS_ERR_INVALID_ARG;
+    if (((uintptr_t)state & 15) || ((uintptr_t)seat_policy & 1) || ((uintptr_t)out & 7)) return SS_ERR_INVALID_ARG;
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t bytes = (size_t)n_policies * n_policies * 8 * sizeof(uint64_t);
+    if (cudaMemsetAsync(out, 0, bytes, st) != cudaSuccess) return SS_ERR_CUDA;
+    league_summary_kernel<<<blocks_for(n_envs, 256), 256, 0, st>>>(state, n_envs, seat_policy, n_policies, tick_limit,
+                                                                    (unsigned long long *)out);
     return check_launch();
 }
 

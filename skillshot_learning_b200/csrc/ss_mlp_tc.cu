@@ -161,10 +161,26 @@ __device__ __forceinline__ void group_units(int64_t n, int64_t group, int64_t up
     u0 = g * upg + tiles * j / k; u1 = g * upg + tiles * (j + 1) / k;
 }
 
+// SEGMENTS: the unit -> (segment, first row) table of ss_actor_forward_segments_tc, passed by value beside FwdArgs.  Segment s
+// = tiles [unit0[s], unit0[s + 1]) = rows [row0[s], row0[s + 1]), worked by CTAs [cta0[s], cta0[s + 1]) (at least one).
+struct SegTable {
+    int n;
+    int64_t unit0[SS_LEAGUE_MAX_POLICIES + 1], row0[SS_LEAGUE_MAX_POLICIES + 1];
+    int cta0[SS_LEAGUE_MAX_POLICIES + 1];
+};
+
+// the segment that holds tile u (the segments are few: a linear walk)
+__device__ __forceinline__ int segment_of(const SegTable &T, int64_t u) {
+    int s = 0;
+    while (s + 1 < T.n && u >= T.unit0[s + 1]) ++s;
+    return s;
+}
+
 // cta / ncta: this CTA's index among the CTAs that share the work of A (the whole grid, or one role's part of a pair launch)
 // GROUPS (actor only): one parameter vector per group of A.group rows instead of one perturbed vector per noise group
-template <int NET, bool FUSED, bool GROUPS = false>
-__device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const int ncta) {
+// SEGS (actor only): one parameter vector per segment of *T instead; no tile mixes two segments
+template <int NET, bool FUSED, bool GROUPS = false, bool SEGS = false>
+__device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const int ncta, const SegTable *T = nullptr) {
     extern __shared__ __align__(128) uint8_t smem[];
     const uint32_t sbase = smem_u32(smem);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -191,13 +207,19 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
     tc_fence_after();
     const uint32_t tmem = *reinterpret_cast<const volatile uint32_t *>(smem + SMP_TMEM);
 
-    const bool noisy = NET == NET_ACTOR && !GROUPS && A.param_sd > 0.f;
+    const bool noisy = NET == NET_ACTOR && !GROUPS && !SEGS && A.param_sd > 0.f;
     const int64_t group = (noisy || GROUPS) ? A.group : A.n;
     const int64_t upg = (group + TM - 1) / TM;
     const int64_t n_groups = (A.n + group - 1) / group;
     const int64_t units = n_groups * upg;
     int64_t u0 = units * cta / ncta, u1 = units * (cta + 1) / ncta;
     if (GROUPS) group_units(A.n, group, upg, cta, ncta, u0, u1);
+    if (SEGS) {                                              // this CTA's share of its segment's tiles
+        int s = 0;
+        while (s + 1 < T->n && cta >= T->cta0[s + 1]) ++s;
+        const int64_t tiles = T->unit0[s + 1] - T->unit0[s], j = cta - T->cta0[s], k = T->cta0[s + 1] - T->cta0[s];
+        u0 = T->unit0[s] + tiles * j / k; u1 = T->unit0[s] + tiles * (j + 1) / k;
+    }
 
     uint32_t tcount = 0;                                     // tiles done by this CTA: buffers = tcount & 1, parities from tcount
     uint32_t xph = 0;                                        // MMA warp: parity of the next X hand-off
@@ -205,11 +227,12 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
     bool waited = false;                                     // griddepcontrol.wait executed (ss_launch.cuh)
 
     for (int64_t u = u0; u < u1;) {
-        const int64_t g = u / upg;
-        const int64_t seg_end = min(u1, (g + 1) * upg);
+        const int64_t g = SEGS ? segment_of(*T, u) : u / upg;
+        const int64_t seg_end = SEGS ? min(u1, T->unit0[g + 1]) : min(u1, (g + 1) * upg);
         const int64_t ntiles = seg_end - u;
-        const int64_t end = min(A.n, (g + 1) * group);
-        const int64_t row0 = g * group + (u - g * upg) * TM;      // first row of the segment's first tile
+        const int64_t end = SEGS ? T->row0[g + 1] : min(A.n, (g + 1) * group);
+        // first row of the segment's first tile
+        const int64_t row0 = SEGS ? T->row0[g] + (u - T->unit0[g]) * TM : g * group + (u - g * upg) * TM;
         const int r = (warp & 3) * 32 + lane;                     // row of the tile = tensor-memory lane
 
         float4 xin[3];
@@ -217,7 +240,7 @@ __device__ __forceinline__ void fwd_body(const FwdArgs &A, const int cta, const 
         // weights are staged ahead of the wait too when the caller knows that grid does not write them
         if (!waited && !A.early_weights) { sslaunch::griddep_wait(); sslaunch::griddep_launch(); waited = true; }
         if (waited && warp < P_WARPS) load_obs(A.obs, row0 + r, end, xin);
-        stage_weights<NET, NTH, true>(Stager{GROUPS ? A.params + g * A.param_stride : A.params, smem + SMP_B1, smem + SMP_B2,
+        stage_weights<NET, NTH, true>(Stager{(GROUPS || SEGS) ? A.params + g * A.param_stride : A.params, smem + SMP_B1, smem + SMP_B2,
                                              reinterpret_cast<float4 *>(smem + SMP_W3), reinterpret_cast<float *>(smem + SMP_B3),
                                              noisy, A.param_sd, A.seed, A.counter, (uint32_t)g});
         if (!waited) {
@@ -477,6 +500,12 @@ __global__ void __launch_bounds__(NTH, 1) mlp_fwd_groups_kernel(const FwdArgs A)
     fwd_body<NET_ACTOR, false, true>(A, (int)blockIdx.x, (int)gridDim.x);
 }
 
+// ss_actor_forward_segments_tc: the actor pipeline with one parameter vector per segment of rows (the table by value: it is
+// read in place from the parameter space)
+__global__ void __launch_bounds__(NTH, 1) mlp_fwd_segments_kernel(const FwdArgs A, const __grid_constant__ SegTable T) {
+    fwd_body<NET_ACTOR, false, false, true>(A, (int)blockIdx.x, (int)gridDim.x, &T);
+}
+
 }  // namespace pipe
 
 template <int NET, bool FUSED = false>
@@ -558,6 +587,52 @@ extern "C" int ss_actor_forward_groups_tc(const float *params, int64_t param_str
         return SS_ERR_CUDA;
     A.early_weights = sslaunch::take_early_weights();
     if (sslaunch::launch(pipe::mlp_fwd_groups_kernel, dim3(grid), dim3(pipe::NTH), pipe::SMP_TOTAL, (cudaStream_t)stream, A) !=
+        cudaSuccess)
+        return SS_ERR_CUDA;
+    return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA;
+}
+
+// One parameter vector per segment.  Launch geometry: as many CTAs as launch_fwd would give the segments' tiles, but at
+// least one per segment; each segment gets one CTA, then the rest go one at a time to the segment with the most tiles per
+// CTA (never more CTAs than tiles), so the CTAs are split in proportion to the tiles and no CTA mixes two segments.
+extern "C" int ss_actor_forward_segments_tc(const float *params, int64_t param_stride, const int64_t *seg_rows_host, int n_segs,
+                                            const float *obs, float *act_out, void *stream) {
+    if (!params || !obs || !act_out || !seg_rows_host || n_segs < 1 || n_segs > SS_LEAGUE_MAX_POLICIES || param_stride < 0)
+        return SS_ERR_INVALID_ARG;
+    if ((param_stride & 3) || (param_stride > 0 && param_stride < SS_ACTOR_PARAMS)) return SS_ERR_INVALID_ARG;
+    if ((((uintptr_t)params | (uintptr_t)obs) & 15) || ((uintptr_t)act_out & 7)) return SS_ERR_INVALID_ARG;
+    pipe::SegTable T{};
+    T.n = n_segs;
+    int64_t tiles[SS_LEAGUE_MAX_POLICIES];
+    for (int s = 0; s < n_segs; ++s) {
+        if (seg_rows_host[s] <= 0) return SS_ERR_INVALID_ARG;
+        tiles[s] = (seg_rows_host[s] + TM - 1) / TM;
+        T.row0[s + 1] = T.row0[s] + seg_rows_host[s];
+        T.unit0[s + 1] = T.unit0[s] + tiles[s];
+    }
+    int dev = 0, sms = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) return SS_ERR_CUDA;
+    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return SS_ERR_CUDA;
+    const int64_t units = T.unit0[n_segs], rounds = (units + sms - 1) / sms;
+    int grid = (int)((units + rounds - 1) / rounds);
+    int ctas[SS_LEAGUE_MAX_POLICIES], given = n_segs;
+    for (int s = 0; s < n_segs; ++s) ctas[s] = 1;
+    while (given < grid) {
+        int best = -1;                                        // the segment with the most tiles per CTA that can take one more
+        for (int s = 0; s < n_segs; ++s)
+            if (ctas[s] < tiles[s] && (best < 0 || tiles[s] * ctas[best] > tiles[best] * ctas[s])) best = s;
+        if (best < 0) break;
+        ++ctas[best];
+        ++given;
+    }
+    for (int s = 0; s < n_segs; ++s) T.cta0[s + 1] = T.cta0[s] + ctas[s];
+    FwdArgs A{};
+    A.params = params; A.obs = obs; A.n = T.row0[n_segs]; A.group = A.n; A.act_out = act_out; A.param_stride = param_stride;
+    if (cudaFuncSetAttribute(pipe::mlp_fwd_segments_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pipe::SMP_TOTAL) !=
+        cudaSuccess)
+        return SS_ERR_CUDA;
+    A.early_weights = sslaunch::take_early_weights();
+    if (sslaunch::launch(pipe::mlp_fwd_segments_kernel, dim3(given), dim3(pipe::NTH), pipe::SMP_TOTAL, (cudaStream_t)stream, A, T) !=
         cudaSuccess)
         return SS_ERR_CUDA;
     return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA;

@@ -1279,6 +1279,30 @@ class SelfPlayTrainer:
         return Match(self.networks.actor, opponent, n_games, device=self.device, precision=self.precision, tick_limit=limit,
                      random_positions=envs.random_positions, seed=seed, speeds=speeds).play()
 
+    def evaluate_league(self, opponents, games_per_pair: int = 8192, seed: int = 0, tick_limit: Optional[int] = None) -> dict:
+        """Play the current actor (policy 0, with this trainer's frames and `precision`) against each of `opponents` (flat
+        actor vectors or six get_weights() arrays, see League) in a gauntlet of games_per_pair seat-balanced games per
+        opponent and return League.play's result (ratings: the current actor's is ratings[0]).  The tick limit (default:
+        the trainer's), start mode and per-env speeds (league env j takes those of the trainer's env j mod n_envs) are the
+        trainer's, as in evaluate().  The league has its own envs, buffers and Philox stream and copies every actor: the
+        trainer's envs, ring, networks and counters are not touched."""
+        from .league import League, gauntlet
+        envs = self.envs
+        limit = envs.tick_limit if tick_limit is None else int(tick_limit)
+        if limit <= 0:
+            raise ValueError("a league needs a positive tick_limit (the trainer has none)")
+        actors = [self.networks.actor] + list(opponents)
+        n_games = (len(actors) - 1) * int(games_per_pair)
+        speeds = None
+        if envs.speeds is not None:
+            n, buf = envs.n_envs, envs.speeds
+            idx = torch.arange(n_games, device=self.device) % n
+            f = buf[:16 * n].view(torch.float64).view(n, 2)
+            g = buf[16 * n:]
+            speeds = (f[idx, 0], f[idx, 1], g.view(torch.float64).view(n, 2)[idx, 0], g.view(torch.int64).view(n, 2)[idx, 1])
+        return League(actors, games_per_pair, pairs=gauntlet(len(actors)), device=self.device, precision=self.precision,
+                      tick_limit=limit, random_positions=envs.random_positions, seed=seed, speeds=speeds).play()
+
     def check_exchange(self):
         """Raises if a rank's gradient failed to arrive in the fused peer exchange (the Adam kernels skip their writes from
         that point on, so the ranks still hold identical weights: reload or stop)."""
