@@ -586,6 +586,73 @@ typedef struct ss_league_args {
 int64_t ss_league_workspace_bytes(const ss_league_args *args);
 int ss_league_play(const ss_league_args *args, void *stream);
 
+/* ---- training against a pool: the self-play learner also plays frozen opponents ----
+ * The last M = pool_envs of the n_envs envs are POOL envs: the learner against one of K = n_opponents frozen 1-frame actors.
+ * Opponent k owns the b = M / K consecutive envs from S + k b (S = n_envs - M); the learner is player 1 in the first b / 2
+ * of them and player 2 in the others, so M % (2K) == 0.  The rows, a fixed formula of (S, M, K):
+ *   learner rows   L = 2S + M:  self-play env i < S: player p is row 2i + p (the layout of ss_env_step_ring);
+ *                               pool env j >= S: the learner's player is row 2S + (j - S)
+ *   opponent rows  M:           pool env j: the opponent's player is row j - S; opponent k's rows are one segment of b rows
+ *
+ *   ss_env_step_pool   one tick of ss_env_step_ring (auto-reset, reward none / looking / terminal, reference speeds) with the
+ *                      rows above: actions float32 [L][2] and opp_actions [M][2] in; obs_out (and obs_out2 when not NULL)
+ *                      [L][12], reward_out [L] (NULL or reward none: not written), done_rows_out uint8 [L] (the terminal
+ *                      flag of ss_env_step_ring, NULL ok) for the learner's rows; opp_obs_out [M][12] for the opponents';
+ *                      done_out / winner_out uint8 [n_envs] per env (NULL ok).  flags: SS_STEP_EPISODE_STATS or 0 (every env
+ *                      counts).  pool_stats: NULL or uint64 [K][SS_POOL_STATS] ADDED TO per finished pool game: {episodes, learner wins
+ *                      (the opponent was hit), learner losses (the learner was hit), tick-limit endings, sum of episode
+ *                      ticks, 0, 0, 0}; winner_id is the player that was HIT, and a double hit records player 1 as hit.
+ *                      M = 0 (n_opponents ignored) is the self-play step of ss_env_step_ring, bit for bit.
+ *
+ * ss_pool_rollout: n_ticks training ticks from one host call (as ss_selfplay_rollout).  Per tick:
+ *   tensor_cores  ss_actor_forward_tc on the L learner rows (the rollout's noise, counter noise_counter + t), then
+ *                 ss_actor_forward_segments_tc on the M opponent rows (K segments of b rows, no noise; skipped when M = 0)
+ *   float32       ss_actor_forward on the learner rows and on each opponent segment
+ * then ss_env_step_pool with counter env_counter + t.  The tensor-core launches form the dependent-launch chain of
+ * ss_selfplay_rollout (ss_set_dependent_launch).  Opponent k acts with opp_params + k opp_param_stride.
+ *   obs [L][12]        the learner rows' current observation on entry and on return
+ *   opp_obs [M][12]    the opponent rows' current observation on entry and on return (updated in place)
+ *   act [L][2], reward [L], opp_act [M][2], done / winner [n_envs]: the last tick's values on return
+ * With a ring (ring_obs != NULL) the learner's transitions are produced IN the ring as in ss_selfplay_rollout: tick t owns
+ * the L rows from write_pos + t L (mod capacity).  capacity and write_pos must be multiples of L, with capacity >= 2 L or
+ * n_ticks == 1.  Without a ring the learner's rows are rewritten in obs / act / reward.  The opponents' transitions are not
+ * stored.  Every argument is checked before anything is enqueued: besides the rules of ss_env_step_pool, speeds must be
+ * NULL (per-env speeds and reward simple run on the per-env step kernel), K <= SS_LEAGUE_MAX_POLICIES and pointers aligned
+ * as ss_selfplay_rollout's.  M = 0 gives ss_selfplay_rollout's results bit for bit. */
+#define SS_POOL_STATS 8        /* uint64 counters per opponent in pool_stats */
+int ss_env_step_pool(void *state, int64_t n_envs, int64_t pool_envs, int n_opponents, const float *actions,
+                     const float *opp_actions, float *obs_out, float *obs_out2, float *reward_out, uint8_t *done_rows_out,
+                     float *opp_obs_out, uint8_t *done_out, uint8_t *winner_out, int reward_mode, int64_t tick_limit,
+                     int reset_mode, uint64_t seed, uint64_t counter, uint32_t *status, int flags, uint64_t *pool_stats,
+                     void *stream);
+typedef struct ss_pool_rollout_args {
+    void *state;
+    int64_t n_envs, pool_envs;
+    int n_opponents;
+    const float *params;                       /* the learner's actor */
+    const float *opp_params;                   /* K opponent vectors, opp_param_stride floats apart */
+    int64_t opp_param_stride;
+    float *obs, *act, *reward;                 /* learner rows */
+    float *opp_obs, *opp_act;                  /* opponent rows */
+    uint8_t *done, *winner;                    /* [n_envs] */
+    float *ring_obs, *ring_act, *ring_reward, *ring_next_obs;
+    uint8_t *ring_done;
+    int64_t capacity, write_pos;
+    int n_ticks;
+    float param_noise_sd;
+    int64_t noise_group;
+    float action_noise_sd;
+    int tensor_cores, reward_mode;
+    int64_t tick_limit;
+    int reset_mode;
+    uint64_t env_seed, env_counter, noise_seed, noise_counter;
+    const void *speeds;                        /* must be NULL */
+    uint32_t *status;                          /* NULL or the status block of ss_env_step */
+    int step_flags;                            /* SS_STEP_EPISODE_STATS or 0 */
+    uint64_t *pool_stats;                      /* NULL or uint64 [K][SS_POOL_STATS], added to */
+} ss_pool_rollout_args;
+int ss_pool_rollout(const ss_pool_rollout_args *args, void *stream);
+
 /* ---- multi-GPU: the gradient all-reduce fused with its neighbours over NVLink peer memory ----
  * One exchange allocation per rank = flags[2][world] | inbox[2][world][capacity floats], made by
  * ss_peer_alloc and shared between the processes of one node through CUDA IPC (export on the owner,

@@ -43,6 +43,7 @@ MATCH_STATS = 16                  # SS_MATCH_STATS: uint64 [2][8] of ss_match_su
 MAX_FRAMES = 20                   # SS_MAX_FRAMES
 LEAGUE_MAX_POLICIES = 64          # SS_LEAGUE_MAX_POLICIES
 STATUS_SEAT_RANGE = 8             # SS_STATUS_SEAT_RANGE
+POOL_STATS = 8                    # uint64 counters per opponent of ss_env_step_pool / ss_pool_rollout
 
 
 class DdpgUpdateArgs(ctypes.Structure):
@@ -73,6 +74,18 @@ class LeagueArgs(ctypes.Structure):
                 ("obs", _vp), ("act", _vp), ("params", _vp), ("param_stride", _i64), ("n_policies", _i32),
                 ("seg_start", ctypes.POINTER(_i64)), ("frames", ctypes.POINTER(_i32)), ("stacks", ctypes.POINTER(_vp)),
                 ("head", _i64), ("workspace", _vp), ("workspace_bytes", _i64), ("tensor_cores", _i32), ("n_ticks", _i32)]
+
+
+class PoolRolloutArgs(ctypes.Structure):
+    """struct ss_pool_rollout_args of include/skillshot_b200.h (same field order)."""
+    _fields_ = ([("state", _vp), ("n_envs", _i64), ("pool_envs", _i64), ("n_opponents", _i32), ("params", _vp), ("opp_params", _vp),
+                 ("opp_param_stride", _i64)] +
+                [(k, _vp) for k in ("obs", "act", "reward", "opp_obs", "opp_act", "done", "winner", "ring_obs", "ring_act",
+                                    "ring_reward", "ring_next_obs", "ring_done")] +
+                [("capacity", _i64), ("write_pos", _i64), ("n_ticks", _i32), ("param_noise_sd", _f32), ("noise_group", _i64),
+                 ("action_noise_sd", _f32), ("tensor_cores", _i32), ("reward_mode", _i32), ("tick_limit", _i64),
+                 ("reset_mode", _i32), ("env_seed", _u64), ("env_counter", _u64), ("noise_seed", _u64), ("noise_counter", _u64),
+                 ("speeds", _vp), ("status", _vp), ("step_flags", _i32), ("pool_stats", _vp)])
 
 
 # name -> (restype, argtypes); every symbol the header declares
@@ -167,6 +180,9 @@ SIGNATURES = {
     "ss_league_summary": (_i32, [_vp, _i64, _vp, _i32, _i64, _vp, _vp]),
     "ss_league_workspace_bytes": (_i64, [ctypes.POINTER(LeagueArgs)]),
     "ss_league_play": (_i32, [ctypes.POINTER(LeagueArgs), _vp]),
+    "ss_env_step_pool": (_i32, [_vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i64, _i32, _u64, _u64,
+                                 _vp, _i32, _vp, _vp]),
+    "ss_pool_rollout": (_i32, [ctypes.POINTER(PoolRolloutArgs), _vp]),
     "ss_replay_sample": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp, _u64, _u64, _i64,
                                  _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
 }

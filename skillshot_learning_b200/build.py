@@ -36,6 +36,7 @@ UNITS = {
     "ss_probe.cu": [],
     "ss_match.cu": [],
     "ss_league.cu": [],
+    "ss_pool.cu": [],
 }
 
 

@@ -428,8 +428,36 @@ __global__ void __launch_bounds__(BLK, 896 / BLK) step_pp_kernel(const StepArgs 
 // float4, staged through shared memory so that a warp's 1,536 bytes leave as three fully coalesced 512-byte requests,
 // to both copies when the replay ring wants two), its terminal byte; the env's done / winner bytes come from the two
 // lanes of the pair.  Bit-identical to step_kernel<OBS = true> (the golden lockstep tests run through this kernel).
-template <bool STATS>
-__global__ void __launch_bounds__(kBlockPP) step_pp_obs_kernel(const StepArgs A) {
+//
+// The body is templated on a ROW RULE: which row of which buffer a lane reads its action from and writes its outputs to.
+//   SelfPlayRows (ss_env_step_ring): row = global lane, every output in the caller's [n][2] rows.
+//   PoolRows (ss_env_step_pool): the training-against-a-pool layout of the header.  Env i < S is
+//     self-play (rows 2i + p of the learner rows); in pool env j >= S the learner's player is learner row 2S + (j - S) and
+//     the frozen opponent's player is row j - S of the opponent rows.  Opponent k owns the b consecutive pool envs from
+//     S + k b, the learner being player 1 in the first b / 2 of them.  An opponent lane writes only its observation (to the
+//     opponent rows); reward and terminal flag are the learner's alone.  A warp's learner rows and its opponent rows are
+//     each one contiguous run, so the observations still leave through the shared-memory tile as coalesced stores.
+struct SelfPlayRows {
+    static constexpr bool kPool = false;
+};
+struct PoolRows {
+    static constexpr bool kPool = true;
+    int64_t S, b;                       // self-play envs; pool envs per opponent (even, >= 2)
+    const float2 *opp_actions;          // [M] opponent rows
+    float4 *opp_obs;                    // [M][3]
+    unsigned long long *pool_stats;     // [K][8] or NULL
+};
+
+// One finished pool game into its opponent's counters {episodes, learner wins, learner losses, tick-limit endings, ticks}.
+// winner_id is the player that was HIT.  Out of line for the reason count_episode is.
+__device__ __noinline__ void count_pool_game(unsigned long long *c, int len, int winner, int learner_player) {
+    atomicAdd(c + 0, 1ull);
+    atomicAdd(c + (winner == 0 ? 3 : winner == learner_player + 1 ? 2 : 1), 1ull);
+    atomicAdd(c + 4, (unsigned long long)len);
+}
+
+template <bool STATS, class Rows>
+__global__ void __launch_bounds__(kBlockPP) step_pp_obs_kernel(const StepArgs A, const Rows R) {
     __shared__ float4 tile[kBlockPP / 32][96];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, P = lane & 1;
     const int64_t g0 = (int64_t)blockIdx.x * kBlockPP + threadIdx.x;
@@ -440,9 +468,25 @@ __global__ void __launch_bounds__(kBlockPP) step_pp_obs_kernel(const StepArgs A)
     // ss_launch.cuh: in the rollout loop this grid is placed while the forward kernel's last CTAs finish, and waits here
     sslaunch::griddep_wait();
     sslaunch::griddep_launch();
+    bool learner = true;                              // this lane's row is a learner row (else an opponent row)
+    int64_t row = gl, block = 0;
+    int learner_player = 0;
+    if constexpr (Rows::kPool) {
+        if (env >= R.S) {
+            const int64_t j = env - R.S;
+            block = j / R.b;
+            learner_player = j - block * R.b >= (R.b >> 1) ? 1 : 0;
+            learner = P == learner_player;
+            row = learner ? 2 * R.S + j : j;
+        }
+    }
     sspp::LaneState L;
     sspp::lane_load((const char *)A.state, A.n, gl, L);
-    const float2 a = __ldg((const float2 *)A.actions + gl);
+    const float2 *act = (const float2 *)A.actions;
+    if constexpr (Rows::kPool) {
+        if (!learner) act = R.opp_actions;
+    }
+    const float2 a = __ldg(act + row);
     uint32_t status = 0;
     sspp::LaneTrig T;
     sspp::lane_trig(L, T);
@@ -451,29 +495,60 @@ __global__ void __launch_bounds__(kBlockPP) step_pp_obs_kernel(const StepArgs A)
     const int v_other = __shfl_xor_sync(0xffffffffu, L.valid, 1);
     if (active) {
         sspp::lane_store((char *)A.state, A.n, gl, L, v_other);
-        if (A.reward_out && A.P.reward_mode != SS_REWARD_NONE) ((float *)A.reward_out)[gl] = out.reward;
+        if (learner && A.reward_out && A.P.reward_mode != SS_REWARD_NONE) ((float *)A.reward_out)[row] = out.reward;
         uint8_t *flag = P ? A.winner_out : A.done_out;
         if (flag) flag[env] = (uint8_t)(P ? out.winner : out.done);
-        if (A.done_rows_out) ((uint8_t *)A.done_rows_out)[gl] = out.winner ? 1 : 0;
+        if (learner && A.done_rows_out) ((uint8_t *)A.done_rows_out)[row] = out.winner ? 1 : 0;
         if (STATS && !P && out.episode_len >= 0) count_episode(A.stats, out.episode_len, out.winner, (int)A.P.tick_limit);
+        if constexpr (Rows::kPool) {
+            if (!P && R.pool_stats && env >= R.S && out.episode_len >= 0)
+                count_pool_game(R.pool_stats + block * 8, out.episode_len, out.winner, learner_player);
+        }
     }
-    // observations: lane's three float4 -> tile -> three coalesced stores per warp and copy
+    if constexpr (Rows::kPool) {
+        // the warp's learner lanes (rows l0 ...) take tile slots [0, nl), its opponent lanes (rows o0 ...) the next no slots
+        const unsigned lmask = __ballot_sync(0xffffffffu, active && learner), omask = __ballot_sync(0xffffffffu, active && !learner);
+        const unsigned below = (1u << lane) - 1u;
+        const int nl = __popc(lmask), no = __popc(omask);
+        const int64_t l0 = __shfl_sync(0xffffffffu, row, lmask ? __ffs(lmask) - 1 : 0);
+        const int64_t o0 = __shfl_sync(0xffffffffu, row, omask ? __ffs(omask) - 1 : 0);
+        const int slot = learner ? __popc(lmask & below) : nl + __popc(omask & below);
+        if (active) {
 #pragma unroll
-    for (int j = 0; j < 3; ++j) tile[warp][lane * 3 + j] = out.obs[j];
-    __syncwarp();
-    const int64_t warp_base = (g0 - lane) * 3;                        // in float4
-    const int64_t total = 2 * A.n * 3;
+            for (int j = 0; j < 3; ++j) tile[warp][slot * 3 + j] = out.obs[j];
+        }
+        __syncwarp();
 #pragma unroll
-    for (int j = 0; j < 3; ++j) {
-        const int64_t idx = warp_base + j * 32 + lane;
-        if (idx < total) {
-            const float4 v = tile[warp][j * 32 + lane];
-            A.obs_out[idx] = v;
-            if (A.obs_out2) A.obs_out2[idx] = v;
+        for (int j = 0; j < 3; ++j) {
+            const int idx = j * 32 + lane;
+            if (idx < 3 * nl) {
+                const float4 v = tile[warp][idx];
+                A.obs_out[l0 * 3 + idx] = v;
+                if (A.obs_out2) A.obs_out2[l0 * 3 + idx] = v;
+            } else if (idx < 3 * (nl + no)) {
+                R.opp_obs[o0 * 3 + (idx - 3 * nl)] = tile[warp][idx];
+            }
+        }
+    } else {
+        // observations: lane's three float4 -> tile -> three coalesced stores per warp and copy
+#pragma unroll
+        for (int j = 0; j < 3; ++j) tile[warp][lane * 3 + j] = out.obs[j];
+        __syncwarp();
+        const int64_t warp_base = (g0 - lane) * 3;                        // in float4
+        const int64_t total = 2 * A.n * 3;
+#pragma unroll
+        for (int j = 0; j < 3; ++j) {
+            const int64_t idx = warp_base + j * 32 + lane;
+            if (idx < total) {
+                const float4 v = tile[warp][j * 32 + lane];
+                A.obs_out[idx] = v;
+                if (A.obs_out2) A.obs_out2[idx] = v;
+            }
         }
     }
     if (status && A.status) atomicOr(A.status, status);
 }
+
 
 // ---------------------------------------------------------------------------------------------------------------------
 // step_pp_tiles_kernel -- the rollout's env step running BESIDE the actor forward kernel that produces its actions.
@@ -924,8 +999,8 @@ int ss_env_step_ring(void *state, int64_t n_envs, const float *actions, float *o
     if (obs_out && n_ticks == 1 && !speeds && reward_mode != SS_REWARD_SIMPLE) {
         // the rollout's env step: one tick with observations, one thread per player
         const dim3 grid_pp(blocks_for(2 * n_envs, kBlockPP));
-        if ((A.stats ? sslaunch::launch(step_pp_obs_kernel<true>, grid_pp, dim3(kBlockPP), 0, st, A)
-                     : sslaunch::launch(step_pp_obs_kernel<false>, grid_pp, dim3(kBlockPP), 0, st, A)) != cudaSuccess)
+        if ((A.stats ? sslaunch::launch(step_pp_obs_kernel<true, SelfPlayRows>, grid_pp, dim3(kBlockPP), 0, st, A, SelfPlayRows{})
+                     : sslaunch::launch(step_pp_obs_kernel<false, SelfPlayRows>, grid_pp, dim3(kBlockPP), 0, st, A, SelfPlayRows{})) != cudaSuccess)
             return SS_ERR_CUDA;
     } else if (obs_out) {
         // 8 CTAs (16 warps) per SM: capping the observation kernel at 128 registers measured
@@ -988,6 +1063,37 @@ int ss_env_step_ring(void *state, int64_t n_envs, const float *actions, float *o
         }
     }
     return check_launch();
+}
+
+int ss_env_step_pool(void *state, int64_t n_envs, int64_t pool_envs, int n_opponents, const float *actions,
+                     const float *opp_actions, float *obs_out, float *obs_out2, float *reward_out, uint8_t *done_rows_out,
+                     float *opp_obs_out, uint8_t *done_out, uint8_t *winner_out, int reward_mode, int64_t tick_limit,
+                     int reset_mode, uint64_t seed, uint64_t counter, uint32_t *status, int flags, uint64_t *pool_stats,
+                     void *stream) {
+    if (!state || !actions || !obs_out || n_envs <= 0 || pool_envs < 0 || pool_envs > n_envs) return SS_ERR_INVALID_ARG;
+    if (pool_envs > 0 && (n_opponents < 1 || n_opponents > SS_LEAGUE_MAX_POLICIES || pool_envs % (2 * n_opponents) != 0 ||
+                          !opp_actions || !opp_obs_out))
+        return SS_ERR_INVALID_ARG;
+    if (reward_mode != SS_REWARD_NONE && reward_mode != SS_REWARD_LOOKING && reward_mode != SS_REWARD_TERMINAL) return SS_ERR_INVALID_ARG;
+    if (reset_mode != SS_RESET_FIXED && reset_mode != SS_RESET_RANDOM) return SS_ERR_INVALID_ARG;
+    if ((((uintptr_t)state | (uintptr_t)obs_out | (uintptr_t)obs_out2 | (uintptr_t)opp_obs_out) & 15) ||
+        (((uintptr_t)actions | (uintptr_t)opp_actions | (uintptr_t)pool_stats) & 7) || (((uintptr_t)reward_out | (uintptr_t)status) & 3))
+        return SS_ERR_INVALID_ARG;
+    StepArgs A{};
+    A.state = state; A.n = n_envs; A.actions = (const float4 *)actions; A.obs_out = (float4 *)obs_out; A.obs_out2 = (float4 *)obs_out2;
+    A.reward_out = (float2 *)reward_out; A.done_out = done_out; A.winner_out = winner_out; A.done_rows_out = (uint16_t *)done_rows_out;
+    A.status = status;
+    A.stats = (status && (flags & SS_STEP_EPISODE_STATS)) ? reinterpret_cast<unsigned long long *>(status) + 1 : nullptr;
+    if (A.stats && ((uintptr_t)status & 7)) return SS_ERR_INVALID_ARG;
+    A.P.seed = seed; A.P.counter = counter; A.P.tick_limit = tick_limit; A.P.reward_mode = reward_mode; A.P.auto_reset = 1;
+    A.P.reset_mode = reset_mode; A.n_ticks = 1;
+    PoolRows R{n_envs - pool_envs, pool_envs > 0 ? pool_envs / n_opponents : 2, (const float2 *)opp_actions, (float4 *)opp_obs_out,
+               pool_envs > 0 ? (unsigned long long *)pool_stats : nullptr};
+    const dim3 grid(blocks_for(2 * n_envs, kBlockPP));
+    if ((A.stats ? sslaunch::launch(step_pp_obs_kernel<true, PoolRows>, grid, dim3(kBlockPP), 0, (cudaStream_t)stream, A, R)
+                 : sslaunch::launch(step_pp_obs_kernel<false, PoolRows>, grid, dim3(kBlockPP), 0, (cudaStream_t)stream, A, R)) != cudaSuccess)
+        return SS_ERR_CUDA;
+    return SS_OK;
 }
 
 int ss_env_step_tiles(void *state, int64_t n_envs, const float *actions, float *obs_out, float *obs_out2,

@@ -26,7 +26,7 @@ import torch
 from . import _lib
 from ._lib import check, lib
 from .game import FEATURE_KEYS, REWARD_MODES, SkillshotEnvs, SkillshotGame
-from .match import Match
+from .match import Match, actor_vector
 
 A_N, C_N = _lib.ACTOR_PARAMS, _lib.CRITIC_PARAMS
 ACTOR_SHAPES = [(12, 256), (256,), (256, 128), (128,), (128, 2), (2,)]       # Keras get_weights() order
@@ -1069,6 +1069,28 @@ class FrameStackActor:
         return stack[:, order, :].reshape(self.n_rows, self.frames * 12)
 
 
+POOL_STRIDE = (A_N + 3) // 4 * 4          # floats between two opponent vectors (16-byte aligned)
+
+
+def pool_layout(n_envs: int, pool_envs: int, n_opponents: int) -> np.ndarray:
+    """int64 [n_envs, 2]: the row of each (env, player) when the last pool_envs envs are played against n_opponents frozen
+    actors (include/skillshot_b200.h, "training against a pool").  Rows [0, L) are the learner's, L = 2 S + M with
+    S = n_envs - M; rows L + r are opponent row r.  Self-play env i keeps rows 2i + p; opponent k owns the b = M / K pool
+    envs from S + k b, the learner being player 1 in the first b / 2 of them."""
+    n, M = int(n_envs), int(pool_envs)
+    S = n - M
+    rows = np.empty((n, 2), np.int64)
+    rows[:S] = np.arange(2 * S).reshape(S, 2)
+    if M:
+        b = M // int(n_opponents)
+        j = np.arange(M)
+        lp = (j % b >= b // 2).astype(np.int64)          # the learner's player in pool env S + j
+        L = 2 * S + M
+        rows[S + j, lp] = 2 * S + j
+        rows[S + j, 1 - lp] = L + j
+    return rows
+
+
 class SelfPlayTrainer:
     """Batched self-play: E games stepped together, both players driven by the shared actor
     with parameter-noise exploration, transitions kept in a device replay ring, critic and
@@ -1080,15 +1102,42 @@ class SelfPlayTrainer:
                  batch_size: int = 4096, gamma: float = 0.0, tau: float = 1.0, param_noise_sd: float = 0.5,
                  noise_group: int = 128, reward_mode: str = "looking", tick_limit: int = 2000,
                  random_positions: bool = True, process_group=None, precision: str = "f32", collective: str = "nccl",
-                 frames: int = 1, update_precision: Optional[str] = None):
+                 frames: int = 1, update_precision: Optional[str] = None, opponents=None, pool_envs: Optional[int] = None):
         """frames > 1: the frame-stacked "planning" networks (readme.md:18-20, BASELINE.json configs[4]): both players act
         from their last `frames` observations (FrameStackActor; `precision` selects its float32 or tensor-core kernels),
         the replay ring stores the stacked observations, and the critic / actor update of SkillshotLearner.py:386-443 runs
         on the 12 * frames-input networks in separate steps.
         update_precision: the kernels of that update, "f32" or "bf16"; None = `precision` when frames = 1, "f32" when
-        frames > 1."""
+        frames > 1.
+        opponents: train against a pool of frozen 1-frame actors (flat vectors or six get_weights() arrays, copied here,
+        at most 64): the last pool_envs envs (default: half of them, rounded down to a multiple of 2 * len(opponents)) are
+        the learner against opponent k in block k of pool_envs / len(opponents) envs, seat-balanced (pool_layout).  The
+        opponents act without noise and only the learner's transitions are stored; see set_opponent / pool_progress."""
         self.device = torch.device(device)
         self.frames = int(frames)
+        self.opponents, self.pool_envs, self.pool_stats = None, 0, None
+        if opponents is not None:
+            K = len(opponents)
+            if self.frames > 1:
+                raise ValueError("training against a pool needs a 1-frame learner")
+            if process_group is not None:
+                raise ValueError("training against a pool runs on one GPU (no process_group)")
+            if reward_mode == "simple":
+                raise ValueError("training against a pool supports reward modes none / looking / terminal")
+            if not 1 <= K <= _lib.LEAGUE_MAX_POLICIES:
+                raise ValueError("1..%d opponents, got %d" % (_lib.LEAGUE_MAX_POLICIES, K))
+            M = (int(n_envs) // 2) // (2 * K) * (2 * K) if pool_envs is None else int(pool_envs)
+            if not 0 <= M <= int(n_envs) or M % (2 * K):
+                raise ValueError("pool_envs must be a multiple of 2 * %d in [0, n_envs], got %d" % (K, M))
+            self.opponents = torch.zeros((K, POOL_STRIDE), dtype=torch.float32, device=self.device)
+            for k, a in enumerate(opponents):
+                self.opponents[k, :A_N] = torch.from_numpy(self._opponent_vector(a)).to(self.device)
+            self.pool_envs = M
+            self.pool_stats = torch.zeros((K, _lib.POOL_STATS), dtype=torch.int64, device=self.device)
+        self.learner_rows = 2 * int(n_envs) - self.pool_envs       # rows of the learner's transitions per tick
+        L = self.learner_rows
+        if replay_capacity is not None and self.opponents is not None and (replay_capacity % L or replay_capacity < 2 * L):
+            raise ValueError("with a pool the replay capacity must be a multiple of the %d learner rows, at least two of them" % L)
         self.envs = SkillshotEnvs(n_envs, device=device, random_positions=random_positions, seed=seed,
                                   reward_mode=reward_mode, tick_limit=tick_limit, auto_reset=True)
         self.envs.collect_episode_stats = True     # the reference's per-episode ticks / winner log, reduced on the device
@@ -1097,7 +1146,7 @@ class SelfPlayTrainer:
                                     update_precision=update_precision or (precision if self.frames == 1 else "f32"),
                                     collective=collective, frames=self.frames)
         self.networks.seed = seed          # exploration / dropout streams differ per rank, weights do not
-        self.replay = ReplayRing(replay_capacity or 2 * n_envs * 8, device=device, seed=seed, frames=self.frames)
+        self.replay = ReplayRing(replay_capacity or L * 8, device=device, seed=seed, frames=self.frames)
         self.batch_size, self.param_noise_sd, self.noise_group = int(batch_size), float(param_noise_sd), int(noise_group)
         self.precision = precision
         self.update_precision = update_precision
@@ -1120,11 +1169,91 @@ class SelfPlayTrainer:
         self.updates = 0
         self.exchange_check_every = 256     # updates between looks at the peer exchange's status word
         self._tile_ready, self._stream2 = None, None      # overlapped rollout (rollout()): allocated on first use
+        if self.opponents is not None:
+            # rows [0, L) the learner's, [L, 2n) the opponents' (pool_layout): observations and actions
+            rows = torch.from_numpy(pool_layout(n, self.pool_envs, len(self.opponents)).reshape(-1)).to(self.device)
+            self.obs = torch.empty((2 * n, 12), dtype=torch.float32, device=self.device)
+            self.obs[rows] = self.envs.observe().reshape(-1, 12)
+            self.prev_obs = None
+            self.actions = torch.empty((2 * n, 2), dtype=torch.float32, device=self.device)
+            self._pool_reward = torch.zeros(L, dtype=torch.float32, device=self.device)
+
+    @staticmethod
+    def _opponent_vector(actor) -> np.ndarray:
+        flat, frames = actor_vector(actor)
+        if frames != 1:
+            raise ValueError("pool opponents must be 1-frame actors, got %d frames" % frames)
+        return flat
+
+    def set_opponent(self, k: int, actor):
+        """Replace opponent k of the pool with a copy of `actor` from the next tick on (the games in flight continue against
+        it), e.g. trainer.set_opponent(i % K, trainer.networks.actor) every few updates."""
+        if self.opponents is None:
+            raise ValueError("this trainer has no opponent pool")
+        k = int(k)
+        if not 0 <= k < len(self.opponents):
+            raise IndexError("opponent %d of %d" % (k, len(self.opponents)))
+        if torch.is_tensor(actor) and actor.dim() == 1 and actor.numel() == A_N:
+            self.opponents[k, :A_N].copy_(actor.detach())
+        else:
+            self.opponents[k, :A_N] = torch.from_numpy(self._opponent_vector(actor)).to(self.device)
+
+    def pool_progress(self, reset: bool = False) -> list:
+        """Per opponent, the training games against it finished so far (device counters): episodes, learner wins (the
+        opponent was hit), learner losses, tick-limit endings (draws), mean episode ticks, and the learner's score with
+        its standard error (win 1, draw 0.5, loss 0)."""
+        from .league import _score
+        if self.opponents is None:
+            raise ValueError("this trainer has no opponent pool")
+        c = self.pool_stats.cpu().numpy()
+        if reset:
+            self.pool_stats.zero_()
+        out = []
+        for k in range(c.shape[0]):
+            games, wins, losses, draws, ticks = (int(v) for v in c[k, :5])
+            score, se = _score(wins, draws, games)
+            out.append(dict(episodes=games, wins=wins, losses=losses, draws=draws,
+                            mean_ticks=ticks / games if games else float("nan"), score=score, stderr=se))
+        return out
+
+    def _rollout_pool(self, n_ticks: int, store: bool):
+        """n_ticks ticks through ss_pool_rollout: the learner's forward, the opponents' segment forward, the pool step."""
+        envs, net, rp = self.envs, self.networks, self.replay
+        if envs.speeds is not None:
+            raise ValueError("training against a pool does not support per-env speeds")
+        L, M = self.learner_rows, self.pool_envs
+        out = envs._buffers(1)
+        a = _lib.PoolRolloutArgs()
+        a.state, a.n_envs, a.pool_envs, a.n_opponents = envs.state.data_ptr(), envs.n_envs, M, len(self.opponents)
+        a.params, a.opp_params, a.opp_param_stride = net.actor.data_ptr(), self.opponents.data_ptr(), POOL_STRIDE
+        a.obs, a.act, a.reward = self.obs.data_ptr(), self.actions.data_ptr(), self._pool_reward.data_ptr()
+        a.opp_obs, a.opp_act = self.obs[L:].data_ptr(), self.actions[L:].data_ptr()
+        a.done, a.winner = out["done"].data_ptr(), out["winner"].data_ptr()
+        if store:
+            a.ring_obs, a.ring_act, a.ring_reward = rp.obs.data_ptr(), rp.act.data_ptr(), rp.reward.data_ptr()
+            a.ring_next_obs, a.ring_done, a.capacity, a.write_pos = rp.next_obs.data_ptr(), rp.done.data_ptr(), rp.capacity, rp.pos
+        a.n_ticks, a.param_noise_sd, a.noise_group, a.action_noise_sd = int(n_ticks), self.param_noise_sd, self.noise_group, 0.0
+        a.tensor_cores, a.reward_mode, a.tick_limit = 1 if self.precision == "bf16" else 0, REWARD_MODES[envs.reward_mode], envs.tick_limit
+        a.reset_mode = _lib.RESET_RANDOM if envs.random_positions else _lib.RESET_FIXED
+        a.env_seed, a.env_counter, a.noise_seed, a.noise_counter = envs.seed, envs.counter, net.seed, net.counter
+        a.status, a.step_flags = envs.status.data_ptr(), _lib.STEP_EPISODE_STATS if envs.collect_episode_stats else 0
+        a.pool_stats = self.pool_stats.data_ptr()
+        with torch.cuda.device(self.device):
+            check(lib.ss_pool_rollout(ctypes.byref(a), _stream(self.device)), "ss_pool_rollout")
+        envs.counter += n_ticks
+        net.counter += n_ticks
+        if store:
+            rp.pos = (rp.pos + L * n_ticks) % rp.capacity
+            rp.size = min(rp.capacity, rp.size + L * n_ticks)
+        self.ticks += n_ticks
+        return dict(obs=self.obs, reward=self._pool_reward, done=out["done"][0], winner=out["winner"][0])
 
     def rollout_tick(self, store: bool = True):
         """One tick of every env: actor forward on both players' observations (fresh parameter
         noise per noise group), env step, transition push."""
         self._ring_clean = False
+        if self.opponents is not None:
+            return self._rollout_pool(1, store)
         if self.frames > 1:
             return self._rollout_tick_frames(store)
         self.prev_obs, self.obs = self.obs, self.prev_obs
@@ -1157,6 +1286,8 @@ class SelfPlayTrainer:
         """n_ticks rollout ticks enqueued by ONE library call (ss_selfplay_rollout): same kernels and Philox
         counters as n_ticks calls of rollout_tick, without the per-tick host work."""
         self._ring_clean = False
+        if self.opponents is not None:
+            return self._rollout_pool(int(n_ticks), store)
         if self.frames > 1:
             for _ in range(int(n_ticks)):
                 out = self._rollout_tick_frames(store)
@@ -1213,9 +1344,16 @@ class SelfPlayTrainer:
             st = self.stack
             sd["stack"] = dict(stack=st.stack.cpu(), stack32=None if st.stack32 is None else st.stack32.cpu(), head=st.head,
                                counter=st.counter, rows=self.rows.cpu())
+        if self.opponents is not None:
+            sd["pool"] = dict(opponents=self.opponents.cpu(), pool_envs=self.pool_envs, stats=self.pool_stats.cpu())
         return sd
 
     def load_state_dict(self, sd):
+        pool = sd.get("pool")            # absent: a trainer without a pool
+        have = (0, 0) if self.opponents is None else (self.pool_envs, len(self.opponents))
+        want = (0, 0) if pool is None else (int(pool["pool_envs"]), int(pool["opponents"].shape[0]))
+        if have != want:
+            raise ValueError("checkpoint pool layout (pool_envs, opponents) = %s, this trainer's %s" % (want, have))
         self.envs.load_state_dict(sd["envs"])
         self.networks.load_state_dict(sd["networks"])
         self.replay.load_state_dict(sd["replay"])
@@ -1231,6 +1369,9 @@ class SelfPlayTrainer:
                 st.stack32.copy_(ss["stack32"].to(self.device))
             st.head, st.counter = int(ss["head"]), int(ss["counter"])
             self.rows.copy_(ss["rows"].to(self.device))
+        if pool is not None:
+            self.opponents.copy_(pool["opponents"].to(self.device))
+            self.pool_stats.copy_(pool["stats"].to(self.device))
         self._batch = None
         self._batches = [None, None]
         self._ring_clean = False
