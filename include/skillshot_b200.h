@@ -653,6 +653,80 @@ typedef struct ss_pool_rollout_args {
 } ss_pool_rollout_args;
 int ss_pool_rollout(const ss_pool_rollout_args *args, void *stream);
 
+/* The same training against a pool with frame-stacked networks: the learner reads its last `frames` (F_l, 1..20)
+ * observations and opponent k its last opp_frames[k] (F_k, 1..20).  Histories are those of ss_obs_stack_push_tc
+ * (tensor_cores) / ss_obs_stack_push (float32); `head` is the slot counter of the newest frame of every history on entry
+ * (after the call: head + n_ticks).
+ *
+ *   ss_obs_stack_push_pool  the learner's history step of one pool tick, for its L = 2S + M rows (S = n_envs - pool_envs):
+ *                           row r belongs to env r < 2S ? r / 2 : S + (r - 2S) and restarts when done[env] is set (any
+ *                           episode end, the per-env done_out of ss_env_step_pool).  obs[r] goes to slot head % frames of
+ *                           stack_tc (NULL: none) and stack32, or to every slot on a restart, with the bytes of
+ *                           ss_obs_stack_push_tc and ss_obs_stack_push; the ordered row [12 frames] (oldest frame first, as
+ *                           ss_obs_stack_ordered) is written to rows_out and, when not NULL, to rows_out2.  M = 0 is the
+ *                           self-play rule (row r <-> env r / 2).  One launch; every history slot is read at most once.
+ *
+ * ss_pool_rollout_frames: ss_pool_rollout (whose all-frames-1 case it is, launch for launch) with these histories.  Per tick:
+ *   learner, F_l > 1    ss_param_noise_groups (counter noise_counter + t; skipped without parameter noise), then
+ *                       ss_actor_forward_frames_tc (float32: ss_actor_forward_frames) over the L rows, one vector per group
+ *   learner, F_l = 1    as ss_pool_rollout
+ *   opponents           one ss_actor_forward_segments_tc per maximal run of consecutive 1-frame opponents, and
+ *                       ss_actor_forward_frames_tc (parameter stride 0) on each F_k > 1 opponent's b rows; float32: the
+ *                       exact forward of each opponent
+ *   ss_env_step_pool    reward and hit flag into the ring segment; observations into it too when F_l = 1, into the staging
+ *                       obs [L][12] when F_l > 1
+ *   pushes              F_l > 1: ss_obs_stack_push_pool, writing the ring's next_obs of segment t and obs of segment t + 1
+ *                       (the caller's `rows` on the last tick; without a ring only `rows`); each F_k > 1 opponent:
+ *                       ss_obs_stack_push_tc / ss_obs_stack_push on its stack with done + S + k b, done_div 1
+ * With F_l > 1 the ring rows hold 12 F_l floats of observation (ss_replay_push_frames' layout) and segment t's obs is filled
+ * from `rows` on entry.  The ring, speed and reward rules are ss_pool_rollout's; action_noise_sd must be 0 when F_l > 1.
+ *   rows [L][12 F_l]    the learner's current ordered rows on entry and on return (F_l > 1)
+ *   opp_frames [K]      HOST array; NULL: every opponent has 1 frame.  opp_stacks [K] HOST array, NULL entries for F_k = 1
+ *   opp_param_stride    % 4 == 0 and (K > 1) at least every opponent's ss_actor_frames_params(F_k)
+ *   workspace           ss_pool_rollout_frames_workspace_bytes(args) bytes, 16-byte aligned (NULL when 0): the learner's
+ *                       noisy parameter vectors and the frame-stacked forward's layer-1 tiles.  That call reads n_envs,
+ *                       pool_envs, n_opponents, frames, opp_frames, tensor_cores, param_noise_sd and noise_group and returns
+ *                       -1 when they are invalid. */
+typedef struct ss_pool_rollout_frames_args {
+    void *state;
+    int64_t n_envs, pool_envs;
+    int n_opponents;
+    const float *params;
+    const float *opp_params;
+    int64_t opp_param_stride;
+    float *obs, *act, *reward;
+    float *opp_obs, *opp_act;
+    uint8_t *done, *winner;
+    float *ring_obs, *ring_act, *ring_reward, *ring_next_obs;
+    uint8_t *ring_done;
+    int64_t capacity, write_pos;
+    int n_ticks;
+    float param_noise_sd;
+    int64_t noise_group;
+    float action_noise_sd;
+    int tensor_cores, reward_mode;
+    int64_t tick_limit;
+    int reset_mode;
+    uint64_t env_seed, env_counter, noise_seed, noise_counter;
+    const void *speeds;                        /* must be NULL */
+    uint32_t *status;
+    int step_flags;
+    uint64_t *pool_stats;
+    int frames;                                /* the learner's F_l */
+    void *stack_tc;                            /* learner history, tensor-core layout (tensor_cores, F_l > 1) */
+    float *stack32;                            /* learner history, float32 [L][F_l][12] (F_l > 1) */
+    float *rows;                               /* [L][12 F_l] (F_l > 1) */
+    int64_t head;
+    const int *opp_frames;                     /* host [K] or NULL */
+    void *const *opp_stacks;                   /* host [K] or NULL */
+    void *workspace;
+    int64_t workspace_bytes;
+} ss_pool_rollout_frames_args;
+int ss_obs_stack_push_pool(void *stack_tc, float *stack32, int64_t n_envs, int64_t pool_envs, int frames, int64_t head,
+                           const float *obs, const uint8_t *done, float *rows_out, float *rows_out2, void *stream);
+int64_t ss_pool_rollout_frames_workspace_bytes(const ss_pool_rollout_frames_args *args);
+int ss_pool_rollout_frames(const ss_pool_rollout_frames_args *args, void *stream);
+
 /* ---- multi-GPU: the gradient all-reduce fused with its neighbours over NVLink peer memory ----
  * One exchange allocation per rank = flags[2][world] | inbox[2][world][capacity floats], made by
  * ss_peer_alloc and shared between the processes of one node through CUDA IPC (export on the owner,

@@ -88,6 +88,14 @@ class PoolRolloutArgs(ctypes.Structure):
                  ("speeds", _vp), ("status", _vp), ("step_flags", _i32), ("pool_stats", _vp)])
 
 
+class PoolRolloutFramesArgs(ctypes.Structure):
+    """struct ss_pool_rollout_frames_args of include/skillshot_b200.h (same field order): ss_pool_rollout_args' fields, then
+    the histories."""
+    _fields_ = PoolRolloutArgs._fields_ + [
+        ("frames", _i32), ("stack_tc", _vp), ("stack32", _vp), ("rows", _vp), ("head", _i64),
+        ("opp_frames", ctypes.POINTER(_i32)), ("opp_stacks", ctypes.POINTER(_vp)), ("workspace", _vp), ("workspace_bytes", _i64)]
+
+
 # name -> (restype, argtypes); every symbol the header declares
 SIGNATURES = {
     "ss_version": (_i32, []),
@@ -183,6 +191,9 @@ SIGNATURES = {
     "ss_env_step_pool": (_i32, [_vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i64, _i32, _u64, _u64,
                                  _vp, _i32, _vp, _vp]),
     "ss_pool_rollout": (_i32, [ctypes.POINTER(PoolRolloutArgs), _vp]),
+    "ss_obs_stack_push_pool": (_i32, [_vp, _vp, _i64, _i64, _i32, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "ss_pool_rollout_frames_workspace_bytes": (_i64, [ctypes.POINTER(PoolRolloutFramesArgs)]),
+    "ss_pool_rollout_frames": (_i32, [ctypes.POINTER(PoolRolloutFramesArgs), _vp]),
     "ss_replay_sample": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp, _u64, _u64, _i64,
                                  _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
 }

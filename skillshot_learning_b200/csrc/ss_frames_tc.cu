@@ -475,6 +475,49 @@ __global__ void obs_stack_push_tc_kernel(uint8_t *xt, int64_t n_rows, int frames
     *reinterpret_cast<uint32_t *>(base + (uint32_t)(kx >> 3) * CHUNK_A + (kx & 7) * 2) = 0x3C003C00u;
 }
 
+// The learner's history step of a pool tick (ss_obs_stack_push_pool): obs_stack_push_tc_kernel, obs_stack_push_kernel and
+// obs_stack_ordered_kernel for the L learner rows in one pass, with each row's restart flag found by the pool row rule.
+// Thread (row, f, part) owns float4 `part` of frame f of the row's ordered output (oldest first), i.e. ring slot
+// (newest + 1 + f) % frames: it takes the newest observation when that slot is the newest one or the game restarted (and then
+// stores it in both histories), the float32 history's value otherwise, and writes it to the ordered row(s).  So every
+// history slot is read at most once and the ordered rows are written straight from registers.  blockIdx.y selects a chunk
+// of PUSH_CHUNK rows, so the index arithmetic within a chunk is 32-bit; `newest` = head % frames comes from the host.
+constexpr int64_t PUSH_CHUNK = 1 << 20;
+
+__global__ void obs_stack_push_pool_kernel(uint8_t *xt, float *stack32, int64_t n_rows, int64_t S, int frames, int newest,
+                                           uint32_t tile_bytes, const float *obs, const uint8_t *done, float *rows_out,
+                                           float *rows_out2) {
+    const uint32_t w4 = 3 * frames, t = blockIdx.x * blockDim.x + threadIdx.x, local = t / w4;
+    const int64_t row = (int64_t)blockIdx.y * PUSH_CHUNK + local;
+    if (local >= PUSH_CHUNK || row >= n_rows) return;
+    const int q = (int)(t - local * w4), f = q / 3, part = q - 3 * f;
+    int slot = newest + 1 + f;
+    if (slot >= frames) slot -= frames;
+    const int64_t env = row < 2 * S ? row >> 1 : row - S;
+    const bool restart = done && done[env];
+    float4 *h = reinterpret_cast<float4 *>(stack32) + (row * frames + slot) * 3 + part;
+    float4 v;
+    if (restart || slot == newest) {
+        v = __ldg(reinterpret_cast<const float4 *>(obs) + row * 3 + part);
+        *h = v;
+        if (xt) {                                           // the same 8 bytes obs_stack_push_tc_kernel's put() stores
+            const int c = DS * slot + 4 * part;
+            *reinterpret_cast<uint2 *>(xt + (row / TM) * (int64_t)tile_bytes + (row % TM) * 16 + (uint32_t)(c >> 3) * CHUNK_A +
+                                       (c & 7) * 2) = make_uint2(pack_f16(v.x, v.y), pack_f16(v.z, v.w));
+        }
+    } else {
+        v = *h;
+    }
+    if (xt && q == 0) {
+        const int kx = DS * frames;
+        *reinterpret_cast<uint32_t *>(xt + (row / TM) * (int64_t)tile_bytes + (row % TM) * 16 + (uint32_t)(kx >> 3) * CHUNK_A +
+                                      (kx & 7) * 2) = 0x3C003C00u;
+    }
+    const int64_t e = row * w4 + q;
+    reinterpret_cast<float4 *>(rows_out)[e] = v;
+    if (rows_out2) reinterpret_cast<float4 *>(rows_out2)[e] = v;
+}
+
 }  // namespace
 
 int sstc::frames_layer1_tc(const float *params, const void *xt, int frames, int64_t n, void *h1, cudaStream_t st) {
@@ -500,6 +543,20 @@ extern "C" int ss_obs_stack_push_tc(void *stack_tc, int64_t n_rows, int frames, 
     if (((uintptr_t)stack_tc | (uintptr_t)obs) & 15) return SS_ERR_INVALID_ARG;
     obs_stack_push_tc_kernel<<<(unsigned)((n_rows + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
         (uint8_t *)stack_tc, n_rows, frames, (int)(head % frames), (uint32_t)(frames_k1(frames) / 8) * CHUNK_A, obs, done, done_div);
+    return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA;
+}
+
+extern "C" int ss_obs_stack_push_pool(void *stack_tc, float *stack32, int64_t n_envs, int64_t pool_envs, int frames, int64_t head,
+                                      const float *obs, const uint8_t *done, float *rows_out, float *rows_out2, void *stream) {
+    if (!stack32 || !obs || !rows_out || n_envs <= 0 || pool_envs < 0 || pool_envs > n_envs || frames < 1 || frames > MAXF || head < 0)
+        return SS_ERR_INVALID_ARG;
+    if (((uintptr_t)stack_tc | (uintptr_t)stack32 | (uintptr_t)obs | (uintptr_t)rows_out | (uintptr_t)rows_out2) & 15)
+        return SS_ERR_INVALID_ARG;
+    const int64_t S = n_envs - pool_envs, L = 2 * S + pool_envs, threads = 3 * frames * (L < PUSH_CHUNK ? L : PUSH_CHUNK);
+    const dim3 grid((unsigned)((threads + 255) / 256), (unsigned)((L + PUSH_CHUNK - 1) / PUSH_CHUNK));
+    obs_stack_push_pool_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>((uint8_t *)stack_tc, stack32, L, S, frames, (int)(head % frames),
+                                                                       (uint32_t)(frames_k1(frames) / 8) * CHUNK_A, obs, done, rows_out,
+                                                                       rows_out2);
     return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA;
 }
 

@@ -1109,17 +1109,16 @@ class SelfPlayTrainer:
         on the 12 * frames-input networks in separate steps.
         update_precision: the kernels of that update, "f32" or "bf16"; None = `precision` when frames = 1, "f32" when
         frames > 1.
-        opponents: train against a pool of frozen 1-frame actors (flat vectors or six get_weights() arrays, copied here,
-        at most 64): the last pool_envs envs (default: half of them, rounded down to a multiple of 2 * len(opponents)) are
-        the learner against opponent k in block k of pool_envs / len(opponents) envs, seat-balanced (pool_layout).  The
-        opponents act without noise and only the learner's transitions are stored; see set_opponent / pool_progress."""
+        opponents: train against a pool of frozen actors (flat vectors or six get_weights() arrays of any frame count,
+        copied here, at most 64): the last pool_envs envs (default: half of them, rounded down to a multiple of
+        2 * len(opponents)) are the learner against opponent k in block k of pool_envs / len(opponents) envs, seat-balanced
+        (pool_layout).  The opponents act without noise and only the learner's transitions are stored; an opponent with
+        more than one frame keeps a history of its rows.  See set_opponent / pool_progress."""
         self.device = torch.device(device)
         self.frames = int(frames)
         self.opponents, self.pool_envs, self.pool_stats = None, 0, None
         if opponents is not None:
             K = len(opponents)
-            if self.frames > 1:
-                raise ValueError("training against a pool needs a 1-frame learner")
             if process_group is not None:
                 raise ValueError("training against a pool runs on one GPU (no process_group)")
             if reward_mode == "simple":
@@ -1129,15 +1128,17 @@ class SelfPlayTrainer:
             M = (int(n_envs) // 2) // (2 * K) * (2 * K) if pool_envs is None else int(pool_envs)
             if not 0 <= M <= int(n_envs) or M % (2 * K):
                 raise ValueError("pool_envs must be a multiple of 2 * %d in [0, n_envs], got %d" % (K, M))
-            self.opponents = torch.zeros((K, POOL_STRIDE), dtype=torch.float32, device=self.device)
-            for k, a in enumerate(opponents):
-                self.opponents[k, :A_N] = torch.from_numpy(self._opponent_vector(a)).to(self.device)
+            if precision == "bf16" and float(param_noise_sd) > 0 and int(noise_group) % 128:
+                raise ValueError("with tensor cores and parameter noise the noise group must be a multiple of 128, got %d" % noise_group)
+            opp_vecs = [actor_vector(a) for a in opponents]
+            self.opp_frames = [f for _, f in opp_vecs]
             self.pool_envs = M
-            self.pool_stats = torch.zeros((K, _lib.POOL_STATS), dtype=torch.int64, device=self.device)
         self.learner_rows = 2 * int(n_envs) - self.pool_envs       # rows of the learner's transitions per tick
         L = self.learner_rows
-        if replay_capacity is not None and self.opponents is not None and (replay_capacity % L or replay_capacity < 2 * L):
+        if replay_capacity is not None and opponents is not None and (replay_capacity % L or replay_capacity < 2 * L):
             raise ValueError("with a pool the replay capacity must be a multiple of the %d learner rows, at least two of them" % L)
+        if opponents is not None and self.device.type != "cuda":
+            raise ValueError("device must be a CUDA device")
         self.envs = SkillshotEnvs(n_envs, device=device, random_positions=random_positions, seed=seed,
                                   reward_mode=reward_mode, tick_limit=tick_limit, auto_reset=True)
         self.envs.collect_episode_stats = True     # the reference's per-episode ticks / winner log, reduced on the device
@@ -1154,22 +1155,13 @@ class SelfPlayTrainer:
         self.obs = self.envs.observe().contiguous()                       # [n,2,12] seen by the actor next
         self.prev_obs = torch.empty_like(self.obs)
         self.actions = torch.empty((n, 2, 2), dtype=torch.float32, device=self.device)
-        self.stack = None
-        if self.frames > 1:
-            # the acting network IS the learner's actor vector; the history lives in the FrameStackActor
-            self.stack = FrameStackActor(2 * n, frames=self.frames, device=device, seed=seed, precision=precision,
-                                         params=self.networks.actor, learner_stack=True)
-            self.stack.push(self.obs.reshape(-1, 12))
-            self.rows = self.stack.ordered_rows()                         # [2n, 12 frames]: the stacked observation now
-            self.prev_rows = torch.empty_like(self.rows)
-        self._batch = None
-        self._batches = [None, None]        # update(): two sets of minibatch buffers used in turn
-        self._ring_clean = False            # no rollout (nothing of this object's that writes the ring) since the last update
-        self.ticks = 0
-        self.updates = 0
-        self.exchange_check_every = 256     # updates between looks at the peer exchange's status word
-        self._tile_ready, self._stream2 = None, None      # overlapped rollout (rollout()): allocated on first use
-        if self.opponents is not None:
+        if opponents is not None:
+            K = len(opp_vecs)
+            # one row per opponent, as wide as the largest vector (16-byte aligned; POOL_STRIDE when all have one frame)
+            self.opponents = torch.zeros((K, max((v.size + 3) // 4 * 4 for v, _ in opp_vecs)), dtype=torch.float32, device=self.device)
+            for k, (v, _) in enumerate(opp_vecs):
+                self.opponents[k, :v.size] = torch.from_numpy(v).to(self.device)
+            self.pool_stats = torch.zeros((K, _lib.POOL_STATS), dtype=torch.int64, device=self.device)
             # rows [0, L) the learner's, [L, 2n) the opponents' (pool_layout): observations and actions
             rows = torch.from_numpy(pool_layout(n, self.pool_envs, len(self.opponents)).reshape(-1)).to(self.device)
             self.obs = torch.empty((2 * n, 12), dtype=torch.float32, device=self.device)
@@ -1177,26 +1169,64 @@ class SelfPlayTrainer:
             self.prev_obs = None
             self.actions = torch.empty((2 * n, 2), dtype=torch.float32, device=self.device)
             self._pool_reward = torch.zeros(L, dtype=torch.float32, device=self.device)
+            self._pool_ws = None
+            # the histories of the opponents with frames > 1, b rows each, filled with the first observation (slot 0);
+            # every history of the pool shares one slot counter
+            self.opp_stacks, self._pool_head = [None] * len(self.opponents), 0      # (see pool_head)
+            b = self.pool_envs // len(self.opponents)
+            for k, f in enumerate(self.opp_frames):
+                if f == 1 or b == 0:
+                    continue
+                if precision == "bf16":
+                    s = torch.zeros(int(lib.ss_obs_stack_tc_bytes(b, f)), dtype=torch.uint8, device=self.device)
+                else:
+                    s = torch.zeros((b, f, 12), dtype=torch.float32, device=self.device)
+                fn = lib.ss_obs_stack_push_tc if precision == "bf16" else lib.ss_obs_stack_push
+                ones = torch.ones(b, dtype=torch.uint8, device=self.device)
+                with torch.cuda.device(self.device):
+                    check(fn(s.data_ptr(), b, f, 0, self.obs[L + k * b:].data_ptr(), ones.data_ptr(), 1, _stream(self.device)),
+                          "ss_obs_stack_push")
+                self.opp_stacks[k] = s
+        self.stack = None
+        if self.frames > 1:
+            # the acting network IS the learner's actor vector; the history lives in the FrameStackActor (its L rows)
+            self.stack = FrameStackActor(L, frames=self.frames, device=device, seed=seed, precision=precision,
+                                         params=self.networks.actor, learner_stack=True)
+            self.stack.push(self.obs[:L] if self.opponents is not None else self.obs.reshape(-1, 12))
+            self.rows = self.stack.ordered_rows()                         # [L, 12 frames]: the stacked observation now
+            self.prev_rows = torch.empty_like(self.rows) if self.opponents is None else None
+        self._batch = None
+        self._batches = [None, None]        # update(): two sets of minibatch buffers used in turn
+        self._ring_clean = False            # no rollout (nothing of this object's that writes the ring) since the last update
+        self.ticks = 0
+        self.updates = 0
+        self.exchange_check_every = 256     # updates between looks at the peer exchange's status word
+        self._tile_ready, self._stream2 = None, None      # overlapped rollout (rollout()): allocated on first use
 
-    @staticmethod
-    def _opponent_vector(actor) -> np.ndarray:
-        flat, frames = actor_vector(actor)
-        if frames != 1:
-            raise ValueError("pool opponents must be 1-frame actors, got %d frames" % frames)
-        return flat
+    @property
+    def pool_head(self) -> int:
+        """The slot counter of the newest frame shared by every history of the pool: the learner's FrameStackActor's when it
+        reads more than one frame, else the trainer's own (then only the opponents' histories use it)."""
+        return self.stack.head if self.stack is not None else self._pool_head
 
     def set_opponent(self, k: int, actor):
         """Replace opponent k of the pool with a copy of `actor` from the next tick on (the games in flight continue against
-        it), e.g. trainer.set_opponent(i % K, trainer.networks.actor) every few updates."""
+        it, with the slot's history), e.g. trainer.set_opponent(i % K, trainer.networks.actor) every few updates.  The actor
+        must have the slot's frame count."""
         if self.opponents is None:
             raise ValueError("this trainer has no opponent pool")
         k = int(k)
         if not 0 <= k < len(self.opponents):
             raise IndexError("opponent %d of %d" % (k, len(self.opponents)))
-        if torch.is_tensor(actor) and actor.dim() == 1 and actor.numel() == A_N:
-            self.opponents[k, :A_N].copy_(actor.detach())
-        else:
-            self.opponents[k, :A_N] = torch.from_numpy(self._opponent_vector(actor)).to(self.device)
+        f = self.opp_frames[k]
+        n_params = int(lib.ss_actor_frames_params(f))
+        if torch.is_tensor(actor) and actor.dim() == 1 and actor.numel() == n_params:
+            self.opponents[k, :n_params].copy_(actor.detach())
+            return
+        flat, frames = actor_vector(actor)
+        if frames != f:
+            raise ValueError("opponent %d has %d frames, the new actor %d" % (k, f, frames))
+        self.opponents[k, :n_params] = torch.from_numpy(flat).to(self.device)
 
     def pool_progress(self, reset: bool = False) -> list:
         """Per opponent, the training games against it finished so far (device counters): episodes, learner wins (the
@@ -1217,15 +1247,16 @@ class SelfPlayTrainer:
         return out
 
     def _rollout_pool(self, n_ticks: int, store: bool):
-        """n_ticks ticks through ss_pool_rollout: the learner's forward, the opponents' segment forward, the pool step."""
-        envs, net, rp = self.envs, self.networks, self.replay
+        """n_ticks ticks through ss_pool_rollout_frames: the learner's forward, the opponents' forwards, the pool step and
+        the history pushes."""
+        envs, net, rp, st = self.envs, self.networks, self.replay, self.stack
         if envs.speeds is not None:
             raise ValueError("training against a pool does not support per-env speeds")
-        L, M = self.learner_rows, self.pool_envs
+        L, M, K = self.learner_rows, self.pool_envs, len(self.opponents)
         out = envs._buffers(1)
-        a = _lib.PoolRolloutArgs()
-        a.state, a.n_envs, a.pool_envs, a.n_opponents = envs.state.data_ptr(), envs.n_envs, M, len(self.opponents)
-        a.params, a.opp_params, a.opp_param_stride = net.actor.data_ptr(), self.opponents.data_ptr(), POOL_STRIDE
+        a = _lib.PoolRolloutFramesArgs()
+        a.state, a.n_envs, a.pool_envs, a.n_opponents = envs.state.data_ptr(), envs.n_envs, M, K
+        a.params, a.opp_params, a.opp_param_stride = net.actor.data_ptr(), self.opponents.data_ptr(), self.opponents.shape[1]
         a.obs, a.act, a.reward = self.obs.data_ptr(), self.actions.data_ptr(), self._pool_reward.data_ptr()
         a.opp_obs, a.opp_act = self.obs[L:].data_ptr(), self.actions[L:].data_ptr()
         a.done, a.winner = out["done"].data_ptr(), out["winner"].data_ptr()
@@ -1238,10 +1269,30 @@ class SelfPlayTrainer:
         a.env_seed, a.env_counter, a.noise_seed, a.noise_counter = envs.seed, envs.counter, net.seed, net.counter
         a.status, a.step_flags = envs.status.data_ptr(), _lib.STEP_EPISODE_STATS if envs.collect_episode_stats else 0
         a.pool_stats = self.pool_stats.data_ptr()
+        a.frames, a.head = self.frames, self.pool_head
+        if st is not None:
+            a.stack_tc = st.stack.data_ptr() if st.precision == "bf16" else None
+            a.stack32 = (st.stack32 if st.precision == "bf16" else st.stack).data_ptr()
+            a.rows = self.rows.data_ptr()
+            a.noise_seed, a.noise_counter = st.seed, st.counter          # the stream FrameStackActor.forward draws from
+        frames = (ctypes.c_int * K)(*self.opp_frames)
+        stacks = (ctypes.c_void_p * K)(*[None if s is None else s.data_ptr() for s in self.opp_stacks])
+        a.opp_frames, a.opp_stacks = frames, stacks
+        need = int(lib.ss_pool_rollout_frames_workspace_bytes(ctypes.byref(a)))
+        if need > 0 and (self._pool_ws is None or self._pool_ws.numel() < need):
+            self._pool_ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+        if need > 0:
+            a.workspace, a.workspace_bytes = self._pool_ws.data_ptr(), self._pool_ws.numel()
         with torch.cuda.device(self.device):
-            check(lib.ss_pool_rollout(ctypes.byref(a), _stream(self.device)), "ss_pool_rollout")
+            check(lib.ss_pool_rollout_frames(ctypes.byref(a), _stream(self.device)), "ss_pool_rollout_frames")
         envs.counter += n_ticks
-        net.counter += n_ticks
+        if st is None:
+            net.counter += n_ticks
+            self._pool_head += n_ticks
+        else:
+            st.head += n_ticks
+            if self.param_noise_sd > 0:
+                st.counter += n_ticks
         if store:
             rp.pos = (rp.pos + L * n_ticks) % rp.capacity
             rp.size = min(rp.capacity, rp.size + L * n_ticks)
@@ -1340,20 +1391,26 @@ class SelfPlayTrainer:
                   obs=self.obs.cpu(), actions=self.actions.cpu(), ticks=self.ticks, batch_size=self.batch_size,
                   param_noise_sd=self.param_noise_sd, noise_group=self.noise_group, precision=self.precision, frames=self.frames,
                   update_precision=self.update_precision)
-        if self.stack is not None:      # the players' observation histories and the noise counter of the stacked actor
+        if self.stack is not None:      # the players' observation histories and the noise stream of the stacked actor
             st = self.stack
             sd["stack"] = dict(stack=st.stack.cpu(), stack32=None if st.stack32 is None else st.stack32.cpu(), head=st.head,
-                               counter=st.counter, rows=self.rows.cpu())
+                               counter=st.counter, seed=st.seed, rows=self.rows.cpu())
         if self.opponents is not None:
-            sd["pool"] = dict(opponents=self.opponents.cpu(), pool_envs=self.pool_envs, stats=self.pool_stats.cpu())
+            sd["pool"] = dict(opponents=self.opponents.cpu(), pool_envs=self.pool_envs, stats=self.pool_stats.cpu(),
+                              frames=list(self.opp_frames), stacks=[None if s is None else s.cpu() for s in self.opp_stacks],
+                              head=self.pool_head)
         return sd
 
     def load_state_dict(self, sd):
         pool = sd.get("pool")            # absent: a trainer without a pool
-        have = (0, 0) if self.opponents is None else (self.pool_envs, len(self.opponents))
-        want = (0, 0) if pool is None else (int(pool["pool_envs"]), int(pool["opponents"].shape[0]))
+        have = (0, 0) if self.opponents is None else (self.pool_envs, len(self.opponents), self.frames, tuple(self.opp_frames))
+        want = (0, 0)
+        if pool is not None:             # (a checkpoint of a pool of 1-frame actors may lack the frame counts)
+            K = int(pool["opponents"].shape[0])
+            want = (int(pool["pool_envs"]), K, int(sd.get("frames", 1)), tuple(int(f) for f in pool.get("frames", [1] * K)))
         if have != want:
-            raise ValueError("checkpoint pool layout (pool_envs, opponents) = %s, this trainer's %s" % (want, have))
+            raise ValueError("checkpoint pool layout (pool_envs, opponents, frames, opponent frames) = %s, this trainer's %s"
+                             % (want, have))
         self.envs.load_state_dict(sd["envs"])
         self.networks.load_state_dict(sd["networks"])
         self.replay.load_state_dict(sd["replay"])
@@ -1368,10 +1425,16 @@ class SelfPlayTrainer:
             if st.stack32 is not None:
                 st.stack32.copy_(ss["stack32"].to(self.device))
             st.head, st.counter = int(ss["head"]), int(ss["counter"])
+            st.seed = int(ss.get("seed", st.seed))       # (absent from older checkpoints: this trainer's seed)
             self.rows.copy_(ss["rows"].to(self.device))
         if pool is not None:
             self.opponents.copy_(pool["opponents"].to(self.device))
             self.pool_stats.copy_(pool["stats"].to(self.device))
+            for s, saved in zip(self.opp_stacks, pool.get("stacks", [None] * len(self.opp_stacks))):
+                if s is not None:
+                    s.copy_(saved.to(self.device))
+            if self.stack is None:      # (a frame-stacked learner's counter came back with its history)
+                self._pool_head = int(pool.get("head", 0))
         self._batch = None
         self._batches = [None, None]
         self._ring_clean = False
