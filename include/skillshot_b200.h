@@ -625,6 +625,26 @@ int ss_env_step_pool(void *state, int64_t n_envs, int64_t pool_envs, int n_oppon
                      float *opp_obs_out, uint8_t *done_out, uint8_t *winner_out, int reward_mode, int64_t tick_limit,
                      int reset_mode, uint64_t seed, uint64_t counter, uint32_t *status, int flags, uint64_t *pool_stats,
                      void *stream);
+
+/* Blocks of any size: opponent k owns the b_k consecutive pool envs from S + B_k, B_k = b_0 + ... + b_{k-1}, with the
+ * learner player 1 in the first b_k / 2 of them and player 2 in the others.  The rows keep the formula above (learner row
+ * 2S + (j - S), opponent row j - S of pool env j), so opponent k's rows are one segment of b_k rows from B_k.  Every b_k
+ * = M / K is the layout above.  A block table opp_envs is a HOST int64 [K] of pool envs per opponent, each even and >= 2,
+ * summing to M (M < 2^31); NULL means M / K each.  An invalid table returns -1 before anything is enqueued.
+ *   ss_env_step_pool_blocks  ss_env_step_pool under the table (M = 0 takes no table).  Bit-identical to ss_env_step_pool
+ *                            for the uniform table.
+ *   ss_pool_restart          every pool env starts a new game: reset_mode FIXED or RANDOM, Philox4x32-10(key = seed,
+ *                            counter = (env, counter)) as the auto-reset of a step with that counter.  The self-play envs are
+ *                            untouched.  obs [L][12] (learner rows) and opp_obs [M][12] receive the new games' observations
+ *                            under the table, the bytes an auto-reset tick writes.  No game ended, so nothing is counted;
+ *                            status is not written (NULL ok). */
+int ss_env_step_pool_blocks(void *state, int64_t n_envs, int64_t pool_envs, int n_opponents, const float *actions,
+                            const float *opp_actions, float *obs_out, float *obs_out2, float *reward_out, uint8_t *done_rows_out,
+                            float *opp_obs_out, uint8_t *done_out, uint8_t *winner_out, int reward_mode, int64_t tick_limit,
+                            int reset_mode, uint64_t seed, uint64_t counter, uint32_t *status, int flags, uint64_t *pool_stats,
+                            const int64_t *opp_envs, void *stream);
+int ss_pool_restart(void *state, int64_t n_envs, int64_t pool_envs, int n_opponents, const int64_t *opp_envs, int reset_mode,
+                    uint64_t seed, uint64_t counter, float *obs, float *opp_obs, uint32_t *status, void *stream);
 typedef struct ss_pool_rollout_args {
     void *state;
     int64_t n_envs, pool_envs;
@@ -686,7 +706,10 @@ int ss_pool_rollout(const ss_pool_rollout_args *args, void *stream);
  *   workspace           ss_pool_rollout_frames_workspace_bytes(args) bytes, 16-byte aligned (NULL when 0): the learner's
  *                       noisy parameter vectors and the frame-stacked forward's layer-1 tiles.  That call reads n_envs,
  *                       pool_envs, n_opponents, frames, opp_frames, tensor_cores, param_noise_sd and noise_group and returns
- *                       -1 when they are invalid. */
+ *                       -1 when they are invalid.
+ *   opp_envs [K]        HOST block table of ss_env_step_pool_blocks (it also reads this); NULL: M / K each, launch for launch
+ *                       the rollout above.  With a table, opponent k's forward, history and workspace use its b_k rows from
+ *                       B_k, and the step is ss_env_step_pool_blocks. */
 typedef struct ss_pool_rollout_frames_args {
     void *state;
     int64_t n_envs, pool_envs;
@@ -721,6 +744,7 @@ typedef struct ss_pool_rollout_frames_args {
     void *const *opp_stacks;                   /* host [K] or NULL */
     void *workspace;
     int64_t workspace_bytes;
+    const int64_t *opp_envs;                   /* host [K]: pool envs per opponent; NULL: M / K each */
 } ss_pool_rollout_frames_args;
 int ss_obs_stack_push_pool(void *stack_tc, float *stack32, int64_t n_envs, int64_t pool_envs, int frames, int64_t head,
                            const float *obs, const uint8_t *done, float *rows_out, float *rows_out2, void *stream);

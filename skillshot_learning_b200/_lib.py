@@ -93,7 +93,8 @@ class PoolRolloutFramesArgs(ctypes.Structure):
     the histories."""
     _fields_ = PoolRolloutArgs._fields_ + [
         ("frames", _i32), ("stack_tc", _vp), ("stack32", _vp), ("rows", _vp), ("head", _i64),
-        ("opp_frames", ctypes.POINTER(_i32)), ("opp_stacks", ctypes.POINTER(_vp)), ("workspace", _vp), ("workspace_bytes", _i64)]
+        ("opp_frames", ctypes.POINTER(_i32)), ("opp_stacks", ctypes.POINTER(_vp)), ("workspace", _vp), ("workspace_bytes", _i64),
+        ("opp_envs", ctypes.POINTER(_i64))]
 
 
 # name -> (restype, argtypes); every symbol the header declares
@@ -190,6 +191,9 @@ SIGNATURES = {
     "ss_league_play": (_i32, [ctypes.POINTER(LeagueArgs), _vp]),
     "ss_env_step_pool": (_i32, [_vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i64, _i32, _u64, _u64,
                                  _vp, _i32, _vp, _vp]),
+    "ss_env_step_pool_blocks": (_i32, [_vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i64, _i32, _u64,
+                                        _u64, _vp, _i32, _vp, ctypes.POINTER(_i64), _vp]),
+    "ss_pool_restart": (_i32, [_vp, _i64, _i64, _i32, ctypes.POINTER(_i64), _i32, _u64, _u64, _vp, _vp, _vp, _vp]),
     "ss_pool_rollout": (_i32, [ctypes.POINTER(PoolRolloutArgs), _vp]),
     "ss_obs_stack_push_pool": (_i32, [_vp, _vp, _i64, _i64, _i32, _i64, _vp, _vp, _vp, _vp, _vp]),
     "ss_pool_rollout_frames_workspace_bytes": (_i64, [ctypes.POINTER(PoolRolloutFramesArgs)]),

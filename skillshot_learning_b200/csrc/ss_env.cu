@@ -16,6 +16,7 @@
 #include "ss_env_core.cuh"
 #include "ss_env_pp.cuh"
 #include "ss_launch.cuh"
+#include "ss_pool_blocks.cuh"
 
 namespace {
 
@@ -437,16 +438,51 @@ __global__ void __launch_bounds__(BLK, 896 / BLK) step_pp_kernel(const StepArgs 
 //     S + k b, the learner being player 1 in the first b / 2 of them.  An opponent lane writes only its observation (to the
 //     opponent rows); reward and terminal flag are the learner's alone.  A warp's learner rows and its opponent rows are
 //     each one contiguous run, so the observations still leave through the shared-memory tile as coalesced stores.
+//   BlockPoolRows (ss_env_step_pool_blocks): PoolRows with one block size per opponent.  Opponent k owns the pool envs
+//     from S + start[k] to S + start[k + 1], the learner being player 1 in the first half of them; the rows are PoolRows'.
+//     The lane finds its block by a 6-step search of the table, a kernel parameter that the search reads in place from
+//     the parameter bank (LDC with a register offset; no copy to the stack, profiles/r7_pool_blocks_ptxas.txt).  Marking
+//     the parameter __grid_constant__ would change the code of the PoolRows instantiations, so it is not marked.
 struct SelfPlayRows {
     static constexpr bool kPool = false;
 };
 struct PoolRows {
-    static constexpr bool kPool = true;
+    static constexpr bool kPool = true, kBlocks = false;
     int64_t S, b;                       // self-play envs; pool envs per opponent (even, >= 2)
     const float2 *opp_actions;          // [M] opponent rows
     float4 *opp_obs;                    // [M][3]
     unsigned long long *pool_stats;     // [K][8] or NULL
 };
+struct BlockPoolRows {
+    static constexpr bool kPool = true, kBlocks = true;
+    int64_t S;
+    const float2 *opp_actions;
+    float4 *opp_obs;
+    unsigned long long *pool_stats;
+    int start[SS_LEAGUE_MAX_POLICIES + 1];   // B_0 = 0 .. B_K = M, then M up to entry 64 (M < 2^31)
+};
+
+// R.S and R.start from the table opp_envs [K] (NULL: M / K each); false: the table is invalid (ss_pool_blocks.cuh) or
+// M >= 2^31.  M = 0 takes no table (every env is self-play).
+bool pool_block_table(int64_t n, int64_t M, int K, const int64_t *opp_envs, BlockPoolRows &R) {
+    int64_t start[SS_LEAGUE_MAX_POLICIES + 1];
+    R.S = n - M;
+    if (M == 0) return !opp_envs;
+    if (M > 0x7fffffff || !sspool::block_starts(M, K, opp_envs, start)) return false;
+    for (int k = 0; k <= SS_LEAGUE_MAX_POLICIES; ++k) R.start[k] = (int)(k <= K ? start[k] : M);
+    return true;
+}
+
+// the block of pool env S + j (0 <= j < M) and the learner's player in it
+__device__ __forceinline__ int pool_block_of(const BlockPoolRows &R, int j, int &learner_player) {
+    int k = 0;
+#pragma unroll
+    for (int s = SS_LEAGUE_MAX_POLICIES / 2; s >= 1; s >>= 1)
+        if (R.start[k + s] <= j) k += s;
+    const int b0 = R.start[k];
+    learner_player = j - b0 >= ((R.start[k + 1] - b0) >> 1) ? 1 : 0;
+    return k;
+}
 
 // One finished pool game into its opponent's counters {episodes, learner wins, learner losses, tick-limit endings, ticks}.
 // winner_id is the player that was HIT.  Out of line for the reason count_episode is.
@@ -474,8 +510,12 @@ __global__ void __launch_bounds__(kBlockPP) step_pp_obs_kernel(const StepArgs A,
     if constexpr (Rows::kPool) {
         if (env >= R.S) {
             const int64_t j = env - R.S;
-            block = j / R.b;
-            learner_player = j - block * R.b >= (R.b >> 1) ? 1 : 0;
+            if constexpr (Rows::kBlocks) {
+                block = pool_block_of(R, (int)j, learner_player);
+            } else {
+                block = j / R.b;
+                learner_player = j - block * R.b >= (R.b >> 1) ? 1 : 0;
+            }
             learner = P == learner_player;
             row = learner ? 2 * R.S + j : j;
         }
@@ -547,6 +587,30 @@ __global__ void __launch_bounds__(kBlockPP) step_pp_obs_kernel(const StepArgs A,
         }
     }
     if (status && A.status) atomicOr(A.status, status);
+}
+
+// pool_restart_kernel -- ss_pool_restart: every pool env starts a new game, one thread per player of the pool envs.  The
+// start state is the auto-reset of lane_obs_tick under Philox counter (env, counter); the observation is the one an
+// auto-reset tick writes for it (the post-reset view, sin 0 and cos 1), to the learner's or the opponent's row of the
+// block layout in R.  No game ended, so nothing is counted.
+__global__ void __launch_bounds__(kBlockPP) pool_restart_kernel(void *state, int64_t n, float4 *obs, int reset_mode, uint64_t seed,
+                                                                uint64_t counter, const __grid_constant__ BlockPoolRows R) {
+    const int64_t g = (int64_t)blockIdx.x * kBlockPP + threadIdx.x;
+    if (g >= 2 * (n - R.S)) return;
+    const int P = (int)(g & 1), j = (int)(g >> 1);
+    const int64_t env = R.S + j;
+    int learner_player;
+    pool_block_of(R, j, learner_player);
+    sspp::LaneState L;
+    int ox, oy;
+    sspp::lane_reset(L, P, (uint64_t)env, counter, reset_mode, seed, ox, oy);
+    sspp::lane_store((char *)state, n, 2 * env + P, L, 0);
+    const sspp::LaneView v = sspp::lane_view(L, ox, oy, 0.0, 1.0, 0.0, 1.0);
+    float4 o[3];
+    sspp::lane_obs(L, v, o);
+    float4 *dst = P == learner_player ? obs + (2 * R.S + j) * 3 : R.opp_obs + (int64_t)j * 3;
+#pragma unroll
+    for (int q = 0; q < 3; ++q) dst[q] = o[q];
 }
 
 
@@ -1065,15 +1129,18 @@ int ss_env_step_ring(void *state, int64_t n_envs, const float *actions, float *o
     return check_launch();
 }
 
-int ss_env_step_pool(void *state, int64_t n_envs, int64_t pool_envs, int n_opponents, const float *actions,
+// ss_env_step_pool (blocks false: PoolRows) and ss_env_step_pool_blocks (blocks true: BlockPoolRows from opp_envs)
+static int step_pool(void *state, int64_t n_envs, int64_t pool_envs, int n_opponents, const float *actions,
                      const float *opp_actions, float *obs_out, float *obs_out2, float *reward_out, uint8_t *done_rows_out,
                      float *opp_obs_out, uint8_t *done_out, uint8_t *winner_out, int reward_mode, int64_t tick_limit,
                      int reset_mode, uint64_t seed, uint64_t counter, uint32_t *status, int flags, uint64_t *pool_stats,
-                     void *stream) {
+                     bool blocks, const int64_t *opp_envs, void *stream) {
     if (!state || !actions || !obs_out || n_envs <= 0 || pool_envs < 0 || pool_envs > n_envs) return SS_ERR_INVALID_ARG;
-    if (pool_envs > 0 && (n_opponents < 1 || n_opponents > SS_LEAGUE_MAX_POLICIES || pool_envs % (2 * n_opponents) != 0 ||
-                          !opp_actions || !opp_obs_out))
+    if (pool_envs > 0 && (n_opponents < 1 || n_opponents > SS_LEAGUE_MAX_POLICIES || !opp_actions || !opp_obs_out))
         return SS_ERR_INVALID_ARG;
+    BlockPoolRows B{};
+    if (blocks && !pool_block_table(n_envs, pool_envs, n_opponents, opp_envs, B)) return SS_ERR_INVALID_ARG;
+    if (!blocks && pool_envs > 0 && pool_envs % (2 * n_opponents) != 0) return SS_ERR_INVALID_ARG;
     if (reward_mode != SS_REWARD_NONE && reward_mode != SS_REWARD_LOOKING && reward_mode != SS_REWARD_TERMINAL) return SS_ERR_INVALID_ARG;
     if (reset_mode != SS_RESET_FIXED && reset_mode != SS_RESET_RANDOM) return SS_ERR_INVALID_ARG;
     if ((((uintptr_t)state | (uintptr_t)obs_out | (uintptr_t)obs_out2 | (uintptr_t)opp_obs_out) & 15) ||
@@ -1087,13 +1154,55 @@ int ss_env_step_pool(void *state, int64_t n_envs, int64_t pool_envs, int n_oppon
     if (A.stats && ((uintptr_t)status & 7)) return SS_ERR_INVALID_ARG;
     A.P.seed = seed; A.P.counter = counter; A.P.tick_limit = tick_limit; A.P.reward_mode = reward_mode; A.P.auto_reset = 1;
     A.P.reset_mode = reset_mode; A.n_ticks = 1;
+    const dim3 grid(blocks_for(2 * n_envs, kBlockPP));
+    if (blocks) {
+        B.opp_actions = (const float2 *)opp_actions; B.opp_obs = (float4 *)opp_obs_out; B.pool_stats = (unsigned long long *)pool_stats;
+        if ((A.stats ? sslaunch::launch(step_pp_obs_kernel<true, BlockPoolRows>, grid, dim3(kBlockPP), 0, (cudaStream_t)stream, A, B)
+                     : sslaunch::launch(step_pp_obs_kernel<false, BlockPoolRows>, grid, dim3(kBlockPP), 0, (cudaStream_t)stream, A, B)) !=
+            cudaSuccess)
+            return SS_ERR_CUDA;
+        return SS_OK;
+    }
     PoolRows R{n_envs - pool_envs, pool_envs > 0 ? pool_envs / n_opponents : 2, (const float2 *)opp_actions, (float4 *)opp_obs_out,
                pool_envs > 0 ? (unsigned long long *)pool_stats : nullptr};
-    const dim3 grid(blocks_for(2 * n_envs, kBlockPP));
     if ((A.stats ? sslaunch::launch(step_pp_obs_kernel<true, PoolRows>, grid, dim3(kBlockPP), 0, (cudaStream_t)stream, A, R)
                  : sslaunch::launch(step_pp_obs_kernel<false, PoolRows>, grid, dim3(kBlockPP), 0, (cudaStream_t)stream, A, R)) != cudaSuccess)
         return SS_ERR_CUDA;
     return SS_OK;
+}
+
+int ss_env_step_pool(void *state, int64_t n_envs, int64_t pool_envs, int n_opponents, const float *actions,
+                     const float *opp_actions, float *obs_out, float *obs_out2, float *reward_out, uint8_t *done_rows_out,
+                     float *opp_obs_out, uint8_t *done_out, uint8_t *winner_out, int reward_mode, int64_t tick_limit,
+                     int reset_mode, uint64_t seed, uint64_t counter, uint32_t *status, int flags, uint64_t *pool_stats,
+                     void *stream) {
+    return step_pool(state, n_envs, pool_envs, n_opponents, actions, opp_actions, obs_out, obs_out2, reward_out, done_rows_out,
+                     opp_obs_out, done_out, winner_out, reward_mode, tick_limit, reset_mode, seed, counter, status, flags, pool_stats,
+                     false, nullptr, stream);
+}
+
+int ss_env_step_pool_blocks(void *state, int64_t n_envs, int64_t pool_envs, int n_opponents, const float *actions,
+                            const float *opp_actions, float *obs_out, float *obs_out2, float *reward_out, uint8_t *done_rows_out,
+                            float *opp_obs_out, uint8_t *done_out, uint8_t *winner_out, int reward_mode, int64_t tick_limit,
+                            int reset_mode, uint64_t seed, uint64_t counter, uint32_t *status, int flags, uint64_t *pool_stats,
+                            const int64_t *opp_envs, void *stream) {
+    return step_pool(state, n_envs, pool_envs, n_opponents, actions, opp_actions, obs_out, obs_out2, reward_out, done_rows_out,
+                     opp_obs_out, done_out, winner_out, reward_mode, tick_limit, reset_mode, seed, counter, status, flags, pool_stats,
+                     true, opp_envs, stream);
+}
+
+int ss_pool_restart(void *state, int64_t n_envs, int64_t pool_envs, int n_opponents, const int64_t *opp_envs, int reset_mode,
+                    uint64_t seed, uint64_t counter, float *obs, float *opp_obs, uint32_t *status, void *stream) {
+    (void)status;          // a restart ends no game: nothing is counted or flagged
+    if (!state || !obs || !opp_obs || n_envs <= 0 || pool_envs <= 0 || pool_envs > n_envs) return SS_ERR_INVALID_ARG;
+    if (reset_mode != SS_RESET_FIXED && reset_mode != SS_RESET_RANDOM) return SS_ERR_INVALID_ARG;
+    if (((uintptr_t)state | (uintptr_t)obs | (uintptr_t)opp_obs) & 15) return SS_ERR_INVALID_ARG;
+    BlockPoolRows B{};
+    if (!pool_block_table(n_envs, pool_envs, n_opponents, opp_envs, B)) return SS_ERR_INVALID_ARG;
+    B.opp_obs = (float4 *)opp_obs;
+    pool_restart_kernel<<<blocks_for(2 * pool_envs, kBlockPP), kBlockPP, 0, (cudaStream_t)stream>>>(state, n_envs, (float4 *)obs,
+                                                                                                  reset_mode, seed, counter, B);
+    return check_launch();
 }
 
 int ss_env_step_tiles(void *state, int64_t n_envs, const float *actions, float *obs_out, float *obs_out2,

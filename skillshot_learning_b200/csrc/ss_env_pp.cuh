@@ -128,6 +128,24 @@ __device__ __forceinline__ void count_episode_pp(unsigned long long *stats, int 
     atomicAdd(stats + 8 + min(63, len / width), 1ull);
 }
 
+// game_reset (SkillshotGame.py:168-169) of this lane's player: the start state, and in (ox, oy) the partner's start
+// position.  SS_RESET_RANDOM draws from Philox4x32-10(key = seed, counter = (env, tick_counter)), as ss_env_reset does.
+// The same statements as the auto-reset in lane_obs_tick below, which keeps its own copy: calling this helper there moves
+// the register allocation of the kernels that inline it.
+__device__ __forceinline__ void lane_reset(LaneState &L, int P, uint64_t env, uint64_t tick_counter, int reset_mode, uint64_t seed,
+                                           int &ox, int &oy) {
+    int x = P ? 200 : 50, y = x;
+    ox = P ? 50 : 200; oy = ox;
+    if (reset_mode == SS_RESET_RANDOM) {
+        const U4 u = philox4x32_10(U4{(uint32_t)env, (uint32_t)(env >> 32), (uint32_t)tick_counter, (uint32_t)(tick_counter >> 32)},
+                                   (uint32_t)seed, (uint32_t)(seed >> 32));
+        x = rand_coord(P ? u.z : u.x); y = rand_coord(P ? u.w : u.y);
+        ox = rand_coord(P ? u.x : u.z); oy = rand_coord(P ? u.y : u.w);
+    }
+    L.px = x; L.py = y; L.rot = 0.0; L.qx = 0; L.qy = 0; L.qrot = 0.0; L.cd = 0; L.age = 0; L.valid = 0;
+    L.ticks = 0; L.live = 1; L.winner = 0;
+}
+
 struct LaneTickOut {
     float4 obs[3];          // the observation the actor sees next (post-reset if the game restarted)
     float reward;           // of the post-tick state

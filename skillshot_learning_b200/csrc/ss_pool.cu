@@ -10,6 +10,7 @@
 
 #include "../../include/skillshot_b200.h"
 #include "ss_launch.cuh"
+#include "ss_pool_blocks.cuh"
 
 namespace {
 
@@ -22,12 +23,22 @@ bool learner_noisy(const Args &R) { return R.frames > 1 && R.param_noise_sd > 0.
 int64_t noisy_stride(const Args &R) { return (ss_actor_frames_params(R.frames) + 3) / 4 * 4; }
 int64_t noise_groups(const Args &R, int64_t L) { return (L + R.noise_group - 1) / R.noise_group; }
 
+// the block starts B_0 .. B_K of opponent k's pool envs (and so of its rows); false: an invalid layout or block table
+// (a table also needs M < 2^31, the step's 32-bit table).  M = 0 takes no table.
+bool block_starts(const Args &R, int64_t *start) {
+    const int64_t M = R.pool_envs;
+    if (M == 0) return !R.opp_envs;
+    if (R.opp_envs && M > 0x7fffffff) return false;
+    return sspool::block_starts(M, R.n_opponents, R.opp_envs, start);
+}
+
 // -1: the layout, frame counts or noise settings are invalid; else the workspace bytes: the learner's noisy vectors, then
 // the frame-stacked tensor-core forward's layer-1 tiles for the largest of its calls (they run one after the other)
 int64_t workspace_bytes(const Args &R) {
     const int64_t n = R.n_envs, M = R.pool_envs, K = R.n_opponents;
     if (n <= 0 || M < 0 || M > n || R.frames < 1 || R.frames > SS_MAX_FRAMES) return -1;
-    if (M > 0 && (K < 1 || K > SS_LEAGUE_MAX_POLICIES || M % (2 * K) != 0)) return -1;
+    int64_t start[SS_LEAGUE_MAX_POLICIES + 1];
+    if (!block_starts(R, start)) return -1;
     if (R.param_noise_sd > 0.f && (R.noise_group <= 0 || (R.tensor_cores && R.noise_group % 128 != 0))) return -1;
     for (int k = 0; k < K && M > 0; ++k)
         if (opp_frames(R, k) < 1 || opp_frames(R, k) > SS_MAX_FRAMES) return -1;
@@ -41,7 +52,7 @@ int64_t workspace_bytes(const Args &R) {
     if (R.frames > 1) tiles = ss_actor_frames_tc_workspace_bytes(L, learner_noisy(R) ? R.noise_group : 0);
     for (int k = 0; k < K && M > 0; ++k) {
         if (opp_frames(R, k) == 1) continue;
-        const int64_t b = ss_actor_frames_tc_workspace_bytes(M / K, 0);
+        const int64_t b = ss_actor_frames_tc_workspace_bytes(start[k + 1] - start[k], 0);
         if (b > tiles) tiles = b;
     }
     return noisy + tiles;
@@ -52,9 +63,11 @@ int rollout(const Args &R, void *stream) {
     if (!R.state || !R.params || !R.obs || !R.act || !R.reward || !R.done || !R.winner || n <= 0 || R.n_ticks <= 0)
         return SS_ERR_INVALID_ARG;
     if (M < 0 || M > n) return SS_ERR_INVALID_ARG;
+    int64_t start[SS_LEAGUE_MAX_POLICIES + 1];
+    if (!block_starts(R, start)) return SS_ERR_INVALID_ARG;
     if (R.frames < 1 || R.frames > SS_MAX_FRAMES || R.head < 0) return SS_ERR_INVALID_ARG;
     if (M > 0) {
-        if (K < 1 || K > SS_LEAGUE_MAX_POLICIES || M % (2 * K) != 0 || !R.opp_params || !R.opp_obs || !R.opp_act) return SS_ERR_INVALID_ARG;
+        if (!R.opp_params || !R.opp_obs || !R.opp_act) return SS_ERR_INVALID_ARG;
         if ((R.opp_param_stride & 3) || R.opp_param_stride < 0) return SS_ERR_INVALID_ARG;
         for (int k = 0; k < K; ++k) {
             const int f = opp_frames(R, k);
@@ -82,7 +95,7 @@ int rollout(const Args &R, void *stream) {
     const int64_t need = workspace_bytes(R);
     if (need < 0) return SS_ERR_INVALID_ARG;
     if (need > 0 && (!R.workspace || R.workspace_bytes < need || ((uintptr_t)R.workspace & 15))) return SS_ERR_INVALID_ARG;
-    const int64_t S = n - M, L = 2 * S + M, b = M > 0 ? M / K : 0, w = 12 * (int64_t)F;
+    const int64_t S = n - M, L = 2 * S + M, w = 12 * (int64_t)F;
     const bool ring = R.ring_obs != nullptr;
     // the transitions are produced in place (see ss_selfplay_rollout: one segment of L rows per tick, and with a single
     // segment the second observation copy would overwrite the rows the actor has just read)
@@ -97,7 +110,7 @@ int rollout(const Args &R, void *stream) {
                     cudaSuccess)
         return SS_ERR_CUDA;
     int64_t seg_rows[SS_LEAGUE_MAX_POLICIES];
-    for (int k = 0; k < K && M > 0; ++k) seg_rows[k] = b;
+    for (int k = 0; k < K && M > 0; ++k) seg_rows[k] = start[k + 1] - start[k];
     float *noisy = (float *)R.workspace;
     void *tiles = learner_noisy(R) ? (void *)(noisy + noise_groups(R, L) * noisy_stride(R)) : R.workspace;
     const int64_t tile_bytes = need - (learner_noisy(R) ? noise_groups(R, L) * noisy_stride(R) * 4 : 0);
@@ -138,7 +151,8 @@ int rollout(const Args &R, void *stream) {
         if (rc != SS_OK) return rc;
         sslaunch::pdl_mode() = kEarly;
         for (int k = 0; k < K && M > 0 && rc == SS_OK;) {
-            float *oo = R.opp_obs + k * b * 12, *oa = R.opp_act + k * b * 2;
+            const int64_t b = seg_rows[k];
+            float *oo = R.opp_obs + start[k] * 12, *oa = R.opp_act + start[k] * 2;
             const int f = opp_frames(R, k);
             if (f > 1) {
                 rc = R.tensor_cores ? ss_actor_forward_frames_tc(opp_prm(k), 0, 0, R.opp_stacks[k], f, head, oa, b, tiles, tile_bytes, stream)
@@ -157,10 +171,14 @@ int rollout(const Args &R, void *stream) {
         if (rc != SS_OK) return rc;
         sslaunch::pdl_mode() = kOn;
         float *step_obs = F > 1 ? R.obs : ring ? R.ring_next_obs + seg * L * 12 : R.obs;
-        rc = ss_env_step_pool(R.state, n, M, (int)K, a, R.opp_act, step_obs, ring && F == 1 ? o_next : nullptr,
-                              ring ? R.ring_reward + seg * L : R.reward, ring ? R.ring_done + seg * L : nullptr, R.opp_obs, R.done,
-                              R.winner, R.reward_mode, R.tick_limit, R.reset_mode, R.env_seed, R.env_counter + (uint64_t)t, R.status,
-                              R.step_flags, R.pool_stats, stream);
+        rc = R.opp_envs ? ss_env_step_pool_blocks(R.state, n, M, (int)K, a, R.opp_act, step_obs, ring && F == 1 ? o_next : nullptr,
+                                                  ring ? R.ring_reward + seg * L : R.reward, ring ? R.ring_done + seg * L : nullptr,
+                                                  R.opp_obs, R.done, R.winner, R.reward_mode, R.tick_limit, R.reset_mode, R.env_seed,
+                                                  R.env_counter + (uint64_t)t, R.status, R.step_flags, R.pool_stats, R.opp_envs, stream)
+                        : ss_env_step_pool(R.state, n, M, (int)K, a, R.opp_act, step_obs, ring && F == 1 ? o_next : nullptr,
+                                           ring ? R.ring_reward + seg * L : R.reward, ring ? R.ring_done + seg * L : nullptr, R.opp_obs,
+                                           R.done, R.winner, R.reward_mode, R.tick_limit, R.reset_mode, R.env_seed,
+                                           R.env_counter + (uint64_t)t, R.status, R.step_flags, R.pool_stats, stream);
         if (rc != SS_OK) return rc;
         if (F > 1) {
             float *r1 = ring ? R.ring_next_obs + seg * L * w : R.rows, *r2 = !ring ? nullptr : !last ? R.ring_obs + nseg * L * w : R.rows;
@@ -170,10 +188,10 @@ int rollout(const Args &R, void *stream) {
         for (int k = 0; k < K && M > 0 && rc == SS_OK; ++k) {
             const int f = opp_frames(R, k);
             if (f == 1) continue;
-            const uint8_t *dk = R.done + S + k * b;
-            float *oo = R.opp_obs + k * b * 12;
-            rc = R.tensor_cores ? ss_obs_stack_push_tc(R.opp_stacks[k], b, f, head + 1, oo, dk, 1, stream)
-                                : ss_obs_stack_push((float *)R.opp_stacks[k], b, f, head + 1, oo, dk, 1, stream);
+            const uint8_t *dk = R.done + S + start[k];
+            float *oo = R.opp_obs + start[k] * 12;
+            rc = R.tensor_cores ? ss_obs_stack_push_tc(R.opp_stacks[k], seg_rows[k], f, head + 1, oo, dk, 1, stream)
+                                : ss_obs_stack_push((float *)R.opp_stacks[k], seg_rows[k], f, head + 1, oo, dk, 1, stream);
         }
         if (rc != SS_OK) return rc;
     }

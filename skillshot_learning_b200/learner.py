@@ -17,6 +17,7 @@ include/skillshot_b200.h); there is no CPU path.
 from __future__ import annotations
 
 import ctypes
+import math
 import os
 from typing import Optional
 
@@ -1072,23 +1073,72 @@ class FrameStackActor:
 POOL_STRIDE = (A_N + 3) // 4 * 4          # floats between two opponent vectors (16-byte aligned)
 
 
-def pool_layout(n_envs: int, pool_envs: int, n_opponents: int) -> np.ndarray:
+def check_pool_blocks(blocks, pool_envs: int, n_opponents: int) -> list:
+    """The block table as a list of ints: one even size >= 2 per opponent, summing to pool_envs; else ValueError."""
+    out = [int(b) for b in blocks]
+    if len(out) != int(n_opponents) or any(b < 2 or b % 2 for b in out) or sum(out) != int(pool_envs):
+        raise ValueError("pool blocks must be %d even sizes >= 2 summing to %d, got %s" % (int(n_opponents), int(pool_envs), out))
+    return out
+
+
+def pool_layout(n_envs: int, pool_envs: int, n_opponents: int, blocks=None) -> np.ndarray:
     """int64 [n_envs, 2]: the row of each (env, player) when the last pool_envs envs are played against n_opponents frozen
     actors (include/skillshot_b200.h, "training against a pool").  Rows [0, L) are the learner's, L = 2 S + M with
-    S = n_envs - M; rows L + r are opponent row r.  Self-play env i keeps rows 2i + p; opponent k owns the b = M / K pool
-    envs from S + k b, the learner being player 1 in the first b / 2 of them."""
+    S = n_envs - M; rows L + r are opponent row r.  Self-play env i keeps rows 2i + p; opponent k owns the b_k pool envs
+    from S + B_k, B_k = b_0 + ... + b_{k-1}, the learner being player 1 in the first b_k / 2 of them.  blocks: the b_k
+    (check_pool_blocks); None: M / K each."""
     n, M = int(n_envs), int(pool_envs)
     S = n - M
     rows = np.empty((n, 2), np.int64)
     rows[:S] = np.arange(2 * S).reshape(S, 2)
     if M:
-        b = M // int(n_opponents)
+        K = int(n_opponents)
         j = np.arange(M)
-        lp = (j % b >= b // 2).astype(np.int64)          # the learner's player in pool env S + j
+        if blocks is None:
+            b = M // K
+            lp = (j % b >= b // 2).astype(np.int64)          # the learner's player in pool env S + j
+        else:
+            sizes = np.array(check_pool_blocks(blocks, M, K), np.int64)
+            starts = np.concatenate([[0], np.cumsum(sizes)])
+            k = np.searchsorted(starts, j, side="right") - 1
+            lp = (j - starts[k] >= sizes[k] // 2).astype(np.int64)
         L = 2 * S + M
         rows[S + j, lp] = 2 * S + j
         rows[S + j, 1 - lp] = L + j
     return rows
+
+
+PFSP_WEIGHTINGS = ("hard", "variance", "uniform")
+
+
+def pfsp_blocks(scores, pool_envs: int, weighting: str = "hard", p: float = 2.0, min_envs: int = 2) -> list:
+    """Prioritized fictitious self-play: the pool envs per opponent from the learner's score against each (1 win, 0.5 draw,
+    0 loss; None or NaN for an opponent without finished games counts as 0.5).  Every opponent gets min_envs (even, >= 2);
+    the rest is split in units of 2 envs in proportion to the weights -- "hard" (1 - s)^p, where play goes to the opponents
+    the learner still loses to, "variance" s (1 - s), where it goes to the even matches, or "uniform" -- by largest
+    remainder, ties to the lower k.  All weights 0 gives the uniform split.  Returns a list of ints summing to pool_envs."""
+    if weighting not in PFSP_WEIGHTINGS:
+        raise ValueError("weighting must be one of %s, got %r" % (PFSP_WEIGHTINGS, weighting))
+    s = np.array([0.5 if v is None or math.isnan(float(v)) else float(v) for v in scores], np.float64)
+    K, M, m, p = len(s), int(pool_envs), int(min_envs), float(p)
+    if not 1 <= K <= _lib.LEAGUE_MAX_POLICIES:
+        raise ValueError("1..%d scores, got %d" % (_lib.LEAGUE_MAX_POLICIES, K))
+    if ((s < 0) | (s > 1)).any():
+        raise ValueError("scores must lie in [0, 1]")
+    if m < 2 or m % 2 or M % 2 or M < K * m:
+        raise ValueError("pool_envs (%d) must be even and at least %d opponents x min_envs (%d, even, >= 2)" % (M, K, m))
+    if not math.isfinite(p) or p < 0:
+        raise ValueError("p must be finite and >= 0, got %r" % p)
+    w = (1.0 - s) ** p if weighting == "hard" else s * (1.0 - s) if weighting == "variance" else np.ones(K)
+    if w.sum() <= 0:
+        w = np.ones(K)
+    units = (M - K * m) // 2
+    quota = units * w / w.sum()
+    share = np.floor(quota).astype(np.int64)
+    order = sorted(range(K), key=lambda k: (-(quota[k] - share[k]), k))
+    for k in order[:units - int(share.sum())]:
+        share[k] += 1
+    return [m + 2 * int(u) for u in share]
 
 
 class SelfPlayTrainer:
@@ -1102,7 +1152,8 @@ class SelfPlayTrainer:
                  batch_size: int = 4096, gamma: float = 0.0, tau: float = 1.0, param_noise_sd: float = 0.5,
                  noise_group: int = 128, reward_mode: str = "looking", tick_limit: int = 2000,
                  random_positions: bool = True, process_group=None, precision: str = "f32", collective: str = "nccl",
-                 frames: int = 1, update_precision: Optional[str] = None, opponents=None, pool_envs: Optional[int] = None):
+                 frames: int = 1, update_precision: Optional[str] = None, opponents=None, pool_envs: Optional[int] = None,
+                 pool_blocks=None):
         """frames > 1: the frame-stacked "planning" networks (readme.md:18-20, BASELINE.json configs[4]): both players act
         from their last `frames` observations (FrameStackActor; `precision` selects its float32 or tensor-core kernels),
         the replay ring stores the stacked observations, and the critic / actor update of SkillshotLearner.py:386-443 runs
@@ -1113,7 +1164,9 @@ class SelfPlayTrainer:
         copied here, at most 64): the last pool_envs envs (default: half of them, rounded down to a multiple of
         2 * len(opponents)) are the learner against opponent k in block k of pool_envs / len(opponents) envs, seat-balanced
         (pool_layout).  The opponents act without noise and only the learner's transitions are stored; an opponent with
-        more than one frame keeps a history of its rows.  See set_opponent / pool_progress."""
+        more than one frame keeps a history of its rows.  See set_opponent / pool_progress.
+        pool_blocks: the pool envs of each opponent (even sizes >= 2 summing to pool_envs, pool_layout) instead of
+        pool_envs / len(opponents) each; see set_pool_blocks / rebalance_pool."""
         self.device = torch.device(device)
         self.frames = int(frames)
         self.opponents, self.pool_envs, self.pool_stats = None, 0, None
@@ -1133,6 +1186,8 @@ class SelfPlayTrainer:
             opp_vecs = [actor_vector(a) for a in opponents]
             self.opp_frames = [f for _, f in opp_vecs]
             self.pool_envs = M
+            # None: M / K envs per opponent, the step of ss_pool_rollout (no block table is passed)
+            self._blocks = None if pool_blocks is None else check_pool_blocks(pool_blocks, M, K)
         self.learner_rows = 2 * int(n_envs) - self.pool_envs       # rows of the learner's transitions per tick
         L = self.learner_rows
         if replay_capacity is not None and opponents is not None and (replay_capacity % L or replay_capacity < 2 * L):
@@ -1163,30 +1218,17 @@ class SelfPlayTrainer:
                 self.opponents[k, :v.size] = torch.from_numpy(v).to(self.device)
             self.pool_stats = torch.zeros((K, _lib.POOL_STATS), dtype=torch.int64, device=self.device)
             # rows [0, L) the learner's, [L, 2n) the opponents' (pool_layout): observations and actions
-            rows = torch.from_numpy(pool_layout(n, self.pool_envs, len(self.opponents)).reshape(-1)).to(self.device)
+            rows = torch.from_numpy(pool_layout(n, self.pool_envs, len(self.opponents), self._blocks).reshape(-1)).to(self.device)
             self.obs = torch.empty((2 * n, 12), dtype=torch.float32, device=self.device)
             self.obs[rows] = self.envs.observe().reshape(-1, 12)
             self.prev_obs = None
             self.actions = torch.empty((2 * n, 2), dtype=torch.float32, device=self.device)
             self._pool_reward = torch.zeros(L, dtype=torch.float32, device=self.device)
             self._pool_ws = None
-            # the histories of the opponents with frames > 1, b rows each, filled with the first observation (slot 0);
+            # the histories of the opponents with frames > 1, b_k rows each, filled with the first observation (slot 0);
             # every history of the pool shares one slot counter
-            self.opp_stacks, self._pool_head = [None] * len(self.opponents), 0      # (see pool_head)
-            b = self.pool_envs // len(self.opponents)
-            for k, f in enumerate(self.opp_frames):
-                if f == 1 or b == 0:
-                    continue
-                if precision == "bf16":
-                    s = torch.zeros(int(lib.ss_obs_stack_tc_bytes(b, f)), dtype=torch.uint8, device=self.device)
-                else:
-                    s = torch.zeros((b, f, 12), dtype=torch.float32, device=self.device)
-                fn = lib.ss_obs_stack_push_tc if precision == "bf16" else lib.ss_obs_stack_push
-                ones = torch.ones(b, dtype=torch.uint8, device=self.device)
-                with torch.cuda.device(self.device):
-                    check(fn(s.data_ptr(), b, f, 0, self.obs[L + k * b:].data_ptr(), ones.data_ptr(), 1, _stream(self.device)),
-                          "ss_obs_stack_push")
-                self.opp_stacks[k] = s
+            self._pool_head = 0      # (see pool_head)
+            self._alloc_opp_stacks(0)
         self.stack = None
         if self.frames > 1:
             # the acting network IS the learner's actor vector; the history lives in the FrameStackActor (its L rows)
@@ -1208,6 +1250,72 @@ class SelfPlayTrainer:
         """The slot counter of the newest frame shared by every history of the pool: the learner's FrameStackActor's when it
         reads more than one frame, else the trainer's own (then only the opponents' histories use it)."""
         return self.stack.head if self.stack is not None else self._pool_head
+
+    @property
+    def pool_blocks(self) -> list:
+        """The pool envs of each opponent (pool_layout's blocks)."""
+        if self.opponents is None:
+            raise ValueError("this trainer has no opponent pool")
+        K = len(self.opponents)
+        return list(self._blocks) if self._blocks is not None else [self.pool_envs // K] * K
+
+    def _alloc_opp_stacks(self, head: int, fill: bool = True):
+        """A history of b_k rows for each opponent with frames > 1, every slot filled with its rows' current observation
+        (fill) or zero (to be loaded)."""
+        L, bf16 = self.learner_rows, self.precision == "bf16"
+        self.opp_stacks = [None] * len(self.opponents)
+        start = 0
+        for k, (f, b) in enumerate(zip(self.opp_frames, self.pool_blocks)):
+            if f > 1 and b > 0:
+                s = (torch.zeros(int(lib.ss_obs_stack_tc_bytes(b, f)), dtype=torch.uint8, device=self.device) if bf16 else
+                     torch.zeros((b, f, 12), dtype=torch.float32, device=self.device))
+                if fill:
+                    fn = lib.ss_obs_stack_push_tc if bf16 else lib.ss_obs_stack_push
+                    ones = torch.ones(b, dtype=torch.uint8, device=self.device)
+                    with torch.cuda.device(self.device):
+                        check(fn(s.data_ptr(), b, f, int(head), self.obs[L + start:].data_ptr(), ones.data_ptr(), 1, _stream(self.device)),
+                              "ss_obs_stack_push")
+                self.opp_stacks[k] = s
+            start += b
+
+    def set_pool_blocks(self, blocks):
+        """Lay the pool out again with blocks[k] envs for opponent k (even, >= 2, summing to pool_envs), between rollouts.
+        Every pool game restarts (ss_pool_restart, Philox counter envs.counter, which then advances by one tick): moving an
+        env between blocks can flip the learner's seat, and an opponent's history is indexed by the env's offset in its
+        block.  The self-play envs, rows and histories are untouched.  The last stored transition of a restarted game keeps
+        its next observation and a 0 done flag, as a tick-limit ending does; nothing is counted in pool_stats or the
+        episode statistics."""
+        if self.opponents is None:
+            raise ValueError("this trainer has no opponent pool")
+        n, M, K, L = self.envs.n_envs, self.pool_envs, len(self.opponents), self.learner_rows
+        blocks = check_pool_blocks(blocks, M, K)
+        envs = self.envs
+        table = (ctypes.c_int64 * K)(*blocks)
+        with torch.cuda.device(self.device):
+            check(lib.ss_pool_restart(envs.state.data_ptr(), n, M, K, table,
+                                      _lib.RESET_RANDOM if envs.random_positions else _lib.RESET_FIXED, envs.seed, envs.counter,
+                                      self.obs.data_ptr(), self.obs[L:].data_ptr(), envs.status.data_ptr(), _stream(self.device)),
+                  "ss_pool_restart")
+            envs.counter += 1
+            st = self.stack
+            if st is not None:
+                # the learner's pool rows restart their histories; the self-play rows push their newest observation again
+                done = torch.zeros(n, dtype=torch.uint8, device=self.device)
+                done[n - M:] = 1
+                check(lib.ss_obs_stack_push_pool(st.stack.data_ptr() if st.precision == "bf16" else None,
+                                                 (st.stack32 if st.precision == "bf16" else st.stack).data_ptr(), n, M, self.frames,
+                                                 st.head, self.obs.data_ptr(), done.data_ptr(), self.rows.data_ptr(), None,
+                                                 _stream(self.device)), "ss_obs_stack_push_pool")
+        self._blocks = blocks
+        self._alloc_opp_stacks(self.pool_head)
+
+    def rebalance_pool(self, weighting: str = "hard", p: float = 2.0, min_envs: int = 2, reset: bool = True) -> list:
+        """Size each opponent's block by the learner's score against it: pool_progress(reset), pfsp_blocks of the scores
+        (an opponent without finished games counts as 0.5), set_pool_blocks.  Returns the new blocks."""
+        prog = self.pool_progress(reset)
+        blocks = pfsp_blocks([q["score"] if q["episodes"] else None for q in prog], self.pool_envs, weighting, p, min_envs)
+        self.set_pool_blocks(blocks)
+        return blocks
 
     def set_opponent(self, k: int, actor):
         """Replace opponent k of the pool with a copy of `actor` from the next tick on (the games in flight continue against
@@ -1278,6 +1386,8 @@ class SelfPlayTrainer:
         frames = (ctypes.c_int * K)(*self.opp_frames)
         stacks = (ctypes.c_void_p * K)(*[None if s is None else s.data_ptr() for s in self.opp_stacks])
         a.opp_frames, a.opp_stacks = frames, stacks
+        table = None if self._blocks is None else (ctypes.c_int64 * K)(*self._blocks)
+        a.opp_envs = table
         need = int(lib.ss_pool_rollout_frames_workspace_bytes(ctypes.byref(a)))
         if need > 0 and (self._pool_ws is None or self._pool_ws.numel() < need):
             self._pool_ws = torch.empty(need, dtype=torch.uint8, device=self.device)
@@ -1398,7 +1508,7 @@ class SelfPlayTrainer:
         if self.opponents is not None:
             sd["pool"] = dict(opponents=self.opponents.cpu(), pool_envs=self.pool_envs, stats=self.pool_stats.cpu(),
                               frames=list(self.opp_frames), stacks=[None if s is None else s.cpu() for s in self.opp_stacks],
-                              head=self.pool_head)
+                              head=self.pool_head, blocks=None if self._blocks is None else list(self._blocks))
         return sd
 
     def load_state_dict(self, sd):
@@ -1428,6 +1538,10 @@ class SelfPlayTrainer:
             st.seed = int(ss.get("seed", st.seed))       # (absent from older checkpoints: this trainer's seed)
             self.rows.copy_(ss["rows"].to(self.device))
         if pool is not None:
+            # the blocks are run state: adopt the checkpoint's (absent: M / K each), with histories of its sizes
+            blocks = pool.get("blocks")
+            self._blocks = None if blocks is None else check_pool_blocks(blocks, self.pool_envs, len(self.opponents))
+            self._alloc_opp_stacks(0, fill=False)
             self.opponents.copy_(pool["opponents"].to(self.device))
             self.pool_stats.copy_(pool["stats"].to(self.device))
             for s, saved in zip(self.opp_stacks, pool.get("stacks", [None] * len(self.opp_stacks))):
