@@ -617,7 +617,7 @@ int ss_league_play(const ss_league_args *args, void *stream);
  * the L rows from write_pos + t L (mod capacity).  capacity and write_pos must be multiples of L, with capacity >= 2 L or
  * n_ticks == 1.  Without a ring the learner's rows are rewritten in obs / act / reward.  The opponents' transitions are not
  * stored.  Every argument is checked before anything is enqueued: besides the rules of ss_env_step_pool, speeds must be
- * NULL (per-env speeds and reward simple run on the per-env step kernel), K <= SS_LEAGUE_MAX_POLICIES and pointers aligned
+ * NULL (per-env speeds: ss_pool_rollout_speeds below), K <= SS_LEAGUE_MAX_POLICIES and pointers aligned
  * as ss_selfplay_rollout's.  M = 0 gives ss_selfplay_rollout's results bit for bit. */
 #define SS_POOL_STATS 8        /* uint64 counters per opponent in pool_stats */
 int ss_env_step_pool(void *state, int64_t n_envs, int64_t pool_envs, int n_opponents, const float *actions,
@@ -645,6 +645,17 @@ int ss_env_step_pool_blocks(void *state, int64_t n_envs, int64_t pool_envs, int 
                             const int64_t *opp_envs, void *stream);
 int ss_pool_restart(void *state, int64_t n_envs, int64_t pool_envs, int n_opponents, const int64_t *opp_envs, int reset_mode,
                     uint64_t seed, uint64_t counter, float *obs, float *opp_obs, uint32_t *status, void *stream);
+/* Per-env speeds: ss_env_step_pool_blocks with the per-env constants of ss_env_step (`speeds`, required: not NULL, 16-byte
+ * aligned, two 16-byte planes of n_envs entries, SkillshotEnvs.set_speeds).  Every other rule is ss_env_step_pool_blocks'
+ * (opp_envs NULL: M / K each; reward none / looking / terminal).  Env i plays with the speeds of entry i whichever block
+ * it is in, and its bytes are those of ss_env_step_ring with the same speeds under the layout's rows.  Without per-env
+ * speeds the step is ss_env_step_pool / ss_env_step_pool_blocks.  ss_pool_restart serves both: a new game has cooldown 0,
+ * so its observation does not depend on the speeds, and no start draw reads them. */
+int ss_env_step_pool_speeds(void *state, int64_t n_envs, int64_t pool_envs, int n_opponents, const float *actions,
+                            const float *opp_actions, float *obs_out, float *obs_out2, float *reward_out, uint8_t *done_rows_out,
+                            float *opp_obs_out, uint8_t *done_out, uint8_t *winner_out, int reward_mode, int64_t tick_limit,
+                            int reset_mode, uint64_t seed, uint64_t counter, uint32_t *status, int flags, uint64_t *pool_stats,
+                            const int64_t *opp_envs, const void *speeds, void *stream);
 typedef struct ss_pool_rollout_args {
     void *state;
     int64_t n_envs, pool_envs;
@@ -666,7 +677,7 @@ typedef struct ss_pool_rollout_args {
     int64_t tick_limit;
     int reset_mode;
     uint64_t env_seed, env_counter, noise_seed, noise_counter;
-    const void *speeds;                        /* must be NULL */
+    const void *speeds;                        /* must be NULL (per-env speeds: ss_pool_rollout_speeds) */
     uint32_t *status;                          /* NULL or the status block of ss_env_step */
     int step_flags;                            /* SS_STEP_EPISODE_STATS or 0 */
     uint64_t *pool_stats;                      /* NULL or uint64 [K][SS_POOL_STATS], added to */
@@ -709,7 +720,11 @@ int ss_pool_rollout(const ss_pool_rollout_args *args, void *stream);
  *                       -1 when they are invalid.
  *   opp_envs [K]        HOST block table of ss_env_step_pool_blocks (it also reads this); NULL: M / K each, launch for launch
  *                       the rollout above.  With a table, opponent k's forward, history and workspace use its b_k rows from
- *                       B_k, and the step is ss_env_step_pool_blocks. */
+ *                       B_k, and the step is ss_env_step_pool_blocks.
+ *
+ * ss_pool_rollout_speeds: ss_pool_rollout_frames with per-env speeds -- args->speeds (required, the layout of ss_env_step)
+ * -- and the env step ss_env_step_pool_speeds in place of ss_env_step_pool / ss_env_step_pool_blocks.  Every other launch,
+ * rule, ring layout and the workspace (ss_pool_rollout_frames_workspace_bytes) are ss_pool_rollout_frames'. */
 typedef struct ss_pool_rollout_frames_args {
     void *state;
     int64_t n_envs, pool_envs;
@@ -731,7 +746,7 @@ typedef struct ss_pool_rollout_frames_args {
     int64_t tick_limit;
     int reset_mode;
     uint64_t env_seed, env_counter, noise_seed, noise_counter;
-    const void *speeds;                        /* must be NULL */
+    const void *speeds;                        /* ss_pool_rollout_speeds: the per-env speeds; ss_pool_rollout_frames: NULL */
     uint32_t *status;
     int step_flags;
     uint64_t *pool_stats;
@@ -750,6 +765,7 @@ int ss_obs_stack_push_pool(void *stack_tc, float *stack32, int64_t n_envs, int64
                            const float *obs, const uint8_t *done, float *rows_out, float *rows_out2, void *stream);
 int64_t ss_pool_rollout_frames_workspace_bytes(const ss_pool_rollout_frames_args *args);
 int ss_pool_rollout_frames(const ss_pool_rollout_frames_args *args, void *stream);
+int ss_pool_rollout_speeds(const ss_pool_rollout_frames_args *args, void *stream);
 
 /* ---- multi-GPU: the gradient all-reduce fused with its neighbours over NVLink peer memory ----
  * One exchange allocation per rank = flags[2][world] | inbox[2][world][capacity floats], made by

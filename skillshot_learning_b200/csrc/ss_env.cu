@@ -969,6 +969,95 @@ __global__ void match_summary_kernel(const void *state, int64_t n, int64_t split
     if (threadIdx.x < SS_MATCH_STATS && acc[threadIdx.x]) atomicAdd(out + threadIdx.x, acc[threadIdx.x]);
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// pool_step_speeds_kernel -- ss_env_step_pool_speeds: one tick of the pool with per-env speeds, ONE THREAD PER ENV.  The
+// per-player kernels fold the reference constants into their arithmetic (ss_env_pp.cuh); per-env speeds run on the core's
+// tick_env, called as step_kernel<OBS, CARRY, SPEEDS> calls it, so the bytes of every env are ss_env_step_ring's.  The
+// rows are BlockPoolRows': self-play env i < S reads its float2 actions from learner rows 2i, 2i + 1; in pool env S + j
+// the learner's float2 is learner row 2S + j and the opponent's opponent row j, seated by the block's learner player.
+// The learner rows of the warp's envs are one contiguous run (env S - 1 ends at row 2S - 1, the pool's start at 2S), and
+// so are its opponent rows: learner row r takes tile slot r - l0 and opponent row o slot nl + o - o0.  Slot s is staged
+// at float4 3s + (s >> 1) of the warp's tile -- for a self-play warp that is step_kernel's conflict-free 7-float4 row per
+// env -- and the warp writes each run with coalesced stores, as step_pp_obs_kernel does.
+__device__ __forceinline__ int slot_at(int s) { return 3 * s + (s >> 1); }
+
+template <bool STATS>
+__global__ void __launch_bounds__(kBlock, 8) pool_step_speeds_kernel(const StepArgs A, const BlockPoolRows R) {
+    __shared__ float4 tile[kBlock / 32][32 * kRowF4];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t i = (int64_t)blockIdx.x * kBlock + threadIdx.x;
+    const int64_t e0 = i - lane, e1 = min(e0 + 32, A.n);           // the warp's envs
+    const bool active = i < A.n;
+    const StatePlanes S = planes_of(A.state, A.n);
+    // first learner row of env e (e = n gives L); an env past the self-play envs has one learner row
+    auto lrow = [&](int64_t e) { return e < R.S ? 2 * e : R.S + e; };
+    const int64_t l0 = lrow(e0), o0 = max(e0, R.S) - R.S;
+    const int nl = (int)(lrow(e1) - l0);
+    const bool pool = i >= R.S;
+    int learner_player = 0, block = 0;
+    if (active && pool) block = pool_block_of(R, (int)(i - R.S), learner_player);
+    // tile slots of player 1's and player 2's rows
+    const int ls = (int)(lrow(i) - l0), os = nl + (int)(i - R.S - o0);
+    const int s1 = !pool ? ls : learner_player == 0 ? ls : os;
+    const int s2 = !pool ? ls + 1 : learner_player == 1 ? ls : os;
+    // ss_launch.cuh: in the rollout loop this grid is placed while the forward kernels' last CTAs finish, and waits here
+    sslaunch::griddep_wait();
+    sslaunch::griddep_launch();
+    uint32_t status = 0;
+    if (active) {
+        Env e;
+        load_env(S, i, e);
+        const Speeds k = load_speeds(A.speeds, A.n, i);
+        const float2 *act = (const float2 *)A.actions;
+        float2 p1, p2;
+        if (!pool) {
+            p1 = __ldg(act + 2 * i); p2 = __ldg(act + 2 * i + 1);
+        } else {
+            const float2 la = __ldg(act + R.S + i), oa = __ldg(R.opp_actions + (i - R.S));
+            p1 = learner_player == 0 ? la : oa; p2 = learner_player == 0 ? oa : la;
+        }
+        // a game that is over before the tick stays "done" and is not an episode end again (step_kernel's STATS rule)
+        const int ticks_before = (!e.live || (A.P.tick_limit > 0 && e.ticks >= A.P.tick_limit)) ? -1 : e.ticks;
+        Trig tr;
+        trig_of(e, tr);
+        float r[2];
+        int done, winner;
+        SeatSink sink{&tile[warp][slot_at(s1)], &tile[warp][slot_at(s2)]};
+        tick_env<true, true>(e, p1.x, p1.y, p2.x, p2.y, k, A.P, (uint64_t)i, 0, true, status, tr, r, done, winner, sink);
+        store_env(S, i, e);
+        const bool write_reward = A.reward_out && A.P.reward_mode != SS_REWARD_NONE;
+        float *reward = (float *)A.reward_out;
+        uint8_t *done_rows = (uint8_t *)A.done_rows_out;
+        if (!pool) {
+            if (write_reward) { reward[2 * i] = r[0]; reward[2 * i + 1] = r[1]; }
+            if (done_rows) { done_rows[2 * i] = winner ? 1 : 0; done_rows[2 * i + 1] = winner ? 1 : 0; }
+        } else {
+            if (write_reward) reward[R.S + i] = r[learner_player];
+            if (done_rows) done_rows[R.S + i] = winner ? 1 : 0;
+        }
+        if (A.done_out) A.done_out[i] = (uint8_t)done;
+        if (A.winner_out) A.winner_out[i] = (uint8_t)winner;
+        if (done && ticks_before >= 0) {                                // rare: a few atomics per finished game
+            if (STATS) count_episode(A.stats, ticks_before + 1, winner, (int)A.P.tick_limit);
+            if (pool && R.pool_stats) count_pool_game(R.pool_stats + block * 8, ticks_before + 1, winner, learner_player);
+        }
+    }
+    __syncwarp();
+    const int n_out = 3 * (nl + (int)(max(e1, R.S) - R.S - o0));
+#pragma unroll
+    for (int j = 0; j < 6; ++j) {
+        const int idx = j * 32 + lane;
+        if (idx < 3 * nl) {
+            const float4 v = tile[warp][idx + (idx / 3 >> 1)];
+            A.obs_out[l0 * 3 + idx] = v;
+            if (A.obs_out2) A.obs_out2[l0 * 3 + idx] = v;
+        } else if (idx < n_out) {
+            R.opp_obs[o0 * 3 + (idx - 3 * nl)] = tile[warp][idx + (idx / 3 >> 1)];
+        }
+    }
+    if (status && A.status) atomicOr(A.status, status);
+}
+
 inline int check_launch() { return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA; }
 inline unsigned blocks_for(int64_t n, int block) { return (unsigned)((n + block - 1) / block); }
 // CTA size of step_pp_kernel for n_envs (see the kernel): 896 when that still makes at least ~one CTA per SM (65,536 envs
@@ -1129,12 +1218,13 @@ int ss_env_step_ring(void *state, int64_t n_envs, const float *actions, float *o
     return check_launch();
 }
 
-// ss_env_step_pool (blocks false: PoolRows) and ss_env_step_pool_blocks (blocks true: BlockPoolRows from opp_envs)
+// ss_env_step_pool (blocks false: PoolRows), ss_env_step_pool_blocks (blocks true: BlockPoolRows from opp_envs) and
+// ss_env_step_pool_speeds (blocks true, speeds not NULL: pool_step_speeds_kernel under BlockPoolRows)
 static int step_pool(void *state, int64_t n_envs, int64_t pool_envs, int n_opponents, const float *actions,
                      const float *opp_actions, float *obs_out, float *obs_out2, float *reward_out, uint8_t *done_rows_out,
                      float *opp_obs_out, uint8_t *done_out, uint8_t *winner_out, int reward_mode, int64_t tick_limit,
                      int reset_mode, uint64_t seed, uint64_t counter, uint32_t *status, int flags, uint64_t *pool_stats,
-                     bool blocks, const int64_t *opp_envs, void *stream) {
+                     bool blocks, const int64_t *opp_envs, const void *speeds, void *stream) {
     if (!state || !actions || !obs_out || n_envs <= 0 || pool_envs < 0 || pool_envs > n_envs) return SS_ERR_INVALID_ARG;
     if (pool_envs > 0 && (n_opponents < 1 || n_opponents > SS_LEAGUE_MAX_POLICIES || !opp_actions || !opp_obs_out))
         return SS_ERR_INVALID_ARG;
@@ -1157,6 +1247,22 @@ static int step_pool(void *state, int64_t n_envs, int64_t pool_envs, int n_oppon
     const dim3 grid(blocks_for(2 * n_envs, kBlockPP));
     if (blocks) {
         B.opp_actions = (const float2 *)opp_actions; B.opp_obs = (float4 *)opp_obs_out; B.pool_stats = (unsigned long long *)pool_stats;
+        if (speeds) {
+            A.speeds = speeds;
+            // the staging tile is step_kernel's: the same carve-out
+            static bool configured = false;
+            if (!configured) {
+                cudaFuncSetAttribute(pool_step_speeds_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 50);
+                cudaFuncSetAttribute(pool_step_speeds_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 50);
+                configured = true;
+            }
+            const dim3 grid_env(blocks_for(n_envs, kBlock));
+            if ((A.stats ? sslaunch::launch(pool_step_speeds_kernel<true>, grid_env, dim3(kBlock), 0, (cudaStream_t)stream, A, B)
+                         : sslaunch::launch(pool_step_speeds_kernel<false>, grid_env, dim3(kBlock), 0, (cudaStream_t)stream, A, B)) !=
+                cudaSuccess)
+                return SS_ERR_CUDA;
+            return SS_OK;
+        }
         if ((A.stats ? sslaunch::launch(step_pp_obs_kernel<true, BlockPoolRows>, grid, dim3(kBlockPP), 0, (cudaStream_t)stream, A, B)
                      : sslaunch::launch(step_pp_obs_kernel<false, BlockPoolRows>, grid, dim3(kBlockPP), 0, (cudaStream_t)stream, A, B)) !=
             cudaSuccess)
@@ -1178,7 +1284,7 @@ int ss_env_step_pool(void *state, int64_t n_envs, int64_t pool_envs, int n_oppon
                      void *stream) {
     return step_pool(state, n_envs, pool_envs, n_opponents, actions, opp_actions, obs_out, obs_out2, reward_out, done_rows_out,
                      opp_obs_out, done_out, winner_out, reward_mode, tick_limit, reset_mode, seed, counter, status, flags, pool_stats,
-                     false, nullptr, stream);
+                     false, nullptr, nullptr, stream);
 }
 
 int ss_env_step_pool_blocks(void *state, int64_t n_envs, int64_t pool_envs, int n_opponents, const float *actions,
@@ -1188,7 +1294,18 @@ int ss_env_step_pool_blocks(void *state, int64_t n_envs, int64_t pool_envs, int 
                             const int64_t *opp_envs, void *stream) {
     return step_pool(state, n_envs, pool_envs, n_opponents, actions, opp_actions, obs_out, obs_out2, reward_out, done_rows_out,
                      opp_obs_out, done_out, winner_out, reward_mode, tick_limit, reset_mode, seed, counter, status, flags, pool_stats,
-                     true, opp_envs, stream);
+                     true, opp_envs, nullptr, stream);
+}
+
+int ss_env_step_pool_speeds(void *state, int64_t n_envs, int64_t pool_envs, int n_opponents, const float *actions,
+                            const float *opp_actions, float *obs_out, float *obs_out2, float *reward_out, uint8_t *done_rows_out,
+                            float *opp_obs_out, uint8_t *done_out, uint8_t *winner_out, int reward_mode, int64_t tick_limit,
+                            int reset_mode, uint64_t seed, uint64_t counter, uint32_t *status, int flags, uint64_t *pool_stats,
+                            const int64_t *opp_envs, const void *speeds, void *stream) {
+    if (!speeds || ((uintptr_t)speeds & 15)) return SS_ERR_INVALID_ARG;
+    return step_pool(state, n_envs, pool_envs, n_opponents, actions, opp_actions, obs_out, obs_out2, reward_out, done_rows_out,
+                     opp_obs_out, done_out, winner_out, reward_mode, tick_limit, reset_mode, seed, counter, status, flags, pool_stats,
+                     true, opp_envs, speeds, stream);
 }
 
 int ss_pool_restart(void *state, int64_t n_envs, int64_t pool_envs, int n_opponents, const int64_t *opp_envs, int reset_mode,

@@ -1,10 +1,12 @@
-// ss_pool.cu -- ss_pool_rollout / ss_pool_rollout_frames: n training ticks of the self-play learner with part of its envs
-// played against a pool of frozen opponents, from one host call (include/skillshot_b200.h, "training against a pool").
+// ss_pool.cu -- ss_pool_rollout / ss_pool_rollout_frames / ss_pool_rollout_speeds: n training ticks of the self-play
+// learner with part of its envs played against a pool of frozen opponents, from one host call (include/skillshot_b200.h,
+// "training against a pool").
 //
 // A tick is the learner's forward over its L rows, the opponents' forwards over their M rows, ss_env_step_pool and, for
 // the networks that read a history of frames, the push of the newest observations.  Every kernel is an existing entry
 // point; this file checks the arguments before anything is enqueued and lays the learner's rows into the replay ring as
-// ss_selfplay_rollout does.  ss_pool_rollout is the case where every network has one frame.
+// ss_selfplay_rollout does.  ss_pool_rollout is the case where every network has one frame; ss_pool_rollout_speeds steps
+// the envs with ss_env_step_pool_speeds and is otherwise the same launches.
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -58,7 +60,8 @@ int64_t workspace_bytes(const Args &R) {
     return noisy + tiles;
 }
 
-int rollout(const Args &R, void *stream) {
+// speeds: the env step is ss_env_step_pool_speeds (R.speeds required), else ss_env_step_pool(_blocks) (R.speeds NULL)
+int rollout(const Args &R, bool speeds, void *stream) {
     const int64_t n = R.n_envs, M = R.pool_envs, K = R.n_opponents;
     if (!R.state || !R.params || !R.obs || !R.act || !R.reward || !R.done || !R.winner || n <= 0 || R.n_ticks <= 0)
         return SS_ERR_INVALID_ARG;
@@ -75,7 +78,7 @@ int rollout(const Args &R, void *stream) {
             if (f > 1 && (!R.opp_stacks || !R.opp_stacks[k] || ((uintptr_t)R.opp_stacks[k] & 15))) return SS_ERR_INVALID_ARG;
         }
     }
-    if (R.speeds) return SS_ERR_INVALID_ARG;
+    if (speeds ? (!R.speeds || ((uintptr_t)R.speeds & 15)) : R.speeds != nullptr) return SS_ERR_INVALID_ARG;
     if (R.reward_mode != SS_REWARD_NONE && R.reward_mode != SS_REWARD_LOOKING && R.reward_mode != SS_REWARD_TERMINAL) return SS_ERR_INVALID_ARG;
     if (R.reset_mode != SS_RESET_FIXED && R.reset_mode != SS_RESET_RANDOM) return SS_ERR_INVALID_ARG;
     if (R.param_noise_sd < 0.f || R.action_noise_sd < 0.f) return SS_ERR_INVALID_ARG;
@@ -171,7 +174,12 @@ int rollout(const Args &R, void *stream) {
         if (rc != SS_OK) return rc;
         sslaunch::pdl_mode() = kOn;
         float *step_obs = F > 1 ? R.obs : ring ? R.ring_next_obs + seg * L * 12 : R.obs;
-        rc = R.opp_envs ? ss_env_step_pool_blocks(R.state, n, M, (int)K, a, R.opp_act, step_obs, ring && F == 1 ? o_next : nullptr,
+        rc = speeds ? ss_env_step_pool_speeds(R.state, n, M, (int)K, a, R.opp_act, step_obs, ring && F == 1 ? o_next : nullptr,
+                                              ring ? R.ring_reward + seg * L : R.reward, ring ? R.ring_done + seg * L : nullptr,
+                                              R.opp_obs, R.done, R.winner, R.reward_mode, R.tick_limit, R.reset_mode, R.env_seed,
+                                              R.env_counter + (uint64_t)t, R.status, R.step_flags, R.pool_stats, R.opp_envs, R.speeds,
+                                              stream)
+           : R.opp_envs ? ss_env_step_pool_blocks(R.state, n, M, (int)K, a, R.opp_act, step_obs, ring && F == 1 ? o_next : nullptr,
                                                   ring ? R.ring_reward + seg * L : R.reward, ring ? R.ring_done + seg * L : nullptr,
                                                   R.opp_obs, R.done, R.winner, R.reward_mode, R.tick_limit, R.reset_mode, R.env_seed,
                                                   R.env_counter + (uint64_t)t, R.status, R.step_flags, R.pool_stats, R.opp_envs, stream)
@@ -211,7 +219,11 @@ extern "C" {
 int64_t ss_pool_rollout_frames_workspace_bytes(const ss_pool_rollout_frames_args *args) { return args ? workspace_bytes(*args) : -1; }
 
 int ss_pool_rollout_frames(const ss_pool_rollout_frames_args *args, void *stream) {
-    return args ? rollout(*args, stream) : SS_ERR_INVALID_ARG;
+    return args ? rollout(*args, false, stream) : SS_ERR_INVALID_ARG;
+}
+
+int ss_pool_rollout_speeds(const ss_pool_rollout_frames_args *args, void *stream) {
+    return args ? rollout(*args, true, stream) : SS_ERR_INVALID_ARG;
 }
 
 int ss_pool_rollout(const ss_pool_rollout_args *args, void *stream) {
@@ -229,7 +241,7 @@ int ss_pool_rollout(const ss_pool_rollout_args *args, void *stream) {
     R.env_seed = P.env_seed; R.env_counter = P.env_counter; R.noise_seed = P.noise_seed; R.noise_counter = P.noise_counter;
     R.speeds = P.speeds; R.status = P.status; R.step_flags = P.step_flags; R.pool_stats = P.pool_stats;
     R.frames = 1;          // every network reads one frame: no history, no workspace
-    return rollout(R, stream);
+    return rollout(R, false, stream);
 }
 
 }  // extern "C"

@@ -1253,7 +1253,8 @@ class SelfPlayTrainer:
 
     @property
     def pool_blocks(self) -> list:
-        """The pool envs of each opponent (pool_layout's blocks)."""
+        """The pool envs of each opponent (pool_layout's blocks).  Per-env speeds (envs.set_speeds) belong to the env, not
+        to the block: each opponent plays at the speeds of the envs its block covers."""
         if self.opponents is None:
             raise ValueError("this trainer has no opponent pool")
         K = len(self.opponents)
@@ -1311,7 +1312,9 @@ class SelfPlayTrainer:
 
     def rebalance_pool(self, weighting: str = "hard", p: float = 2.0, min_envs: int = 2, reset: bool = True) -> list:
         """Size each opponent's block by the learner's score against it: pool_progress(reset), pfsp_blocks of the scores
-        (an opponent without finished games counts as 0.5), set_pool_blocks.  Returns the new blocks."""
+        (an opponent without finished games counts as 0.5), set_pool_blocks.  Returns the new blocks.  With per-env speeds
+        each opponent was scored at the speeds of the envs its block covered; when the speeds are drawn independently per
+        env (a random sweep), every block samples the same distribution and the scores stay comparable."""
         prog = self.pool_progress(reset)
         blocks = pfsp_blocks([q["score"] if q["episodes"] else None for q in prog], self.pool_envs, weighting, p, min_envs)
         self.set_pool_blocks(blocks)
@@ -1355,11 +1358,9 @@ class SelfPlayTrainer:
         return out
 
     def _rollout_pool(self, n_ticks: int, store: bool):
-        """n_ticks ticks through ss_pool_rollout_frames: the learner's forward, the opponents' forwards, the pool step and
-        the history pushes."""
+        """n_ticks ticks through ss_pool_rollout_frames (ss_pool_rollout_speeds when the envs have per-env speeds): the
+        learner's forward, the opponents' forwards, the pool step and the history pushes."""
         envs, net, rp, st = self.envs, self.networks, self.replay, self.stack
-        if envs.speeds is not None:
-            raise ValueError("training against a pool does not support per-env speeds")
         L, M, K = self.learner_rows, self.pool_envs, len(self.opponents)
         out = envs._buffers(1)
         a = _lib.PoolRolloutFramesArgs()
@@ -1394,7 +1395,11 @@ class SelfPlayTrainer:
         if need > 0:
             a.workspace, a.workspace_bytes = self._pool_ws.data_ptr(), self._pool_ws.numel()
         with torch.cuda.device(self.device):
-            check(lib.ss_pool_rollout_frames(ctypes.byref(a), _stream(self.device)), "ss_pool_rollout_frames")
+            if envs.speeds is not None:
+                a.speeds = envs.speeds.data_ptr()
+                check(lib.ss_pool_rollout_speeds(ctypes.byref(a), _stream(self.device)), "ss_pool_rollout_speeds")
+            else:
+                check(lib.ss_pool_rollout_frames(ctypes.byref(a), _stream(self.device)), "ss_pool_rollout_frames")
         envs.counter += n_ticks
         if st is None:
             net.counter += n_ticks
