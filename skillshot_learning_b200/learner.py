@@ -81,6 +81,66 @@ def allreduce_sum(t: torch.Tensor, group=None):
     return t
 
 
+def check_process_group(group):
+    """ValueError unless `group` is True (the default group) or a torch.distributed ProcessGroup this process belongs to,
+    with torch.distributed initialised."""
+    import torch.distributed as dist
+    if not (dist.is_available() and dist.is_initialized()):
+        raise ValueError("process_group needs an initialised torch.distributed")
+    if group is not True and not isinstance(group, dist.ProcessGroup):
+        raise ValueError("process_group must be True (the default group) or a torch.distributed ProcessGroup, got %r" % (group,))
+    if dist.get_rank(None if group is True else group) < 0:
+        raise ValueError("this process is not a member of process_group")
+
+
+def ranks_agree(refusal: Optional[str], config, group=True):
+    """The agreement check of a collective call over the ranks of `group` (True: the default group): ONE
+    all_gather_object of (this rank's refusal message or None, this rank's config as (field, value) pairs in a fixed
+    order).  Every rank reads the same gathered list, so every rank raises the same ValueError -- naming the first rank
+    that refused, or else the first rank and field that differ from group rank 0's -- or none does; no rank is left
+    waiting in a later collective."""
+    import torch.distributed as dist
+    g = None if group is True else group
+    got = [None] * dist.get_world_size(g)
+    dist.all_gather_object(got, (refusal, tuple(config)), group=g)
+    for r, (msg, _) in enumerate(got):
+        if msg is not None:
+            raise ValueError("rank %d refused: %s" % (r, msg))
+    base = dict(got[0][1])
+    for r, (_, cfg) in enumerate(got[1:], 1):
+        for field, value in cfg:
+            if value != base.get(field):
+                raise ValueError("rank %d passed %s = %r, rank 0 %r" % (r, field, value, base.get(field)))
+
+
+def _device_collective(t: torch.Tensor, g) -> bool:
+    """True when a collective of group `g` takes `t` where it lies (a CUDA tensor and an NCCL backend); gloo takes a CPU copy."""
+    import torch.distributed as dist
+    return t.is_cuda and "nccl" in str(dist.get_backend(g))
+
+
+def allreduce_counters(t: torch.Tensor, group=True) -> torch.Tensor:
+    """The sum of an int64 counter tensor over the ranks of `group` (True: the default group) as a new CPU tensor; `t`
+    itself is not changed.  One all-reduce: on the device for an NCCL group, on a CPU copy for gloo."""
+    import torch.distributed as dist
+    g = None if group is True else group
+    s = t.clone() if _device_collective(t, g) else t.cpu().clone()
+    dist.all_reduce(s, op=dist.ReduceOp.SUM, group=g)
+    return s.cpu()
+
+
+def _broadcast_rank0(t: torch.Tensor, group=True):
+    """Overwrite `t` in place with group rank 0's `t` (on the device for an NCCL group, through a CPU copy for gloo)."""
+    import torch.distributed as dist
+    g = None if group is True else group
+    if _device_collective(t, g):
+        dist.broadcast(t, group=g, group_src=0)
+    else:
+        c = t.cpu()
+        dist.broadcast(c, group=g, group_src=0)
+        t.copy_(c)
+
+
 class PeerExchange:
     """The gradient exchange of a sharded update over NVLink peer memory (csrc/ss_peer.cu): every rank
     owns an inbox {flags | 2 x world x capacity floats} shared with the other processes of the node
@@ -1166,34 +1226,62 @@ class SelfPlayTrainer:
         (pool_layout).  The opponents act without noise and only the learner's transitions are stored; an opponent with
         more than one frame keeps a history of its rows.  See set_opponent / pool_progress.
         pool_blocks: the pool envs of each opponent (even sizes >= 2 summing to pool_envs, pool_layout) instead of
-        pool_envs / len(opponents) each; see set_pool_blocks / rebalance_pool."""
+        pool_envs / len(opponents) each; see set_pool_blocks / rebalance_pool.
+        process_group with opponents (a sharded pool, DESIGN.md section 6.13): one rank per GPU, every rank passing the same
+        n_envs, pool_envs, number of opponents, frames, opponent frame counts, pool_blocks and collective, and its own seed.
+        The pool is replicated: every rank plays all K opponents on its own pool_envs envs with the same blocks, so a
+        rank's rollout is the single-GPU pool rollout of its envs and the update sums gradients over the ranks as for
+        sharded self-play.  process_group must be True (the default group) or a ProcessGroup of an initialised
+        torch.distributed, else ValueError.  Every rank then checks the pool rules and one all_gather_object compares the
+        ranks' refusals and configurations: when any rank refused or one differs, every rank raises the same ValueError
+        before anything is allocated.  The opponents are then broadcast from group rank 0.  Every pool method
+        (set_opponent, set_pool_blocks, rebalance_pool, pool_progress) is collective: call it on every rank with the same
+        arguments, as update().  save / load write and read each rank's own file."""
         self.device = torch.device(device)
         self.frames = int(frames)
         self.opponents, self.pool_envs, self.pool_stats = None, 0, None
         if opponents is not None:
-            K = len(opponents)
             if process_group is not None:
-                raise ValueError("training against a pool runs on one GPU (no process_group)")
-            if reward_mode == "simple":
-                raise ValueError("training against a pool supports reward modes none / looking / terminal")
-            if not 1 <= K <= _lib.LEAGUE_MAX_POLICIES:
-                raise ValueError("1..%d opponents, got %d" % (_lib.LEAGUE_MAX_POLICIES, K))
-            M = (int(n_envs) // 2) // (2 * K) * (2 * K) if pool_envs is None else int(pool_envs)
-            if not 0 <= M <= int(n_envs) or M % (2 * K):
-                raise ValueError("pool_envs must be a multiple of 2 * %d in [0, n_envs], got %d" % (K, M))
-            if precision == "bf16" and float(param_noise_sd) > 0 and int(noise_group) % 128:
-                raise ValueError("with tensor cores and parameter noise the noise group must be a multiple of 128, got %d" % noise_group)
-            opp_vecs = [actor_vector(a) for a in opponents]
+                check_process_group(process_group)
+
+            def pool_rules():
+                K = len(opponents)
+                if reward_mode == "simple":
+                    raise ValueError("training against a pool supports reward modes none / looking / terminal")
+                if not 1 <= K <= _lib.LEAGUE_MAX_POLICIES:
+                    raise ValueError("1..%d opponents, got %d" % (_lib.LEAGUE_MAX_POLICIES, K))
+                M = (int(n_envs) // 2) // (2 * K) * (2 * K) if pool_envs is None else int(pool_envs)
+                if not 0 <= M <= int(n_envs) or M % (2 * K):
+                    raise ValueError("pool_envs must be a multiple of 2 * %d in [0, n_envs], got %d" % (K, M))
+                if precision == "bf16" and float(param_noise_sd) > 0 and int(noise_group) % 128:
+                    raise ValueError("with tensor cores and parameter noise the noise group must be a multiple of 128, got %d" % noise_group)
+                vecs = [actor_vector(a) for a in opponents]
+                # None: M / K envs per opponent, the step of ss_pool_rollout (no block table is passed)
+                blocks = None if pool_blocks is None else check_pool_blocks(pool_blocks, M, K)
+                L = 2 * int(n_envs) - M
+                if replay_capacity is not None and (replay_capacity % L or replay_capacity < 2 * L):
+                    raise ValueError("with a pool the replay capacity must be a multiple of the %d learner rows, at least two of them" % L)
+                if self.device.type != "cuda":
+                    raise ValueError("device must be a CUDA device")
+                return vecs, M, blocks
+
+            if process_group is None:
+                opp_vecs, M, self._blocks = pool_rules()
+            else:
+                # sharded: every rank runs the rules, then one exchange makes every rank raise, or none
+                refusal, config = None, ()
+                try:
+                    opp_vecs, M, self._blocks = pool_rules()
+                    config = (("n_envs", int(n_envs)), ("pool_envs", M), ("opponents", len(opp_vecs)), ("frames", self.frames),
+                              ("opponent frames", [f for _, f in opp_vecs]),
+                              ("pool_blocks", self._blocks or [M // len(opp_vecs)] * len(opp_vecs)), ("collective", collective))
+                except ValueError as e:
+                    refusal = str(e)
+                ranks_agree(refusal, config, process_group)
             self.opp_frames = [f for _, f in opp_vecs]
             self.pool_envs = M
-            # None: M / K envs per opponent, the step of ss_pool_rollout (no block table is passed)
-            self._blocks = None if pool_blocks is None else check_pool_blocks(pool_blocks, M, K)
         self.learner_rows = 2 * int(n_envs) - self.pool_envs       # rows of the learner's transitions per tick
         L = self.learner_rows
-        if replay_capacity is not None and opponents is not None and (replay_capacity % L or replay_capacity < 2 * L):
-            raise ValueError("with a pool the replay capacity must be a multiple of the %d learner rows, at least two of them" % L)
-        if opponents is not None and self.device.type != "cuda":
-            raise ValueError("device must be a CUDA device")
         self.envs = SkillshotEnvs(n_envs, device=device, random_positions=random_positions, seed=seed,
                                   reward_mode=reward_mode, tick_limit=tick_limit, auto_reset=True)
         self.envs.collect_episode_stats = True     # the reference's per-episode ticks / winner log, reduced on the device
@@ -1216,6 +1304,8 @@ class SelfPlayTrainer:
             self.opponents = torch.zeros((K, max((v.size + 3) // 4 * 4 for v, _ in opp_vecs)), dtype=torch.float32, device=self.device)
             for k, (v, _) in enumerate(opp_vecs):
                 self.opponents[k, :v.size] = torch.from_numpy(v).to(self.device)
+            if process_group is not None:
+                _broadcast_rank0(self.opponents, process_group)      # the same pool on every rank by construction
             self.pool_stats = torch.zeros((K, _lib.POOL_STATS), dtype=torch.int64, device=self.device)
             # rows [0, L) the learner's, [L, 2n) the opponents' (pool_layout): observations and actions
             rows = torch.from_numpy(pool_layout(n, self.pool_envs, len(self.opponents), self._blocks).reshape(-1)).to(self.device)
@@ -1285,11 +1375,21 @@ class SelfPlayTrainer:
         env between blocks can flip the learner's seat, and an opponent's history is indexed by the env's offset in its
         block.  The self-play envs, rows and histories are untouched.  The last stored transition of a restarted game keeps
         its next observation and a 0 done flag, as a tick-limit ending does; nothing is counted in pool_stats or the
-        episode statistics."""
+        episode statistics.  Sharded: collective; one all-gather checks that every rank passed the same valid table, and
+        otherwise every rank raises ValueError and nothing restarts."""
         if self.opponents is None:
             raise ValueError("this trainer has no opponent pool")
         n, M, K, L = self.envs.n_envs, self.pool_envs, len(self.opponents), self.learner_rows
-        blocks = check_pool_blocks(blocks, M, K)
+        group = self.networks.group
+        if group is None:
+            blocks = check_pool_blocks(blocks, M, K)
+        else:
+            refusal = None
+            try:
+                blocks = check_pool_blocks(blocks, M, K)
+            except ValueError as e:
+                refusal, blocks = str(e), None
+            ranks_agree(refusal, (("pool_blocks", blocks),), group)
         envs = self.envs
         table = (ctypes.c_int64 * K)(*blocks)
         with torch.cuda.device(self.device):
@@ -1314,7 +1414,9 @@ class SelfPlayTrainer:
         """Size each opponent's block by the learner's score against it: pool_progress(reset), pfsp_blocks of the scores
         (an opponent without finished games counts as 0.5), set_pool_blocks.  Returns the new blocks.  With per-env speeds
         each opponent was scored at the speeds of the envs its block covered; when the speeds are drawn independently per
-        env (a random sweep), every block samples the same distribution and the scores stay comparable."""
+        env (a random sweep), every block samples the same distribution and the scores stay comparable.  Sharded:
+        collective; pool_progress sums the counters over the ranks and pfsp_blocks is deterministic, so every rank computes
+        the same blocks."""
         prog = self.pool_progress(reset)
         blocks = pfsp_blocks([q["score"] if q["episodes"] else None for q in prog], self.pool_envs, weighting, p, min_envs)
         self.set_pool_blocks(blocks)
@@ -1323,30 +1425,47 @@ class SelfPlayTrainer:
     def set_opponent(self, k: int, actor):
         """Replace opponent k of the pool with a copy of `actor` from the next tick on (the games in flight continue against
         it, with the slot's history), e.g. trainer.set_opponent(i % K, trainer.networks.actor) every few updates.  The actor
-        must have the slot's frame count."""
+        must have the slot's frame count.  Sharded: collective; slot k then holds group rank 0's actor on every rank (one
+        broadcast), and a refusal on any rank, or a different k, raises ValueError on every rank."""
         if self.opponents is None:
             raise ValueError("this trainer has no opponent pool")
-        k = int(k)
+        k, group = int(k), self.networks.group
+        if group is None:
+            v = self._opponent_vector(k, actor)
+        else:
+            refusal, v = None, None
+            try:
+                v = self._opponent_vector(k, actor)
+            except (IndexError, ValueError) as e:
+                refusal = str(e)
+            ranks_agree(refusal, (("k", k),), group)
+        self.opponents[k, :v.numel()].copy_(v)
+        if group is not None:
+            _broadcast_rank0(self.opponents[k], group)
+
+    def _opponent_vector(self, k: int, actor) -> torch.Tensor:
+        """`actor` as a flat vector for slot k (IndexError / ValueError when it does not fit the slot)."""
         if not 0 <= k < len(self.opponents):
             raise IndexError("opponent %d of %d" % (k, len(self.opponents)))
         f = self.opp_frames[k]
         n_params = int(lib.ss_actor_frames_params(f))
         if torch.is_tensor(actor) and actor.dim() == 1 and actor.numel() == n_params:
-            self.opponents[k, :n_params].copy_(actor.detach())
-            return
+            return actor.detach()
         flat, frames = actor_vector(actor)
         if frames != f:
             raise ValueError("opponent %d has %d frames, the new actor %d" % (k, f, frames))
-        self.opponents[k, :n_params] = torch.from_numpy(flat).to(self.device)
+        return torch.from_numpy(flat)
 
     def pool_progress(self, reset: bool = False) -> list:
         """Per opponent, the training games against it finished so far (device counters): episodes, learner wins (the
         opponent was hit), learner losses, tick-limit endings (draws), mean episode ticks, and the learner's score with
-        its standard error (win 1, draw 0.5, loss 0)."""
+        its standard error (win 1, draw 0.5, loss 0).  Sharded: collective; the figures are those of the counters summed
+        over the ranks (one all-reduce), the same list on every rank, and `reset` zeroes each rank's own counters."""
         from .league import _score
         if self.opponents is None:
             raise ValueError("this trainer has no opponent pool")
-        c = self.pool_stats.cpu().numpy()
+        group = self.networks.group
+        c = (self.pool_stats.cpu() if group is None else allreduce_counters(self.pool_stats, group)).numpy()
         if reset:
             self.pool_stats.zero_()
         out = []
