@@ -448,6 +448,38 @@ int ss_critic_grad_frames_tc(const float *critic_params, int frames, const float
                              void *workspace, int64_t workspace_bytes, void *stream);
 int ss_actor_grad_frames_tc(const float *actor_params, const float *critic_params, int frames, const float *obs, int64_t n,
                             float *grad_out, float *q_sum_out, void *workspace, int64_t workspace_bytes, void *stream);
+
+/* ---- TD3 target (twin critics, target policy smoothing; no reference code, DESIGN.md section 6.14) ----
+ *   a~[i] = clamp(mu'(s'_i) + clamp(noise_sd * eps_i, -noise_clip, noise_clip), -1, 1)
+ *   y_out[i] = reward[i] + gamma * (1 - done[i]) * min(Q1'(s'_i, a~[i]), Q2'(s'_i, a~[i]))
+ * target_critic2_params NULL: the minimum is over Q1' alone.  eps_i: the first two of the four Box-Muller normals of
+ * Philox4x32-10(seed; row_offset + i, (row_offset + i) >> 32, counter) with tag SS_TAG_TARGET_NOISE (the keying of the
+ * action noise of ss_actor_forward, by the GLOBAL row as dropout is: a shard of a batch draws what the whole batch draws);
+ * noise_sd == 0 draws nothing.  With target_critic2_params == NULL and noise_sd == 0 each entry point returns, bit for
+ * bit, what its ss_ddpg_targets* counterpart returns.  Every argument is checked before anything is enqueued; a bad one
+ * (NULL pointer, n <= 0, frames out of range, noise_sd < 0, noise_clip < 0, row_offset < 0, a misaligned parameter vector,
+ * a short workspace) returns SS_ERR_INVALID_ARG.
+ *   ss_td3_targets_frames     float32 CUDA cores, frames 1..SS_MAX_FRAMES (frames = 1: the 12-input networks).
+ *                             The workspace is not used (may be NULL).
+ *   ss_td3_targets_tc         tcgen05, the 12-input networks: ss_ddpg_targets_tc's forwards; workspace (16-byte aligned)
+ *                             of at least SS_TD3_TC_WORKSPACE_BYTES(n) bytes (8 n rounded up to 16 is enough for one critic).
+ *   ss_td3_targets_frames_tc  tcgen05, frames 2..SS_MAX_FRAMES: ss_ddpg_targets_frames_tc's forwards with its workspace,
+ *                             ss_learner_frames_tc_workspace_bytes(frames, n). */
+#define SS_TAG_TARGET_NOISE 5
+#define SS_TD3_TC_WORKSPACE_BYTES(n) (((int64_t)(n) * 8 + 15) / 16 * 16 + 2 * (((int64_t)(n) * 4 + 15) / 16 * 16))
+int ss_td3_targets_frames(const float *target_actor_params, const float *target_critic_params, const float *target_critic2_params,
+                          int frames, const float *reward, const float *next_obs, const uint8_t *done, float gamma,
+                          float noise_sd, float noise_clip, uint64_t seed, uint64_t counter, int64_t row_offset, float *y_out,
+                          int64_t n, void *workspace, int64_t workspace_bytes, void *stream);
+int ss_td3_targets_tc(const float *target_actor_params, const float *target_critic_params, const float *target_critic2_params,
+                      const float *reward, const float *next_obs, const uint8_t *done, float gamma, float noise_sd, float noise_clip,
+                      uint64_t seed, uint64_t counter, int64_t row_offset, float *y_out, int64_t n, void *workspace,
+                      int64_t workspace_bytes, void *stream);
+int ss_td3_targets_frames_tc(const float *target_actor_params, const float *target_critic_params, const float *target_critic2_params,
+                             int frames, const float *reward, const float *next_obs, const uint8_t *done, float gamma, float noise_sd,
+                             float noise_clip, uint64_t seed, uint64_t counter, int64_t row_offset, float *y_out, int64_t n,
+                             void *workspace, int64_t workspace_bytes, void *stream);
+
 int ss_replay_push_frames(float *ring_obs, float *ring_act, float *ring_reward, float *ring_next_obs, uint8_t *ring_done,
                           int64_t capacity, int64_t write_pos, int frames, const float *obs, const float *act,
                           const float *reward, const float *next_obs, const uint8_t *done, int done_div, int64_t n,

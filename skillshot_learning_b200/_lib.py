@@ -44,6 +44,12 @@ MAX_FRAMES = 20                   # SS_MAX_FRAMES
 LEAGUE_MAX_POLICIES = 64          # SS_LEAGUE_MAX_POLICIES
 STATUS_SEAT_RANGE = 8             # SS_STATUS_SEAT_RANGE
 POOL_STATS = 8                    # uint64 counters per opponent of ss_env_step_pool / ss_pool_rollout
+TAG_TARGET_NOISE = 5              # SS_TAG_TARGET_NOISE: Philox tag of the TD3 target policy smoothing
+
+
+def td3_tc_workspace_bytes(n: int) -> int:
+    """SS_TD3_TC_WORKSPACE_BYTES(n): the workspace of ss_td3_targets_tc with two critics."""
+    return (n * 8 + 15) // 16 * 16 + 2 * ((n * 4 + 15) // 16 * 16)
 
 
 class DdpgUpdateArgs(ctypes.Structure):
@@ -166,6 +172,11 @@ SIGNATURES = {
     "ss_critic_grad_frames_tc": (_i32, [_vp, _i32, _vp, _vp, _vp, _vp, _f32, _u64, _u64, _i64, _i64, _i64, _vp, _vp, _vp, _i64,
                                          _vp]),
     "ss_actor_grad_frames_tc": (_i32, [_vp, _vp, _i32, _vp, _i64, _vp, _vp, _vp, _i64, _vp]),
+    "ss_td3_targets_frames": (_i32, [_vp, _vp, _vp, _i32, _vp, _vp, _vp, _f32, _f32, _f32, _u64, _u64, _i64, _vp, _i64, _vp, _i64,
+                                      _vp]),
+    "ss_td3_targets_tc": (_i32, [_vp, _vp, _vp, _vp, _vp, _vp, _f32, _f32, _f32, _u64, _u64, _i64, _vp, _i64, _vp, _i64, _vp]),
+    "ss_td3_targets_frames_tc": (_i32, [_vp, _vp, _vp, _i32, _vp, _vp, _vp, _f32, _f32, _f32, _u64, _u64, _i64, _vp, _i64, _vp,
+                                         _i64, _vp]),
     "ss_replay_push_frames": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _i32, _i64, _vp]),
     "ss_replay_sample_frames": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _vp, _u64, _u64, _i64,
                                         _vp, _vp, _vp, _vp, _vp, _vp, _vp]),

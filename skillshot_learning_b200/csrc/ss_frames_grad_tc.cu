@@ -717,6 +717,36 @@ int ss_ddpg_targets_frames_tc(const float *target_actor_params, const float *tar
     return rc;
 }
 
+// ss_ddpg_targets_frames_tc with the smoothing on a' and, with a second critic, both critics' q (in the q and -dQ/da
+// regions of the workspace) -> td3_min_target
+int ss_td3_targets_frames_tc(const float *target_actor_params, const float *target_critic_params, const float *target_critic2_params,
+                             int frames, const float *reward, const float *next_obs, const uint8_t *done, float gamma, float noise_sd,
+                             float noise_clip, uint64_t seed, uint64_t counter, int64_t row_offset, float *y_out, int64_t n,
+                             void *workspace, int64_t workspace_bytes, void *stream) {
+    Ctx C{};
+    if (!target_actor_params || !target_critic_params || !reward || !next_obs || !y_out) return SS_ERR_INVALID_ARG;
+    if (frames < 2 || !(noise_sd >= 0.f) || !(noise_clip >= 0.f) || row_offset < 0) return SS_ERR_INVALID_ARG;
+    if (((uintptr_t)target_actor_params | (uintptr_t)target_critic_params | (uintptr_t)target_critic2_params | (uintptr_t)next_obs) & 15)
+        return SS_ERR_INVALID_ARG;
+    if (prepare(frames, n, workspace, workspace_bytes, stream, C) != SS_OK) return SS_ERR_INVALID_ARG;
+    int sms = 0, rc = device_sms(sms);
+    if (rc == SS_OK) rc = pack(C, next_obs, frames, n, false);
+    if (rc == SS_OK)
+        rc = ss_actor_forward_frames_tc(target_actor_params, 0, 0, C.at(C.L.xf), frames, frames - 1, C.at<float>(C.L.act), n,
+                                        C.at(C.L.h1b), C.L.act - C.L.h1b, stream);
+    if (rc == SS_OK && noise_sd > 0.f)
+        rc = td3_smooth_actions(C.at<float>(C.L.act), n, noise_sd, noise_clip, seed, counter, row_offset, C.st);
+    if (rc != SS_OK) return rc;
+    if (!target_critic2_params)
+        return critic_forward(C, target_critic_params, frames, n, C.at<float>(C.L.act), nullptr, nullptr, reward, done, gamma, y_out, sms);
+    float *q1 = C.at<float>(C.L.q), *q2 = C.at<float>(C.L.up);
+    rc = critic_forward(C, target_critic_params, frames, n, C.at<float>(C.L.act), q1, nullptr, nullptr, nullptr, 0.f, nullptr, sms);
+    if (rc == SS_OK)
+        rc = critic_forward(C, target_critic2_params, frames, n, C.at<float>(C.L.act), q2, nullptr, nullptr, nullptr, 0.f, nullptr, sms);
+    if (rc != SS_OK) return rc;
+    return td3_min_target(q1, q2, reward, done, gamma, y_out, n, C.st);
+}
+
 int ss_critic_grad_frames_tc(const float *critic_params, int frames, const float *obs, const float *act, const float *target,
                              const uint8_t *dropout_keep, float dropout_rate, uint64_t seed, uint64_t counter,
                              int64_t n, int64_t n_global, int64_t row_offset, float *grad_out, float *sse_out,

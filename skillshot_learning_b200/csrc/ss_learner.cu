@@ -429,6 +429,70 @@ __global__ void __launch_bounds__(NT) critic_fwd_kernel(const CriticFwdArgs A) {
 }
 
 // ---------------------------------------------------------------------------
+// TD3 target (no reference code, DESIGN.md section 6.14):
+//   a~ = clamp(mu'(s') + clamp(sigma eps, -c, c), -1, 1);  y = r + gamma (1 - d) min(Q1'(s', a~), Q2'(s', a~))
+// critic_fwd_kernel<true>'s tile loop with the smoothing between the actor and the critic and a second critic pass;
+// with phi2 == NULL and sigma == 0 every operation is that kernel's, so y is ss_ddpg_targets_frames' bit for bit.
+// ---------------------------------------------------------------------------
+struct Td3TargetArgs {
+    const float *theta, *phi, *phi2;     // target actor, target critics (phi2 NULL: one critic)
+    const float *reward, *obs;           // obs = s'
+    const uint8_t *done;
+    float gamma, sigma, clip;
+    uint64_t seed, counter;
+    int64_t row_offset;                  // global index of row 0 (the smoothing draw of a shard)
+    float *out;
+    int64_t n;
+    int ds;
+};
+
+__global__ void __launch_bounds__(NT) td3_target_kernel(const Td3TargetArgs A) {
+    extern __shared__ __align__(16) float smem[];
+    const Lay L = lay_of(A.ds);
+    float *sT = smem, *x2T = sT + L.ds * PITCH, *c2T = x2T + (H1 + DA) * PITCH, *qv = c2T + H2 * PITCH;
+    float *h1T = qv + TB, *h2T = h1T + H1 * PITCH, *qv2 = h2T + H2 * PITCH;
+    const int64_t tiles = (A.n + TB - 1) / TB;
+    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
+        const int64_t base = tile * TB;
+        __syncthreads();
+        load_tile_rt(A.obs, base, A.n, sT, L.ds);
+        __syncthreads();
+        dense_fwd<H1, ACT_RELU>(A.theta, A.theta + L.a_b1, sT, L.ds, h1T);
+        __syncthreads();
+        dense_fwd<H2, ACT_RELU>(A.theta + L.a_w2, A.theta + L.a_b2, h1T, H1, h2T);
+        __syncthreads();
+        actor_out(A.theta + L.a_w3, A.theta + L.a_b3, h2T, x2T + H1 * PITCH);
+        if (A.sigma > 0.f) {                      // (uniform over the CTA) one thread per row smooths both actions
+            __syncthreads();
+            if (threadIdx.x < TB && base + threadIdx.x < A.n) {
+                float *a = x2T + H1 * PITCH + threadIdx.x;
+                td3_smooth(A.seed, A.counter, A.row_offset + base + threadIdx.x, A.sigma, A.clip, a, a + PITCH);
+            }
+        }
+        dense_fwd<H1, ACT_RELU>(A.phi, A.phi + L.c_b1, sT, L.ds, x2T);
+        __syncthreads();
+        dense_fwd<H2, ACT_RELU>(A.phi + L.c_w2, A.phi + L.c_b2, x2T, H1 + DA, c2T);
+        __syncthreads();
+        critic_out(A.phi + L.c_w3, A.phi + L.c_b3, c2T, qv);
+        if (A.phi2) {
+            dense_fwd<H1, ACT_RELU>(A.phi2, A.phi2 + L.c_b1, sT, L.ds, x2T);
+            __syncthreads();
+            dense_fwd<H2, ACT_RELU>(A.phi2 + L.c_w2, A.phi2 + L.c_b2, x2T, H1 + DA, c2T);
+            __syncthreads();
+            critic_out(A.phi2 + L.c_w3, A.phi2 + L.c_b3, c2T, qv2);
+        }
+        __syncthreads();
+        if (threadIdx.x < TB && base + threadIdx.x < A.n) {
+            const int64_t row = base + threadIdx.x;
+            float q = qv[threadIdx.x];
+            if (A.phi2) q = fminf(q, qv2[threadIdx.x]);
+            q = A.reward[row] + A.gamma * (A.done && A.done[row] ? 0.f : 1.f) * q;
+            A.out[row] = q;
+        }
+    }
+}
+
+// ---------------------------------------------------------------------------
 // critic MSE gradient (one Keras fit batch, SkillshotLearner.py:434)
 // ---------------------------------------------------------------------------
 struct CriticGradArgs {
@@ -859,6 +923,24 @@ int ss_ddpg_targets_frames(const float *target_actor_params, const float *target
     const int grid = grid_for(critic_fwd_kernel<true>, smem_critic_fwd_actor(ds), (n + TB - 1) / TB, 0);
     if (grid < 0) return SS_ERR_CUDA;
     critic_fwd_kernel<true><<<grid, NT, smem_critic_fwd_actor(ds), (cudaStream_t)stream>>>(A);
+    return check_launch();
+}
+
+int ss_td3_targets_frames(const float *target_actor_params, const float *target_critic_params, const float *target_critic2_params,
+                          int frames, const float *reward, const float *next_obs, const uint8_t *done, float gamma,
+                          float noise_sd, float noise_clip, uint64_t seed, uint64_t counter, int64_t row_offset, float *y_out,
+                          int64_t n, void *workspace, int64_t workspace_bytes, void *stream) {
+    (void)workspace; (void)workspace_bytes;       // (the float32 kernel keeps everything in shared memory)
+    if (!target_actor_params || !target_critic_params || !reward || !next_obs || !y_out || n <= 0 || frames < 1 ||
+        frames > SS_MAX_FRAMES || !(noise_sd >= 0.f) || !(noise_clip >= 0.f) || row_offset < 0)
+        return SS_ERR_INVALID_ARG;
+    const int ds = DS * frames;
+    const size_t smem = smem_critic_fwd_actor(ds) + TB * 4;
+    Td3TargetArgs A{target_actor_params, target_critic_params, target_critic2_params, reward, next_obs, done, gamma, noise_sd,
+                    noise_clip, seed, counter, row_offset, y_out, n, ds};
+    const int grid = grid_for(td3_target_kernel, smem, (n + TB - 1) / TB, 0);
+    if (grid < 0) return SS_ERR_CUDA;
+    td3_target_kernel<<<grid, NT, smem, (cudaStream_t)stream>>>(A);
     return check_launch();
 }
 

@@ -558,10 +558,40 @@ int launch_grad(const GradArgs &A0, float *grad_out, float *aux_out, int64_t wor
     return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA;
 }
 
+// TD3 target policy smoothing of the target actions, one thread per row (ss_rng.cuh td3_smooth)
+__global__ void td3_smooth_kernel(float2 *act, int64_t n, float sigma, float clip, uint64_t seed, uint64_t counter,
+                                  int64_t row_offset) {
+    const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (row >= n) return;
+    float2 a = act[row];
+    ss::td3_smooth(seed, counter, row_offset + row, sigma, clip, &a.x, &a.y);
+    act[row] = a;
+}
+
+// the TD3 target from the two target critics' values: the TD epilogue of the forward kernels on min(q1, q2)
+__global__ void td3_min_target_kernel(const float *q1, const float *q2, const float *reward, const uint8_t *done, float gamma,
+                                      float *y, int64_t n) {
+    const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (row >= n) return;
+    y[row] = reward[row] + gamma * (done && done[row] ? 0.f : 1.f) * fminf(q1[row], q2[row]);
+}
+
 }  // namespace
 
 int sstc::reduce_slices(const float *work, int parts, int n_params, float *grad, float *aux, cudaStream_t st) {
     reduce_parts_kernel<<<(n_params + 1 + 63) / 64, dim3(64, 4), 0, st>>>(work, parts, n_params, grad, aux);
+    return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA;
+}
+
+int sstc::td3_smooth_actions(float *act, int64_t n, float sigma, float clip, uint64_t seed, uint64_t counter, int64_t row_offset,
+                             cudaStream_t st) {
+    td3_smooth_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>((float2 *)act, n, sigma, clip, seed, counter, row_offset);
+    return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA;
+}
+
+int sstc::td3_min_target(const float *q1, const float *q2, const float *reward, const uint8_t *done, float gamma, float *y, int64_t n,
+                         cudaStream_t st) {
+    td3_min_target_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(q1, q2, reward, done, gamma, y, n);
     return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA;
 }
 
@@ -652,6 +682,35 @@ int ss_ddpg_targets_tc_paired(const float *target_actor_params, const float *tar
     int rc = ss_actor_forward_tc(target_actor_params, next_obs, act, n, 0.f, 0, 0.f, 0, 0, stream);
     if (rc != SS_OK) return rc;
     return ss_critic_forward_tc(target_critic_params, next_obs, act, n, nullptr, nullptr, reward, done, gamma, y_out, stream);
+}
+
+// actor'(s') -> [smoothing] -> critic'(s', a~) with the TD epilogue (one critic: ss_ddpg_targets_tc's two launches), or both
+// critics' q -> td3_min_target.  workspace: [act n x 2 | q1 n | q2 n], each 16-byte aligned.
+int ss_td3_targets_tc(const float *target_actor_params, const float *target_critic_params, const float *target_critic2_params,
+                      const float *reward, const float *next_obs, const uint8_t *done, float gamma, float noise_sd, float noise_clip,
+                      uint64_t seed, uint64_t counter, int64_t row_offset, float *y_out, int64_t n, void *workspace,
+                      int64_t workspace_bytes, void *stream) {
+    if (!target_actor_params || !target_critic_params || !reward || !next_obs || !y_out || !workspace || n <= 0 ||
+        !(noise_sd >= 0.f) || !(noise_clip >= 0.f) || row_offset < 0)
+        return SS_ERR_INVALID_ARG;
+    if (((uintptr_t)target_actor_params | (uintptr_t)target_critic_params | (uintptr_t)target_critic2_params | (uintptr_t)next_obs |
+         (uintptr_t)workspace) & 15)
+        return SS_ERR_INVALID_ARG;
+    const int64_t act_bytes = (n * 8 + 15) / 16 * 16, q_bytes = (n * 4 + 15) / 16 * 16;
+    if (workspace_bytes < (target_critic2_params ? SS_TD3_TC_WORKSPACE_BYTES(n) : act_bytes)) return SS_ERR_INVALID_ARG;
+    cudaStream_t st = (cudaStream_t)stream;
+    float *act = (float *)workspace;
+    int rc = ss_actor_forward_tc(target_actor_params, next_obs, act, n, 0.f, 0, 0.f, 0, 0, stream);
+    if (rc == SS_OK && noise_sd > 0.f) rc = td3_smooth_actions(act, n, noise_sd, noise_clip, seed, counter, row_offset, st);
+    if (rc != SS_OK) return rc;
+    if (!target_critic2_params)
+        return ss_critic_forward_tc(target_critic_params, next_obs, act, n, nullptr, nullptr, reward, done, gamma, y_out, stream);
+    float *q1 = (float *)((char *)workspace + act_bytes), *q2 = (float *)((char *)workspace + act_bytes + q_bytes);
+    rc = ss_critic_forward_tc(target_critic_params, next_obs, act, n, q1, nullptr, nullptr, nullptr, 0.f, nullptr, stream);
+    if (rc == SS_OK)
+        rc = ss_critic_forward_tc(target_critic2_params, next_obs, act, n, q2, nullptr, nullptr, nullptr, 0.f, nullptr, stream);
+    if (rc != SS_OK) return rc;
+    return td3_min_target(q1, q2, reward, done, gamma, y_out, n, st);
 }
 
 }  // extern "C"

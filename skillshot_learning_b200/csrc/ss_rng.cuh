@@ -15,6 +15,7 @@ constexpr uint32_t kTagParamNoise = 1;   // model_act_param_noise, SkillshotLear
 constexpr uint32_t kTagDropout = 2;      // Dropout(0.2) during critic.fit, SkillshotLearner.py:105, 434
 constexpr uint32_t kTagActionNoise = 3;  // model_act_action_noise, SkillshotLearner.py:238
 constexpr uint32_t kTagReplay = 4;       // minibatch row choice (np.random.shuffle at :427 in the reference)
+constexpr uint32_t kTagTargetNoise = 5;  // TD3 target policy smoothing (no reference code, DESIGN.md section 6.14)
 
 SS_HD U4 draw4(uint64_t seed, uint32_t tag, uint32_t a, uint32_t b, uint64_t counter) {
     return philox4x32_10(U4{a, b, (uint32_t)counter, tag ^ (uint32_t)(counter >> 32)},
@@ -42,6 +43,16 @@ SS_HD void normal4(uint64_t seed, uint32_t tag, uint32_t a, uint32_t b, uint64_t
     const U4 u = draw4(seed, tag, a, b, counter);
     box_muller(u.x, u.y, z + 0, z + 1);
     box_muller(u.z, u.w, z + 2, z + 3);
+}
+
+// TD3 target policy smoothing of one row's target action, in place: a_m = clamp(a_m + clamp(sigma z_m, -c, c), -1, 1)
+// with z_0, z_1 the first two normals of normal4(seed, kTagTargetNoise, row, row >> 32, counter) -- keyed by the GLOBAL
+// row, as dropout is, so a shard of a batch draws what the whole batch draws.  Every TD3 target entry point applies it.
+SS_HD void td3_smooth(uint64_t seed, uint64_t counter, int64_t row, float sigma, float clip, float *a0, float *a1) {
+    float z[4];
+    normal4(seed, kTagTargetNoise, (uint32_t)row, (uint32_t)((uint64_t)row >> 32), counter, z);
+    *a0 = fminf(fmaxf(*a0 + fminf(fmaxf(sigma * z[0], -clip), clip), -1.0f), 1.0f);
+    *a1 = fminf(fmaxf(*a1 + fminf(fmaxf(sigma * z[1], -clip), clip), -1.0f), 1.0f);
 }
 
 #ifdef __CUDACC__

@@ -375,5 +375,11 @@ __device__ __forceinline__ void stage_weights(const Stager &S) {
 int frames_layer1_tc(const float *params, const void *xt, int frames, int64_t n, void *h1, cudaStream_t st);
 // reduce_parts_kernel (ss_mlp_grad_tc.cu): grad[p] = fixed-order sum of `parts` slices of n_params + 1 floats, aux = extra slot
 int reduce_slices(const float *work, int parts, int n_params, float *grad, float *aux, cudaStream_t st);
+// the TD3 target's two CUDA-core steps around the tensor-core forwards (ss_mlp_grad_tc.cu): td3_smooth (ss_rng.cuh) on the
+// target actions act[n][2] of global rows row_offset.., in place; y = reward + gamma (1 - done) min(q1, q2)
+int td3_smooth_actions(float *act, int64_t n, float sigma, float clip, uint64_t seed, uint64_t counter, int64_t row_offset,
+                       cudaStream_t st);
+int td3_min_target(const float *q1, const float *q2, const float *reward, const uint8_t *done, float gamma, float *y, int64_t n,
+                   cudaStream_t st);
 
 }  // namespace sstc

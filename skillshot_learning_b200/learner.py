@@ -113,6 +113,27 @@ def ranks_agree(refusal: Optional[str], config, group=True):
                 raise ValueError("rank %d passed %s = %r, rank 0 %r" % (r, field, value, base.get(field)))
 
 
+def check_td3_options(twin_critics, policy_delay, target_noise, target_noise_clip, group=None):
+    """ValueError unless policy_delay >= 1, target_noise >= 0 and target_noise_clip >= 0.  Sharded (group not None): every
+    rank checks its own arguments and ranks_agree compares the refusals and the four values, so every rank raises the
+    same ValueError or none does -- a rank with another twin_critics or policy_delay would otherwise wait forever in a
+    collective of a step the others do not run."""
+    refusal = None
+    if int(policy_delay) != policy_delay or policy_delay < 1:
+        refusal = "policy_delay must be an integer >= 1, got %r" % (policy_delay,)
+    elif not float(target_noise) >= 0.0:
+        refusal = "target_noise must be >= 0, got %r" % (target_noise,)
+    elif not float(target_noise_clip) >= 0.0:
+        refusal = "target_noise_clip must be >= 0, got %r" % (target_noise_clip,)
+    if group is None:
+        if refusal is not None:
+            raise ValueError(refusal)
+        return
+    check_process_group(group)
+    ranks_agree(refusal, (("twin_critics", bool(twin_critics)), ("policy_delay", policy_delay), ("target_noise", float(target_noise)),
+                          ("target_noise_clip", float(target_noise_clip))), group)
+
+
 def _device_collective(t: torch.Tensor, g) -> bool:
     """True when a collective of group `g` takes `t` where it lies (a CUDA tensor and an NCCL backend); gloo takes a CPU copy."""
     import torch.distributed as dist
@@ -213,11 +234,27 @@ class ActorCritic:
     Dropout(0.2) in the critic (SkillshotLearner.py:105).  gamma = 0 and tau = 1
     are the reference's update (critic regresses on the immediate reward, no
     target network); other values give DDPG proper.
+
+    TD3 (no reference code, DESIGN.md section 6.14): twin_critics adds a second critic with its own slices of every
+    buffer, [actor | pad | critic | pad | critic2], its own Adam step counter and its own initialisation (the critic's
+    initialisers from a seed derived from `seed`).  One TD3 update (td3_step) computes
+        y = r + gamma (1 - done) min(Q1'(s', a~), Q2'(s', a~)),  a~ = clamp(mu'(s') + clamp(target_noise eps, -c, c), -1, 1)
+    with c = target_noise_clip (one critic without twin_critics; no draw when target_noise = 0), runs a critic step on
+    critic 1 and then on critic 2 against that y, and on every policy_delay-th update only the actor step against
+    critic 1.  The targets of all networks are soft-updated on those delayed updates only: the other updates pass tau = 0
+    to the Adam kernels, and target = 0 w + 1 target leaves every target byte-identical.  The defaults (False, 1, 0, any
+    clip) are the DDPG update of this class, with the same allocations and checkpoints.
     """
 
     def __init__(self, device="cuda", seed: int = 0, lr_actor: float = 1e-3, lr_critic: float = 1e-3,
                  gamma: float = 0.0, tau: float = 1.0, dropout: float = 0.2, process_group=None,
-                 update_precision: str = "f32", collective: str = "nccl", frames: int = 1):
+                 update_precision: str = "f32", collective: str = "nccl", frames: int = 1, twin_critics: bool = False,
+                 policy_delay: int = 1, target_noise: float = 0.0, target_noise_clip: float = 0.5):
+        check_td3_options(twin_critics, policy_delay, target_noise, target_noise_clip, process_group)
+        self.twin_critics, self.policy_delay = bool(twin_critics), int(policy_delay)
+        self.target_noise, self.target_noise_clip = float(target_noise), float(target_noise_clip)
+        # any non-default option: the TD3 update (td3_step) instead of the DDPG one
+        self.td3 = self.twin_critics or self.policy_delay > 1 or self.target_noise > 0.0
         if not torch.cuda.is_available():
             raise RuntimeError("skillshot_learning_b200 needs a CUDA device (no CPU fallback)")
         # frames > 1: the frame-stacked "planning" networks of readme.md:18-20 (no reference code): both first layers read
@@ -247,9 +284,12 @@ class ActorCritic:
                      if (process_group is not None and collective == "peer") else None)
         dev = self.device
         A_N, C_N = self.a_n, self.c_n
-        # one allocation: [actor | pad | critic] so both vectors are 16-byte aligned
+        # one allocation: [actor | pad | critic] so both vectors are 16-byte aligned (twin critics: [.. | pad | critic2])
         self._a_off, self._c_off = 0, (A_N + 3) // 4 * 4
         total = self._c_off + C_N
+        if self.twin_critics:
+            self._c2_off = (total + 3) // 4 * 4
+            total = self._c2_off + C_N
         self.params = torch.zeros(total, dtype=torch.float32, device=dev)
         self.grads = torch.zeros(total, dtype=torch.float32, device=dev)
         self.adam_m = torch.zeros(total, dtype=torch.float32, device=dev)
@@ -262,6 +302,10 @@ class ActorCritic:
         self.workspace = torch.empty(self._ws_base, dtype=torch.uint8, device=dev)
         self.step_actor = 0
         self.step_critic = 0
+        if self.twin_critics:
+            self.step_critic2 = 0
+            self.critic2_sse = torch.zeros(1, dtype=torch.float32, device=dev)    # critic 2's sum sq err of its last step
+        self.td3_updates = 0        # TD3 updates so far: phases the delayed actor / target updates
         self.counter = 0            # Philox counter: advances with every noisy call
         self._update_args = None    # cached ss_ddpg_update argument block (pointers change rarely)
         self._pair_mail = None      # ss_actor_critic_forward_tc's mailbox, allocated with the argument block
@@ -284,16 +328,24 @@ class ActorCritic:
     def target_critic(self):
         return self.target[self._c_off:self._c_off + self.c_n]
 
-    def _slice(self, buf, which):
-        return buf[self._a_off:self._a_off + self.a_n] if which == "actor" else buf[self._c_off:self._c_off + self.c_n]
+    @property
+    def critic2(self):
+        return self._slice(self.params, "critic2")
 
-    def init_weights(self, seed: int):
-        """Keras initialisers of the reference's layers: actor kernels RandomNormal(0, 0.05)
-        (SkillshotLearner.py:74), critic hidden kernels glorot-uniform (the Dense default),
-        critic output kernel "RandomNormal" = N(0, 0.05) (SkillshotLearner.py:113), biases 0."""
-        g = torch.Generator(device="cpu")
-        g.manual_seed(int(seed))
-        a = [torch.randn(s, generator=g) * 0.05 if len(s) == 2 else torch.zeros(s) for s in self.actor_shapes]
+    @property
+    def target_critic2(self):
+        return self._slice(self.target, "critic2")
+
+    def _slice(self, buf, which):
+        if which == "actor":
+            return buf[self._a_off:self._a_off + self.a_n]
+        if which == "critic2":
+            if not self.twin_critics:
+                raise ValueError("critic2 exists with twin_critics=True only")
+            return buf[self._c2_off:self._c2_off + self.c_n]
+        return buf[self._c_off:self._c_off + self.c_n]
+
+    def _critic_init(self, g):
         c = []
         for i, s in enumerate(self.critic_shapes):
             if len(s) == 1:
@@ -303,22 +355,46 @@ class ActorCritic:
             else:
                 lim = float(np.sqrt(6.0 / (s[0] + s[1])))
                 c.append((torch.rand(s, generator=g) * 2.0 - 1.0) * lim)
-        self.set_weights(torch.cat([t.reshape(-1) for t in a]), torch.cat([t.reshape(-1) for t in c]))
+        return torch.cat([t.reshape(-1) for t in c])
 
-    def set_weights(self, actor=None, critic=None, reset_optimizer: bool = True):
-        """Install flat parameter vectors (Keras get_weights() order); targets are set equal."""
+    def init_weights(self, seed: int):
+        """Keras initialisers of the reference's layers: actor kernels RandomNormal(0, 0.05)
+        (SkillshotLearner.py:74), critic hidden kernels glorot-uniform (the Dense default),
+        critic output kernel "RandomNormal" = N(0, 0.05) (SkillshotLearner.py:113), biases 0.
+        Twin critics: critic 2 takes the critic's initialisers from its own generator, seeded with `seed` mixed by a
+        64-bit odd constant, so that it differs from critic 1."""
+        g = torch.Generator(device="cpu")
+        g.manual_seed(int(seed))
+        a = [torch.randn(s, generator=g) * 0.05 if len(s) == 2 else torch.zeros(s) for s in self.actor_shapes]
+        c = self._critic_init(g)
+        c2 = None
+        if self.twin_critics:
+            g2 = torch.Generator(device="cpu")
+            g2.manual_seed((int(seed) * 0x9E3779B97F4A7C15 + 0x632BE59BD9B4E019) % (1 << 63))
+            c2 = self._critic_init(g2)
+        self.set_weights(torch.cat([t.reshape(-1) for t in a]), c, critic2=c2)
+
+    def set_weights(self, actor=None, critic=None, reset_optimizer: bool = True, *, critic2=None):
+        """Install flat parameter vectors (Keras get_weights() order); targets are set equal.  critic2: the second critic
+        of twin critics (ValueError without them)."""
+        if critic2 is not None and not self.twin_critics:
+            raise ValueError("critic2 needs twin_critics=True")
         if actor is not None:
             self.actor.copy_(_f32(actor, self.device, (self.a_n,)))
         if critic is not None:
             self.critic.copy_(_f32(critic, self.device, (self.c_n,)))
+        if critic2 is not None:
+            self.critic2.copy_(_f32(critic2, self.device, (self.c_n,)))
         self.target.copy_(self.params)
         if reset_optimizer:
             self.adam_m.zero_()
             self.adam_v.zero_()
             self.step_actor = self.step_critic = 0
+            if self.twin_critics:
+                self.step_critic2 = 0
 
     def get_weights(self, which="actor"):
-        """List of numpy arrays like keras Model.get_weights()."""
+        """List of numpy arrays like keras Model.get_weights() ("actor", "critic" or, with twin critics, "critic2")."""
         flat = self._slice(self.params, which).detach().cpu().numpy()
         return [w.copy() for w in split_params(flat, self.actor_shapes if which == "actor" else self.critic_shapes)]
 
@@ -390,9 +466,11 @@ class ActorCritic:
                                         _stream(self.device)), "ss_critic_forward")
         return q
 
-    def td_targets(self, reward, next_obs, done=None):
+    def td_targets(self, reward, next_obs, done=None, row_offset: int = 0):
         """y = r + gamma (1 - done) Q'(s', mu'(s')); gamma = 0 returns the reward itself
-        (the reference's critic target, SkillshotLearner.py:434)."""
+        (the reference's critic target, SkillshotLearner.py:434).  With the TD3 options the target is the class
+        docstring's (ss_td3_targets*): the smoothing draw is keyed by the global row (row_offset + i) and the Philox
+        counter, which then advances; target_noise = 0 draws nothing."""
         reward = _f32(reward, self.device).reshape(-1)
         if self.gamma == 0.0:
             return reward
@@ -401,6 +479,21 @@ class ActorCritic:
         if done is not None:
             done = done.to(device=self.device, dtype=torch.uint8).contiguous()
         n = reward.shape[0]
+        if self.td3:
+            if self.update_precision == "bf16":
+                ws = self._workspace_for(n)
+                fn, args = ((lib.ss_td3_targets_frames_tc, (self.frames,)) if self.frames > 1 else (lib.ss_td3_targets_tc, ()))
+            else:
+                ws, fn, args = None, lib.ss_td3_targets_frames, (self.frames,)
+            with torch.cuda.device(self.device):
+                check(fn(self.target_actor.data_ptr(), self.target_critic.data_ptr(),
+                         self.target_critic2.data_ptr() if self.twin_critics else None, *args, reward.data_ptr(),
+                         next_obs.data_ptr(), _ptr(done), self.gamma, self.target_noise, self.target_noise_clip, self.seed,
+                         self.counter, int(row_offset), y.data_ptr(), n, _ptr(ws), 0 if ws is None else ws.numel(),
+                         _stream(self.device)), "ss_td3_targets")
+            if self.target_noise > 0.0:
+                self.counter += 1
+            return y
         with torch.cuda.device(self.device):
             if self.update_precision == "bf16" and self.frames > 1:
                 ws = self._workspace_for(n)
@@ -436,26 +529,33 @@ class ActorCritic:
     def _allreduce(self, t):
         allreduce_sum(t, self.group)
 
-    def critic_grad(self, obs, act, y, keep=None, n_global: int = 0, row_offset: int = 0, slices_only: bool = False):
+    def _sse(self, which: str) -> torch.Tensor:
+        """The device slot of a critic's sum of squared errors: stats[0] for critic 1, critic2_sse for critic 2."""
+        return self.critic2_sse if which == "critic2" else self.stats[0:1]
+
+    def critic_grad(self, obs, act, y, keep=None, n_global: int = 0, row_offset: int = 0, slices_only: bool = False,
+                    which: str = "critic"):
         """grads[critic] <- d/dphi mean (q - y)^2 of this (shard of a) batch; returns the gradient view.
-        slices_only: leave the per-CTA slices in the workspace and return their number (peer exchange)."""
+        slices_only: leave the per-CTA slices in the workspace and return their number (peer exchange).
+        which: "critic", or "critic2" with twin critics (its own slices of params / grads, its sum in critic2_sse)."""
         obs, act = _f32(obs, self.device).reshape(-1, 12 * self.frames), _f32(act, self.device).reshape(-1, 2)
         y = _f32(y, self.device).reshape(-1)
         n = obs.shape[0]
         if keep is not None:
             keep = torch.as_tensor(keep).to(device=self.device, dtype=torch.uint8).contiguous()
-        g = self._slice(self.grads, "critic")
+        g = self._slice(self.grads, which)
+        phi = self._slice(self.params, which)
         ws = self._workspace_for(n)
         tail = (_ptr(keep), self.dropout, self.seed, self.counter, n, int(n_global), int(row_offset),
-                None if slices_only else g.data_ptr(), self.stats[0:1].data_ptr(), ws.data_ptr(), ws.numel(), _stream(self.device))
+                None if slices_only else g.data_ptr(), self._sse(which).data_ptr(), ws.data_ptr(), ws.numel(), _stream(self.device))
         with torch.cuda.device(self.device):
             if self.update_precision == "bf16" and self.frames > 1:
-                rc = lib.ss_critic_grad_frames_tc(self.critic.data_ptr(), self.frames, obs.data_ptr(), act.data_ptr(), y.data_ptr(),
+                rc = lib.ss_critic_grad_frames_tc(phi.data_ptr(), self.frames, obs.data_ptr(), act.data_ptr(), y.data_ptr(),
                                                   *tail)
             elif self.update_precision == "bf16":
-                rc = lib.ss_critic_grad_tc(self.critic.data_ptr(), obs.data_ptr(), act.data_ptr(), y.data_ptr(), *tail)
+                rc = lib.ss_critic_grad_tc(phi.data_ptr(), obs.data_ptr(), act.data_ptr(), y.data_ptr(), *tail)
             else:
-                rc = lib.ss_critic_grad_frames(self.critic.data_ptr(), self.frames, obs.data_ptr(), act.data_ptr(), y.data_ptr(), *tail)
+                rc = lib.ss_critic_grad_frames(phi.data_ptr(), self.frames, obs.data_ptr(), act.data_ptr(), y.data_ptr(), *tail)
         self.counter += 1
         if slices_only and rc > 0:
             return rc
@@ -481,16 +581,23 @@ class ActorCritic:
         check(rc, "ss_actor_grad")
         return g
 
-    def apply_adam(self, which: str, grad_scale: float = 1.0, from_peers: bool = False):
-        """tf.keras Adam.apply_gradients on one network (+ soft target update with self.tau).
-        from_peers: the gradient is the rank-ordered sum of this rank's peer inbox (fused exchange)."""
-        n = self.a_n if which == "actor" else self.c_n
+    def _next_step(self, which: str):
+        """Advance the Adam step counter of network `which`; returns (step, learning rate)."""
         if which == "actor":
             self.step_actor += 1
-            step, lr = self.step_actor, self.lr_actor
-        else:
-            self.step_critic += 1
-            step, lr = self.step_critic, self.lr_critic
+            return self.step_actor, self.lr_actor
+        if which == "critic2":
+            self.step_critic2 += 1
+            return self.step_critic2, self.lr_critic
+        self.step_critic += 1
+        return self.step_critic, self.lr_critic
+
+    def apply_adam(self, which: str, grad_scale: float = 1.0, from_peers: bool = False, tau: Optional[float] = None):
+        """tf.keras Adam.apply_gradients on one network (+ soft target update with self.tau, or `tau` when given).
+        from_peers: the gradient is the rank-ordered sum of this rank's peer inbox (fused exchange)."""
+        n = self.a_n if which == "actor" else self.c_n
+        step, lr = self._next_step(which)
+        tau = self.tau if tau is None else float(tau)
         if from_peers:
             px = self.peer
             with torch.cuda.device(self.device):
@@ -498,64 +605,82 @@ class ActorCritic:
                                           self._slice(self.params, which).data_ptr(), self._slice(self.adam_m, which).data_ptr(),
                                           self._slice(self.adam_v, which).data_ptr(), self._slice(self.target, which).data_ptr(),
                                           self._slice(self.grads, which).data_ptr(), n, step, lr, self.beta1, self.beta2,
-                                          self.eps, self.tau, float(grad_scale), px.status.data_ptr(), _stream(self.device)),
+                                          self.eps, tau, float(grad_scale), px.status.data_ptr(), _stream(self.device)),
                       "ss_peer_adam_tf")
             return
         with torch.cuda.device(self.device):
             check(lib.ss_adam_tf(self._slice(self.params, which).data_ptr(), self._slice(self.grads, which).data_ptr(),
                                  self._slice(self.adam_m, which).data_ptr(), self._slice(self.adam_v, which).data_ptr(),
                                  self._slice(self.target, which).data_ptr(), n, step, lr, self.beta1, self.beta2,
-                                 self.eps, self.tau, float(grad_scale), _stream(self.device)), "ss_adam_tf")
+                                 self.eps, tau, float(grad_scale), _stream(self.device)), "ss_adam_tf")
 
-    def reduce_adam(self, which: str, parts: int, aux: Optional[torch.Tensor], grad_scale: float = 1.0):
+    def reduce_adam(self, which: str, parts: int, aux: Optional[torch.Tensor], grad_scale: float = 1.0,
+                    tau: Optional[float] = None):
         """Single GPU: fixed-order sum of the `parts` gradient slices in the workspace + Adam + soft update, one kernel."""
         n = self.a_n if which == "actor" else self.c_n
-        if which == "actor":
-            self.step_actor += 1
-            step, lr = self.step_actor, self.lr_actor
-        else:
-            self.step_critic += 1
-            step, lr = self.step_critic, self.lr_critic
+        step, lr = self._next_step(which)
+        tau = self.tau if tau is None else float(tau)
         with torch.cuda.device(self.device):
             check(lib.ss_reduce_adam_tf(self.workspace.data_ptr(), int(parts), n, _ptr(aux), self._slice(self.grads, which).data_ptr(),
                                         self._slice(self.params, which).data_ptr(), self._slice(self.adam_m, which).data_ptr(),
                                         self._slice(self.adam_v, which).data_ptr(), self._slice(self.target, which).data_ptr(),
-                                        step, lr, self.beta1, self.beta2, self.eps, self.tau, float(grad_scale),
+                                        step, lr, self.beta1, self.beta2, self.eps, tau, float(grad_scale),
                                         _stream(self.device)), "ss_reduce_adam_tf")
 
-    def critic_step(self, obs, act, y, keep=None):
+    def critic_step(self, obs, act, y, keep=None, which: str = "critic", tau: Optional[float] = None):
         """One batch of model_critic.fit (SkillshotLearner.py:434): gradient of the batch-mean
-        squared error, summed over the ranks when sharded, then Adam.  Returns the (device) sum of squared errors."""
+        squared error, summed over the ranks when sharded, then Adam.  Returns the (device) sum of squared errors.
+        which: "critic" or "critic2" (twin critics); tau: the soft update's tau instead of self.tau (TD3: 0 between
+        delayed updates)."""
         _, n_global, row_offset = shard_info(int(np.prod(y.shape)), self.group)
+        sse = self._sse(which)
         if self.group is not None and self.peer is None:      # NCCL: gradient -> all-reduce -> Adam
-            g = self.critic_grad(obs, act, y, keep, n_global=n_global, row_offset=row_offset)
+            g = self.critic_grad(obs, act, y, keep, n_global=n_global, row_offset=row_offset, which=which)
             self._allreduce(g)
-            self.apply_adam("critic")
-            return self.stats[0]
+            self.apply_adam(which, tau=tau)
+            return sse[0]
         # per-CTA slices -> one kernel that sums them and applies Adam (single GPU), or pushes the sum into every
         # rank's inbox for the peers' Adam kernel (fused exchange)
-        parts = self.critic_grad(obs, act, y, keep, n_global=n_global, row_offset=row_offset, slices_only=True)
+        parts = self.critic_grad(obs, act, y, keep, n_global=n_global, row_offset=row_offset, slices_only=True, which=which)
         if self.peer is not None:
-            self.peer.reduce_push(self.workspace, parts, self.c_n, self.stats[0:1])
-            self.apply_adam("critic", from_peers=True)
+            self.peer.reduce_push(self.workspace, parts, self.c_n, sse)
+            self.apply_adam(which, from_peers=True, tau=tau)
         else:
-            self.reduce_adam("critic", parts, self.stats[0:1])
-        return self.stats[0]
+            self.reduce_adam(which, parts, sse, tau=tau)
+        return sse[0]
 
-    def actor_step(self, obs):
+    def actor_step(self, obs, tau: Optional[float] = None):
         """model_actor_fit_step (SkillshotLearner.py:386-417).  Returns the (device) sum of q."""
         if self.group is not None and self.peer is None:
             g = self.actor_grad(obs)
             self._allreduce(g)
-            self.apply_adam("actor")
+            self.apply_adam("actor", tau=tau)
             return self.stats[1]
         parts = self.actor_grad(obs, slices_only=True)
         if self.peer is not None:
             self.peer.reduce_push(self.workspace, parts, self.a_n, self.stats[1:2])
-            self.apply_adam("actor", from_peers=True)
+            self.apply_adam("actor", from_peers=True, tau=tau)
         else:
-            self.reduce_adam("actor", parts, self.stats[1:2])
+            self.reduce_adam("actor", parts, self.stats[1:2], tau=tau)
         return self.stats[1]
+
+    def td3_step(self, obs, act, reward, next_obs, done=None):
+        """One TD3 update on a (shard of a) minibatch (class docstring): the target, a critic step on critic 1 and one on
+        critic 2 against the same y (each with its own Philox dropout draw: the counter advances per call), and on every
+        policy_delay-th update the actor step against critic 1.  Only those delayed updates soft-update the targets; the
+        others pass tau = 0, which leaves every target byte-identical.  Returns (critic 1's sum of squared errors, the
+        sum of q of the last actor step), device scalars; critic 2's sum is in critic2_sse."""
+        _, _, row_offset = shard_info(int(np.prod(reward.shape)), self.group)
+        y = self.td_targets(reward, next_obs, done, row_offset=row_offset)
+        delayed = (self.td3_updates + 1) % self.policy_delay == 0
+        tau = self.tau if delayed else 0.0
+        sse = self.critic_step(obs, act, y, tau=tau)
+        if self.twin_critics:
+            self.critic_step(obs, act, y, which="critic2", tau=tau)
+        if delayed:
+            self.actor_step(obs, tau=tau)
+        self.td3_updates += 1
+        return sse, self.stats[1]
 
     def update_from_ring(self, ring: "ReplayRing", batch: int, out: Optional[dict] = None, sample_early: bool = False):
         """One whole update step from ONE library call (ss_ddpg_update): sample `batch` rows of `ring`,
@@ -640,11 +765,32 @@ class ActorCritic:
 
     # -- checkpoint ------------------------------------------------------------
     def state_dict(self):
-        return dict(params=self.params.cpu(), target=self.target.cpu(), adam_m=self.adam_m.cpu(),
-                    adam_v=self.adam_v.cpu(), step_actor=self.step_actor, step_critic=self.step_critic,
-                    counter=self.counter, seed=self.seed)
+        sd = dict(params=self.params.cpu(), target=self.target.cpu(), adam_m=self.adam_m.cpu(),
+                  adam_v=self.adam_v.cpu(), step_actor=self.step_actor, step_critic=self.step_critic,
+                  counter=self.counter, seed=self.seed)
+        if self.td3:            # (the flat buffers above already hold critic 2's slices)
+            sd["td3_updates"] = self.td3_updates
+        if self.twin_critics:
+            sd["step_critic2"] = self.step_critic2
+        return sd
+
+    def check_state_dict(self, sd):
+        """ValueError for a checkpoint of one critic into a twin-critic learner, of twin critics into a one-critic
+        learner, or of another parameter layout."""
+        twin = "step_critic2" in sd
+        if twin != self.twin_critics:
+            raise ValueError("a checkpoint of %s does not load into a learner with %s"
+                             % (("twin critics", "one critic") if twin else ("one critic", "twin critics")))
+        if sd["params"].numel() != self.params.numel():
+            raise ValueError("checkpoint parameter layout of %d floats, this learner's %d" % (sd["params"].numel(), self.params.numel()))
 
     def load_state_dict(self, sd):
+        """check_state_dict's refusals come before anything is copied."""
+        self.check_state_dict(sd)
+        twin = "step_critic2" in sd
+        if twin:
+            self.step_critic2 = int(sd["step_critic2"])
+        self.td3_updates = int(sd.get("td3_updates", 0))
         for k in ("params", "target", "adam_m", "adam_v"):
             getattr(self, k).copy_(sd[k].to(self.device))
         self.step_actor, self.step_critic = int(sd["step_actor"]), int(sd["step_critic"])
@@ -1213,7 +1359,8 @@ class SelfPlayTrainer:
                  noise_group: int = 128, reward_mode: str = "looking", tick_limit: int = 2000,
                  random_positions: bool = True, process_group=None, precision: str = "f32", collective: str = "nccl",
                  frames: int = 1, update_precision: Optional[str] = None, opponents=None, pool_envs: Optional[int] = None,
-                 pool_blocks=None):
+                 pool_blocks=None, twin_critics: bool = False, policy_delay: int = 1, target_noise: float = 0.0,
+                 target_noise_clip: float = 0.5):
         """frames > 1: the frame-stacked "planning" networks (readme.md:18-20, BASELINE.json configs[4]): both players act
         from their last `frames` observations (FrameStackActor; `precision` selects its float32 or tensor-core kernels),
         the replay ring stores the stacked observations, and the critic / actor update of SkillshotLearner.py:386-443 runs
@@ -1236,7 +1383,11 @@ class SelfPlayTrainer:
         ranks' refusals and configurations: when any rank refused or one differs, every rank raises the same ValueError
         before anything is allocated.  The opponents are then broadcast from group rank 0.  Every pool method
         (set_opponent, set_pool_blocks, rebalance_pool, pool_progress) is collective: call it on every rank with the same
-        arguments, as update().  save / load write and read each rank's own file."""
+        arguments, as update().  save / load write and read each rank's own file.
+        twin_critics, policy_delay, target_noise, target_noise_clip: the TD3 update of ActorCritic (DESIGN.md section 6.14),
+        which update() then runs through update_stepwise; the defaults are the DDPG update.  Bad values raise ValueError
+        before anything is allocated (sharded: on every rank, when any rank refused or passed other values)."""
+        check_td3_options(twin_critics, policy_delay, target_noise, target_noise_clip, process_group)
         self.device = torch.device(device)
         self.frames = int(frames)
         self.opponents, self.pool_envs, self.pool_stats = None, 0, None
@@ -1288,7 +1439,8 @@ class SelfPlayTrainer:
         self.networks = ActorCritic(device=device, seed=seed if process_group is None else 0, gamma=gamma, tau=tau,
                                     process_group=process_group,
                                     update_precision=update_precision or (precision if self.frames == 1 else "f32"),
-                                    collective=collective, frames=self.frames)
+                                    collective=collective, frames=self.frames, twin_critics=twin_critics,
+                                    policy_delay=policy_delay, target_noise=target_noise, target_noise_clip=target_noise_clip)
         self.networks.seed = seed          # exploration / dropout streams differ per rank, weights do not
         self.replay = ReplayRing(replay_capacity or L * 8, device=device, seed=seed, frames=self.frames)
         self.batch_size, self.param_noise_sd, self.noise_group = int(batch_size), float(param_noise_sd), int(noise_group)
@@ -1645,6 +1797,7 @@ class SelfPlayTrainer:
         if have != want:
             raise ValueError("checkpoint pool layout (pool_envs, opponents, frames, opponent frames) = %s, this trainer's %s"
                              % (want, have))
+        self.networks.check_state_dict(sd["networks"])
         self.envs.load_state_dict(sd["envs"])
         self.networks.load_state_dict(sd["networks"])
         self.replay.load_state_dict(sd["replay"])
@@ -1763,9 +1916,10 @@ class SelfPlayTrainer:
 
     def update(self):
         """One critic step and one actor step on a sampled minibatch: a single library call on one GPU or
-        with the fused peer exchange, the separate steps (update_stepwise) around an NCCL all-reduce."""
+        with the fused peer exchange, the separate steps (update_stepwise) around an NCCL all-reduce, for frames > 1 and
+        for the TD3 update (any of the four TD3 options not at its default)."""
         net = self.networks
-        if (net.group is not None and net.peer is None) or self.frames > 1:
+        if (net.group is not None and net.peer is None) or self.frames > 1 or net.td3:
             return self.update_stepwise()
         # two sets of minibatch buffers in turn: when no rollout has touched the ring since the previous update, this
         # update's rows are drawn while that update's last kernels still run (ss_ddpg_update_args.sample_early)
@@ -1781,10 +1935,13 @@ class SelfPlayTrainer:
         return net.stats[0], net.stats[1]
 
     def update_stepwise(self):
-        """The same update as one library call per step (sample, target, critic step, actor step)."""
+        """The same update as one library call per step (sample, target, critic step, actor step); with the TD3 options,
+        ActorCritic.td3_step on the minibatch."""
         self._ring_clean = False
         self._batch = b = self.replay.sample(self.batch_size, out=self._batch)
         net = self.networks
+        if net.td3:
+            return net.td3_step(b["obs"], b["act"], b["reward"], b["next_obs"], b["done"])
         y = net.td_targets(b["reward"], b["next_obs"], b["done"])
         sse = net.critic_step(b["obs"], b["act"], y)
         q = net.actor_step(b["obs"])
