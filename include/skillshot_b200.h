@@ -490,6 +490,34 @@ int ss_replay_sample_frames(const float *ring_obs, const float *ring_act, const 
                             float *obs, float *act, float *reward, float *next_obs, uint8_t *done, int64_t *indices_out,
                             void *stream);
 
+/* ---- n-step rows of the replay ring (no reference code, DESIGN.md section 6.15) ----
+ * A ring written one block of tick_rows rows per tick (2 n_envs for self-play, the learner's rows of a pool) holds the same
+ * player's next transition after row r at row (r + tick_rows) mod capacity.  Row r is drawn uniformly from the eligible rows:
+ * the runs [start, start + length) of ring positions in runs_host[2 n_runs] = {start_0, length_0, start_1, ...}, taken in
+ * order; the draw is ss_replay_sample's Philox word x (tag kTagReplay, row b, counter) as j = (x * total) >> 32 with total
+ * = the sum of the lengths, and j picks the j-th row of the runs.  With one run [0, size) the rows are ss_replay_sample's,
+ * bit for bit.  The walk then visits r_t = (r + t tick_rows) mod capacity, t = 0 .. n_step - 1, and stops after the first
+ * row whose done flag is set; k rows visited.
+ *   obs, act, indices_out  row r's (indices_out may be NULL)
+ *   reward                 sum over t < k of g_t reward[r_t] in float32, increasing t, each product and sum rounded
+ *                          (no FMA); g_0 = 1, g_{t+1} = g_t * gamma in float32
+ *   next_obs, done         row r_{k-1}'s
+ *   steps_out              k (uint8, may be NULL)
+ * The TD target is then reward + g_n (1 - done) Q'(next_obs, .) with g_n of the same recurrence: pass it as the gamma of
+ * ss_ddpg_targets* / ss_td3_targets* / ss_ddpg_update.  Which rows are eligible (no walk passes the newest stored tick or a
+ * break in the players' trajectories) is the caller's; the library checks only that every run lies inside the ring.
+ * Every argument is checked before anything is enqueued: NULL pointers (but indices_out, steps_out), frames out of
+ * 1..SS_MAX_FRAMES, n_step out of 1..SS_REPLAY_MAX_NSTEP, tick_rows < 1, n_step * tick_rows > capacity, n_runs out of
+ * 1..SS_REPLAY_MAX_RUNS, a run with start < 0, length < 1 or past the capacity, a total of 2^32 rows or more, a gamma that
+ * is not finite and observation pointers that are not 16-byte aligned return SS_ERR_INVALID_ARG. */
+#define SS_REPLAY_MAX_RUNS 16
+#define SS_REPLAY_MAX_NSTEP 32
+int ss_replay_sample_nstep(const float *ring_obs, const float *ring_act, const float *ring_reward, const float *ring_next_obs,
+                           const uint8_t *ring_done, int64_t capacity, int frames, int64_t tick_rows, int n_step, float gamma,
+                           const int64_t *runs_host, int n_runs, uint64_t seed, uint64_t counter, int64_t batch, float *obs,
+                           float *act, float *reward, float *next_obs, uint8_t *done, int64_t *indices_out, uint8_t *steps_out,
+                           void *stream);
+
 /* ---- matches: two actors against each other (no reference code; the readme's "does the planning actor play better" question) ----
  * A match is n_envs games between policy A and policy B, ONE game per env (no auto-reset: every game starts at tick 0 and
  * is played to a hit or to tick_limit ticks, so no outcome is sampled by its length).  Seat map, split index 0 <= split <= n_envs:
@@ -906,6 +934,13 @@ typedef struct ss_ddpg_update_args {
                                                   (obs .. y, indices) -- e.g. the previous ss_ddpg_update used another set of
                                                   buffers and no rollout came between: the minibatch is then gathered while
                                                   that launch still runs.  0: the gather waits for it */
+    int n_step;                                /* 0 or 1: one-step rows (ss_replay_sample), the fields below unused;
+                                                  2..SS_REPLAY_MAX_NSTEP: n-step rows (ss_replay_sample_nstep), and gamma
+                                                  above is then the bootstrap factor g_n of that recurrence */
+    int64_t tick_rows;                         /* ring rows per tick (ss_replay_sample_nstep) */
+    int n_runs;                                /* eligible runs: runs_host[2 n_runs] = {start, length, ...} (host memory) */
+    const int64_t *runs_host;
+    float step_gamma;                          /* the per-tick gamma of the n-step reward sum's weights */
 } ss_ddpg_update_args;
 int ss_ddpg_update(const ss_ddpg_update_args *args, void *stream);
 

@@ -45,6 +45,8 @@ LEAGUE_MAX_POLICIES = 64          # SS_LEAGUE_MAX_POLICIES
 STATUS_SEAT_RANGE = 8             # SS_STATUS_SEAT_RANGE
 POOL_STATS = 8                    # uint64 counters per opponent of ss_env_step_pool / ss_pool_rollout
 TAG_TARGET_NOISE = 5              # SS_TAG_TARGET_NOISE: Philox tag of the TD3 target policy smoothing
+REPLAY_MAX_RUNS = 16              # SS_REPLAY_MAX_RUNS: runs of eligible rows of one ss_replay_sample_nstep call
+REPLAY_MAX_NSTEP = 32             # SS_REPLAY_MAX_NSTEP: the longest n-step walk
 
 
 def td3_tc_workspace_bytes(n: int) -> int:
@@ -63,7 +65,10 @@ class DdpgUpdateArgs(ctypes.Structure):
                 [("seed", _u64), ("counter", _u64), ("step_critic", _i64), ("step_actor", _i64), ("n_global", _i64),
                  ("row_offset", _i64), ("workspace", _vp), ("workspace_bytes", _i64), ("tensor_cores", _i32),
                  ("world", _i32), ("rank", _i32), ("peer_bases", _vp), ("peer_capacity", _i64), ("epoch", _u32),
-                 ("done_counter", _vp), ("status", _vp), ("pair_mail", _vp), ("sample_early", _i32)])
+                 ("done_counter", _vp), ("status", _vp), ("pair_mail", _vp), ("sample_early", _i32),
+                 # n-step rows: n_step 0 / 1 one-step (the other four unused), else gamma above is g_n
+                 ("n_step", _i32), ("tick_rows", _i64), ("n_runs", _i32), ("runs_host", ctypes.POINTER(_i64)),
+                 ("step_gamma", _f32)])
 
 
 class MatchArgs(ctypes.Structure):
@@ -212,6 +217,8 @@ SIGNATURES = {
     "ss_env_step_pool_speeds": (_i32, [_vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i64, _i32, _u64,
                                         _u64, _vp, _i32, _vp, ctypes.POINTER(_i64), _vp, _vp]),
     "ss_pool_rollout_speeds": (_i32, [ctypes.POINTER(PoolRolloutFramesArgs), _vp]),
+    "ss_replay_sample_nstep": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i32, _i64, _i32, _f32, ctypes.POINTER(_i64), _i32, _u64,
+                                       _u64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "ss_replay_sample": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp, _u64, _u64, _i64,
                                  _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
 }

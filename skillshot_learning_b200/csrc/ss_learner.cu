@@ -20,6 +20,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <cmath>
+
 #include "../../include/skillshot_b200.h"
 #include "ss_launch.cuh"
 #include "ss_rng.cuh"
@@ -821,6 +823,68 @@ __global__ void replay_sample_kernel(Ring R, int64_t size, const int64_t *indice
     }
 }
 
+// n-step rows (DESIGN.md section 6.15): the eligible rows are up to SS_REPLAY_MAX_RUNS runs of ring positions; draw j of
+// their total length picks the j-th eligible row in run order
+struct NstepRuns {
+    int64_t start[SS_REPLAY_MAX_RUNS], length[SS_REPLAY_MAX_RUNS];
+    int n;
+};
+
+// replay_sample_kernel's thread per (row, float4) and draw.  The walk visits src + t * tick_rows (mod capacity) and stops
+// after the first row with its done flag set or after n_step rows; every lane of a row walks the done bytes itself (the
+// row's other lanes find them in L1) because each needs the walk's last row for its part of next_obs.  The reward sum
+// rounds each product and each sum on its own (no FMA), so that a float32 restatement of the recurrence is exact.
+__global__ void replay_sample_nstep_kernel(Ring R, NstepRuns runs, int64_t total, int64_t tick_rows, int n_step, float gamma,
+                                           uint64_t seed, uint64_t counter, int64_t batch, float *s, float *a, float *r, float *s2,
+                                           uint8_t *done, int64_t *indices_out, uint8_t *steps_out, int w4, int early) {
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (!early) {
+        sslaunch::griddep_wait();
+        sslaunch::griddep_launch();
+    }
+    if (e < w4 * batch) {
+        const int64_t b = e / w4, part = e - b * w4;
+        const U4 u = draw4(seed, kTagReplay, (uint32_t)(b / 4), (uint32_t)((b / 4) >> 32), counter);
+        const uint32_t x = (b & 3) == 0 ? u.x : (b & 3) == 1 ? u.y : (b & 3) == 2 ? u.z : u.w;
+        int64_t j = (int64_t)(((uint64_t)x * (uint64_t)total) >> 32);      // total < 2^32 rows
+        int64_t src = runs.start[0] + j;
+        for (int i = 0; i < runs.n; ++i) {
+            if (j < runs.length[i]) {
+                src = runs.start[i] + j;
+                break;
+            }
+            j -= runs.length[i];
+        }
+        int64_t last = src;
+        int k = 1;
+        for (; k < n_step && !R.done[last]; ++k) {
+            last += tick_rows;
+            if (last >= R.capacity) last -= R.capacity;
+        }
+        reinterpret_cast<float4 *>(s)[e] = reinterpret_cast<const float4 *>(R.s)[src * w4 + part];
+        reinterpret_cast<float4 *>(s2)[e] = reinterpret_cast<const float4 *>(R.s2)[last * w4 + part];
+        if (part == 0) {
+            float sum = R.r[src], g = 1.0f;
+            int64_t row = src;
+            for (int t = 1; t < k; ++t) {
+                row += tick_rows;
+                if (row >= R.capacity) row -= R.capacity;
+                g = __fmul_rn(g, gamma);
+                sum = __fadd_rn(sum, __fmul_rn(g, R.r[row]));
+            }
+            reinterpret_cast<float2 *>(a)[b] = reinterpret_cast<const float2 *>(R.a)[src];
+            r[b] = sum;
+            done[b] = R.done[last];
+            if (indices_out) indices_out[b] = src;
+            if (steps_out) steps_out[b] = (uint8_t)k;
+        }
+    }
+    if (early) {
+        sslaunch::griddep_wait();
+        sslaunch::griddep_launch();
+    }
+}
+
 // ---------------------------------------------------------------------------
 // launch helpers
 // ---------------------------------------------------------------------------
@@ -1068,6 +1132,40 @@ int ss_replay_sample_frames(const float *ring_obs, const float *ring_act, const 
     const int early = (sslaunch::pdl_mode() & sslaunch::kPdlOn) && (sslaunch::pdl_mode() & sslaunch::kPdlSampleEarly) ? 1 : 0;
     if (sslaunch::launch(replay_sample_kernel, dim3((unsigned)((w4 * batch + 255) / 256)), dim3(256), 0, (cudaStream_t)stream, R,
                          size, indices, seed, counter, batch, obs, act, reward, next_obs, done, indices_out, w4, early) != cudaSuccess)
+        return SS_ERR_CUDA;
+    return check_launch();
+}
+
+int ss_replay_sample_nstep(const float *ring_obs, const float *ring_act, const float *ring_reward, const float *ring_next_obs,
+                           const uint8_t *ring_done, int64_t capacity, int frames, int64_t tick_rows, int n_step, float gamma,
+                           const int64_t *runs_host, int n_runs, uint64_t seed, uint64_t counter, int64_t batch, float *obs,
+                           float *act, float *reward, float *next_obs, uint8_t *done, int64_t *indices_out, uint8_t *steps_out,
+                           void *stream) {
+    if (!ring_obs || !ring_act || !ring_reward || !ring_next_obs || !ring_done || !obs || !act || !reward || !next_obs ||
+        !done || !runs_host)
+        return SS_ERR_INVALID_ARG;
+    if (capacity <= 0 || batch <= 0 || frames < 1 || frames > SS_MAX_FRAMES || tick_rows < 1 || n_step < 1 ||
+        n_step > SS_REPLAY_MAX_NSTEP || tick_rows > capacity / n_step || n_runs < 1 || n_runs > SS_REPLAY_MAX_RUNS ||
+        !std::isfinite(gamma))
+        return SS_ERR_INVALID_ARG;
+    if (((uintptr_t)ring_obs | (uintptr_t)ring_next_obs | (uintptr_t)obs | (uintptr_t)next_obs) & 15) return SS_ERR_INVALID_ARG;
+    NstepRuns runs{};
+    int64_t total = 0;
+    for (int i = 0; i < n_runs; ++i) {
+        const int64_t st = runs_host[2 * i], len = runs_host[2 * i + 1];
+        if (st < 0 || len < 1 || st >= capacity || len > capacity - st) return SS_ERR_INVALID_ARG;
+        runs.start[i] = st;
+        runs.length[i] = len;
+        total += len;
+    }
+    runs.n = n_runs;
+    if (total >= ((int64_t)1 << 32)) return SS_ERR_INVALID_ARG;
+    Ring R{(float *)ring_obs, (float *)ring_act, (float *)ring_reward, (float *)ring_next_obs, (uint8_t *)ring_done, capacity};
+    const int w4 = 3 * frames;
+    const int early = (sslaunch::pdl_mode() & sslaunch::kPdlOn) && (sslaunch::pdl_mode() & sslaunch::kPdlSampleEarly) ? 1 : 0;
+    if (sslaunch::launch(replay_sample_nstep_kernel, dim3((unsigned)((w4 * batch + 255) / 256)), dim3(256), 0, (cudaStream_t)stream,
+                         R, runs, total, tick_rows, n_step, gamma, seed, counter, batch, obs, act, reward, next_obs, done,
+                         indices_out, steps_out, w4, early) != cudaSuccess)
         return SS_ERR_CUDA;
     return check_launch();
 }

@@ -41,6 +41,7 @@ extern "C" int ss_ddpg_update(const ss_ddpg_update_args *a, void *stream) {
                   !a->done_counter))
         return SS_ERR_INVALID_ARG;
     if (a->gamma != 0.f && (!a->y || !a->target_actor || !a->target_critic)) return SS_ERR_INVALID_ARG;
+    if (a->n_step < 0 || a->n_step > SS_REPLAY_MAX_NSTEP) return SS_ERR_INVALID_ARG;
     const int64_t n = a->batch;
     const bool tc = a->tensor_cores != 0;
     int rc;
@@ -63,9 +64,16 @@ extern "C" int ss_ddpg_update(const ss_ddpg_update_args *a, void *stream) {
     // minibatch (uniform with replacement from the filled part of the ring); drawn beside the previous launch's tail when the
     // caller vouches for it (args.sample_early)
     if (kOn && a->sample_early) sslaunch::pdl_mode() = kOn | sslaunch::kPdlSampleEarly;
-    rc = ss_replay_sample(a->ring_obs, a->ring_act, a->ring_reward, a->ring_next_obs, a->ring_done, a->capacity, a->size,
-                          nullptr, a->replay_seed, a->replay_counter, n, a->obs, a->act, a->reward, a->next_obs, a->done,
-                          a->indices, stream);
+    // (n-step rows: the same draw over the eligible runs, then the walk; a->gamma is g_n)
+    if (a->n_step > 1)
+        rc = ss_replay_sample_nstep(a->ring_obs, a->ring_act, a->ring_reward, a->ring_next_obs, a->ring_done, a->capacity, 1,
+                                    a->tick_rows, a->n_step, a->step_gamma, a->runs_host, a->n_runs, a->replay_seed,
+                                    a->replay_counter, n, a->obs, a->act, a->reward, a->next_obs, a->done, a->indices, nullptr,
+                                    stream);
+    else
+        rc = ss_replay_sample(a->ring_obs, a->ring_act, a->ring_reward, a->ring_next_obs, a->ring_done, a->capacity, a->size,
+                              nullptr, a->replay_seed, a->replay_counter, n, a->obs, a->act, a->reward, a->next_obs, a->done,
+                              a->indices, stream);
     if (rc != SS_OK) return rc;
 
     // critic target: the reference regresses on the reward itself (gamma = 0, SkillshotLearner.py:434)

@@ -134,6 +134,73 @@ def check_td3_options(twin_critics, policy_delay, target_noise, target_noise_cli
                           ("target_noise_clip", float(target_noise_clip))), group)
 
 
+def nstep_refusal(n_step, capacity: int, tick_rows: int) -> Optional[str]:
+    """The message of the ValueError for an n_step that is not an integer in 1..SS_REPLAY_MAX_NSTEP, or for a ring of
+    `capacity` rows shorter than n_step ticks of tick_rows rows; None when both are fine."""
+    try:
+        ok = not isinstance(n_step, bool) and int(n_step) == n_step and 1 <= int(n_step) <= _lib.REPLAY_MAX_NSTEP
+    except (TypeError, ValueError):
+        ok = False
+    if not ok:
+        return "n_step must be an integer in 1..%d, got %r" % (_lib.REPLAY_MAX_NSTEP, n_step)
+    if int(n_step) > 1 and int(capacity) < int(n_step) * int(tick_rows):
+        return "n_step = %d needs a replay capacity of at least %d rows (n_step ticks of %d), got %d" % (
+            n_step, int(n_step) * int(tick_rows), tick_rows, capacity)
+    return None
+
+
+def nstep_discount(gamma: float, n_step: int) -> float:
+    """g_n of the n-step target: g_0 = 1, g_{j+1} = g_j * gamma, each product rounded to float32 (the recurrence of the
+    reward weights of ss_replay_sample_nstep)."""
+    g, gm = np.float32(1.0), np.float32(gamma)
+    for _ in range(int(n_step)):
+        g = np.float32(g * gm)
+    return float(g)
+
+
+def nstep_runs(capacity: int, size: int, pos: int, tick_rows: int, n_step: int, breaks) -> list:
+    """The rows an n-step walk may start from, as at most SS_REPLAY_MAX_RUNS runs (start, length) of ring positions in
+    increasing order.
+
+    The ring holds `size` rows written in order, the newest just before `pos` (mod capacity), one block of tick_rows rows
+    per tick.  A walk from row r visits r, r + W, ..., r + (n_step - 1) W (W = tick_rows, mod capacity).  Each entry of
+    `breaks` is a ring position where the players' trajectories do not continue from the rows written before it into the
+    rows written from it on; the write head `pos` is one too.  A row is eligible when its walk neither passes the newest
+    row nor crosses a break: the filled rows minus the (n_step - 1) W rows written just before each break.  (A break
+    whose rows before it are all overwritten, or one at the oldest row, takes nothing away.)  With n_step = 1 every filled
+    row is eligible and the one run is (0, size).  When the eligible rows form more than SS_REPLAY_MAX_RUNS runs, the
+    oldest runs (by write order of their first row) are left out, and those rows are not drawn until the breaks between
+    them are overwritten."""
+    capacity, size, pos, W, n = int(capacity), int(size), int(pos), int(tick_rows), int(n_step)
+    if size <= 0:
+        return []
+    D = (n - 1) * W
+    oldest = (pos - size) % capacity
+    # every break as the write order of its first row after it (0 = the oldest row, size = the head)
+    cuts = sorted({o for o in ((int(b) - oldest) % capacity for b in breaks) if 0 < o < size}) + [size]
+    pieces, prev = [], 0                        # (position, length, write order of the first row)
+    for c in cuts:
+        end = c - D
+        if end > prev:
+            p, m = (oldest + prev) % capacity, end - prev
+            head = min(m, capacity - p)         # a run that wraps past the ring's last position is two runs
+            pieces.append([p, head, prev])
+            if m > head:
+                pieces.append([0, m - head, prev + head])
+        prev = c
+    pieces.sort()
+    runs = []
+    for p in pieces:                            # (adjacent only with n_step = 1: the runs of a full ring join into one)
+        if runs and runs[-1][0] + runs[-1][1] == p[0]:
+            runs[-1][1] += p[1]
+            runs[-1][2] = min(runs[-1][2], p[2])
+        else:
+            runs.append(p)
+    if len(runs) > _lib.REPLAY_MAX_RUNS:
+        runs = sorted(sorted(runs, key=lambda q: q[2])[-_lib.REPLAY_MAX_RUNS:])
+    return [(p, m) for p, m, _ in runs]
+
+
 def _device_collective(t: torch.Tensor, g) -> bool:
     """True when a collective of group `g` takes `t` where it lies (a CUDA tensor and an NCCL backend); gloo takes a CPU copy."""
     import torch.distributed as dist
@@ -466,13 +533,15 @@ class ActorCritic:
                                         _stream(self.device)), "ss_critic_forward")
         return q
 
-    def td_targets(self, reward, next_obs, done=None, row_offset: int = 0):
+    def td_targets(self, reward, next_obs, done=None, row_offset: int = 0, discount: Optional[float] = None):
         """y = r + gamma (1 - done) Q'(s', mu'(s')); gamma = 0 returns the reward itself
         (the reference's critic target, SkillshotLearner.py:434).  With the TD3 options the target is the class
         docstring's (ss_td3_targets*): the smoothing draw is keyed by the global row (row_offset + i) and the Philox
-        counter, which then advances; target_noise = 0 draws nothing."""
+        counter, which then advances; target_noise = 0 draws nothing.
+        discount: the bootstrap factor in place of gamma, e.g. nstep_discount(gamma, n) for n-step rows."""
         reward = _f32(reward, self.device).reshape(-1)
-        if self.gamma == 0.0:
+        gamma = self.gamma if discount is None else float(discount)
+        if gamma == 0.0:
             return reward
         next_obs = _f32(next_obs, self.device).reshape(-1, 12 * self.frames)
         y = torch.empty_like(reward)
@@ -488,7 +557,7 @@ class ActorCritic:
             with torch.cuda.device(self.device):
                 check(fn(self.target_actor.data_ptr(), self.target_critic.data_ptr(),
                          self.target_critic2.data_ptr() if self.twin_critics else None, *args, reward.data_ptr(),
-                         next_obs.data_ptr(), _ptr(done), self.gamma, self.target_noise, self.target_noise_clip, self.seed,
+                         next_obs.data_ptr(), _ptr(done), gamma, self.target_noise, self.target_noise_clip, self.seed,
                          self.counter, int(row_offset), y.data_ptr(), n, _ptr(ws), 0 if ws is None else ws.numel(),
                          _stream(self.device)), "ss_td3_targets")
             if self.target_noise > 0.0:
@@ -498,17 +567,17 @@ class ActorCritic:
             if self.update_precision == "bf16" and self.frames > 1:
                 ws = self._workspace_for(n)
                 check(lib.ss_ddpg_targets_frames_tc(self.target_actor.data_ptr(), self.target_critic.data_ptr(), self.frames,
-                                                    reward.data_ptr(), next_obs.data_ptr(), _ptr(done), self.gamma, y.data_ptr(),
+                                                    reward.data_ptr(), next_obs.data_ptr(), _ptr(done), gamma, y.data_ptr(),
                                                     n, ws.data_ptr(), ws.numel(), _stream(self.device)), "ss_ddpg_targets_frames_tc")
             elif self.update_precision == "bf16":
                 ws = self._workspace_for(n)
                 check(lib.ss_ddpg_targets_tc(self.target_actor.data_ptr(), self.target_critic.data_ptr(),
-                                             reward.data_ptr(), next_obs.data_ptr(), _ptr(done), self.gamma,
+                                             reward.data_ptr(), next_obs.data_ptr(), _ptr(done), gamma,
                                              y.data_ptr(), n, ws.data_ptr(), ws.numel(), _stream(self.device)),
                       "ss_ddpg_targets_tc")
             else:
                 check(lib.ss_ddpg_targets_frames(self.target_actor.data_ptr(), self.target_critic.data_ptr(), self.frames,
-                                                 reward.data_ptr(), next_obs.data_ptr(), _ptr(done), self.gamma, y.data_ptr(), n,
+                                                 reward.data_ptr(), next_obs.data_ptr(), _ptr(done), gamma, y.data_ptr(), n,
                                                  _stream(self.device)), "ss_ddpg_targets")
         return y
 
@@ -664,14 +733,14 @@ class ActorCritic:
             self.reduce_adam("actor", parts, self.stats[1:2], tau=tau)
         return self.stats[1]
 
-    def td3_step(self, obs, act, reward, next_obs, done=None):
+    def td3_step(self, obs, act, reward, next_obs, done=None, discount: Optional[float] = None):
         """One TD3 update on a (shard of a) minibatch (class docstring): the target, a critic step on critic 1 and one on
         critic 2 against the same y (each with its own Philox dropout draw: the counter advances per call), and on every
         policy_delay-th update the actor step against critic 1.  Only those delayed updates soft-update the targets; the
         others pass tau = 0, which leaves every target byte-identical.  Returns (critic 1's sum of squared errors, the
-        sum of q of the last actor step), device scalars; critic 2's sum is in critic2_sse."""
+        sum of q of the last actor step), device scalars; critic 2's sum is in critic2_sse.  discount: as for td_targets."""
         _, _, row_offset = shard_info(int(np.prod(reward.shape)), self.group)
-        y = self.td_targets(reward, next_obs, done, row_offset=row_offset)
+        y = self.td_targets(reward, next_obs, done, row_offset=row_offset, discount=discount)
         delayed = (self.td3_updates + 1) % self.policy_delay == 0
         tau = self.tau if delayed else 0.0
         sse = self.critic_step(obs, act, y, tau=tau)
@@ -682,17 +751,22 @@ class ActorCritic:
         self.td3_updates += 1
         return sse, self.stats[1]
 
-    def update_from_ring(self, ring: "ReplayRing", batch: int, out: Optional[dict] = None, sample_early: bool = False):
+    def update_from_ring(self, ring: "ReplayRing", batch: int, out: Optional[dict] = None, sample_early: bool = False,
+                         n_step: int = 1):
         """One whole update step from ONE library call (ss_ddpg_update): sample `batch` rows of `ring`,
         TD target, critic step, actor step -- the launches critic_step / actor_step make, without the
         interpreter time between them.  Single GPU or the fused peer exchange (an NCCL all-reduce needs
         the host between the gradient and Adam: use the separate steps).  Returns the minibatch dict.
         sample_early: the caller guarantees that the previous launch on the stream neither writes the ring nor touches
-        `out` (ss_ddpg_update_args.sample_early): the minibatch is gathered while that launch still runs."""
+        `out` (ss_ddpg_update_args.sample_early): the minibatch is gathered while that launch still runs.
+        n_step > 1: n-step rows of a ring with tick_rows (ReplayRing.sample), bootstrapped with nstep_discount(gamma, n_step)."""
         if self.group is not None and self.peer is None:
             raise ValueError("update_from_ring needs collective='peer' when the update is sharded")
         if self.frames > 1:
             raise ValueError("the single-call update is built for the reference's 12-input networks: use the separate steps")
+        runs = None
+        if n_step != 1:
+            runs, n_runs = ring.nstep_table(n_step)
         if ring.size == 0:
             raise ValueError("sampling from an empty ring")
         dev = self.device
@@ -753,6 +827,11 @@ class ActorCritic:
         a.sample_early = 1 if sample_early else 0
         if self.peer is not None:
             a.epoch = self.peer.epoch + 1
+        if runs is None:
+            a.n_step = 0
+        else:
+            a.n_step, a.tick_rows, a.n_runs, a.runs_host, a.step_gamma = int(n_step), ring.tick_rows, n_runs, runs, self.gamma
+            a.gamma = nstep_discount(self.gamma, n_step)
         with torch.cuda.device(dev):
             check(lib.ss_ddpg_update(ctypes.byref(a), _stream(dev)), "ss_ddpg_update")
         ring.counter += 1
@@ -800,12 +879,21 @@ class ActorCritic:
 class ReplayRing:
     """Device-resident replay ring (structure of arrays).  The reference keeps one episode in
     Python lists and uses it once (SkillshotLearner.py:292-361); a ring sized to the episode and
-    read back in order is that buffer."""
+    read back in order is that buffer.
 
-    def __init__(self, capacity: int, device="cuda", seed: int = 0, frames: int = 1):
+    tick_rows (DESIGN.md section 6.15): the ring is written one block of tick_rows rows per tick, so that the same
+    player's next transition after row r is row (r + tick_rows) mod capacity; sample(n_step > 1) then draws n-step rows.
+    Such a ring keeps its breaks (mark_break) as a host-side list of ring positions, and drops a break once the rows
+    written before it are overwritten.  A ring without tick_rows keeps no breaks and draws one-step rows only."""
+
+    def __init__(self, capacity: int, device="cuda", seed: int = 0, frames: int = 1, tick_rows: Optional[int] = None):
+        if tick_rows is not None and not 1 <= int(tick_rows) <= int(capacity):
+            raise ValueError("tick_rows must be in 1..capacity, got %r" % (tick_rows,))
         self.capacity, self.device, self.seed = int(capacity), torch.device(device), int(seed)
         self.frames = int(frames)          # observation rows of 12 * frames floats (the frame-stacked networks' inputs)
         self.width = 12 * self.frames
+        self.tick_rows = None if tick_rows is None else int(tick_rows)
+        self.breaks = []                   # ring positions, oldest first
         c, dev = self.capacity, self.device
         self.obs = torch.zeros((c, self.width), dtype=torch.float32, device=dev)
         self.act = torch.zeros((c, 2), dtype=torch.float32, device=dev)
@@ -815,6 +903,40 @@ class ReplayRing:
         self.pos = 0
         self.size = 0
         self.counter = 0
+
+    def advance(self, n: int):
+        """Account for n rows written at pos (by push, or in place by a rollout kernel): pos and size move on, and a break
+        whose last row before it was among them is dropped."""
+        if self.breaks:
+            c = self.capacity
+            self.breaks = [b for b in self.breaks if n < c and (b - 1 - self.pos) % c >= n]
+        self.pos = (self.pos + n) % self.capacity
+        self.size = min(self.capacity, self.size + n)
+
+    def mark_break(self):
+        """Record that the trajectories of the rows written before pos do not continue into the rows written from pos on
+        (ticks played without storing them, restarted games).  Nothing without tick_rows or in an empty ring."""
+        if self.tick_rows is not None and self.size > 0 and self.pos not in self.breaks:
+            self.breaks.append(self.pos)
+
+    def eligible_runs(self, n_step: int) -> list:
+        """nstep_runs of this ring: the runs (start, length) of the rows an n_step walk may start from."""
+        if self.tick_rows is None:
+            raise ValueError("n-step rows need a ring with tick_rows")
+        return nstep_runs(self.capacity, self.size, self.pos, self.tick_rows, n_step, self.breaks)
+
+    def nstep_table(self, n_step: int):
+        """(host run table, number of runs) of ss_replay_sample_nstep; ValueError for a bad n_step, a ring without
+        tick_rows, one shorter than n_step ticks, or one without an eligible row."""
+        if self.tick_rows is None:
+            raise ValueError("n-step rows need a ring with tick_rows")
+        refusal = nstep_refusal(n_step, self.capacity, self.tick_rows)
+        if refusal is not None:
+            raise ValueError(refusal)
+        runs = self.eligible_runs(n_step)
+        if not runs:
+            raise ValueError("no row of the ring can start a %d-step walk (%d rows stored)" % (n_step, self.size))
+        return (ctypes.c_int64 * (2 * len(runs)))(*[v for run in runs for v in run]), len(runs)
 
     def push(self, obs, act, reward, next_obs, done=None, done_div: int = 1):
         obs, next_obs = _f32(obs, self.device).reshape(-1, self.width), _f32(next_obs, self.device).reshape(-1, self.width)
@@ -829,33 +951,64 @@ class ReplayRing:
                                             self.next_obs.data_ptr(), self.done.data_ptr(), self.capacity, self.pos, self.frames,
                                             obs.data_ptr(), act.data_ptr(), reward.data_ptr(), next_obs.data_ptr(),
                                             _ptr(done), int(done_div), n, _stream(self.device)), "ss_replay_push")
-        self.pos = (self.pos + n) % self.capacity
-        self.size = min(self.capacity, self.size + n)
+        self.advance(n)
 
     def state_dict(self):
-        return dict(capacity=self.capacity, seed=self.seed, pos=self.pos, size=self.size, counter=self.counter, frames=self.frames,
-                    **{k: getattr(self, k).cpu() for k in ("obs", "act", "reward", "next_obs", "done")})
+        sd = dict(capacity=self.capacity, seed=self.seed, pos=self.pos, size=self.size, counter=self.counter, frames=self.frames,
+                  **{k: getattr(self, k).cpu() for k in ("obs", "act", "reward", "next_obs", "done")})
+        if self.tick_rows is not None:
+            sd.update(tick_rows=self.tick_rows, breaks=list(self.breaks))
+        return sd
 
     def load_state_dict(self, sd):
+        """A ring with tick_rows loads the checkpoint's breaks; from a checkpoint without them (a ring without tick_rows)
+        it loads empty (pos = size = 0), because the breaks of its rows are unknown."""
         if int(sd["capacity"]) != self.capacity:
             raise ValueError("checkpoint ring holds %d rows, this ring %d" % (sd["capacity"], self.capacity))
+        if self.tick_rows is not None and "breaks" in sd and int(sd["tick_rows"]) != self.tick_rows:
+            raise ValueError("checkpoint ring of %d rows per tick, this ring %d" % (sd["tick_rows"], self.tick_rows))
         for k in ("obs", "act", "reward", "next_obs", "done"):
             getattr(self, k).copy_(sd[k].to(self.device))
         self.seed, self.pos, self.size, self.counter = int(sd["seed"]), int(sd["pos"]), int(sd["size"]), int(sd["counter"])
+        if self.tick_rows is not None:
+            if "breaks" in sd:
+                self.breaks = [int(b) for b in sd["breaks"]]
+            else:
+                self.pos, self.size, self.breaks = 0, 0, []
 
-    def sample(self, batch: int, indices=None, out: Optional[dict] = None):
+    def sample(self, batch: int, indices=None, out: Optional[dict] = None, n_step: int = 1, gamma: float = 0.0):
         """dict(obs, act, reward, next_obs, done, indices) of `batch` rows: the rows `indices` or a
-        uniform draw with replacement from the filled part of the ring."""
+        uniform draw with replacement from the filled part of the ring.
+        n_step > 1 (a ring with tick_rows): n-step rows (ss_replay_sample_nstep) drawn uniformly from eligible_runs(n_step),
+        with the reward summed with the weights 1, gamma, gamma^2, ... (float32 recurrence) and next_obs / done of the
+        walk's last row; the dict also holds `steps`, the rows each walk visited.  Bootstrap such rows with
+        nstep_discount(gamma, n_step)."""
+        if n_step != 1:
+            runs, n_runs = self.nstep_table(n_step)
+            if indices is not None:
+                raise ValueError("n-step rows are drawn by the sampler: indices must be None")
         if self.size == 0:
             raise ValueError("sampling from an empty ring")
         dev = self.device
-        if out is None or out["reward"].shape[0] != batch:
+        if out is None or out["reward"].shape[0] != batch or (n_step != 1 and "steps" not in out):
             out = dict(obs=torch.empty((batch, self.width), dtype=torch.float32, device=dev),
                        act=torch.empty((batch, 2), dtype=torch.float32, device=dev),
                        reward=torch.empty(batch, dtype=torch.float32, device=dev),
                        next_obs=torch.empty((batch, self.width), dtype=torch.float32, device=dev),
                        done=torch.empty(batch, dtype=torch.uint8, device=dev),
                        indices=torch.empty(batch, dtype=torch.int64, device=dev))
+            if n_step != 1:
+                out["steps"] = torch.empty(batch, dtype=torch.uint8, device=dev)
+        if n_step != 1:
+            with torch.cuda.device(dev):
+                check(lib.ss_replay_sample_nstep(self.obs.data_ptr(), self.act.data_ptr(), self.reward.data_ptr(),
+                                                 self.next_obs.data_ptr(), self.done.data_ptr(), self.capacity, self.frames,
+                                                 self.tick_rows, int(n_step), float(gamma), runs, n_runs, self.seed, self.counter,
+                                                 batch, out["obs"].data_ptr(), out["act"].data_ptr(), out["reward"].data_ptr(),
+                                                 out["next_obs"].data_ptr(), out["done"].data_ptr(), out["indices"].data_ptr(),
+                                                 out["steps"].data_ptr(), _stream(dev)), "ss_replay_sample_nstep")
+            self.counter += 1
+            return out
         if indices is not None:
             indices = torch.as_tensor(indices).to(device=dev, dtype=torch.int64).contiguous()
             if indices.numel() != batch:
@@ -1360,7 +1513,7 @@ class SelfPlayTrainer:
                  random_positions: bool = True, process_group=None, precision: str = "f32", collective: str = "nccl",
                  frames: int = 1, update_precision: Optional[str] = None, opponents=None, pool_envs: Optional[int] = None,
                  pool_blocks=None, twin_critics: bool = False, policy_delay: int = 1, target_noise: float = 0.0,
-                 target_noise_clip: float = 0.5):
+                 target_noise_clip: float = 0.5, n_step: int = 1):
         """frames > 1: the frame-stacked "planning" networks (readme.md:18-20, BASELINE.json configs[4]): both players act
         from their last `frames` observations (FrameStackActor; `precision` selects its float32 or tensor-core kernels),
         the replay ring stores the stacked observations, and the critic / actor update of SkillshotLearner.py:386-443 runs
@@ -1386,7 +1539,14 @@ class SelfPlayTrainer:
         arguments, as update().  save / load write and read each rank's own file.
         twin_critics, policy_delay, target_noise, target_noise_clip: the TD3 update of ActorCritic (DESIGN.md section 6.14),
         which update() then runs through update_stepwise; the defaults are the DDPG update.  Bad values raise ValueError
-        before anything is allocated (sharded: on every rank, when any rank refused or passed other values)."""
+        before anything is allocated (sharded: on every rank, when any rank refused or passed other values).
+        n_step (DESIGN.md section 6.15): every update path trains on n-step rows of the replay ring (ReplayRing.sample),
+        bootstrapped with nstep_discount(gamma, n_step).  The ring is then built with tick_rows = the learner's rows per
+        tick and records a break at every rollout, rollout_tick or record_boards call with store=False and at every
+        set_pool_blocks / rebalance_pool; a checkpoint holds the breaks, and a checkpoint without them (an older one, or one
+        of an n_step = 1 run) loads with an empty ring.  n_step must be an integer in 1..32 and the replay capacity at least
+        n_step ticks of rows, else ValueError before anything is allocated (sharded: on every rank when any rank refused
+        or passed another n_step).  n_step = 1 is the one-step update, with the same allocations and checkpoints."""
         check_td3_options(twin_critics, policy_delay, target_noise, target_noise_clip, process_group)
         self.device = torch.device(device)
         self.frames = int(frames)
@@ -1433,6 +1593,13 @@ class SelfPlayTrainer:
             self.pool_envs = M
         self.learner_rows = 2 * int(n_envs) - self.pool_envs       # rows of the learner's transitions per tick
         L = self.learner_rows
+        refusal = nstep_refusal(n_step, replay_capacity or L * 8, L)
+        if process_group is not None:
+            check_process_group(process_group)
+            ranks_agree(refusal, (("n_step", n_step if refusal else int(n_step)),), process_group)
+        elif refusal is not None:
+            raise ValueError(refusal)
+        self.n_step = int(n_step)
         self.envs = SkillshotEnvs(n_envs, device=device, random_positions=random_positions, seed=seed,
                                   reward_mode=reward_mode, tick_limit=tick_limit, auto_reset=True)
         self.envs.collect_episode_stats = True     # the reference's per-episode ticks / winner log, reduced on the device
@@ -1442,7 +1609,8 @@ class SelfPlayTrainer:
                                     collective=collective, frames=self.frames, twin_critics=twin_critics,
                                     policy_delay=policy_delay, target_noise=target_noise, target_noise_clip=target_noise_clip)
         self.networks.seed = seed          # exploration / dropout streams differ per rank, weights do not
-        self.replay = ReplayRing(replay_capacity or L * 8, device=device, seed=seed, frames=self.frames)
+        self.replay = ReplayRing(replay_capacity or L * 8, device=device, seed=seed, frames=self.frames,
+                                 tick_rows=L if self.n_step > 1 else None)
         self.batch_size, self.param_noise_sd, self.noise_group = int(batch_size), float(param_noise_sd), int(noise_group)
         self.precision = precision
         self.update_precision = update_precision
@@ -1561,6 +1729,7 @@ class SelfPlayTrainer:
                                                  _stream(self.device)), "ss_obs_stack_push_pool")
         self._blocks = blocks
         self._alloc_opp_stacks(self.pool_head)
+        self.replay.mark_break()          # the learner's pool rows now belong to other games
 
     def rebalance_pool(self, weighting: str = "hard", p: float = 2.0, min_envs: int = 2, reset: bool = True) -> list:
         """Size each opponent's block by the learner's score against it: pool_progress(reset), pfsp_blocks of the scores
@@ -1680,15 +1849,17 @@ class SelfPlayTrainer:
             if self.param_noise_sd > 0:
                 st.counter += n_ticks
         if store:
-            rp.pos = (rp.pos + L * n_ticks) % rp.capacity
-            rp.size = min(rp.capacity, rp.size + L * n_ticks)
+            rp.advance(L * n_ticks)
         self.ticks += n_ticks
         return dict(obs=self.obs, reward=self._pool_reward, done=out["done"][0], winner=out["winner"][0])
 
     def rollout_tick(self, store: bool = True):
         """One tick of every env: actor forward on both players' observations (fresh parameter
-        noise per noise group), env step, transition push."""
+        noise per noise group), env step, transition push.  store=False: the tick is played but not stored (a break of
+        the ring's trajectories, ReplayRing.mark_break)."""
         self._ring_clean = False
+        if not store:
+            self.replay.mark_break()
         if self.opponents is not None:
             return self._rollout_pool(1, store)
         if self.frames > 1:
@@ -1723,6 +1894,8 @@ class SelfPlayTrainer:
         """n_ticks rollout ticks enqueued by ONE library call (ss_selfplay_rollout): same kernels and Philox
         counters as n_ticks calls of rollout_tick, without the per-tick host work."""
         self._ring_clean = False
+        if not store:
+            self.replay.mark_break()
         if self.opponents is not None:
             return self._rollout_pool(int(n_ticks), store)
         if self.frames > 1:
@@ -1760,8 +1933,7 @@ class SelfPlayTrainer:
         envs.counter += n_ticks
         net.counter += n_ticks
         if store:
-            rp.pos = (rp.pos + 2 * envs.n_envs * n_ticks) % rp.capacity
-            rp.size = min(rp.capacity, rp.size + 2 * envs.n_envs * n_ticks)
+            rp.advance(2 * envs.n_envs * n_ticks)
         rows = 2 * envs.n_envs
         in_place = (store and rp.capacity % rows == 0 and (rp.pos - rows * n_ticks) % rows == 0
                     and (rp.capacity // rows >= 2 or n_ticks == 1))       # the library's own condition (ss_selfplay_rollout)
@@ -1927,7 +2099,8 @@ class SelfPlayTrainer:
         # (measured, profiles/r2_update_sample_early_ab.txt: 158.1 -> 152.1 us at 65,536 rows; at 524,288 rows the gather
         #  competes with what it runs beside, 759 -> 764 us: small minibatches only)
         early = self._ring_clean and self._batches[k] is not None and self.batch_size <= 131072
-        self._batch = self._batches[k] = net.update_from_ring(self.replay, self.batch_size, out=self._batches[k], sample_early=early)
+        self._batch = self._batches[k] = net.update_from_ring(self.replay, self.batch_size, out=self._batches[k], sample_early=early,
+                                                              n_step=self.n_step)
         self._ring_clean = True
         self.updates += 1
         if net.peer is not None and self.updates % self.exchange_check_every == 0:
@@ -1936,13 +2109,14 @@ class SelfPlayTrainer:
 
     def update_stepwise(self):
         """The same update as one library call per step (sample, target, critic step, actor step); with the TD3 options,
-        ActorCritic.td3_step on the minibatch."""
+        ActorCritic.td3_step on the minibatch; with n_step > 1, on n-step rows with the bootstrap factor g_n."""
         self._ring_clean = False
-        self._batch = b = self.replay.sample(self.batch_size, out=self._batch)
         net = self.networks
+        self._batch = b = self.replay.sample(self.batch_size, out=self._batch, n_step=self.n_step, gamma=net.gamma)
+        disc = None if self.n_step == 1 else nstep_discount(net.gamma, self.n_step)
         if net.td3:
-            return net.td3_step(b["obs"], b["act"], b["reward"], b["next_obs"], b["done"])
-        y = net.td_targets(b["reward"], b["next_obs"], b["done"])
+            return net.td3_step(b["obs"], b["act"], b["reward"], b["next_obs"], b["done"], discount=disc)
+        y = net.td_targets(b["reward"], b["next_obs"], b["done"], discount=disc)
         sse = net.critic_step(b["obs"], b["act"], y)
         q = net.actor_step(b["obs"])
         return sse, q
