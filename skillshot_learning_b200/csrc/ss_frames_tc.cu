@@ -259,7 +259,7 @@ __global__ void __launch_bounds__(NTH, 1) frames_l1_kernel(const FramesArgs A) {
                     __syncwarp();
                     if (sg + 1 < nstages) {
                         mbar_wait(bar(B_XFULL + sg + 1), tc & 1);
-                    } else if (i + 1 < ntiles) {
+                    } else if (i + 1 < ntiles && nstages > 1) {
                         mbar_wait(bar(B_DFREE + (slot ^ 1)), (((tc + 1) >> 1) & 1) ^ 1);      // the epilogue has drained the other D
                         mbar_wait(bar(B_XFULL + 0), (tc + 1) & 1);
                     }
@@ -274,6 +274,13 @@ __global__ void __launch_bounds__(NTH, 1) frames_l1_kernel(const FramesArgs A) {
                         if (sg == nstages - 1) umma_commit(bar(B_DFULL + slot));
                     }
                     __syncwarp();
+                }
+                // One K stage (k1 <= 64, frames <= 5): the next tile's X lands in the stage this tile releases with the
+                // commit above, so its wait cannot come before that commit -- the copy thread would wait for it forever.
+                if (nstages == 1 && i + 1 < ntiles) {
+                    mbar_wait(bar(B_DFREE + (slot ^ 1)), (((tc + 1) >> 1) & 1) ^ 1);
+                    mbar_wait(bar(B_XFULL + 0), (tc + 1) & 1);
+                    tc_fence_after();
                 }
             }
         } else if (warp == COPY_W && lane == 0) {

@@ -46,6 +46,16 @@ def _scale_close(got, want, rel):
     np.testing.assert_allclose(got / scale, want / scale, rtol=0, atol=rel)
 
 
+def _arrays_close(got, want, shapes, rel):
+    """_scale_close per Keras array, so that an error in a small array (db3, the critic's action rows) cannot hide
+    behind the largest entry of another.  Below ~1,000 rows single rows are not averaged out and dW2 lands at up to ~2.7 %
+    of its own scale (as in tests/test_gpu_frames_learner_tc.py): callers pass 3e-2 there, beside the global 2e-2 check."""
+    for k, (g, w) in enumerate(zip(lo.split(np.asarray(got), shapes), lo.split(np.asarray(want), shapes))):
+        scale = np.abs(w).max() + 1e-12
+        err = np.abs(g - w).max() / scale
+        assert err <= rel, "array %d (shape %s): %.3g of its scale" % (k, w.shape, err)
+
+
 @pytest.mark.parametrize("n", [1, 16, 33, 1000, 40000])
 def test_actor_and_critic_forward(net, n):
     ac, theta, phi = net
@@ -414,6 +424,7 @@ def test_tensor_core_critic_gradient(net, n):
     sse = float(ac.stats[0])
     want, want_sse = lo.critic_grad(phi.astype(np.float64), s, a, r, keep.astype(np.float64), 0.2, dtype=torch.float64)
     _scale_close(g, want, 2e-2)
+    _arrays_close(g, want, lo.CRITIC_SHAPES, 2e-2 if n > 1000 else 3e-2)
     assert np.abs(g - want).mean() < 2e-3 * np.abs(want).max()
     assert abs(sse - want_sse) <= 2e-2 * max(1.0, want_sse)
     again = ac.critic_grad(s, a, r, keep=keep).cpu().numpy()
@@ -431,6 +442,7 @@ def test_tensor_core_critic_gradient_philox_dropout_matches_float32_path(net):
     ac32.counter = 77
     want = ac32.critic_grad(s, a, r, row_offset=5).cpu().numpy()      # same Philox mask in both kernels
     _scale_close(g, want, 2e-2)
+    _arrays_close(g, want, lo.CRITIC_SHAPES, 2e-2)
 
 
 @pytest.mark.parametrize("n", [128, 45, 3000, 20000])
@@ -442,6 +454,7 @@ def test_tensor_core_actor_policy_gradient(net, n):
     qsum = float(ac.stats[1])
     want, want_q = lo.actor_grad(theta.astype(np.float64), phi.astype(np.float64), s, dtype=torch.float64)
     _scale_close(g, want, 2e-2)
+    _arrays_close(g, want, lo.ACTOR_SHAPES, 2e-2 if n > 1000 else 3e-2)
     assert np.abs(g - want).mean() < 2e-3 * np.abs(want).max()
     assert abs(qsum - want_q) <= 2e-2 * max(1.0, abs(want_q))
 
