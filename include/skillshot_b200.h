@@ -518,6 +518,58 @@ int ss_replay_sample_nstep(const float *ring_obs, const float *ring_act, const f
                            float *act, float *reward, float *next_obs, uint8_t *done, int64_t *indices_out, uint8_t *steps_out,
                            void *stream);
 
+/* ---- prioritized replay (Schaul et al. 2016, proportional; no reference code, DESIGN.md section 6.16) ----
+ * A prioritized ring keeps one float32 leaf per ring position, priority[capacity] = p^alpha, and a device scalar
+ * priority_max (1.0 at the start).  Every row written gets the leaf priority_max (ss_replay_priority_fill); a priority update
+ * sets leaf[idx_b] = powf(|delta_b| + eps, alpha) and raises priority_max to the largest leaf it wrote.
+ *
+ * ss_replay_sample_prioritized: ss_replay_sample_nstep's arguments (n_step = 1: one-step rows; pass one run [0, size) for
+ * the rows ss_replay_sample draws from) and
+ *   priority               the leaves (4-byte aligned)
+ *   scratch                at least ss_replay_priority_scratch_bytes(capacity) bytes, 8-byte aligned (float64 prefix)
+ *   beta                   importance-weight exponent in [0, 1]
+ *   weights_out[batch]     w_b = (leaf_min / leaf[src_b])^beta in float64, rounded to float32; leaf_min is the smallest
+ *                          non-zero eligible leaf, so every w is in (0, 1]
+ * The eligible rows are those of the runs, in run order; eligible row j maps to its ring position as in
+ * ss_replay_sample_nstep.  P[j] is the float64 inclusive prefix of their leaves, summed in a fixed order (bit-identical from
+ * run to run) and total = P[last].  Row b of B draws the smallest j with P[j] > u_b, where
+ *   u_b = ((double)b + x_b * 2^-32) / (double)B * total,   x_b = word b & 3 of Philox4x32-10 with tag SS_TAG_PRIORITY,
+ *         keyed (b / 4, (b / 4) >> 32, counter) like ss_replay_sample's draw,
+ * or, when u_b rounds up to total, the last eligible row with a non-zero leaf.  The row is then gathered (and walked for
+ * n_step > 1) exactly as by ss_replay_sample_nstep.  (Every eligible leaf 0: row 0 of the runs, weight 1.)  The draw is
+ * three launches: a block scan of the leaves, one block over the blocks' sums, and the search + gather.
+ * ss_replay_priority_update: leaf[indices[b]] = powf(|td_abs[b]| + eps, alpha) for b < batch; when an index occurs more than
+ * once, the largest b wins.  scratch: int32[capacity] (contents need not be set).  Indices outside [0, capacity) are skipped.
+ * ss_replay_priority_fill: leaf[(pos + i) mod capacity] = *priority_max for i < n.
+ * Every argument is checked before anything is enqueued: NULL pointers (but indices_out, steps_out), the ranges of
+ * ss_replay_sample_nstep, a beta outside [0, 1], an alpha < 0, an eps <= 0, any of them not finite, runs holding more
+ * rows than the ring, a short scratch and misaligned pointers return SS_ERR_INVALID_ARG. */
+#define SS_TAG_PRIORITY 6
+int64_t ss_replay_priority_scratch_bytes(int64_t capacity);
+int ss_replay_sample_prioritized(const float *ring_obs, const float *ring_act, const float *ring_reward, const float *ring_next_obs,
+                                 const uint8_t *ring_done, int64_t capacity, int frames, int64_t tick_rows, int n_step, float gamma,
+                                 const int64_t *runs_host, int n_runs, uint64_t seed, uint64_t counter, int64_t batch, float *obs,
+                                 float *act, float *reward, float *next_obs, uint8_t *done, int64_t *indices_out, uint8_t *steps_out,
+                                 const float *priority, void *scratch, int64_t scratch_bytes, float beta, float *weights_out,
+                                 void *stream);
+int ss_replay_priority_update(float *priority, float *priority_max, int64_t capacity, const int64_t *indices, const float *td_abs,
+                              int64_t batch, float alpha, float eps, int32_t *scratch, void *stream);
+int ss_replay_priority_fill(float *priority, const float *priority_max, int64_t capacity, int64_t pos, int64_t n, void *stream);
+
+/* ss_critic_grad_weighted: the critic gradient of the row-weighted loss (prioritized replay's importance weights):
+ * d_b = (2 e_b / n_global) * row_weight[b], the weight multiplied last, so that row_weight = 1 gives the unweighted d bit
+ * for bit; sse_out stays the unweighted sum of e_b^2.  td_abs_out[b] = |e_b| = |q_b - target_b| of the same forward
+ * (with its dropout mask).  Either may be NULL (row_weight NULL: weight 1).  One entry point for the three families:
+ *   tensor_cores = 0        float32 CUDA cores, frames 1..SS_MAX_FRAMES (ss_critic_grad_frames)
+ *   tensor_cores, frames 1  tcgen05, 12 inputs (ss_critic_grad_tc, its workspace)
+ *   tensor_cores, frames>1  tcgen05, frame-stacked (ss_critic_grad_frames_tc, ss_learner_frames_tc_workspace_bytes)
+ * The other arguments, the return value and the checks are those of the family's unweighted entry point; row_weight and
+ * td_abs_out must be 4-byte aligned. */
+int ss_critic_grad_weighted(const float *critic_params, int frames, int tensor_cores, const float *obs, const float *act,
+                            const float *target, const float *row_weight, float *td_abs_out, const uint8_t *dropout_keep,
+                            float dropout_rate, uint64_t seed, uint64_t counter, int64_t n, int64_t n_global, int64_t row_offset,
+                            float *grad_out, float *sse_out, void *workspace, int64_t workspace_bytes, void *stream);
+
 /* ---- matches: two actors against each other (no reference code; the readme's "does the planning actor play better" question) ----
  * A match is n_envs games between policy A and policy B, ONE game per env (no auto-reset: every game starts at tick 0 and
  * is played to a hit or to tick_limit ticks, so no outcome is sampled by its length).  Seat map, split index 0 <= split <= n_envs:
@@ -941,6 +993,19 @@ typedef struct ss_ddpg_update_args {
     int n_runs;                                /* eligible runs: runs_host[2 n_runs] = {start, length, ...} (host memory) */
     const int64_t *runs_host;
     float step_gamma;                          /* the per-tick gamma of the n-step reward sum's weights */
+    int prioritized;                           /* 0: the uniform draw, the fields below unused.  1: prioritized replay
+                                                  (DESIGN.md section 6.16): ss_replay_sample_prioritized over [0, size) (or the
+                                                  n-step runs), the critic gradient weighted by `weights` with |e| into
+                                                  td_abs (ss_critic_grad_weighted), and after the critic's Adam
+                                                  ss_replay_priority_update at `indices`.  Refused with sample_early. */
+    float *priority;                           /* leaves [capacity] */
+    float *priority_max;
+    void *priority_scratch;                    /* ss_replay_priority_scratch_bytes(capacity) bytes */
+    int64_t priority_scratch_bytes;
+    int32_t *priority_update_scratch;          /* int32[capacity] */
+    float priority_alpha, priority_beta, priority_eps;
+    float *weights;                            /* [batch] importance weights out */
+    float *td_abs;                             /* [batch] |q - y| out */
 } ss_ddpg_update_args;
 int ss_ddpg_update(const ss_ddpg_update_args *args, void *stream);
 

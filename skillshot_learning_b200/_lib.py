@@ -47,6 +47,7 @@ POOL_STATS = 8                    # uint64 counters per opponent of ss_env_step_
 TAG_TARGET_NOISE = 5              # SS_TAG_TARGET_NOISE: Philox tag of the TD3 target policy smoothing
 REPLAY_MAX_RUNS = 16              # SS_REPLAY_MAX_RUNS: runs of eligible rows of one ss_replay_sample_nstep call
 REPLAY_MAX_NSTEP = 32             # SS_REPLAY_MAX_NSTEP: the longest n-step walk
+TAG_PRIORITY = 6                  # SS_TAG_PRIORITY: Philox tag of the stratified prioritized replay draw
 
 
 def td3_tc_workspace_bytes(n: int) -> int:
@@ -68,7 +69,11 @@ class DdpgUpdateArgs(ctypes.Structure):
                  ("done_counter", _vp), ("status", _vp), ("pair_mail", _vp), ("sample_early", _i32),
                  # n-step rows: n_step 0 / 1 one-step (the other four unused), else gamma above is g_n
                  ("n_step", _i32), ("tick_rows", _i64), ("n_runs", _i32), ("runs_host", ctypes.POINTER(_i64)),
-                 ("step_gamma", _f32)])
+                 ("step_gamma", _f32),
+                 # prioritized replay: prioritized 0, the rest unused
+                 ("prioritized", _i32), ("priority", _vp), ("priority_max", _vp), ("priority_scratch", _vp),
+                 ("priority_scratch_bytes", _i64), ("priority_update_scratch", _vp), ("priority_alpha", _f32),
+                 ("priority_beta", _f32), ("priority_eps", _f32), ("weights", _vp), ("td_abs", _vp)])
 
 
 class MatchArgs(ctypes.Structure):
@@ -219,6 +224,13 @@ SIGNATURES = {
     "ss_pool_rollout_speeds": (_i32, [ctypes.POINTER(PoolRolloutFramesArgs), _vp]),
     "ss_replay_sample_nstep": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i32, _i64, _i32, _f32, ctypes.POINTER(_i64), _i32, _u64,
                                        _u64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "ss_replay_priority_scratch_bytes": (_i64, [_i64]),
+    "ss_replay_sample_prioritized": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i32, _i64, _i32, _f32, ctypes.POINTER(_i64), _i32,
+                                             _u64, _u64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _f32, _vp, _vp]),
+    "ss_replay_priority_update": (_i32, [_vp, _vp, _i64, _vp, _vp, _i64, _f32, _f32, _vp, _vp]),
+    "ss_replay_priority_fill": (_i32, [_vp, _vp, _i64, _i64, _i64, _vp]),
+    "ss_critic_grad_weighted": (_i32, [_vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _f32, _u64, _u64, _i64, _i64, _i64, _vp, _vp,
+                                        _vp, _i64, _vp]),
     "ss_replay_sample": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp, _u64, _u64, _i64,
                                  _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
 }

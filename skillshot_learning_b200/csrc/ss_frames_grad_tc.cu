@@ -79,6 +79,8 @@ __global__ void frames_pack_kernel(const float *x, int64_t n, int frames, int64_
 namespace mid {
 
 constexpr int MODE_FWD = 0, MODE_CRITIC = 1, MODE_ACTOR = 2;
+// MODE_CRITIC with row weights and |e| out (ss_critic_grad_weighted)
+constexpr int MODE_CRITIC_W = 3;
 // eight epilogue warps as in ss_mlp_grad_tc.cu: warps w and w + 4 share lane quadrant w & 3 and split the columns
 constexpr int EPI_WARPS = 8, NSLICE = 2, MMA_WARP = EPI_WARPS, NTH = 32 * (EPI_WARPS + 1);
 
@@ -117,6 +119,8 @@ struct MidArgs {
     const uint8_t *done;
     float gamma;
     int frames;
+    const float *row_weight;         // CRITIC_W: the loss weight of each row [n] or NULL (1)
+    float *td_abs;                   // CRITIC_W: |q - target| of each row [n] or NULL
 };
 
 // the keep bits of 8 consecutive hidden-1 units of one row: ss_mlp_grad_tc.cu's keep8, the same Philox draw
@@ -155,6 +159,8 @@ template <int MODE>
 __global__ void __launch_bounds__(NTH, 1) frames_mid_kernel(const MidArgs A) {
     constexpr int NET = MODE == MODE_ACTOR ? NET_ACTOR : NET_CRITIC;
     constexpr bool GRAD = MODE != MODE_FWD;
+    constexpr bool WEIGHTED = MODE == MODE_CRITIC_W;
+    constexpr bool CRITIC_GRAD = MODE == MODE_CRITIC || WEIGHTED;
     extern __shared__ __align__(128) uint8_t smem[];
     const uint32_t sbase = smem_u32(smem);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -195,7 +201,7 @@ __global__ void __launch_bounds__(NTH, 1) frames_mid_kernel(const MidArgs A) {
         const float4 *w3x = reinterpret_cast<const float4 *>(smem + SM_W3);      // critic layout
         const float2 *w3a = reinterpret_cast<const float2 *>(smem + SM_W3);      // actor layout: W3[128][2] as stored
         const float *b3 = reinterpret_cast<const float *>(smem + SM_B3);
-        const bool dropout = MODE == MODE_CRITIC && A.rate > 0.f;
+        const bool dropout = CRITIC_GRAD && A.rate > 0.f;
         const float inv_keep = dropout ? 1.0f / (1.0f - A.rate) : 1.0f;
         const uint32_t thresh16 = (uint32_t)(A.rate * 65536.0f);
         uint32_t ph = 0;
@@ -260,7 +266,7 @@ __global__ void __launch_bounds__(NTH, 1) frames_mid_kernel(const MidArgs A) {
             if (valid) {
                 if (NET == NET_CRITIC) side = __ldg(reinterpret_cast<const float2 *>(A.act) + row);
                 else side = __ldg(reinterpret_cast<const float2 *>(A.up) + row);
-                if (MODE == MODE_CRITIC) tgt = __ldg(A.target + row);
+                if (CRITIC_GRAD) tgt = __ldg(A.target + row);
                 if (MODE == MODE_ACTOR) tgt = __ldg(A.q + row);
             }
             if (NET == NET_CRITIC && cs == 0)
@@ -303,11 +309,15 @@ __global__ void __launch_bounds__(NTH, 1) frames_mid_kernel(const MidArgs A) {
                 continue;
             }
             float d0 = 0.f, d1 = 0.f;
-            if (MODE == MODE_CRITIC) {
+            if (CRITIC_GRAD) {
                 if (valid) {                              // loss "mse": mean over the global batch
                     const float e = (z0 + b3[0]) - tgt;
                     stat += e * e;
                     d0 = 2.0f * e / (float)A.n_global;
+                    if (WEIGHTED) {                       // (the weight last: w = 1 leaves d0 as it is)
+                        if (A.row_weight) d0 = d0 * __ldg(A.row_weight + row);
+                        if (A.td_abs && cs == 0) A.td_abs[row] = fabsf(e);
+                    }
                 }
             } else if (valid) {                           // through tanh, upstream = -dQ/da
                 stat += tgt;
@@ -766,6 +776,28 @@ int ss_critic_grad_frames_tc(const float *critic_params, int frames, const float
     A.seed = seed; A.counter = counter; A.n_global = n_global > 0 ? n_global : n; A.row_offset = row_offset;
     return gradient<mid::MODE_CRITIC>(C, A, frames, n, critic_n(frames), grad_out, sse_out, sms);
 }
+
+}  // extern "C"
+
+int sstc::critic_grad_frames_tc_weighted(const float *critic_params, int frames, const float *obs, const float *act,
+                                         const float *target, const float *row_weight, float *td_abs_out,
+                                         const uint8_t *dropout_keep, float dropout_rate, uint64_t seed, uint64_t counter, int64_t n,
+                                         int64_t n_global, int64_t row_offset, float *grad_out, float *sse_out, void *workspace,
+                                         int64_t workspace_bytes, cudaStream_t stream) {
+    Ctx C{};
+    if (prepare(frames, n, workspace, workspace_bytes, stream, C) != SS_OK) return SS_ERR_INVALID_ARG;
+    int sms = 0, rc = device_sms(sms);
+    if (rc == SS_OK) rc = pack(C, obs, frames, n, true);
+    if (rc == SS_OK) rc = frames_layer1_tc(critic_params, C.at(C.L.xf), frames, n, C.at(C.L.h1a), C.st);
+    if (rc != SS_OK) return rc;
+    mid::MidArgs A{};
+    A.params = critic_params; A.h1 = C.at(C.L.h1a); A.act = act; A.target = target; A.keep = dropout_keep; A.rate = dropout_rate;
+    A.seed = seed; A.counter = counter; A.n_global = n_global > 0 ? n_global : n; A.row_offset = row_offset;
+    A.row_weight = row_weight; A.td_abs = td_abs_out;
+    return gradient<mid::MODE_CRITIC_W>(C, A, frames, n, critic_n(frames), grad_out, sse_out, sms);
+}
+
+extern "C" {
 
 int ss_actor_grad_frames_tc(const float *actor_params, const float *critic_params, int frames, const float *obs, int64_t n,
                             float *grad_out, float *q_sum_out, void *workspace, int64_t workspace_bytes, void *stream) {

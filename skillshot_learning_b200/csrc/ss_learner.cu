@@ -26,6 +26,17 @@
 #include "ss_launch.cuh"
 #include "ss_rng.cuh"
 
+namespace sstc {   // the tensor-core families of ss_critic_grad_weighted (ss_tc_common.cuh)
+int critic_grad_tc_weighted(const float *critic_params, const float *obs, const float *act, const float *target,
+                            const float *row_weight, float *td_abs_out, const uint8_t *dropout_keep, float dropout_rate,
+                            uint64_t seed, uint64_t counter, int64_t n, int64_t n_global, int64_t row_offset, float *grad_out,
+                            float *sse_out, void *workspace, int64_t workspace_bytes, cudaStream_t stream);
+int critic_grad_frames_tc_weighted(const float *critic_params, int frames, const float *obs, const float *act, const float *target,
+                                   const float *row_weight, float *td_abs_out, const uint8_t *dropout_keep, float dropout_rate,
+                                   uint64_t seed, uint64_t counter, int64_t n, int64_t n_global, int64_t row_offset,
+                                   float *grad_out, float *sse_out, void *workspace, int64_t workspace_bytes, cudaStream_t stream);
+}  // namespace sstc
+
 namespace {
 
 using namespace ss;
@@ -505,9 +516,14 @@ struct CriticGradArgs {
     int64_t n, n_global, row_offset;   // row_offset: global index of row 0 (Philox dropout of a shard)
     float *work;             // [gridDim.x][c_n + 1]
     int ds;                  // input width: 12 (reference) or 12 * frames
+    const float *row_weight; // WEIGHTED: the loss weight of each row [n] or NULL (1)
+    float *td_abs;           // WEIGHTED: |q - target| of each row [n] or NULL
 };
 
-__global__ void __launch_bounds__(NT) critic_grad_kernel(const CriticGradArgs A) {
+// critic_grad_kernel's body; WEIGHTED (critic_grad_weighted_kernel, ss_critic_grad_weighted) multiplies each row's loss
+// gradient by its weight and stores |e|
+template <bool WEIGHTED>
+__device__ __forceinline__ void critic_grad_tiles(const CriticGradArgs &A) {
     extern __shared__ __align__(16) float smem[];
     const Lay L = lay_of(A.ds);
     const int C_B1 = L.c_b1, C_W2 = L.c_w2, C_B2 = L.c_b2, C_W3 = L.c_w3, C_B3 = L.c_b3, C_N = L.c_n, C_W1 = 0;
@@ -557,6 +573,10 @@ __global__ void __launch_bounds__(NT) critic_grad_kernel(const CriticGradArgs A)
                 const float e = qv[t] - A.target[base + t];
                 sse += e * e;
                 d = 2.0f * e / (float)A.n_global;
+                if (WEIGHTED) {                             // (the weight last: w = 1 leaves d as it is)
+                    if (A.row_weight) d = d * A.row_weight[base + t];
+                    if (A.td_abs) A.td_abs[base + t] = fabsf(e);
+                }
             }
             dq[t] = d;
         }
@@ -594,6 +614,9 @@ __global__ void __launch_bounds__(NT) critic_grad_kernel(const CriticGradArgs A)
         for (int p = threadIdx.x; p < C_N; p += NT) g[p] = 0.f;
     }
 }
+
+__global__ void __launch_bounds__(NT) critic_grad_kernel(const CriticGradArgs A) { critic_grad_tiles<false>(A); }
+__global__ void __launch_bounds__(NT) critic_grad_weighted_kernel(const CriticGradArgs A) { critic_grad_tiles<true>(A); }
 
 // ---------------------------------------------------------------------------
 // actor deterministic-policy-gradient (model_actor_fit_step, SkillshotLearner.py:386-417)
@@ -886,6 +909,291 @@ __global__ void replay_sample_nstep_kernel(Ring R, NstepRuns runs, int64_t total
 }
 
 // ---------------------------------------------------------------------------
+// prioritized replay (DESIGN.md section 6.16): one float32 leaf p^alpha per ring position
+// ---------------------------------------------------------------------------
+constexpr int kPriThreads = 256, kPriItems = 8, kPriChunk = kPriThreads * kPriItems;   // eligible rows per scan block
+constexpr int kPriRows = 64;                                                            // minibatch rows per draw block
+
+// the float64 scratch of one prioritized draw over total_n eligible rows (capacity bounds total_n)
+struct PriScratch {
+    double *prefix;          // [total_n] inclusive prefix of the leaves WITHIN each kPriChunk block
+    double *start;           // [blocks + 1] prefix before each block: start[0] = 0, start[k + 1] = start[k] + block k's sum
+    float *bmin;             // [blocks] smallest non-zero leaf of each block (+inf: none)
+    int64_t *blast;          // [blocks] last eligible row with a non-zero leaf of each block (-1: none)
+    float *leaf_min;         // smallest non-zero eligible leaf
+    int64_t *last_nz;        // last eligible row with a non-zero leaf (-1: none)
+};
+
+inline int64_t pri_blocks(int64_t capacity) { return (capacity + kPriChunk - 1) / kPriChunk; }
+inline int64_t pri_scratch_bytes(int64_t capacity) {
+    const int64_t nb = pri_blocks(capacity);
+    return 8 * capacity + 8 * (nb + 1) + 8 * nb + 8 * nb + 16;
+}
+inline PriScratch pri_scratch(void *base, int64_t capacity) {
+    const int64_t nb = pri_blocks(capacity);
+    char *p = (char *)base;
+    PriScratch S;
+    S.prefix = (double *)p;
+    S.start = (double *)(p + 8 * capacity);
+    S.blast = (int64_t *)(p + 8 * capacity + 8 * (nb + 1));
+    S.bmin = (float *)(p + 8 * capacity + 8 * (nb + 1) + 8 * nb);
+    S.last_nz = (int64_t *)(p + 8 * capacity + 8 * (nb + 1) + 16 * nb);
+    S.leaf_min = (float *)(p + 8 * capacity + 8 * (nb + 1) + 16 * nb + 8);
+    return S;
+}
+
+// ring position of eligible row j (the mapping of replay_sample_nstep_kernel)
+__device__ __forceinline__ int64_t run_position(const NstepRuns &runs, int64_t j) {
+    int64_t src = runs.start[0] + j;
+    for (int i = 0; i < runs.n; ++i) {
+        if (j < runs.length[i]) {
+            src = runs.start[i] + j;
+            break;
+        }
+        j -= runs.length[i];
+    }
+    return src;
+}
+
+// block k: the inclusive prefix of eligible rows [k kPriChunk, (k + 1) kPriChunk) in a fixed order (each thread's eight rows
+// in sequence, then the threads' sums by a fixed shuffle / shared-memory scan), its smallest non-zero leaf and its last
+// row with a non-zero leaf
+__global__ void __launch_bounds__(kPriThreads) priority_scan_kernel(const float *leaf, NstepRuns runs, int64_t total_n, PriScratch S) {
+    __shared__ double wsum[kPriThreads / 32];
+    __shared__ float wmin[kPriThreads / 32];
+    __shared__ long long wlast[kPriThreads / 32];
+    sslaunch::griddep_wait();
+    sslaunch::griddep_launch();
+    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    const int64_t j0 = (int64_t)blockIdx.x * kPriChunk + (int64_t)t * kPriItems;
+    double loc[kPriItems], acc = 0.0;
+    float mn = INFINITY;
+    long long last = -1;
+#pragma unroll
+    for (int i = 0; i < kPriItems; ++i) {
+        const int64_t j = j0 + i;
+        const float v = j < total_n ? leaf[run_position(runs, j)] : 0.f;
+        acc += (double)v;
+        loc[i] = acc;
+        if (v > 0.f) {
+            mn = fminf(mn, v);
+            last = j;
+        }
+    }
+    // inclusive scan of the thread sums: within the warp, then over the warps
+    double inc = acc;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const double y = __shfl_up_sync(0xffffffffu, inc, o);
+        if (lane >= o) inc += y;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
+        last = max(last, __shfl_xor_sync(0xffffffffu, last, o));
+    }
+    if (lane == 31) wsum[warp] = inc;
+    if (lane == 0) {
+        wmin[warp] = mn;
+        wlast[warp] = last;
+    }
+    __syncthreads();
+    double before = 0.0;                                  // the earlier warps' sums, in order
+    for (int w = 0; w < warp; ++w) before += wsum[w];
+    const double below = __shfl_up_sync(0xffffffffu, inc, 1);
+    const double base = lane == 0 ? before : before + below;
+#pragma unroll
+    for (int i = 0; i < kPriItems; ++i) {
+        const int64_t j = j0 + i;
+        if (j < total_n) S.prefix[j] = base + loc[i];
+    }
+    if (t == kPriThreads - 1) S.start[blockIdx.x + 1] = base + loc[kPriItems - 1];     // this block's sum (start fixed up below)
+    if (t == 0) {
+        float m = wmin[0];
+        long long l = wlast[0];
+        for (int w = 1; w < kPriThreads / 32; ++w) {
+            m = fminf(m, wmin[w]);
+            l = max(l, wlast[w]);
+        }
+        S.bmin[blockIdx.x] = m;
+        S.blast[blockIdx.x] = l;
+    }
+}
+
+// start[k + 1] = start[k] + sum_k in block order (the blocks' sums are in start[1 ..] on entry), by one thread from shared
+// memory, 1,024 blocks at a time (the running sum is a chain of float64 additions; its operands are staged by every thread);
+// the smallest non-zero leaf and the last row with one
+constexpr int kPriBlocksThreads = 1024;
+__global__ void __launch_bounds__(kPriBlocksThreads) priority_blocks_kernel(int64_t nb, PriScratch S) {
+    __shared__ double sums[kPriBlocksThreads], starts[kPriBlocksThreads];
+    __shared__ float wmin[kPriBlocksThreads / 32];
+    __shared__ long long wlast[kPriBlocksThreads / 32];
+    sslaunch::griddep_wait();
+    sslaunch::griddep_launch();
+    const int t = threadIdx.x;
+    float mn = INFINITY;
+    long long last = -1;
+    for (int64_t k = t; k < nb; k += kPriBlocksThreads) {
+        mn = fminf(mn, S.bmin[k]);
+        last = max(last, (long long)S.blast[k]);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
+        last = max(last, __shfl_xor_sync(0xffffffffu, last, o));
+    }
+    if ((t & 31) == 0) {
+        wmin[t >> 5] = mn;
+        wlast[t >> 5] = last;
+    }
+    double run = 0.0;
+    for (int64_t c0 = 0; c0 < nb; c0 += kPriBlocksThreads) {
+        const int n = (int)min((int64_t)kPriBlocksThreads, nb - c0);
+        if (t < n) sums[t] = S.start[c0 + t + 1];
+        __syncthreads();
+        if (t == 0) {
+#pragma unroll 16
+            for (int i = 0; i < n; ++i) {
+                run += sums[i];
+                starts[i] = run;
+            }
+        }
+        __syncthreads();
+        if (t < n) S.start[c0 + t + 1] = starts[t];
+        __syncthreads();
+    }
+    if (t == 0) {
+        for (int w = 1; w < kPriBlocksThreads / 32; ++w) {
+            mn = fminf(mn, wmin[w]);
+            last = max(last, wlast[w]);
+        }
+        S.start[0] = 0.0;
+        *S.leaf_min = mn;
+        *S.last_nz = last;
+    }
+}
+
+// One minibatch row per thread of the first kPriRows: the stratified draw u_b = (b + U_b) / B * total, the smallest eligible
+// j with P[j] > u_b (binary search over the blocks' starts, then inside the block), the walk and reward sum of
+// replay_sample_nstep_kernel (n_step = 1: the one-step row) and the importance weight; then every thread of the block copies
+// the rows' observations, one float4 per (row, part)
+__global__ void __launch_bounds__(256) replay_sample_prioritized_kernel(Ring R, NstepRuns runs, int64_t total_n, int64_t nb,
+                                                                        PriScratch S, const float *leaf, int64_t tick_rows,
+                                                                        int n_step, float gamma, uint64_t seed, uint64_t counter,
+                                                                        int64_t batch, float beta, float *s, float *a, float *r,
+                                                                        float *s2, uint8_t *done, int64_t *indices_out,
+                                                                        uint8_t *steps_out, float *w_out, int w4) {
+    __shared__ int64_t src_s[kPriRows], last_s[kPriRows];
+    sslaunch::griddep_wait();
+    sslaunch::griddep_launch();
+    const int64_t b0 = (int64_t)blockIdx.x * kPriRows;
+    if (threadIdx.x < kPriRows && b0 + threadIdx.x < batch) {
+        const int64_t b = b0 + threadIdx.x;
+        const U4 u4 = draw4(seed, kTagPriority, (uint32_t)(b / 4), (uint32_t)((b / 4) >> 32), counter);
+        const uint32_t x = (b & 3) == 0 ? u4.x : (b & 3) == 1 ? u4.y : (b & 3) == 2 ? u4.z : u4.w;
+        const double total = S.start[nb];
+        const double u = ((double)b + (double)x * 0x1p-32) / (double)batch * total;
+        int64_t j;
+        if (!(u < total)) {
+            j = *S.last_nz;                              // (u rounded up to total)
+        } else {
+            int64_t lo = 0, hi = nb - 1;                 // the first block whose end start[k + 1] exceeds u
+            while (lo < hi) {
+                const int64_t mid = (lo + hi) >> 1;
+                if (S.start[mid + 1] > u) hi = mid;
+                else lo = mid + 1;
+            }
+            const double st = S.start[lo];
+            int64_t jl = lo * kPriChunk, jh = min(total_n, jl + kPriChunk) - 1;
+            while (jl < jh) {
+                const int64_t mid = (jl + jh) >> 1;
+                if (st + S.prefix[mid] > u) jh = mid;
+                else jl = mid + 1;
+            }
+            j = jl;
+        }
+        float w = 1.0f;
+        if (j < 0) {
+            j = 0;                                       // no non-zero leaf: row 0 of the runs, weight 1
+        }
+        const int64_t src = run_position(runs, j);
+        const float p = leaf[src];
+        if (p > 0.f) w = (float)pow((double)*S.leaf_min / (double)p, (double)beta);
+        int64_t last = src;
+        int k = 1;
+        for (; k < n_step && !R.done[last]; ++k) {
+            last += tick_rows;
+            if (last >= R.capacity) last -= R.capacity;
+        }
+        float sum = R.r[src], g = 1.0f;
+        int64_t row = src;
+        for (int t = 1; t < k; ++t) {
+            row += tick_rows;
+            if (row >= R.capacity) row -= R.capacity;
+            g = __fmul_rn(g, gamma);
+            sum = __fadd_rn(sum, __fmul_rn(g, R.r[row]));
+        }
+        reinterpret_cast<float2 *>(a)[b] = reinterpret_cast<const float2 *>(R.a)[src];
+        r[b] = sum;
+        done[b] = R.done[last];
+        w_out[b] = w;
+        if (indices_out) indices_out[b] = src;
+        if (steps_out) steps_out[b] = (uint8_t)k;
+        src_s[threadIdx.x] = src;
+        last_s[threadIdx.x] = last;
+    }
+    __syncthreads();
+    const int64_t rows = min((int64_t)kPriRows, batch - b0);
+    for (int64_t e = threadIdx.x; e < rows * w4; e += blockDim.x) {
+        const int64_t bl = e / w4, part = e - bl * w4, o = (b0 + bl) * w4 + part;
+        reinterpret_cast<float4 *>(s)[o] = reinterpret_cast<const float4 *>(R.s)[src_s[bl] * w4 + part];
+        reinterpret_cast<float4 *>(s2)[o] = reinterpret_cast<const float4 *>(R.s2)[last_s[bl] * w4 + part];
+    }
+}
+
+// priority update, in three launches: mark every drawn position, let the largest batch position claim it, and write the
+// claimed leaves (and raise priority_max: non-negative floats order as their bit patterns)
+__global__ void priority_mark_kernel(const int64_t *idx, int64_t batch, int64_t capacity, int *claim) {
+    const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    sslaunch::griddep_wait();
+    sslaunch::griddep_launch();
+    if (b < batch && idx[b] >= 0 && idx[b] < capacity) claim[idx[b]] = -1;
+}
+
+__global__ void priority_claim_kernel(const int64_t *idx, int64_t batch, int64_t capacity, int *claim) {
+    const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    sslaunch::griddep_wait();
+    sslaunch::griddep_launch();
+    if (b < batch && idx[b] >= 0 && idx[b] < capacity) atomicMax(claim + idx[b], (int)b);
+}
+
+__global__ void priority_write_kernel(const int64_t *idx, const float *td_abs, int64_t batch, int64_t capacity, const int *claim,
+                                      float alpha, float eps, float *leaf, float *leaf_max) {
+    const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    sslaunch::griddep_wait();
+    sslaunch::griddep_launch();
+    if (b < batch) {
+        const int64_t i = idx[b];
+        if (i >= 0 && i < capacity && claim[i] == (int)b) {
+            const float p = powf(__fadd_rn(fabsf(td_abs[b]), eps), alpha);
+            leaf[i] = p;
+            atomicMax(reinterpret_cast<int *>(leaf_max), __float_as_int(p));
+        }
+    }
+}
+
+__global__ void priority_fill_kernel(float *leaf, const float *leaf_max, int64_t capacity, int64_t pos, int64_t n) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    sslaunch::griddep_wait();
+    sslaunch::griddep_launch();
+    if (i < n) {
+        int64_t dst = pos + i;
+        if (dst >= capacity) dst -= capacity;
+        leaf[dst] = *leaf_max;
+    }
+}
+
+// ---------------------------------------------------------------------------
 // launch helpers
 // ---------------------------------------------------------------------------
 constexpr size_t kSmemActorFwd = (size_t)(DS + H1 + H2 + DA) * PITCH * 4;
@@ -1008,10 +1316,10 @@ int ss_td3_targets_frames(const float *target_actor_params, const float *target_
     return check_launch();
 }
 
-int ss_critic_grad_frames(const float *critic_params, int frames, const float *obs, const float *act, const float *target,
-                          const uint8_t *dropout_keep, float dropout_rate, uint64_t seed, uint64_t counter,
-                          int64_t n, int64_t n_global, int64_t row_offset, float *grad_out, float *sse_out,
-                          void *workspace, int64_t workspace_bytes, void *stream) {
+static int critic_grad_f32(const float *critic_params, int frames, const float *obs, const float *act, const float *target,
+                           const float *row_weight, float *td_abs_out, bool weighted, const uint8_t *dropout_keep,
+                           float dropout_rate, uint64_t seed, uint64_t counter, int64_t n, int64_t n_global, int64_t row_offset,
+                           float *grad_out, float *sse_out, void *workspace, int64_t workspace_bytes, void *stream) {
     if (!critic_params || !obs || !act || !target || !workspace || n <= 0 || frames < 1 || frames > SS_MAX_FRAMES)
         return SS_ERR_INVALID_ARG;
     if (dropout_rate < 0.f || dropout_rate >= 1.f) return SS_ERR_INVALID_ARG;
@@ -1019,16 +1327,51 @@ int ss_critic_grad_frames(const float *critic_params, int frames, const float *o
     const Lay L = lay_of(DS * frames);
     const int cap = (int)(workspace_bytes / ((int64_t)(L.c_n + 1) * 4));
     if (cap < 1) return SS_ERR_INVALID_ARG;
-    const int grid = grid_for(critic_grad_kernel, smem_critic_grad(L.ds), (n + TB - 1) / TB,
-                              cap < SS_LEARNER_MAX_PARTS ? cap : SS_LEARNER_MAX_PARTS);
+    auto kernel = weighted ? critic_grad_weighted_kernel : critic_grad_kernel;
+    const int grid = grid_for(kernel, smem_critic_grad(L.ds), (n + TB - 1) / TB, cap < SS_LEARNER_MAX_PARTS ? cap : SS_LEARNER_MAX_PARTS);
     if (grid < 0) return SS_ERR_CUDA;
     CriticGradArgs A{critic_params, obs, act, target, dropout_keep, dropout_rate, seed, counter,
-                     n, n_global > 0 ? n_global : n, row_offset, (float *)workspace, L.ds};
+                     n, n_global > 0 ? n_global : n, row_offset, (float *)workspace, L.ds, row_weight, td_abs_out};
     cudaStream_t st = (cudaStream_t)stream;
-    critic_grad_kernel<<<grid, NT, smem_critic_grad(L.ds), st>>>(A);
+    kernel<<<grid, NT, smem_critic_grad(L.ds), st>>>(A);
     if (!grad_out) return check_launch() == SS_OK ? grid : SS_ERR_CUDA;      // slices only (ss_peer_reduce_push follows)
     reduce_kernel<<<(L.c_n + 1 + 63) / 64, dim3(64, 4), 0, st>>>((const float *)workspace, grid, L.c_n, grad_out, sse_out);
     return check_launch();
+}
+
+int ss_critic_grad_frames(const float *critic_params, int frames, const float *obs, const float *act, const float *target,
+                          const uint8_t *dropout_keep, float dropout_rate, uint64_t seed, uint64_t counter,
+                          int64_t n, int64_t n_global, int64_t row_offset, float *grad_out, float *sse_out,
+                          void *workspace, int64_t workspace_bytes, void *stream) {
+    return critic_grad_f32(critic_params, frames, obs, act, target, nullptr, nullptr, false, dropout_keep, dropout_rate, seed, counter,
+                           n, n_global, row_offset, grad_out, sse_out, workspace, workspace_bytes, stream);
+}
+
+int ss_critic_grad_weighted(const float *critic_params, int frames, int tensor_cores, const float *obs, const float *act,
+                            const float *target, const float *row_weight, float *td_abs_out, const uint8_t *dropout_keep,
+                            float dropout_rate, uint64_t seed, uint64_t counter, int64_t n, int64_t n_global, int64_t row_offset,
+                            float *grad_out, float *sse_out, void *workspace, int64_t workspace_bytes, void *stream) {
+    if (!critic_params || !obs || !act || !target || !workspace || n <= 0 || frames < 1 || frames > SS_MAX_FRAMES)
+        return SS_ERR_INVALID_ARG;
+    if (!(dropout_rate >= 0.f && dropout_rate < 1.f) || n_global < 0 || row_offset < 0) return SS_ERR_INVALID_ARG;
+    if (((uintptr_t)row_weight | (uintptr_t)td_abs_out) & 3) return SS_ERR_INVALID_ARG;
+    if (!tensor_cores)
+        return critic_grad_f32(critic_params, frames, obs, act, target, row_weight, td_abs_out, true, dropout_keep, dropout_rate, seed,
+                               counter, n, n_global, row_offset, grad_out, sse_out, workspace, workspace_bytes, stream);
+    // the checks of ss_critic_grad_tc / ss_critic_grad_frames_tc
+    if (((uintptr_t)critic_params | (uintptr_t)obs) & 15 || ((uintptr_t)act & 7)) return SS_ERR_INVALID_ARG;
+    if (frames == 1) {
+        if ((uintptr_t)dropout_keep & 15) return SS_ERR_INVALID_ARG;
+        if (workspace_bytes / ((int64_t)(SS_CRITIC_PARAMS + 1) * 4) < 1) return SS_ERR_INVALID_ARG;
+        return sstc::critic_grad_tc_weighted(critic_params, obs, act, target, row_weight, td_abs_out, dropout_keep, dropout_rate, seed,
+                                             counter, n, n_global, row_offset, grad_out, sse_out, workspace, workspace_bytes,
+                                             (cudaStream_t)stream);
+    }
+    if (((uintptr_t)dropout_keep & 7) || ((uintptr_t)workspace & 15) || workspace_bytes < ss_learner_frames_tc_workspace_bytes(frames, n))
+        return SS_ERR_INVALID_ARG;
+    return sstc::critic_grad_frames_tc_weighted(critic_params, frames, obs, act, target, row_weight, td_abs_out, dropout_keep,
+                                                dropout_rate, seed, counter, n, n_global, row_offset, grad_out, sse_out, workspace,
+                                                workspace_bytes, (cudaStream_t)stream);
 }
 
 int ss_actor_grad_frames(const float *actor_params, const float *critic_params, int frames, const float *obs, int64_t n,
@@ -1166,6 +1509,78 @@ int ss_replay_sample_nstep(const float *ring_obs, const float *ring_act, const f
     if (sslaunch::launch(replay_sample_nstep_kernel, dim3((unsigned)((w4 * batch + 255) / 256)), dim3(256), 0, (cudaStream_t)stream,
                          R, runs, total, tick_rows, n_step, gamma, seed, counter, batch, obs, act, reward, next_obs, done,
                          indices_out, steps_out, w4, early) != cudaSuccess)
+        return SS_ERR_CUDA;
+    return check_launch();
+}
+
+int64_t ss_replay_priority_scratch_bytes(int64_t capacity) { return capacity < 1 ? -1 : pri_scratch_bytes(capacity); }
+
+int ss_replay_sample_prioritized(const float *ring_obs, const float *ring_act, const float *ring_reward, const float *ring_next_obs,
+                                 const uint8_t *ring_done, int64_t capacity, int frames, int64_t tick_rows, int n_step, float gamma,
+                                 const int64_t *runs_host, int n_runs, uint64_t seed, uint64_t counter, int64_t batch, float *obs,
+                                 float *act, float *reward, float *next_obs, uint8_t *done, int64_t *indices_out, uint8_t *steps_out,
+                                 const float *priority, void *scratch, int64_t scratch_bytes, float beta, float *weights_out,
+                                 void *stream) {
+    if (!ring_obs || !ring_act || !ring_reward || !ring_next_obs || !ring_done || !obs || !act || !reward || !next_obs ||
+        !done || !runs_host || !priority || !scratch || !weights_out)
+        return SS_ERR_INVALID_ARG;
+    if (capacity <= 0 || batch <= 0 || frames < 1 || frames > SS_MAX_FRAMES || tick_rows < 1 || n_step < 1 ||
+        n_step > SS_REPLAY_MAX_NSTEP || tick_rows > capacity / n_step || n_runs < 1 || n_runs > SS_REPLAY_MAX_RUNS ||
+        !std::isfinite(gamma) || !std::isfinite(beta) || beta < 0.f || beta > 1.f)
+        return SS_ERR_INVALID_ARG;
+    if (((uintptr_t)ring_obs | (uintptr_t)ring_next_obs | (uintptr_t)obs | (uintptr_t)next_obs) & 15) return SS_ERR_INVALID_ARG;
+    if (((uintptr_t)scratch & 7) || ((uintptr_t)priority & 3) || ((uintptr_t)weights_out & 3) || ((uintptr_t)indices_out & 7) ||
+        ((uintptr_t)act & 7))
+        return SS_ERR_INVALID_ARG;
+    if (scratch_bytes < pri_scratch_bytes(capacity)) return SS_ERR_INVALID_ARG;
+    NstepRuns runs{};
+    int64_t total = 0;
+    for (int i = 0; i < n_runs; ++i) {
+        const int64_t st = runs_host[2 * i], len = runs_host[2 * i + 1];
+        if (st < 0 || len < 1 || st >= capacity || len > capacity - st) return SS_ERR_INVALID_ARG;
+        runs.start[i] = st;
+        runs.length[i] = len;
+        total += len;
+    }
+    runs.n = n_runs;
+    if (total > capacity) return SS_ERR_INVALID_ARG;          // (runs that overlap)
+    Ring R{(float *)ring_obs, (float *)ring_act, (float *)ring_reward, (float *)ring_next_obs, (uint8_t *)ring_done, capacity};
+    const PriScratch S = pri_scratch(scratch, capacity);
+    const int64_t nb = (total + kPriChunk - 1) / kPriChunk;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (sslaunch::launch(priority_scan_kernel, dim3((unsigned)nb), dim3(kPriThreads), 0, st, priority, runs, total, S) != cudaSuccess)
+        return SS_ERR_CUDA;
+    if (sslaunch::launch(priority_blocks_kernel, dim3(1), dim3(kPriBlocksThreads), 0, st, nb, S) != cudaSuccess)
+        return SS_ERR_CUDA;
+    if (sslaunch::launch(replay_sample_prioritized_kernel, dim3((unsigned)((batch + kPriRows - 1) / kPriRows)), dim3(256), 0, st, R,
+                         runs, total, nb, S, priority, tick_rows, n_step, gamma, seed, counter, batch, beta, obs, act, reward,
+                         next_obs, done, indices_out, steps_out, weights_out, 3 * frames) != cudaSuccess)
+        return SS_ERR_CUDA;
+    return check_launch();
+}
+
+int ss_replay_priority_update(float *priority, float *priority_max, int64_t capacity, const int64_t *indices, const float *td_abs,
+                              int64_t batch, float alpha, float eps, int32_t *scratch, void *stream) {
+    if (!priority || !priority_max || !indices || !td_abs || !scratch || capacity < 1 || batch < 1 || batch > INT32_MAX)
+        return SS_ERR_INVALID_ARG;
+    if (!std::isfinite(alpha) || alpha < 0.f || !std::isfinite(eps) || !(eps > 0.f)) return SS_ERR_INVALID_ARG;
+    if (((uintptr_t)priority | (uintptr_t)priority_max | (uintptr_t)td_abs | (uintptr_t)scratch) & 3 || ((uintptr_t)indices & 7))
+        return SS_ERR_INVALID_ARG;
+    const dim3 grid((unsigned)((batch + 255) / 256));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (sslaunch::launch(priority_mark_kernel, grid, dim3(256), 0, st, indices, batch, capacity, (int *)scratch) != cudaSuccess ||
+        sslaunch::launch(priority_claim_kernel, grid, dim3(256), 0, st, indices, batch, capacity, (int *)scratch) != cudaSuccess ||
+        sslaunch::launch(priority_write_kernel, grid, dim3(256), 0, st, indices, td_abs, batch, capacity, (const int *)scratch, alpha,
+                         eps, priority, priority_max) != cudaSuccess)
+        return SS_ERR_CUDA;
+    return check_launch();
+}
+
+int ss_replay_priority_fill(float *priority, const float *priority_max, int64_t capacity, int64_t pos, int64_t n, void *stream) {
+    if (!priority || !priority_max || capacity < 1 || pos < 0 || pos >= capacity || n < 1 || n > capacity) return SS_ERR_INVALID_ARG;
+    if (((uintptr_t)priority | (uintptr_t)priority_max) & 3) return SS_ERR_INVALID_ARG;
+    if (sslaunch::launch(priority_fill_kernel, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, (cudaStream_t)stream, priority,
+                         priority_max, capacity, pos, n) != cudaSuccess)
         return SS_ERR_CUDA;
     return check_launch();
 }

@@ -69,8 +69,14 @@ constexpr uint32_t T_WORK = 384;     // z1 halves, z2, dx2 halves  [128 rows][12
 struct GradArgs {
     const float *params, *obs;
     const float *act, *target;       // critic: actions [n][2], regression target [n]
-    const float *up;                 // actor: upstream gradient on the action [n][2] (= -dQ/da)
-    const float *q;                  // actor: Q(s, actor(s)) per row [n] or NULL; its sum goes out through the slices' extra slot
+    union {                          // (the weighted critic's pointers share the actor's slots: the struct keeps its layout)
+        const float *up;             // actor: upstream gradient on the action [n][2] (= -dQ/da)
+        float *td_abs;               // WEIGHTED: |q - target| of each row [n] or NULL
+    };
+    union {
+        const float *q;              // actor: Q(s, actor(s)) per row [n] or NULL; its sum goes out through the slices' extra slot
+        const float *row_weight;     // WEIGHTED: the loss weight of each row [n] or NULL (1)
+    };
     const uint8_t *keep;             // critic: injected dropout mask [n][256] or NULL (Philox)
     float rate;
     uint64_t seed, counter;
@@ -78,6 +84,7 @@ struct GradArgs {
     float *work;                     // [gridDim.x][params + 1]
     int early_weights;               // ss_launch.cuh: the parameters may be staged ahead of griddepcontrol.wait (set by launch_grad)
 };
+
 
 // inverted-dropout keep bits of 8 consecutive hidden-1 units of one row: one Philox draw, 16 bits per unit
 __device__ __forceinline__ uint32_t keep8(const GradArgs &A, int64_t grow, int chunk, uint32_t thresh16) {
@@ -113,7 +120,8 @@ __device__ __forceinline__ void sweep_work(uint32_t taddr, int cs, F &&f) {
     }
 }
 
-template <int NET>
+// WEIGHTED (the critic only): ss_critic_grad_weighted's row weights and |e| out
+template <int NET, bool WEIGHTED>
 __global__ void __launch_bounds__(NTHREADS, 1) mlp_grad_tc_kernel(const GradArgs A) {
     constexpr int PN = NET == NET_ACTOR ? A_N : C_N;
     extern __shared__ __align__(128) uint8_t smem[];
@@ -305,6 +313,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_grad_tc_kernel(const GradArgs
                     const float e = (z0 + b3[0]) - tgt;
                     stat += e * e;
                     d0 = 2.0f * e / (float)A.n_global;
+                    if constexpr (WEIGHTED) {             // (the weight last: w = 1 leaves d0 as it is)
+                        if (A.row_weight) d0 = d0 * __ldg(A.row_weight + row);
+                        if (A.td_abs && cs == 0) A.td_abs[row] = fabsf(e);
+                    }
                 }
             } else if (valid) {                           // through tanh, upstream = -dQ/da (SkillshotLearner.py:408-410)
                 stat += tgt;                              // Q of the row (reported sum)
@@ -533,13 +545,13 @@ __global__ void reduce_parts_kernel(const float *work, int parts, int n_params, 
     }
 }
 
-template <int NET>
+template <int NET, bool WEIGHTED = false>
 int launch_grad(const GradArgs &A0, float *grad_out, float *aux_out, int64_t workspace_bytes, void *stream) {
     constexpr int PN = NET == NET_ACTOR ? A_N : C_N;
     int dev = 0, sms = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) return SS_ERR_CUDA;
     if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return SS_ERR_CUDA;
-    if (cudaFuncSetAttribute(mlp_grad_tc_kernel<NET>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SM_TOTAL) != cudaSuccess)
+    if (cudaFuncSetAttribute(mlp_grad_tc_kernel<NET, WEIGHTED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SM_TOTAL) != cudaSuccess)
         return SS_ERR_CUDA;
     const int64_t tiles = (A0.n + TM - 1) / TM;
     int64_t cap = workspace_bytes / ((int64_t)(PN + 1) * 4);
@@ -552,7 +564,7 @@ int launch_grad(const GradArgs &A0, float *grad_out, float *aux_out, int64_t wor
     cudaStream_t st = (cudaStream_t)stream;
     GradArgs A1 = A0;
     A1.early_weights = sslaunch::take_early_weights();
-    if (sslaunch::launch(mlp_grad_tc_kernel<NET>, dim3(grid), dim3(NTHREADS), SM_TOTAL, st, A1) != cudaSuccess) return SS_ERR_CUDA;
+    if (sslaunch::launch(mlp_grad_tc_kernel<NET, WEIGHTED>, dim3(grid), dim3(NTHREADS), SM_TOTAL, st, A1) != cudaSuccess) return SS_ERR_CUDA;
     if (!grad_out) return cudaGetLastError() == cudaSuccess ? grid : SS_ERR_CUDA;   // slices only (ss_peer_reduce_push follows)
     reduce_parts_kernel<<<(PN + 1 + 63) / 64, dim3(64, 4), 0, st>>>(A0.work, grid, PN, grad_out, aux_out);
     return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA;
@@ -581,6 +593,17 @@ __global__ void td3_min_target_kernel(const float *q1, const float *q2, const fl
 int sstc::reduce_slices(const float *work, int parts, int n_params, float *grad, float *aux, cudaStream_t st) {
     reduce_parts_kernel<<<(n_params + 1 + 63) / 64, dim3(64, 4), 0, st>>>(work, parts, n_params, grad, aux);
     return cudaGetLastError() == cudaSuccess ? SS_OK : SS_ERR_CUDA;
+}
+
+int sstc::critic_grad_tc_weighted(const float *critic_params, const float *obs, const float *act, const float *target,
+                                   const float *row_weight, float *td_abs_out, const uint8_t *dropout_keep, float dropout_rate,
+                                   uint64_t seed, uint64_t counter, int64_t n, int64_t n_global, int64_t row_offset, float *grad_out,
+                                   float *sse_out, void *workspace, int64_t workspace_bytes, cudaStream_t stream) {
+    GradArgs A{};
+    A.params = critic_params; A.obs = obs; A.act = act; A.target = target; A.keep = dropout_keep; A.rate = dropout_rate;
+    A.seed = seed; A.counter = counter; A.n = n; A.n_global = n_global > 0 ? n_global : n; A.row_offset = row_offset;
+    A.work = (float *)workspace; A.row_weight = row_weight; A.td_abs = td_abs_out;
+    return launch_grad<NET_CRITIC, true>(A, grad_out, sse_out, workspace_bytes, stream);
 }
 
 int sstc::td3_smooth_actions(float *act, int64_t n, float sigma, float clip, uint64_t seed, uint64_t counter, int64_t row_offset,

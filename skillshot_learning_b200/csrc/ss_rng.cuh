@@ -16,6 +16,7 @@ constexpr uint32_t kTagDropout = 2;      // Dropout(0.2) during critic.fit, Skil
 constexpr uint32_t kTagActionNoise = 3;  // model_act_action_noise, SkillshotLearner.py:238
 constexpr uint32_t kTagReplay = 4;       // minibatch row choice (np.random.shuffle at :427 in the reference)
 constexpr uint32_t kTagTargetNoise = 5;  // TD3 target policy smoothing (no reference code, DESIGN.md section 6.14)
+constexpr uint32_t kTagPriority = 6;     // stratified prioritized replay draw (no reference code, DESIGN.md section 6.16)
 
 SS_HD U4 draw4(uint64_t seed, uint32_t tag, uint32_t a, uint32_t b, uint64_t counter) {
     return philox4x32_10(U4{a, b, (uint32_t)counter, tag ^ (uint32_t)(counter >> 32)},

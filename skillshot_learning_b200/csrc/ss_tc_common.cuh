@@ -381,5 +381,16 @@ int td3_smooth_actions(float *act, int64_t n, float sigma, float clip, uint64_t 
                        cudaStream_t st);
 int td3_min_target(const float *q1, const float *q2, const float *reward, const uint8_t *done, float gamma, float *y, int64_t n,
                    cudaStream_t st);
+// ss_critic_grad_weighted's tensor-core families, arguments checked by the caller: the 12-input gradient kernel
+// (ss_mlp_grad_tc.cu) and the frame-stacked one (ss_frames_grad_tc.cu), with d = (2 e / n_global) * row_weight[row] and
+// td_abs_out[row] = |e| (either pointer may be NULL)
+int critic_grad_tc_weighted(const float *critic_params, const float *obs, const float *act, const float *target,
+                            const float *row_weight, float *td_abs_out, const uint8_t *dropout_keep, float dropout_rate,
+                            uint64_t seed, uint64_t counter, int64_t n, int64_t n_global, int64_t row_offset, float *grad_out,
+                            float *sse_out, void *workspace, int64_t workspace_bytes, cudaStream_t stream);
+int critic_grad_frames_tc_weighted(const float *critic_params, int frames, const float *obs, const float *act, const float *target,
+                                   const float *row_weight, float *td_abs_out, const uint8_t *dropout_keep, float dropout_rate,
+                                   uint64_t seed, uint64_t counter, int64_t n, int64_t n_global, int64_t row_offset,
+                                   float *grad_out, float *sse_out, void *workspace, int64_t workspace_bytes, cudaStream_t stream);
 
 }  // namespace sstc

@@ -15,6 +15,7 @@
 #include "ss_launch.cuh"
 
 #include <atomic>
+#include <cmath>
 #include <string.h>
 
 int &sslaunch::pdl_mode() {
@@ -42,6 +43,13 @@ extern "C" int ss_ddpg_update(const ss_ddpg_update_args *a, void *stream) {
         return SS_ERR_INVALID_ARG;
     if (a->gamma != 0.f && (!a->y || !a->target_actor || !a->target_critic)) return SS_ERR_INVALID_ARG;
     if (a->n_step < 0 || a->n_step > SS_REPLAY_MAX_NSTEP) return SS_ERR_INVALID_ARG;
+    // prioritized replay: the previous update's priority write must land before this draw builds its prefix, so the draw
+    // cannot start beside that update's tail (sample_early)
+    const bool pri = a->prioritized != 0;
+    if (pri && (a->sample_early || !a->indices || !a->priority || !a->priority_max || !a->priority_scratch ||
+                !a->priority_update_scratch || !a->weights || !a->td_abs || !std::isfinite(a->priority_alpha) ||
+                a->priority_alpha < 0.f || !std::isfinite(a->priority_eps) || !(a->priority_eps > 0.f)))
+        return SS_ERR_INVALID_ARG;
     const int64_t n = a->batch;
     const bool tc = a->tensor_cores != 0;
     int rc;
@@ -65,7 +73,15 @@ extern "C" int ss_ddpg_update(const ss_ddpg_update_args *a, void *stream) {
     // caller vouches for it (args.sample_early)
     if (kOn && a->sample_early) sslaunch::pdl_mode() = kOn | sslaunch::kPdlSampleEarly;
     // (n-step rows: the same draw over the eligible runs, then the walk; a->gamma is g_n)
-    if (a->n_step > 1)
+    if (pri) {
+        const int64_t whole[2] = {0, a->size};
+        const bool nstep = a->n_step > 1;
+        rc = ss_replay_sample_prioritized(a->ring_obs, a->ring_act, a->ring_reward, a->ring_next_obs, a->ring_done, a->capacity, 1,
+                                          nstep ? a->tick_rows : 1, nstep ? a->n_step : 1, nstep ? a->step_gamma : 0.f,
+                                          nstep ? a->runs_host : whole, nstep ? a->n_runs : 1, a->replay_seed, a->replay_counter, n,
+                                          a->obs, a->act, a->reward, a->next_obs, a->done, a->indices, nullptr, a->priority,
+                                          a->priority_scratch, a->priority_scratch_bytes, a->priority_beta, a->weights, stream);
+    } else if (a->n_step > 1)
         rc = ss_replay_sample_nstep(a->ring_obs, a->ring_act, a->ring_reward, a->ring_next_obs, a->ring_done, a->capacity, 1,
                                     a->tick_rows, a->n_step, a->step_gamma, a->runs_host, a->n_runs, a->replay_seed,
                                     a->replay_counter, n, a->obs, a->act, a->reward, a->next_obs, a->done, a->indices, nullptr,
@@ -90,9 +106,15 @@ extern "C" int ss_ddpg_update(const ss_ddpg_update_args *a, void *stream) {
     // critic: gradient of the batch-mean squared error -> (exchange) -> Adam (+ soft target update).  The gradient
     // kernels leave per-CTA slices; one more kernel sums them in a fixed order and applies Adam (ss_reduce_adam_tf), or
     // pushes the sum to every rank's inbox (ss_peer_reduce_push) for the peers' Adam kernel.
+    // (prioritized: the loss of each row weighted by its importance weight, and its |e| kept for the priority update)
     auto critic_grad = tc ? ss_critic_grad_tc : ss_critic_grad;
-    rc = critic_grad(a->critic, a->obs, a->act, y, nullptr, a->dropout_rate, a->seed, a->counter, n, a->n_global, a->row_offset,
-                     nullptr, a->stats, a->workspace, a->workspace_bytes, stream);
+    if (pri)
+        rc = ss_critic_grad_weighted(a->critic, 1, tc ? 1 : 0, a->obs, a->act, y, a->weights, a->td_abs, nullptr, a->dropout_rate,
+                                     a->seed, a->counter, n, a->n_global, a->row_offset, nullptr, a->stats, a->workspace,
+                                     a->workspace_bytes, stream);
+    else
+        rc = critic_grad(a->critic, a->obs, a->act, y, nullptr, a->dropout_rate, a->seed, a->counter, n, a->n_global, a->row_offset,
+                         nullptr, a->stats, a->workspace, a->workspace_bytes, stream);
     if (rc <= 0) return rc < 0 ? rc : SS_ERR_INVALID_ARG;
     sslaunch::pdl_mode() = kOn;
     // The actor step begins with a = actor(s), which needs neither the critic's new weights nor anything the exchange
@@ -123,6 +145,11 @@ extern "C" int ss_ddpg_update(const ss_ddpg_update_args *a, void *stream) {
                                a->target_critic, a->step_critic, a->lr_critic, a->beta1, a->beta2, a->eps, a->tau, 1.0f, stream);
     }
     if (rc != SS_OK) return rc;
+    if (pri) {         // the drawn rows' new leaves from this step's |e|
+        rc = ss_replay_priority_update(a->priority, a->priority_max, a->capacity, a->indices, a->td_abs, n, a->priority_alpha,
+                                       a->priority_eps, a->priority_update_scratch, stream);
+        if (rc != SS_OK) return rc;
+    }
 
     // actor: model_actor_fit_step with the critic just updated (SkillshotLearner.py:440-443 follows 434)
     sslaunch::pdl_mode() = kEarly;

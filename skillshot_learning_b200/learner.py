@@ -134,6 +134,36 @@ def check_td3_options(twin_critics, policy_delay, target_noise, target_noise_cli
                           ("target_noise_clip", float(target_noise_clip))), group)
 
 
+def check_priority_options(prioritized, alpha, beta, eps, group=None):
+    """ValueError unless alpha >= 0, 0 <= beta <= 1 and eps > 0, all finite (prioritized replay, DESIGN.md section 6.16).
+    Sharded (group not None): every rank checks its own arguments and ranks_agree compares the refusals and the four
+    values, so every rank raises the same ValueError or none does."""
+    refusal = None
+    vals = []
+    for name, v in (("priority_alpha", alpha), ("priority_beta", beta), ("priority_eps", eps)):
+        try:
+            vals.append(float(v))
+        except (TypeError, ValueError):
+            refusal = "%s must be a finite number, got %r" % (name, v)
+            break
+    if refusal is None:
+        a, b, e = vals
+        if not math.isfinite(a) or a < 0.0:
+            refusal = "priority_alpha must be finite and >= 0, got %r" % (alpha,)
+        elif not math.isfinite(b) or not 0.0 <= b <= 1.0:
+            refusal = "priority_beta must be in [0, 1], got %r" % (beta,)
+        elif not math.isfinite(e) or not e > 0.0:
+            refusal = "priority_eps must be finite and > 0, got %r" % (eps,)
+    if group is None:
+        if refusal is not None:
+            raise ValueError(refusal)
+        return
+    check_process_group(group)
+    ranks_agree(refusal, (("prioritized_replay", bool(prioritized)), ("priority_alpha", alpha if refusal else float(alpha)),
+                          ("priority_beta", beta if refusal else float(beta)), ("priority_eps", eps if refusal else float(eps))),
+                group)
+
+
 def nstep_refusal(n_step, capacity: int, tick_rows: int) -> Optional[str]:
     """The message of the ValueError for an n_step that is not an integer in 1..SS_REPLAY_MAX_NSTEP, or for a ring of
     `capacity` rows shorter than n_step ticks of tick_rows rows; None when both are fine."""
@@ -603,10 +633,12 @@ class ActorCritic:
         return self.critic2_sse if which == "critic2" else self.stats[0:1]
 
     def critic_grad(self, obs, act, y, keep=None, n_global: int = 0, row_offset: int = 0, slices_only: bool = False,
-                    which: str = "critic"):
+                    which: str = "critic", weights=None, td_abs_out: Optional[torch.Tensor] = None):
         """grads[critic] <- d/dphi mean (q - y)^2 of this (shard of a) batch; returns the gradient view.
         slices_only: leave the per-CTA slices in the workspace and return their number (peer exchange).
-        which: "critic", or "critic2" with twin critics (its own slices of params / grads, its sum in critic2_sse)."""
+        which: "critic", or "critic2" with twin critics (its own slices of params / grads, its sum in critic2_sse).
+        weights / td_abs_out (prioritized replay, ss_critic_grad_weighted): each row's loss gradient times its weight, and
+        |q - y| of each row written to the float32 device tensor td_abs_out."""
         obs, act = _f32(obs, self.device).reshape(-1, 12 * self.frames), _f32(act, self.device).reshape(-1, 2)
         y = _f32(y, self.device).reshape(-1)
         n = obs.shape[0]
@@ -617,8 +649,18 @@ class ActorCritic:
         ws = self._workspace_for(n)
         tail = (_ptr(keep), self.dropout, self.seed, self.counter, n, int(n_global), int(row_offset),
                 None if slices_only else g.data_ptr(), self._sse(which).data_ptr(), ws.data_ptr(), ws.numel(), _stream(self.device))
+        if weights is not None:
+            weights = _f32(weights, self.device).reshape(-1)
+            if weights.shape[0] != n:
+                raise ValueError("weights must have one entry per row")
+        if td_abs_out is not None and (td_abs_out.dtype != torch.float32 or td_abs_out.numel() < n or not td_abs_out.is_contiguous()):
+            raise ValueError("td_abs_out must be a contiguous float32 tensor of at least %d entries" % n)
         with torch.cuda.device(self.device):
-            if self.update_precision == "bf16" and self.frames > 1:
+            if weights is not None or td_abs_out is not None:
+                rc = lib.ss_critic_grad_weighted(phi.data_ptr(), self.frames, 1 if self.update_precision == "bf16" else 0,
+                                                 obs.data_ptr(), act.data_ptr(), y.data_ptr(), _ptr(weights), _ptr(td_abs_out),
+                                                 *tail)
+            elif self.update_precision == "bf16" and self.frames > 1:
                 rc = lib.ss_critic_grad_frames_tc(phi.data_ptr(), self.frames, obs.data_ptr(), act.data_ptr(), y.data_ptr(),
                                                   *tail)
             elif self.update_precision == "bf16":
@@ -696,21 +738,23 @@ class ActorCritic:
                                         step, lr, self.beta1, self.beta2, self.eps, tau, float(grad_scale),
                                         _stream(self.device)), "ss_reduce_adam_tf")
 
-    def critic_step(self, obs, act, y, keep=None, which: str = "critic", tau: Optional[float] = None):
+    def critic_step(self, obs, act, y, keep=None, which: str = "critic", tau: Optional[float] = None, weights=None,
+                    td_abs_out: Optional[torch.Tensor] = None):
         """One batch of model_critic.fit (SkillshotLearner.py:434): gradient of the batch-mean
         squared error, summed over the ranks when sharded, then Adam.  Returns the (device) sum of squared errors.
         which: "critic" or "critic2" (twin critics); tau: the soft update's tau instead of self.tau (TD3: 0 between
-        delayed updates)."""
+        delayed updates).  weights / td_abs_out: prioritized replay's importance weights and |q - y| (critic_grad)."""
         _, n_global, row_offset = shard_info(int(np.prod(y.shape)), self.group)
         sse = self._sse(which)
+        wt = dict(weights=weights, td_abs_out=td_abs_out)
         if self.group is not None and self.peer is None:      # NCCL: gradient -> all-reduce -> Adam
-            g = self.critic_grad(obs, act, y, keep, n_global=n_global, row_offset=row_offset, which=which)
+            g = self.critic_grad(obs, act, y, keep, n_global=n_global, row_offset=row_offset, which=which, **wt)
             self._allreduce(g)
             self.apply_adam(which, tau=tau)
             return sse[0]
         # per-CTA slices -> one kernel that sums them and applies Adam (single GPU), or pushes the sum into every
         # rank's inbox for the peers' Adam kernel (fused exchange)
-        parts = self.critic_grad(obs, act, y, keep, n_global=n_global, row_offset=row_offset, slices_only=True, which=which)
+        parts = self.critic_grad(obs, act, y, keep, n_global=n_global, row_offset=row_offset, slices_only=True, which=which, **wt)
         if self.peer is not None:
             self.peer.reduce_push(self.workspace, parts, self.c_n, sse)
             self.apply_adam(which, from_peers=True, tau=tau)
@@ -733,33 +777,40 @@ class ActorCritic:
             self.reduce_adam("actor", parts, self.stats[1:2], tau=tau)
         return self.stats[1]
 
-    def td3_step(self, obs, act, reward, next_obs, done=None, discount: Optional[float] = None):
+    def td3_step(self, obs, act, reward, next_obs, done=None, discount: Optional[float] = None, weights=None,
+                 td_abs_out: Optional[torch.Tensor] = None):
         """One TD3 update on a (shard of a) minibatch (class docstring): the target, a critic step on critic 1 and one on
         critic 2 against the same y (each with its own Philox dropout draw: the counter advances per call), and on every
         policy_delay-th update the actor step against critic 1.  Only those delayed updates soft-update the targets; the
         others pass tau = 0, which leaves every target byte-identical.  Returns (critic 1's sum of squared errors, the
-        sum of q of the last actor step), device scalars; critic 2's sum is in critic2_sse.  discount: as for td_targets."""
+        sum of q of the last actor step), device scalars; critic 2's sum is in critic2_sse.  discount: as for td_targets.
+        weights: prioritized replay's importance weights, for both critics; td_abs_out: critic 1's |q - y|."""
         _, _, row_offset = shard_info(int(np.prod(reward.shape)), self.group)
         y = self.td_targets(reward, next_obs, done, row_offset=row_offset, discount=discount)
         delayed = (self.td3_updates + 1) % self.policy_delay == 0
         tau = self.tau if delayed else 0.0
-        sse = self.critic_step(obs, act, y, tau=tau)
+        sse = self.critic_step(obs, act, y, tau=tau, weights=weights, td_abs_out=td_abs_out)
         if self.twin_critics:
-            self.critic_step(obs, act, y, which="critic2", tau=tau)
+            self.critic_step(obs, act, y, which="critic2", tau=tau, weights=weights)
         if delayed:
             self.actor_step(obs, tau=tau)
         self.td3_updates += 1
         return sse, self.stats[1]
 
     def update_from_ring(self, ring: "ReplayRing", batch: int, out: Optional[dict] = None, sample_early: bool = False,
-                         n_step: int = 1):
+                         n_step: int = 1, priority_beta: Optional[float] = None, priority_alpha: float = 0.6,
+                         priority_eps: float = 1e-6):
         """One whole update step from ONE library call (ss_ddpg_update): sample `batch` rows of `ring`,
         TD target, critic step, actor step -- the launches critic_step / actor_step make, without the
         interpreter time between them.  Single GPU or the fused peer exchange (an NCCL all-reduce needs
         the host between the gradient and Adam: use the separate steps).  Returns the minibatch dict.
         sample_early: the caller guarantees that the previous launch on the stream neither writes the ring nor touches
         `out` (ss_ddpg_update_args.sample_early): the minibatch is gathered while that launch still runs.
-        n_step > 1: n-step rows of a ring with tick_rows (ReplayRing.sample), bootstrapped with nstep_discount(gamma, n_step)."""
+        n_step > 1: n-step rows of a ring with tick_rows (ReplayRing.sample), bootstrapped with nstep_discount(gamma, n_step).
+        priority_beta (a prioritized ring, DESIGN.md section 6.16): the prioritized draw with importance-weight exponent
+        priority_beta, the critic's loss weighted by those weights, and the drawn rows' leaves set from the critic step's
+        |q - y| with priority_alpha and priority_eps; the dict also holds `weights` and `td_abs`.  Refused with
+        sample_early (the previous update's priority write must land before the draw)."""
         if self.group is not None and self.peer is None:
             raise ValueError("update_from_ring needs collective='peer' when the update is sharded")
         if self.frames > 1:
@@ -767,10 +818,16 @@ class ActorCritic:
         runs = None
         if n_step != 1:
             runs, n_runs = ring.nstep_table(n_step)
+        pri = priority_beta is not None
+        if pri:
+            ring.check_priority_draw(priority_beta)
+            check_priority_options(True, priority_alpha, priority_beta, priority_eps)
+            if sample_early:
+                raise ValueError("a prioritized update cannot draw beside the previous update (sample_early)")
         if ring.size == 0:
             raise ValueError("sampling from an empty ring")
         dev = self.device
-        if out is None or out["reward"].shape[0] != batch or "y" not in out:
+        if out is None or out["reward"].shape[0] != batch or "y" not in out or (pri and "weights" not in out):
             out = dict(obs=torch.empty((batch, 12), dtype=torch.float32, device=dev),
                        act=torch.empty((batch, 2), dtype=torch.float32, device=dev),
                        reward=torch.empty(batch, dtype=torch.float32, device=dev),
@@ -778,10 +835,13 @@ class ActorCritic:
                        done=torch.empty(batch, dtype=torch.uint8, device=dev),
                        indices=torch.empty(batch, dtype=torch.int64, device=dev),
                        y=torch.empty(batch, dtype=torch.float32, device=dev))
+            if pri:
+                out["weights"] = torch.empty(batch, dtype=torch.float32, device=dev)
+                out["td_abs"] = torch.empty(batch, dtype=torch.float32, device=dev)
         _, n_global, row_offset = shard_info(batch, self.group)
         ws = self._workspace_for(batch)
         key = (ring.obs.data_ptr(), ring.next_obs.data_ptr(), ring.capacity, out["obs"].data_ptr(), out["y"].data_ptr(), ws.data_ptr(),
-               ws.numel(), batch, id(self.peer))
+               ws.numel(), batch, id(self.peer), pri and out["weights"].data_ptr())
         if self._update_args is None:
             self._update_args = {}
         a = self._update_args.get(key)      # one cached argument block per set of minibatch buffers (callers alternate two)
@@ -832,6 +892,13 @@ class ActorCritic:
         else:
             a.n_step, a.tick_rows, a.n_runs, a.runs_host, a.step_gamma = int(n_step), ring.tick_rows, n_runs, runs, self.gamma
             a.gamma = nstep_discount(self.gamma, n_step)
+        a.prioritized = 1 if pri else 0
+        if pri:
+            a.priority, a.priority_max = ring.priority.data_ptr(), ring.priority_max.data_ptr()
+            a.priority_scratch, a.priority_scratch_bytes = ring.priority_scratch.data_ptr(), ring.priority_scratch.numel()
+            a.priority_update_scratch = ring.priority_claim.data_ptr()
+            a.priority_alpha, a.priority_beta, a.priority_eps = priority_alpha, priority_beta, priority_eps
+            a.weights, a.td_abs = out["weights"].data_ptr(), out["td_abs"].data_ptr()
         with torch.cuda.device(dev):
             check(lib.ss_ddpg_update(ctypes.byref(a), _stream(dev)), "ss_ddpg_update")
         ring.counter += 1
@@ -884,9 +951,15 @@ class ReplayRing:
     tick_rows (DESIGN.md section 6.15): the ring is written one block of tick_rows rows per tick, so that the same
     player's next transition after row r is row (r + tick_rows) mod capacity; sample(n_step > 1) then draws n-step rows.
     Such a ring keeps its breaks (mark_break) as a host-side list of ring positions, and drops a break once the rows
-    written before it are overwritten.  A ring without tick_rows keeps no breaks and draws one-step rows only."""
+    written before it are overwritten.  A ring without tick_rows keeps no breaks and draws one-step rows only.
 
-    def __init__(self, capacity: int, device="cuda", seed: int = 0, frames: int = 1, tick_rows: Optional[int] = None):
+    prioritized (DESIGN.md section 6.16): the ring also keeps one float32 leaf p^alpha per row (`priority`) and the device
+    scalar `priority_max` (1.0 at the start).  Every row written gets the leaf priority_max (advance enqueues the fill, so
+    every writer that calls advance is covered); sample(..., beta=...) draws rows in proportion to their leaves and
+    update_priorities writes new ones.  A uniform ring allocates none of this."""
+
+    def __init__(self, capacity: int, device="cuda", seed: int = 0, frames: int = 1, tick_rows: Optional[int] = None,
+                 prioritized: bool = False):
         if tick_rows is not None and not 1 <= int(tick_rows) <= int(capacity):
             raise ValueError("tick_rows must be in 1..capacity, got %r" % (tick_rows,))
         self.capacity, self.device, self.seed = int(capacity), torch.device(device), int(seed)
@@ -903,10 +976,20 @@ class ReplayRing:
         self.pos = 0
         self.size = 0
         self.counter = 0
+        self.prioritized = bool(prioritized)
+        if self.prioritized:
+            self.priority = torch.zeros(c, dtype=torch.float32, device=dev)
+            self.priority_max = torch.ones(1, dtype=torch.float32, device=dev)
+            self.priority_scratch = torch.empty(int(lib.ss_replay_priority_scratch_bytes(c)), dtype=torch.uint8, device=dev)
+            self.priority_claim = torch.empty(c, dtype=torch.int32, device=dev)      # the update's int32 scratch
 
     def advance(self, n: int):
         """Account for n rows written at pos (by push, or in place by a rollout kernel): pos and size move on, and a break
-        whose last row before it was among them is dropped."""
+        whose last row before it was among them is dropped.  A prioritized ring gives the rows the leaf priority_max."""
+        if self.prioritized and n > 0:
+            with torch.cuda.device(self.device):
+                check(lib.ss_replay_priority_fill(self.priority.data_ptr(), self.priority_max.data_ptr(), self.capacity, self.pos,
+                                                  min(int(n), self.capacity), _stream(self.device)), "ss_replay_priority_fill")
         if self.breaks:
             c = self.capacity
             self.breaks = [b for b in self.breaks if n < c and (b - 1 - self.pos) % c >= n]
@@ -938,6 +1021,32 @@ class ReplayRing:
             raise ValueError("no row of the ring can start a %d-step walk (%d rows stored)" % (n_step, self.size))
         return (ctypes.c_int64 * (2 * len(runs)))(*[v for run in runs for v in run]), len(runs)
 
+    def check_priority_draw(self, beta):
+        """ValueError unless this ring is prioritized and beta is a finite number in [0, 1]."""
+        if not self.prioritized:
+            raise ValueError("a prioritized draw needs a ring built with prioritized=True")
+        try:
+            b = float(beta)
+        except (TypeError, ValueError):
+            b = math.nan
+        if not 0.0 <= b <= 1.0:
+            raise ValueError("beta must be in [0, 1], got %r" % (beta,))
+
+    def update_priorities(self, indices, td_abs, alpha: float, eps: float):
+        """leaf[indices[b]] = (|td_abs[b]| + eps)^alpha (powf, float32), the largest b winning for a repeated index, and
+        priority_max raised to the largest leaf written (ss_replay_priority_update)."""
+        if not self.prioritized:
+            raise ValueError("update_priorities needs a ring built with prioritized=True")
+        check_priority_options(True, alpha, 0.0, eps)
+        idx = torch.as_tensor(indices).to(device=self.device, dtype=torch.int64).contiguous().reshape(-1)
+        td = _f32(td_abs, self.device).reshape(-1)
+        if idx.numel() != td.numel() or idx.numel() == 0:
+            raise ValueError("indices and td_abs must have the same number of entries (at least one)")
+        with torch.cuda.device(self.device):
+            check(lib.ss_replay_priority_update(self.priority.data_ptr(), self.priority_max.data_ptr(), self.capacity,
+                                                idx.data_ptr(), td.data_ptr(), idx.numel(), float(alpha), float(eps),
+                                                self.priority_claim.data_ptr(), _stream(self.device)), "ss_replay_priority_update")
+
     def push(self, obs, act, reward, next_obs, done=None, done_div: int = 1):
         obs, next_obs = _f32(obs, self.device).reshape(-1, self.width), _f32(next_obs, self.device).reshape(-1, self.width)
         act, reward = _f32(act, self.device).reshape(-1, 2), _f32(reward, self.device).reshape(-1)
@@ -958,15 +1067,21 @@ class ReplayRing:
                   **{k: getattr(self, k).cpu() for k in ("obs", "act", "reward", "next_obs", "done")})
         if self.tick_rows is not None:
             sd.update(tick_rows=self.tick_rows, breaks=list(self.breaks))
+        if self.prioritized:
+            sd.update(priority=self.priority.cpu(), priority_max=self.priority_max.cpu())
         return sd
 
     def load_state_dict(self, sd):
         """A ring with tick_rows loads the checkpoint's breaks; from a checkpoint without them (a ring without tick_rows)
-        it loads empty (pos = size = 0), because the breaks of its rows are unknown."""
+        it loads empty (pos = size = 0), because the breaks of its rows are unknown.  A prioritized ring loads the
+        checkpoint's leaves and priority_max; from a checkpoint without them every leaf and priority_max are 1.0.  A uniform
+        ring ignores them."""
         if int(sd["capacity"]) != self.capacity:
             raise ValueError("checkpoint ring holds %d rows, this ring %d" % (sd["capacity"], self.capacity))
         if self.tick_rows is not None and "breaks" in sd and int(sd["tick_rows"]) != self.tick_rows:
             raise ValueError("checkpoint ring of %d rows per tick, this ring %d" % (sd["tick_rows"], self.tick_rows))
+        if self.prioritized and "priority" in sd and (sd["priority"].numel() != self.capacity or sd["priority_max"].numel() != 1):
+            raise ValueError("checkpoint priority leaves of %d rows, this ring %d" % (sd["priority"].numel(), self.capacity))
         for k in ("obs", "act", "reward", "next_obs", "done"):
             getattr(self, k).copy_(sd[k].to(self.device))
         self.seed, self.pos, self.size, self.counter = int(sd["seed"]), int(sd["pos"]), int(sd["size"]), int(sd["counter"])
@@ -975,14 +1090,29 @@ class ReplayRing:
                 self.breaks = [int(b) for b in sd["breaks"]]
             else:
                 self.pos, self.size, self.breaks = 0, 0, []
+        if self.prioritized:
+            if "priority" in sd:
+                self.priority.copy_(sd["priority"].to(self.device))
+                self.priority_max.copy_(sd["priority_max"].to(self.device))
+            else:
+                self.priority.fill_(1.0)
+                self.priority_max.fill_(1.0)
 
-    def sample(self, batch: int, indices=None, out: Optional[dict] = None, n_step: int = 1, gamma: float = 0.0):
+    def sample(self, batch: int, indices=None, out: Optional[dict] = None, n_step: int = 1, gamma: float = 0.0,
+               beta: Optional[float] = None):
         """dict(obs, act, reward, next_obs, done, indices) of `batch` rows: the rows `indices` or a
         uniform draw with replacement from the filled part of the ring.
         n_step > 1 (a ring with tick_rows): n-step rows (ss_replay_sample_nstep) drawn uniformly from eligible_runs(n_step),
         with the reward summed with the weights 1, gamma, gamma^2, ... (float32 recurrence) and next_obs / done of the
         walk's last row; the dict also holds `steps`, the rows each walk visited.  Bootstrap such rows with
-        nstep_discount(gamma, n_step)."""
+        nstep_discount(gamma, n_step).
+        beta (a prioritized ring, DESIGN.md section 6.16): the prioritized draw (ss_replay_sample_prioritized) over the same
+        eligible rows, in proportion to their leaves; the dict also holds `weights`, the importance weights
+        (leaf_min / leaf)^beta.  indices must then be None.  Without beta the draw is uniform, also on a prioritized ring."""
+        if beta is not None:
+            self.check_priority_draw(beta)
+            if indices is not None:
+                raise ValueError("prioritized rows are drawn by the sampler: indices must be None")
         if n_step != 1:
             runs, n_runs = self.nstep_table(n_step)
             if indices is not None:
@@ -990,7 +1120,8 @@ class ReplayRing:
         if self.size == 0:
             raise ValueError("sampling from an empty ring")
         dev = self.device
-        if out is None or out["reward"].shape[0] != batch or (n_step != 1 and "steps" not in out):
+        if (out is None or out["reward"].shape[0] != batch or (n_step != 1 and "steps" not in out) or
+                (beta is not None and "weights" not in out)):
             out = dict(obs=torch.empty((batch, self.width), dtype=torch.float32, device=dev),
                        act=torch.empty((batch, 2), dtype=torch.float32, device=dev),
                        reward=torch.empty(batch, dtype=torch.float32, device=dev),
@@ -999,6 +1130,22 @@ class ReplayRing:
                        indices=torch.empty(batch, dtype=torch.int64, device=dev))
             if n_step != 1:
                 out["steps"] = torch.empty(batch, dtype=torch.uint8, device=dev)
+            if beta is not None:
+                out["weights"] = torch.empty(batch, dtype=torch.float32, device=dev)
+        if beta is not None:
+            if n_step == 1:
+                runs, n_runs = (ctypes.c_int64 * 2)(0, self.size), 1
+            with torch.cuda.device(dev):
+                check(lib.ss_replay_sample_prioritized(
+                    self.obs.data_ptr(), self.act.data_ptr(), self.reward.data_ptr(), self.next_obs.data_ptr(), self.done.data_ptr(),
+                    self.capacity, self.frames, self.tick_rows if n_step != 1 else 1, int(n_step), float(gamma), runs, n_runs,
+                    self.seed, self.counter, batch, out["obs"].data_ptr(), out["act"].data_ptr(), out["reward"].data_ptr(),
+                    out["next_obs"].data_ptr(), out["done"].data_ptr(), out["indices"].data_ptr(),
+                    out["steps"].data_ptr() if n_step != 1 else None, self.priority.data_ptr(), self.priority_scratch.data_ptr(),
+                    self.priority_scratch.numel(), float(beta), out["weights"].data_ptr(), _stream(dev)),
+                      "ss_replay_sample_prioritized")
+            self.counter += 1
+            return out
         if n_step != 1:
             with torch.cuda.device(dev):
                 check(lib.ss_replay_sample_nstep(self.obs.data_ptr(), self.act.data_ptr(), self.reward.data_ptr(),
@@ -1513,7 +1660,8 @@ class SelfPlayTrainer:
                  random_positions: bool = True, process_group=None, precision: str = "f32", collective: str = "nccl",
                  frames: int = 1, update_precision: Optional[str] = None, opponents=None, pool_envs: Optional[int] = None,
                  pool_blocks=None, twin_critics: bool = False, policy_delay: int = 1, target_noise: float = 0.0,
-                 target_noise_clip: float = 0.5, n_step: int = 1):
+                 target_noise_clip: float = 0.5, n_step: int = 1, prioritized_replay: bool = False,
+                 priority_alpha: float = 0.6, priority_beta: float = 0.4, priority_eps: float = 1e-6):
         """frames > 1: the frame-stacked "planning" networks (readme.md:18-20, BASELINE.json configs[4]): both players act
         from their last `frames` observations (FrameStackActor; `precision` selects its float32 or tensor-core kernels),
         the replay ring stores the stacked observations, and the critic / actor update of SkillshotLearner.py:386-443 runs
@@ -1546,8 +1694,16 @@ class SelfPlayTrainer:
         set_pool_blocks / rebalance_pool; a checkpoint holds the breaks, and a checkpoint without them (an older one, or one
         of an n_step = 1 run) loads with an empty ring.  n_step must be an integer in 1..32 and the replay capacity at least
         n_step ticks of rows, else ValueError before anything is allocated (sharded: on every rank when any rank refused
-        or passed another n_step).  n_step = 1 is the one-step update, with the same allocations and checkpoints."""
+        or passed another n_step).  n_step = 1 is the one-step update, with the same allocations and checkpoints.
+        prioritized_replay (DESIGN.md section 6.16): every update path draws its minibatch in proportion to the rows'
+        leaves (|delta| + priority_eps)^priority_alpha (ReplayRing(prioritized=True)), weights the critic's loss by the
+        importance weights (leaf_min / leaf)^beta with beta = self.priority_beta read at every update (set it to anneal
+        beta), and writes the minibatch's new leaves from critic 1's |q - y| after the critic step.  Sharded, each rank
+        draws from and normalises by its own ring.  alpha >= 0, 0 <= beta <= 1 and eps > 0, all finite, else ValueError
+        before anything is allocated (sharded: on every rank when any rank refused or passed other values).  Off: the
+        uniform update, with the same allocations and checkpoints."""
         check_td3_options(twin_critics, policy_delay, target_noise, target_noise_clip, process_group)
+        check_priority_options(prioritized_replay, priority_alpha, priority_beta, priority_eps, process_group)
         self.device = torch.device(device)
         self.frames = int(frames)
         self.opponents, self.pool_envs, self.pool_stats = None, 0, None
@@ -1610,7 +1766,9 @@ class SelfPlayTrainer:
                                     policy_delay=policy_delay, target_noise=target_noise, target_noise_clip=target_noise_clip)
         self.networks.seed = seed          # exploration / dropout streams differ per rank, weights do not
         self.replay = ReplayRing(replay_capacity or L * 8, device=device, seed=seed, frames=self.frames,
-                                 tick_rows=L if self.n_step > 1 else None)
+                                 tick_rows=L if self.n_step > 1 else None, prioritized=prioritized_replay)
+        self.prioritized_replay = bool(prioritized_replay)
+        self.priority_alpha, self.priority_beta, self.priority_eps = float(priority_alpha), float(priority_beta), float(priority_eps)
         self.batch_size, self.param_noise_sd, self.noise_group = int(batch_size), float(param_noise_sd), int(noise_group)
         self.precision = precision
         self.update_precision = update_precision
@@ -2098,9 +2256,11 @@ class SelfPlayTrainer:
         k = self.updates & 1
         # (measured, profiles/r2_update_sample_early_ab.txt: 158.1 -> 152.1 us at 65,536 rows; at 524,288 rows the gather
         #  competes with what it runs beside, 759 -> 764 us: small minibatches only)
-        early = self._ring_clean and self._batches[k] is not None and self.batch_size <= 131072
+        early = self._ring_clean and self._batches[k] is not None and self.batch_size <= 131072 and not self.prioritized_replay
+        pri = dict(priority_beta=self.priority_beta, priority_alpha=self.priority_alpha,
+                   priority_eps=self.priority_eps) if self.prioritized_replay else {}
         self._batch = self._batches[k] = net.update_from_ring(self.replay, self.batch_size, out=self._batches[k], sample_early=early,
-                                                              n_step=self.n_step)
+                                                              n_step=self.n_step, **pri)
         self._ring_clean = True
         self.updates += 1
         if net.peer is not None and self.updates % self.exchange_check_every == 0:
@@ -2109,14 +2269,27 @@ class SelfPlayTrainer:
 
     def update_stepwise(self):
         """The same update as one library call per step (sample, target, critic step, actor step); with the TD3 options,
-        ActorCritic.td3_step on the minibatch; with n_step > 1, on n-step rows with the bootstrap factor g_n."""
+        ActorCritic.td3_step on the minibatch; with n_step > 1, on n-step rows with the bootstrap factor g_n; with
+        prioritized replay, the prioritized draw, the weighted critic step(s) and the priority write after them."""
         self._ring_clean = False
         net = self.networks
-        self._batch = b = self.replay.sample(self.batch_size, out=self._batch, n_step=self.n_step, gamma=net.gamma)
+        pri = self.prioritized_replay
+        self._batch = b = self.replay.sample(self.batch_size, out=self._batch, n_step=self.n_step, gamma=net.gamma,
+                                             beta=self.priority_beta if pri else None)
+        wt = {}
+        if pri:
+            if "td_abs" not in b:
+                b["td_abs"] = torch.empty(self.batch_size, dtype=torch.float32, device=self.device)
+            wt = dict(weights=b["weights"], td_abs_out=b["td_abs"])
         disc = None if self.n_step == 1 else nstep_discount(net.gamma, self.n_step)
         if net.td3:
-            return net.td3_step(b["obs"], b["act"], b["reward"], b["next_obs"], b["done"], discount=disc)
+            out = net.td3_step(b["obs"], b["act"], b["reward"], b["next_obs"], b["done"], discount=disc, **wt)
+            if pri:
+                self.replay.update_priorities(b["indices"], b["td_abs"], self.priority_alpha, self.priority_eps)
+            return out
         y = net.td_targets(b["reward"], b["next_obs"], b["done"], discount=disc)
-        sse = net.critic_step(b["obs"], b["act"], y)
+        sse = net.critic_step(b["obs"], b["act"], y, **wt)
+        if pri:
+            self.replay.update_priorities(b["indices"], b["td_abs"], self.priority_alpha, self.priority_eps)
         q = net.actor_step(b["obs"])
         return sse, q
