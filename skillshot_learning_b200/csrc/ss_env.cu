@@ -10,6 +10,7 @@
 // The step is HBM-bound by design (SURVEY.md 8(d)): no tensor-core work here.
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <atomic>
 #include <stdlib.h>
 
 #include "../../include/skillshot_b200.h"
@@ -330,36 +331,63 @@ __device__ __forceinline__ void lane_tick(Lane &L, double *qrot, const float mov
     }
 }
 
-template <int TERMINAL, bool CHECKED>
-__device__ __forceinline__ void lane_loop(Lane &L, double *qrot, const StepArgs &A, LaneIo &io, int lane, int P, int64_t env,
-                                          bool &nan_seen) {
+// The action stream of step_pp_kernel goes through a ring of kRingD slots per lane in shared memory: slot s of a lane is
+// ring[s * BLK + threadIdx.x], so a warp's 32 float2 of one slot are 256 contiguous bytes (no bank conflicts).  Each lane
+// copies the 8 bytes it will read itself with cp.async and waits only on its own copies (cp.async.wait_group): no barrier,
+// no other thread involved.  The copy of tick k is issued during tick k - kRingD + 1 and first read during tick k - 1,
+// kRingD - 2 ticks (~250 cycles of a warp's own time each) ahead of its use.  8 slots measured as fast as 16 at 256 and
+// 1,024 ticks per launch and faster at 32 (the prologue waits for its first copies once per launch), in half the shared
+// memory (profiles/r13_step_ring_step0.txt).
+constexpr int kRingD = 8;
+static_assert((kRingD & (kRingD - 1)) == 0 && kRingD >= 4, "kRingD is a power of two >= 4");
+
+__device__ __forceinline__ void ring_copy(float2 *dst, const float2 *src, bool valid) {   // 8 bytes; zero-filled when !valid
+    const uint32_t d = (uint32_t)__cvta_generic_to_shared(dst);
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;\n" ::"r"(d), "l"(src), "r"(valid ? 8 : 0) : "memory");
+    asm volatile("cp.async.commit_group;\n" ::: "memory");
+}
+__device__ __forceinline__ float2 ring_read(const float2 *slot) {       // after this lane's copies up to `slot` have landed
+    asm volatile("cp.async.wait_group %0;\n" ::"n"(kRingD - 2) : "memory");
+    return *slot;
+}
+
+template <int TERMINAL, bool CHECKED, int BLK>
+__device__ __forceinline__ void lane_loop(Lane &L, double *qrot, const StepArgs &A, LaneIo &io, float2 *ring, int lane, int P,
+                                          int64_t env, bool &nan_seen) {
     const int limit = A.P.tick_limit > 0 ? (int)min((int64_t)0x7fffffff, A.P.tick_limit) : 0x7fffffff;
     const bool write_zero = TERMINAL == OUT_FLAGS && A.reward_out && A.P.reward_mode != SS_REWARD_NONE;
     const int T = A.n_ticks;
-    const float2 zero = make_float2(0.f, 0.f);
     // tick t needs move(t) and look(t + 1): the action of tick t + 1 is consumed during tick t (its look half now, its
-    // move half one tick later) and the action of tick t + 2 is in flight.  The loop is unrolled by two so that the two
-    // action registers and the two Turn records alternate by renaming.
-    float2 a0 = __ldg(io.actions + io.idx);
-    float2 qa = T > 1 ? __ldg(io.actions + (io.idx + io.n2)) : zero;          // action of tick 1
-    float2 qb = T > 2 ? __ldg(io.actions + (io.idx + 2 * io.n2)) : zero;      // action of tick 2
+    // move half one tick later).  The ring holds ticks t ... t + kRingD - 1 during tick t.  Ticks >= T are zero-filled
+    // copies from index 0 (a valid address), so every lane commits one group per tick and no tick branches on the end.
+    // src is the element index of the next tick to copy; it is only dereferenced while that tick is < T, where it is below
+    // 2n * T (the launch checks that 2n * (n_ticks + 2) fits 32 bits).
+    uint32_t src = io.idx;
+#pragma unroll
+    for (int k = 0; k < kRingD - 1; ++k, src += io.n2) ring_copy(ring + k * BLK, io.actions + (k < T ? src : 0u), k < T);
+    float2 a0 = ring_read(ring);
     Turn ta, tb;
     turn_from<CHECKED>(ta, L.rot, a0.y);
     float move = a0.x;
-    // (The register loads run one tick ahead of their use, ~500 cycles of a warp's own time, less than a DRAM access under
-    //  load, and ncu attributes 36 % of the stall samples to the first use of a loaded action.  That is where a warp that
-    //  ran ahead parks, not what bounds the kernel: four loads in flight per lane, and an L2 prefetch eight ticks ahead,
-    //  were both measured and left the launch time unchanged -- 119 / 108.5 us -- while costing registers / issue slots.)
+    // Tick t refills the slot of tick t - 1 with tick t + kRingD - 1.  That slot was last read by the shared-memory load
+    // of tick t - 2, whose two values were consumed by arithmetic before tick t began, so the load has completed and the
+    // asynchronous write cannot overtake it.  Its own slot t + 1 is then read after waiting for all but the kRingD - 2
+    // newest groups, which leaves the copies of ticks 0 ... t + 1 landed.
     for (int t = 0; t < T; t += 2) {
-        lane_tick<TERMINAL, CHECKED>(L, qrot, move, qa.y, ta, tb, A, io, lane, P, env, t, limit, write_zero, nan_seen);
-        move = qa.x;
-        qa = (t + 3 < T) ? __ldg(io.actions + (io.idx + 2 * io.n2)) : zero;      // action of tick t + 3 (idx is at tick t + 1 now)
+        ring_copy(ring + ((t - 1) & (kRingD - 1)) * BLK, io.actions + (t + kRingD - 1 < T ? src : 0u), t + kRingD - 1 < T);
+        src += io.n2;
+        float2 q = ring_read(ring + ((t + 1) & (kRingD - 1)) * BLK);
+        lane_tick<TERMINAL, CHECKED>(L, qrot, move, q.y, ta, tb, A, io, lane, P, env, t, limit, write_zero, nan_seen);
+        move = q.x;
         if (t + 1 < T) {
-            lane_tick<TERMINAL, CHECKED>(L, qrot, move, qb.y, tb, ta, A, io, lane, P, env, t + 1, limit, write_zero, nan_seen);
-            move = qb.x;
-            qb = (t + 4 < T) ? __ldg(io.actions + (io.idx + 2 * io.n2)) : zero;  // action of tick t + 4 (idx is at tick t + 2 now)
+            ring_copy(ring + (t & (kRingD - 1)) * BLK, io.actions + (t + kRingD < T ? src : 0u), t + kRingD < T);
+            src += io.n2;
+            q = ring_read(ring + ((t + 2) & (kRingD - 1)) * BLK);
+            lane_tick<TERMINAL, CHECKED>(L, qrot, move, q.y, tb, ta, A, io, lane, P, env, t + 1, limit, write_zero, nan_seen);
+            move = q.x;
         }
     }
+    asm volatile("cp.async.wait_all;\n" ::: "memory");              // the zero-fill copies past the end
 }
 
 // TERMINAL: one of OUT_FLAGS / OUT_TERMINAL / OUT_PACKED.
@@ -408,8 +436,10 @@ __global__ void __launch_bounds__(BLK, 896 / BLK) step_pp_kernel(const StepArgs 
     // boundary it puts in the middle of the tick) then goes.  Otherwise (400,000 ticks of one-sided turning without a
     // reset, or a NaN) the warp runs the checked loop.
     const bool in_range = fabs(L.rot) + 0.25 * (double)A.n_ticks + 1.0 < 1.0e5;
-    if (__all_sync(0xffffffffu, in_range)) lane_loop<TERMINAL, false>(L, qrot, A, io, lane, P, env, nan_seen);
-    else lane_loop<TERMINAL, true>(L, qrot, A, io, lane, P, env, nan_seen);
+    extern __shared__ float2 ring_sh[];                                 // kRingD * BLK float2: the action ring (lane_loop)
+    float2 *const ring = ring_sh + threadIdx.x;
+    if (__all_sync(0xffffffffu, in_range)) lane_loop<TERMINAL, false, BLK>(L, qrot, A, io, ring, lane, P, env, nan_seen);
+    else lane_loop<TERMINAL, true, BLK>(L, qrot, A, io, ring, lane, P, env, nan_seen);
     // the partner's valid bit for the env's flag word
     const int v_other = __shfl_xor_sync(0xffffffffu, L.valid, 1);
     ((double *)base)[gl] = L.rot;
@@ -1086,12 +1116,29 @@ inline int pp_block_for(int64_t n_envs) {
     if (c448 * 20 >= (int64_t)sms * 19) return 448;
     return 64;
 }
+template <int OUT, int BLK>
+inline int launch_step_pp_blk(const StepArgs &A, int64_t n_envs, cudaStream_t st) {
+    constexpr int ring_bytes = kRingD * BLK * (int)sizeof(float2);      // 56 KB at 896 threads: above the 48 KB default
+    // The launch needs the function's dynamic shared-memory limit raised, and that limit belongs to the function on one
+    // device: it is set the first time this process launches the kernel on each device (devices past 63 on every call).
+    static std::atomic<uint64_t> configured{0};
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) return SS_ERR_CUDA;
+    const uint64_t bit = dev < 64 ? 1ull << dev : 0;
+    if (!(configured.load(std::memory_order_acquire) & bit)) {
+        if (cudaFuncSetAttribute(step_pp_kernel<OUT, BLK>, cudaFuncAttributeMaxDynamicSharedMemorySize, ring_bytes) != cudaSuccess)
+            return SS_ERR_CUDA;
+        configured.fetch_or(bit, std::memory_order_acq_rel);
+    }
+    step_pp_kernel<OUT, BLK><<<blocks_for(2 * n_envs, BLK), BLK, ring_bytes, st>>>(A);
+    return check_launch();
+}
 template <int OUT>
-inline void launch_step_pp(const StepArgs &A, int64_t n_envs, cudaStream_t st) {
+inline int launch_step_pp(const StepArgs &A, int64_t n_envs, cudaStream_t st) {
     switch (pp_block_for(n_envs)) {
-        case 896: step_pp_kernel<OUT, 896><<<blocks_for(2 * n_envs, 896), 896, 0, st>>>(A); break;
-        case 448: step_pp_kernel<OUT, 448><<<blocks_for(2 * n_envs, 448), 448, 0, st>>>(A); break;
-        default: step_pp_kernel<OUT, 64><<<blocks_for(2 * n_envs, 64), 64, 0, st>>>(A); break;
+        case 896: return launch_step_pp_blk<OUT, 896>(A, n_envs, st);
+        case 448: return launch_step_pp_blk<OUT, 448>(A, n_envs, st);
+        default: return launch_step_pp_blk<OUT, 64>(A, n_envs, st);
     }
 }
 
@@ -1169,8 +1216,9 @@ int ss_env_step_ring(void *state, int64_t n_envs, const float *actions, float *o
                2 * n_envs * ((int64_t)n_ticks + 2) < (int64_t)0x7fffffff) {     // (32-bit running index)
         // physics-only fused ticks (bench.py's timed shape): one thread per player.  (A single tick per launch stays on
         // the one-thread-per-env kernel: a launch then pays 3 sincos per lane to set up what it carries, measured 4.1 vs 3.9 us.)
-        if (reward_out && reward_mode == SS_REWARD_TERMINAL) launch_step_pp<OUT_TERMINAL>(A, n_envs, st);
-        else launch_step_pp<OUT_FLAGS>(A, n_envs, st);
+        if ((reward_out && reward_mode == SS_REWARD_TERMINAL ? launch_step_pp<OUT_TERMINAL>(A, n_envs, st)
+                                                             : launch_step_pp<OUT_FLAGS>(A, n_envs, st)) != SS_OK)
+            return SS_ERR_CUDA;
     } else if (carry) {
         if (A.stats) {
             if (speeds) step_kernel<false, true, true, 1, true><<<grid, block, 0, st>>>(A);
@@ -1377,8 +1425,7 @@ int ss_env_step_packed(void *state, int64_t n_envs, const float *actions, uint8_
     A.state = state; A.n = n_envs; A.actions = (const float4 *)actions; A.packed_out = packed_out; A.status = status;
     A.P.seed = seed; A.P.counter = counter; A.P.tick_limit = tick_limit; A.P.reward_mode = SS_REWARD_TERMINAL;
     A.P.auto_reset = auto_reset ? 1 : 0; A.P.reset_mode = reset_mode; A.n_ticks = n_ticks;
-    launch_step_pp<OUT_PACKED>(A, n_envs, (cudaStream_t)stream);
-    return check_launch();
+    return launch_step_pp<OUT_PACKED>(A, n_envs, (cudaStream_t)stream);
 }
 
 int ss_env_features(const void *state, int64_t n_envs, double *feat_out, double *obs_out,
